@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py — corrected Mpx/s of the CameraCalibration.correct() chain on B200 (BASELINE.json metric).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--frames F] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--frames F] [--impl reference] [--dump-outputs DIR]
 
 Headline workload (BASELINE.json configs[2]): a batch of 4096x3000 uint16 frames per GPU through the full chain
 (dark subtract, flat-field divide, nan_to_num, 3x3 median-threshold, lens undistortion).  One step = one pass
@@ -24,6 +24,10 @@ One JSON line on rank 0:
   cpu_baseline the oracle's restatement of the reference path (scipy + OpenCV, float64) on one host core
 `--impl reference` times that reference path on all host cores instead (rank 0 only), after re-checking it against the
 golden outputs of the unmodified reference (tests/golden).
+
+`--dump-outputs DIR` writes, after the timed steps, what the headline correct_batch() call returned in its last step on
+rank 0, as float32 .npy files (see dump_outputs).  The inputs are seeded, so two builds run with the same arguments can
+be compared file for file.
 """
 import argparse
 import json
@@ -319,6 +323,23 @@ def pcie_probe(dev, in_bytes, out_bytes, seconds=0.25):
     return res
 
 
+DUMP_SAMPLE = 1 << 21      # pixels in the seeded sample of the whole batch: 8 MB of float32
+
+
+def dump_outputs(path, out):
+    """write the (F, H, W) float32 result of the timed call as two .npy files, 57.5 MB in all at the 4096x3000 frame size:
+    out_last_frame.npy, the whole last frame (every tile and strip seam of one frame), and out_sample.npy, the values at
+    DUMP_SAMPLE flat positions of the batch drawn by a fixed-seed generator (every frame group).  The positions depend on
+    the output's shape only."""
+    import numpy as np
+    import torch
+    os.makedirs(path, exist_ok=True)
+    idx = np.sort(np.random.default_rng(20240607).integers(0, out.numel(), DUMP_SAMPLE))
+    sample = out.reshape(-1)[torch.from_numpy(idx).to(out.device)]
+    np.save(os.path.join(path, 'out_last_frame.npy'), out[-1].cpu().numpy())
+    np.save(os.path.join(path, 'out_sample.npy'), sample.cpu().numpy())
+
+
 def run_ours(args):
     import numpy as np
     import torch
@@ -401,6 +422,8 @@ def run_ours(args):
         torch.cuda.synchronize()
     ms_total = ev0.elapsed_time(ev1)
     barrier()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, out)
     launches = eng.launch_count - launches0
     k1_ms, k1_frames, k2_ms, k2_frames = eng.profile_read()
     eng.set_option(_lib.OPT_PROFILE, 0)
@@ -656,7 +679,12 @@ def main():
     ap.add_argument('--c4-frames', type=int, default=256, help='6000x4000 frames streamed per GPU in the timed region of c4')
     ap.add_argument('--no-configs', action='store_true', help='headline only (skip c0 / c1 / c3 / c4)')
     ap.add_argument('--no-cpu-baseline', action='store_true')
+    ap.add_argument('--dump-outputs', metavar='DIR', help='write the last timed step\'s output (rank 0) as .npy files into DIR')
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error('--steps must be at least 1')
+    if args.dump_outputs and args.impl != 'ours':
+        ap.error('--dump-outputs needs --impl ours')
     if args.gpus > 1 and 'WORLD_SIZE' not in os.environ and args.impl == 'ours':
         # started as plain `python bench.py --gpus N`: relaunch under torchrun, one rank per GPU (the driver does this itself)
         import socket
