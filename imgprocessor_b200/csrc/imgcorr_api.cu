@@ -75,6 +75,9 @@ struct imgcorr_ctx {
     double dark_absmax = 0.0, flat_absmin = 1.0;   // over finite entries (flat: non-zero entries)
     long long launches = 0;
     float* mid[2] = {nullptr, nullptr};
+    // the chain's last use of mid[] (recorded on the stream of that call): a call on another stream waits for it
+    cudaEvent_t ev_mid = nullptr;
+    cudaStream_t mid_st = nullptr;
     int chain_overlap = 1;                    // K1 of group g+1 on the internal stream while K2 of group g runs: +2-3.5 % on batches
     cudaStream_t s_chain = nullptr;           // high-priority stream of K1 in overlap mode
     cudaEvent_t ev_k1[2] = {nullptr, nullptr}, ev_k2[2] = {nullptr, nullptr}, ev_entry = nullptr;
@@ -171,6 +174,7 @@ extern "C" IMGCORR_API int imgcorr_ctx_destroy(imgcorr_ctx* c) {
     if (c->s_chain) cudaStreamDestroy(c->s_chain);
     for (int i = 0; i < 2; ++i) { if (c->ev_k1[i]) cudaEventDestroy(c->ev_k1[i]); if (c->ev_k2[i]) cudaEventDestroy(c->ev_k2[i]); }
     if (c->ev_entry) cudaEventDestroy(c->ev_entry);
+    if (c->ev_mid) cudaEventDestroy(c->ev_mid);
     cudaFree(c->dark);
     cudaFree(c->ascent);
     cudaFree(c->flat);
@@ -723,13 +727,21 @@ static int chain_frames(imgcorr_ctx* c, const void* raw, int raw_dtype, void* ou
     // buffers (L2-resident for small groups); K2 evaluates each pixel's map once per group.
     const int grp = c->chain_group < n ? c->chain_group : (n > 0 ? n : 1);
     if (c->mid_frames < (size_t)grp) {
-        CK(cudaStreamSynchronize(st));
+        CK(cudaDeviceSynchronize());                   // calls on other streams (correct_host, other torch streams) may still use mid[]
         for (int i = 0; i < 2; ++i) {
             if (c->mid[i]) { CK(cudaFree(c->mid[i])); c->mid[i] = nullptr; }
             CK(cudaMalloc((void**)&c->mid[i], npx * sizeof(float) * grp));
         }
         c->mid_frames = grp;
     }
+    // mid[] is one pair per context: a call on another stream than the last one first waits until that call's K2 has
+    // read it.  The wait precedes ev_entry, so the overlap stream inherits it.
+    if (!c->ev_mid) CK(cudaEventCreateWithFlags(&c->ev_mid, cudaEventDisableTiming));
+    else if (c->mid_st != st) CK(cudaStreamWaitEvent(st, c->ev_mid, 0));
+    struct MidRelease {                                // every K1 / K2 of this call is ordered before the end of `st`
+        imgcorr_ctx* c; cudaStream_t st;
+        ~MidRelease() { cudaEventRecord(c->ev_mid, st); c->mid_st = st; }
+    } release{c, st};
     const size_t out_stride = (size_t)ow * oh * dtype_size(out_dtype);
     // Overlap mode: K1 of group g+1 runs on an internal high-priority stream while K2 of group g runs on the caller's
     // stream, so that K2's blocks fill the SM slots K1's last, partially filled wave leaves idle (and vice versa).  The

@@ -150,7 +150,10 @@ IMGCORR_API int imgcorr_undistort_maps(imgcorr_ctx* ctx, float* mapx_dev, float*
  * image branch; a stack of frames is a batch here, not the STE average of :385-406).
  *   threshold > 0 : median-threshold with ksize (3 in correct(), :556-563) after nan_to_num
  *   use_lens      : apply K2 if a lens is set (missing lens -> frames pass through, :570-575)
- *   out_dtype     : F32 or F64 (float64 is what the reference returns, :459) */
+ *   out_dtype     : F32 or F64 (float64 is what the reference returns, :459)
+ * Asynchronous on `stream`.  The context's K1 scratch is shared by every chain call: a call on another stream than
+ * the previous chain call (imgcorr_correct_host included) first waits for that call's work on the scratch, so calls
+ * of one context on several streams are correct and run one after the other on the device. */
 IMGCORR_API int imgcorr_correct_batch(imgcorr_ctx* ctx, const void* raw_dev, int raw_dtype, void* out_dev, int out_dtype,
                           int n_frames, double threshold, int ksize, int flags, int use_lens, double border_value,
                           int x0, int y0, int ow, int oh, void* stream);
@@ -158,7 +161,8 @@ IMGCORR_API int imgcorr_correct_batch(imgcorr_ctx* ctx, const void* raw_dev, int
 /* Same chain with HOST buffers: frames are staged through a ring of pinned buffers, H2D copy,
  * kernels and D2H copy of consecutive frames (small frames: chunks of up to 16 frames) overlap on three streams.  Synchronous: returns
  * when out_host is complete.  Fastest when raw_host / out_host come from imgcorr_host_alloc
- * (or are otherwise page-locked). */
+ * (or are otherwise page-locked).  Its kernels wait for an earlier imgcorr_correct_batch of the same context that is
+ * still queued on another stream (they share the K1 scratch), so the call also waits for that batch to finish. */
 IMGCORR_API int imgcorr_correct_host(imgcorr_ctx* ctx, const void* raw_host, int raw_dtype, void* out_host, int out_dtype,
                          int n_frames, double threshold, int ksize, int flags, int use_lens, double border_value,
                          int x0, int y0, int ow, int oh);
