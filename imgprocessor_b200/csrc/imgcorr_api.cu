@@ -7,6 +7,8 @@
 #include <string.h>
 #include <string>
 #include <algorithm>
+#include <memory>
+#include <type_traits>
 #include <vector>
 #include <thread>
 
@@ -35,62 +37,129 @@ static int cuda_fail(cudaError_t e, const char* what) {
         if (e__ != cudaSuccess) return cuda_fail(e__, #call); \
     } while (0)
 
+// ---- owning handles: every CUDA resource the library keeps is released by its handle's destructor ---------------------
+struct DevFree { void operator()(void* p) const { cudaFree(p); } };
+struct HostFree { void operator()(void* p) const { cudaFreeHost(p); } };
+struct EventFree { void operator()(cudaEvent_t e) const { cudaEventDestroy(e); } };
+struct StreamFree { void operator()(cudaStream_t s) const { cudaStreamDestroy(s); } };
+template <class T> using DevPtr = std::unique_ptr<T, DevFree>;
+using PinnedPtr = std::unique_ptr<void, HostFree>;
+using Event = std::unique_ptr<std::remove_pointer_t<cudaEvent_t>, EventFree>;
+using Stream = std::unique_ptr<std::remove_pointer_t<cudaStream_t>, StreamFree>;
+
+// creation fills an empty handle and returns the CUDA error (nothing throws); on failure the handle stays empty
+template <class H, class Create> static cudaError_t create(H& h, Create&& make) {
+    typename H::pointer raw = nullptr;
+    const cudaError_t e = make(&raw);
+    h.reset(e == cudaSuccess ? raw : nullptr);
+    return e;
+}
+template <class T> static cudaError_t dev_alloc(DevPtr<T>& p, size_t bytes) {
+    return create(p, [&](T** raw) { return cudaMalloc((void**)raw, bytes); });
+}
+static cudaError_t host_alloc(PinnedPtr& p, size_t bytes) {
+    return create(p, [&](void** raw) { return cudaHostAlloc(raw, bytes, cudaHostAllocDefault); });
+}
+static cudaError_t new_event(Event& ev, unsigned flags = cudaEventDisableTiming) {
+    return create(ev, [&](cudaEvent_t* raw) { return cudaEventCreateWithFlags(raw, flags); });
+}
+static cudaError_t new_stream(Stream& s, int priority = 0) {      // non-blocking; 0 is the default priority
+    return create(s, [&](cudaStream_t* raw) { return cudaStreamCreateWithPriority(raw, cudaStreamNonBlocking, priority); });
+}
+
+// 256 bytes, the alignment cudaMalloc gives: K1's TMA paths and K2's tiled path need 16-byte aligned frames and quietly
+// take slower kernels otherwise, so every part of a split allocation starts on such a boundary
+static size_t round256(size_t bytes) { return (bytes + 255) & ~(size_t)255; }
+
+// Device memory that every call of one kind shares, one per context.  Calls may come on different streams: a call on
+// another stream than the last user first waits until that user's launches are done with it.
+struct SharedScratch {
+    DevPtr<char> buf;
+    size_t bytes = 0;
+    Event last_use;                                 // recorded on the last user's stream after its last launch
+    cudaStream_t last_st = nullptr;
+
+    // at least `need` bytes, ordered on `st` after the last use
+    cudaError_t acquire(size_t need, cudaStream_t st) {
+        cudaError_t e;
+        if (bytes < need) {
+            // launches on other streams may still use the old buffer; it goes before the new one is allocated, so
+            // peak memory stays one buffer, and a failed allocation leaves the scratch empty for the next call to retry
+            if (buf && (e = cudaDeviceSynchronize()) != cudaSuccess) return e;
+            buf.reset();
+            bytes = 0;
+            if ((e = dev_alloc(buf, need)) != cudaSuccess) return e;
+            bytes = need;
+        }
+        if (!last_use) return new_event(last_use);
+        return last_st == st ? cudaSuccess : cudaStreamWaitEvent(st, last_use.get(), 0);
+    }
+    void release(cudaStream_t st) { cudaEventRecord(last_use.get(), st); last_st = st; }
+    struct Guard {                                  // releases on every exit path of the call that acquired the scratch
+        SharedScratch& s;
+        cudaStream_t st;
+        ~Guard() { s.release(st); }
+    };
+};
+
 struct HostSlot {
-    void* d_raw = nullptr;
-    void* d_out = nullptr;
-    void* h_raw = nullptr;
-    void* h_out = nullptr;
-    cudaEvent_t ev_in = nullptr, ev_k = nullptr, ev_out = nullptr;
+    DevPtr<void> d_raw, d_out;
+    PinnedPtr h_raw, h_out;
+    Event ev_in, ev_k, ev_out;
 };
 
 struct imgcorr_ctx {
     int device = 0, H = 0, W = 0, sm_count = 148;
-    float* dark = nullptr;
-    float* ascent = nullptr;
-    float* flat = nullptr;
+    DevPtr<float> dark, ascent, flat;
     double exposure = 0.0, maxval = 65535.0;
     bool has_lens = false;
     LensConst lens{};
     double lens_in[23] = {0};                 // K, dist, P as last given to imgcorr_set_lens (an identical call is a no-op)
-    double* lens_dev = nullptr;
-    float4* k2_wtab = nullptr;                // OpenCV's BilinearTab_f [32][32] (K2 tiles)
+    DevPtr<double> lens_dev;
+    DevPtr<float4> k2_wtab;                   // OpenCV's BilinearTab_f [32][32] (K2 tiles)
     struct GeomKey { int x0, y0, ow, oh, esz, g; };
     std::vector<GeomKey> k2_geom;             // staged-box geometry per output window (k2_pick_geometry), reset by set_lens
     // K2 coordinate cache: packed per-pixel source coordinates of the current lens for an output window (4 bytes per pixel),
     // written by the first tiled launch, read by the following ones; dropped by set_lens
-    struct K2Cache { int x0, y0, ow, oh, g, esz; unsigned* pack; int2* hdr; cudaEvent_t ev; cudaStream_t st; unsigned long long stamp; };
+    struct K2Cache { int x0, y0, ow, oh, g, esz; DevPtr<unsigned> pack; DevPtr<int2> hdr; Event ev; cudaStream_t st; unsigned long long stamp; };
     std::vector<K2Cache> k2_cache;
     int k2_cache_on = 1, k2_tma_store = 0;
     unsigned long long k2_stamp = 0;
-    void* dump = nullptr;                     // scratch for stores of lanes that own no output pixel
+    DevPtr<void> dump;                        // scratch for stores of lanes that own no output pixel
     int raw_big_endian = 0;
     long long raw_gap = 0;
     int k1_variant = 0, k2_variant = 0, k3_variant = 0, host_slots = 4, k1_seg_rows = 0, profile = 0, chain_group = 16;
     long long chain_groups_seen = 0;
     double prof_frames[2] = {0.0, 0.0};
-    std::vector<cudaEvent_t> prof_ev[2];      // [kernel] start/stop pairs
-    size_t mid_frames = 0;
+    std::vector<Event> prof_ev[2];            // [kernel] start/stop pairs (timing events)
     bool dark_finite = true, flat_finite = true;
-    float* flat_nz = nullptr;                 // flat with zeros replaced by 1.0
+    DevPtr<float> flat_nz;                    // flat with zeros replaced by 1.0
     double dark_absmax = 0.0, flat_absmin = 1.0;   // over finite entries (flat: non-zero entries)
     long long launches = 0;
-    float* mid[2] = {nullptr, nullptr};
-    // the chain's last use of mid[] (recorded on the stream of that call): a call on another stream waits for it
-    cudaEvent_t ev_mid = nullptr;
-    cudaStream_t mid_st = nullptr;
+    SharedScratch chain_scratch;              // the chain's K1 output: two halves of `chain_group` float32 frames each
     int chain_overlap = 1;                    // K1 of group g+1 on the internal stream while K2 of group g runs: +2-3.5 % on batches
-    cudaStream_t s_chain = nullptr;           // high-priority stream of K1 in overlap mode
-    cudaEvent_t ev_k1[2] = {nullptr, nullptr}, ev_k2[2] = {nullptr, nullptr}, ev_entry = nullptr;
-    double* ste_avg = nullptr;                // K4 scratch: second running-average buffer, thresholds, counts
-    double* ste_thr = nullptr;
-    int* ste_n = nullptr;
-    int16_t* warp_itab[2] = {nullptr, nullptr};   // [bicubic, Lanczos4] fixed-point weights for uint8 images (K3)
-    float* warp_tab = nullptr;                // [32][8] Lanczos4 then [32][4] bicubic coefficient tables (K3)
+    struct ChainOverlap { Stream st; Event k1[2], k2[2], entry; };
+    ChainOverlap ov;                          // high-priority stream of K1 in overlap mode and its hand-off events
+    SharedScratch ste_scratch;                // K4: second running-average buffer, thresholds, counts
+    DevPtr<int16_t> warp_itab[2];             // [bicubic, Lanczos4] fixed-point weights for uint8 images (K3)
+    DevPtr<float> warp_tab;                   // [32][8] Lanczos4 then [32][4] bicubic coefficient tables (K3)
     // host pipeline
-    cudaStream_t s_in = nullptr, s_k = nullptr, s_out = nullptr;
+    Stream s_in, s_k, s_out;
     std::vector<HostSlot> slots;
     size_t slot_raw_bytes = 0, slot_out_bytes = 0;
 };
+
+// The end of every launch: count the kernels the launch helper issued and map its error to a status.  K1, K2 and K3 name
+// the errors they can explain: a requested variant that is not eligible, and a dtype pair no kernel implements (`pair`,
+// formatted with the two dtypes).
+static int launched(imgcorr_ctx* c, int l, cudaError_t e, const char* what, const char* ineligible = nullptr,
+                    const char* pair = nullptr, int dt_in = 0, int dt_out = 0) {
+    c->launches += l;
+    if (e == cudaSuccess) return IMGCORR_OK;
+    if (pair && e == cudaErrorInvalidValue && l == 0) return fail(IMGCORR_ERR_INVALID, pair, dt_in, dt_out);
+    if (ineligible && e == cudaErrorNotSupported) return fail(IMGCORR_ERR_INVALID, "%s", ineligible);
+    return cuda_fail(e, what);
+}
 
 struct DeviceGuard {
     int prev = -1;
@@ -140,58 +209,10 @@ extern "C" IMGCORR_API int imgcorr_ctx_create(int device, int height, int width,
     return IMGCORR_OK;
 }
 
-static void free_k2_cache(imgcorr_ctx* c) {
-    for (auto& k : c->k2_cache) {
-        cudaFree(k.pack);
-        cudaFree(k.hdr);
-        if (k.ev) cudaEventDestroy(k.ev);
-    }
-    c->k2_cache.clear();
-}
-
-static void free_slots(imgcorr_ctx* c) {
-    for (auto& s : c->slots) {
-        if (s.d_raw) cudaFree(s.d_raw);
-        if (s.d_out) cudaFree(s.d_out);
-        if (s.h_raw) cudaFreeHost(s.h_raw);
-        if (s.h_out) cudaFreeHost(s.h_out);
-        if (s.ev_in) cudaEventDestroy(s.ev_in);
-        if (s.ev_k) cudaEventDestroy(s.ev_k);
-        if (s.ev_out) cudaEventDestroy(s.ev_out);
-    }
-    c->slots.clear();
-    c->slot_raw_bytes = c->slot_out_bytes = 0;
-}
-
 extern "C" IMGCORR_API int imgcorr_ctx_destroy(imgcorr_ctx* c) {
     if (!c) return IMGCORR_OK;
     DeviceGuard g(c->device);
     cudaDeviceSynchronize();
-    free_slots(c);
-    if (c->s_in) cudaStreamDestroy(c->s_in);
-    if (c->s_k) cudaStreamDestroy(c->s_k);
-    if (c->s_out) cudaStreamDestroy(c->s_out);
-    if (c->s_chain) cudaStreamDestroy(c->s_chain);
-    for (int i = 0; i < 2; ++i) { if (c->ev_k1[i]) cudaEventDestroy(c->ev_k1[i]); if (c->ev_k2[i]) cudaEventDestroy(c->ev_k2[i]); }
-    if (c->ev_entry) cudaEventDestroy(c->ev_entry);
-    if (c->ev_mid) cudaEventDestroy(c->ev_mid);
-    cudaFree(c->dark);
-    cudaFree(c->ascent);
-    cudaFree(c->flat);
-    cudaFree(c->flat_nz);
-    cudaFree(c->mid[0]);
-    cudaFree(c->mid[1]);
-    cudaFree(c->lens_dev);
-    cudaFree(c->k2_wtab);
-    free_k2_cache(c);
-    cudaFree(c->warp_tab);
-    cudaFree(c->warp_itab[0]);
-    cudaFree(c->warp_itab[1]);
-    cudaFree(c->ste_avg);
-    cudaFree(c->ste_thr);
-    cudaFree(c->ste_n);
-    cudaFree(c->dump);
-    for (int k = 0; k < 2; ++k) for (auto e : c->prof_ev[k]) cudaEventDestroy(e);
     delete c;
     return IMGCORR_OK;
 }
@@ -218,7 +239,7 @@ extern "C" IMGCORR_API int imgcorr_set_option(imgcorr_ctx* c, int key, int value
             if (!value && !c->k2_cache.empty()) {
                 DeviceGuard g(c->device);
                 cudaDeviceSynchronize();
-                free_k2_cache(c);
+                c->k2_cache.clear();
             }
             return IMGCORR_OK;
         case IMGCORR_OPT_K3_VARIANT:
@@ -249,7 +270,7 @@ extern "C" IMGCORR_API int imgcorr_set_option(imgcorr_ctx* c, int key, int value
             if (value != c->host_slots) {
                 DeviceGuard g(c->device);
                 cudaDeviceSynchronize();
-                free_slots(c);
+                c->slots.clear();
                 c->host_slots = value;
             }
             return IMGCORR_OK;
@@ -260,10 +281,10 @@ extern "C" IMGCORR_API int imgcorr_set_option(imgcorr_ctx* c, int key, int value
 extern "C" IMGCORR_API long long imgcorr_launch_count(const imgcorr_ctx* c) { return c ? c->launches : 0; }
 
 static void prof_mark(imgcorr_ctx* c, int which, cudaStream_t st) {
-    cudaEvent_t e = nullptr;
-    if (cudaEventCreate(&e) != cudaSuccess) return;
-    cudaEventRecord(e, st);
-    c->prof_ev[which].push_back(e);
+    Event e;
+    if (new_event(e, cudaEventDefault) != cudaSuccess) return;
+    cudaEventRecord(e.get(), st);
+    c->prof_ev[which].push_back(std::move(e));
 }
 
 extern "C" IMGCORR_API int imgcorr_profile_read(imgcorr_ctx* c, double out[4]) {
@@ -275,11 +296,10 @@ extern "C" IMGCORR_API int imgcorr_profile_read(imgcorr_ctx* c, double out[4]) {
         const size_t pairs = v.size() / 2;
         for (size_t i = 0; i < pairs; ++i) {
             float t = 0.f;
-            CK(cudaEventSynchronize(v[2 * i + 1]));
-            CK(cudaEventElapsedTime(&t, v[2 * i], v[2 * i + 1]));
+            CK(cudaEventSynchronize(v[2 * i + 1].get()));
+            CK(cudaEventElapsedTime(&t, v[2 * i].get(), v[2 * i + 1].get()));
             ms += t;
         }
-        for (auto e : v) cudaEventDestroy(e);
         v.clear();
         out[2 * k] = ms;
         out[2 * k + 1] = c->prof_frames[k];
@@ -295,23 +315,23 @@ static bool all_finite(const float* p, size_t n) {
     return ok;
 }
 
-static int upload_map(imgcorr_ctx* c, float** slot, const float* src, int on_device, bool* finite,
+static int upload_map(imgcorr_ctx* c, DevPtr<float>& slot, const float* src, int on_device, bool* finite,
                       std::vector<float>* host_copy = nullptr) {
     const size_t n = (size_t)c->H * c->W, bytes = n * sizeof(float);
     *finite = true;
     if (!src) {
-        if (*slot) { CK(cudaDeviceSynchronize()); CK(cudaFree(*slot)); *slot = nullptr; }
+        if (slot) { CK(cudaDeviceSynchronize()); slot.reset(); }
         return IMGCORR_OK;
     }
-    if (!*slot) CK(cudaMalloc((void**)slot, bytes));
+    if (!slot) CK(dev_alloc(slot, bytes));
     else CK(cudaDeviceSynchronize());      // launches on other (non-blocking) streams may still read the map being replaced
-    CK(cudaMemcpy(*slot, src, bytes, on_device ? cudaMemcpyDeviceToDevice : cudaMemcpyHostToDevice));
+    CK(cudaMemcpy(slot.get(), src, bytes, on_device ? cudaMemcpyDeviceToDevice : cudaMemcpyHostToDevice));
     std::vector<float> tmp;
     const float* h = src;
     if (on_device || host_copy) {
         std::vector<float>& dst = host_copy ? *host_copy : tmp;
         dst.resize(n);
-        if (on_device) CK(cudaMemcpy(dst.data(), *slot, bytes, cudaMemcpyDeviceToHost));
+        if (on_device) CK(cudaMemcpy(dst.data(), slot.get(), bytes, cudaMemcpyDeviceToHost));
         else memcpy(dst.data(), src, bytes);
         h = dst.data();
     }
@@ -327,11 +347,11 @@ extern "C" IMGCORR_API int imgcorr_set_dark(imgcorr_ctx* c, const float* dark, c
     if (ascent && !(exposure_time == exposure_time)) return fail(IMGCORR_ERR_INVALID, "exposure_time is NaN");
     bool fin2 = true;
     std::vector<float> h;
-    int r = upload_map(c, &c->dark, dark, on_device, &c->dark_finite, &h);
+    int r = upload_map(c, c->dark, dark, on_device, &c->dark_finite, &h);
     if (r) return r;
     c->dark_absmax = 0.0;
     for (float v : h) { const float av = fabsf(v); if (av <= 3.402823466e+38f && av > c->dark_absmax) c->dark_absmax = av; }
-    r = upload_map(c, &c->ascent, ascent, on_device, &fin2);
+    r = upload_map(c, c->ascent, ascent, on_device, &fin2);
     if (r) return r;
     c->exposure = exposure_time;
     c->maxval = ascent ? ldexp(1.0, depth_bits) - 1.0 : 65535.0;
@@ -341,10 +361,10 @@ extern "C" IMGCORR_API int imgcorr_set_dark(imgcorr_ctx* c, const float* dark, c
 extern "C" IMGCORR_API int imgcorr_set_flat(imgcorr_ctx* c, const float* flat, int on_device) {
     GUARD(c);
     std::vector<float> h;
-    int r = upload_map(c, &c->flat, flat, on_device, &c->flat_finite, &h);
+    int r = upload_map(c, c->flat, flat, on_device, &c->flat_finite, &h);
     if (r) return r;
     if (!flat) {
-        if (c->flat_nz) { CK(cudaFree(c->flat_nz)); c->flat_nz = nullptr; }
+        c->flat_nz.reset();                        // upload_map synchronised the device before it dropped the flat
         return IMGCORR_OK;
     }
     // zero-free copy for the streaming kernel + the smallest non-zero magnitude (overflow proof)
@@ -355,9 +375,9 @@ extern "C" IMGCORR_API int imgcorr_set_flat(imgcorr_ctx* c, const float* flat, i
         if (av <= 3.402823466e+38f && av < mn) mn = av;
     }
     c->flat_absmin = mn;
-    if (!c->flat_nz) CK(cudaMalloc((void**)&c->flat_nz, h.size() * sizeof(float)));
+    if (!c->flat_nz) CK(dev_alloc(c->flat_nz, h.size() * sizeof(float)));
     else CK(cudaDeviceSynchronize());
-    CK(cudaMemcpy(c->flat_nz, h.data(), h.size() * sizeof(float), cudaMemcpyHostToDevice));
+    CK(cudaMemcpy(c->flat_nz.get(), h.data(), h.size() * sizeof(float), cudaMemcpyHostToDevice));
     return IMGCORR_OK;
 }
 
@@ -385,8 +405,8 @@ extern "C" IMGCORR_API int imgcorr_set_lens(imgcorr_ctx* c, const double K[9], c
     {
         DeviceGuard g(c->device);
         if (!g.ok) return cuda_fail(cudaGetLastError(), "cudaSetDevice");
-        if (!c->lens_dev) CK(cudaMalloc((void**)&c->lens_dev, sizeof pack));
-        CK(cudaMemcpy(c->lens_dev, pack, sizeof pack, cudaMemcpyHostToDevice));
+        if (!c->lens_dev) CK(dev_alloc(c->lens_dev, sizeof pack));
+        CK(cudaMemcpy(c->lens_dev.get(), pack, sizeof pack, cudaMemcpyHostToDevice));
     }
     c->lens = L;
     c->has_lens = true;
@@ -395,7 +415,7 @@ extern "C" IMGCORR_API int imgcorr_set_lens(imgcorr_ctx* c, const double K[9], c
     if (!c->k2_cache.empty()) {
         DeviceGuard g(c->device);
         cudaDeviceSynchronize();                       // launches that still read the old lens' coordinates
-        free_k2_cache(c);
+        c->k2_cache.clear();
     }
     return IMGCORR_OK;
 }
@@ -417,16 +437,16 @@ static int fill_k1(imgcorr_ctx* c, K1Args& a, const void* raw, int raw_dtype, vo
     if (c->raw_gap % (long long)dtype_size(raw_dtype)) return fail(IMGCORR_ERR_INVALID, "frame gap must be a multiple of the sample size");
     int f = 0;
     if ((flags & IMGCORR_DO_DARK) && c->dark) {
-        f |= FLAG_DARK; a.dark = c->dark;
-        if (c->ascent) { f |= FLAG_DARK_LINEAR; a.ascent = c->ascent; }
+        f |= FLAG_DARK; a.dark = c->dark.get();
+        if (c->ascent) { f |= FLAG_DARK_LINEAR; a.ascent = c->ascent.get(); }
     }
-    if ((flags & IMGCORR_DO_FLAT) && c->flat) { f |= FLAG_FLAT; a.flat = c->flat; }
+    if ((flags & IMGCORR_DO_FLAT) && c->flat) { f |= FLAG_FLAT; a.flat = c->flat.get(); }
     if (flags & IMGCORR_DO_NAN_TO_NUM) f |= FLAG_NAN_TO_NUM;
     a.pw.flags = f; a.pw.exposure_time = c->exposure; a.pw.max_value = c->maxval;
     a.maps_finite = ((!a.dark || c->dark_finite) && (!a.flat || c->flat_finite)) ? 1 : 0;
-    a.flat_nz = a.flat ? c->flat_nz : nullptr;
-    if (!c->dump) CK(cudaMalloc(&c->dump, (size_t)4 << 20));
-    a.dump = c->dump;
+    a.flat_nz = a.flat ? c->flat_nz.get() : nullptr;
+    if (!c->dump) CK(dev_alloc(c->dump, (size_t)4 << 20));
+    a.dump = c->dump.get();
     // integer frames: |raw - dark| <= raw_max + max|dark|; divided by min|flat| it must stay below FLT_MAX
     a.no_overflow = 0;
     if (a.maps_finite && (raw_dtype == DT_U8 || raw_dtype == DT_U16)) {
@@ -448,12 +468,8 @@ extern "C" IMGCORR_API int imgcorr_pointwise_median(imgcorr_ctx* c, const void* 
     a.out_streaming = 1;
     int l = 0;
     cudaError_t e = launch_k1(a, raw_dtype, out_dtype, c->k1_variant, c->sm_count, c->k1_seg_rows, (cudaStream_t)stream, &l);
-    c->launches += l;
-    if (e == cudaErrorInvalidValue && l == 0)
-        return fail(IMGCORR_ERR_INVALID, "unsupported dtype pair raw=%d out=%d", raw_dtype, out_dtype);
-    if (e == cudaErrorNotSupported) return fail(IMGCORR_ERR_INVALID, "requested K1 variant is not eligible for this shape / dtype / alignment");
-    if (e != cudaSuccess) return cuda_fail(e, "K1 launch");
-    return IMGCORR_OK;
+    return launched(c, l, e, "K1 launch", "requested K1 variant is not eligible for this shape / dtype / alignment",
+                    "unsupported dtype pair raw=%d out=%d", raw_dtype, out_dtype);
 }
 
 static int run_k2(imgcorr_ctx* c, const void* src, int sdt, void* dst, int ddt, int n, const float* mapx,
@@ -469,7 +485,7 @@ static int run_k2(imgcorr_ctx* c, const void* src, int sdt, void* dst, int ddt, 
     a.x0 = x0; a.y0 = y0; a.ow = ow; a.oh = oh;
     a.border = border_for_dtype(sdt == DT_U8, sdt == DT_U16, border);
     a.lens = c->lens;
-    a.lens_dev = c->lens_dev;
+    a.lens_dev = c->lens_dev.get();
     a.sm_count = c->sm_count;
     a.tma_store = c->k2_tma_store;
     if (!c->k2_wtab) {
@@ -480,10 +496,12 @@ static int run_k2(imgcorr_ctx* c, const void* src, int sdt, void* dst, int ddt, 
                 bilinear_weights(fx, fy, w.x, w.y, w.z, w.w);
                 t[fy * 32 + fx] = w;
             }
-        CK(cudaMalloc((void**)&c->k2_wtab, t.size() * sizeof(float4)));
-        CK(cudaMemcpy(c->k2_wtab, t.data(), t.size() * sizeof(float4), cudaMemcpyHostToDevice));
+        DevPtr<float4> d;
+        CK(dev_alloc(d, t.size() * sizeof(float4)));
+        CK(cudaMemcpy(d.get(), t.data(), t.size() * sizeof(float4), cudaMemcpyHostToDevice));
+        c->k2_wtab = std::move(d);
     }
-    a.wtab = c->k2_wtab;
+    a.wtab = c->k2_wtab.get();
     a.geometry = 0;
     if (!mapx) {
         bool found = false;
@@ -497,7 +515,7 @@ static int run_k2(imgcorr_ctx* c, const void* src, int sdt, void* dst, int ddt, 
         }
     }
     // coordinate cache (tiled variant, analytic map): the first launch for this lens / window writes it, later ones read it
-    imgcorr_ctx::K2Cache* building = nullptr;
+    imgcorr_ctx::K2Cache fresh{};                      // the entry this launch writes; it joins the cache once its event is recorded
     // Only launches of one or two frames use it: a batch amortises the analytic evaluation over its frames and the
     // per-tile kernel then streams faster (19 vs 33 us per 4096x3000 frame) than the cached one (49 vs 65 us for one frame).
     if (!mapx && c->k2_cache_on && n > 0 && n <= 2 && ow > 0 && oh > 0 && k2_will_tile(a, sdt, ddt, c->k2_variant)) {
@@ -506,49 +524,36 @@ static int run_k2(imgcorr_ctx* c, const void* src, int sdt, void* dst, int ddt, 
         for (auto& k : c->k2_cache)
             if (k.x0 == x0 && k.y0 == y0 && k.ow == ow && k.oh == oh && k.g == a.geometry && k.esz == esz) { hit = &k; break; }
         if (hit) {
-            if (hit->st != st) CK(cudaStreamWaitEvent(st, hit->ev, 0));       // written on another stream
+            if (hit->st != st) CK(cudaStreamWaitEvent(st, hit->ev.get(), 0));       // written on another stream
             hit->stamp = ++c->k2_stamp;
-            a.cpack = hit->pack; a.chdr = hit->hdr;
+            a.cpack = hit->pack.get(); a.chdr = hit->hdr.get();
         } else {
             if (c->k2_cache.size() >= 2) {             // keep at most two windows (keep_size True / False): drop the older one
                 size_t old = c->k2_cache[0].stamp < c->k2_cache[1].stamp ? 0 : 1;
                 CK(cudaDeviceSynchronize());
-                cudaFree(c->k2_cache[old].pack); cudaFree(c->k2_cache[old].hdr);
-                if (c->k2_cache[old].ev) cudaEventDestroy(c->k2_cache[old].ev);
                 c->k2_cache.erase(c->k2_cache.begin() + old);
             }
             size_t words = 0, tiles = 0;
             k2_cache_size(a.geometry, ow, oh, &words, &tiles);
-            imgcorr_ctx::K2Cache k{x0, y0, ow, oh, a.geometry, esz, nullptr, nullptr, nullptr, st, ++c->k2_stamp};
-            if (cudaMalloc((void**)&k.pack, words * sizeof(unsigned)) == cudaSuccess &&
-                cudaMalloc((void**)&k.hdr, tiles * sizeof(int2)) == cudaSuccess &&
-                cudaEventCreateWithFlags(&k.ev, cudaEventDisableTiming) == cudaSuccess) {
-                c->k2_cache.push_back(k);
-                building = &c->k2_cache.back();
-                a.cpack_w = k.pack; a.chdr_w = k.hdr;
+            imgcorr_ctx::K2Cache k{x0, y0, ow, oh, a.geometry, esz, {}, {}, {}, st, ++c->k2_stamp};
+            if (dev_alloc(k.pack, words * sizeof(unsigned)) == cudaSuccess && dev_alloc(k.hdr, tiles * sizeof(int2)) == cudaSuccess &&
+                new_event(k.ev) == cudaSuccess) {
+                fresh = std::move(k);
+                a.cpack_w = fresh.pack.get(); a.chdr_w = fresh.hdr.get();
             } else {                                   // no memory for the cache: compute every time
                 cudaGetLastError();
-                cudaFree(k.pack); cudaFree(k.hdr);
-                if (k.ev) cudaEventDestroy(k.ev);
             }
         }
     }
     int l = 0;
     cudaError_t e = launch_k2(a, sdt, ddt, c->k2_variant, st, &l);
-    if (building) {
-        if (e == cudaSuccess) e = cudaEventRecord(building->ev, st);
-        if (e != cudaSuccess) {                        // never leave a half-written cache behind
-            cudaDeviceSynchronize();
-            cudaFree(building->pack); cudaFree(building->hdr); cudaEventDestroy(building->ev);
-            c->k2_cache.pop_back();
-        }
+    if (fresh.ev) {                                    // never leave a half-written cache behind
+        if (e == cudaSuccess) e = cudaEventRecord(fresh.ev.get(), st);
+        if (e == cudaSuccess) c->k2_cache.push_back(std::move(fresh));
+        else cudaDeviceSynchronize();                  // a queued kernel may still write the buffers `fresh` frees on return
     }
-    c->launches += l;
-    if (e == cudaErrorInvalidValue && l == 0)
-        return fail(IMGCORR_ERR_INVALID, "unsupported dtype pair src=%d dst=%d", sdt, ddt);
-    if (e == cudaErrorNotSupported) return fail(IMGCORR_ERR_INVALID, "requested K2 variant is not eligible for this dtype / alignment");
-    if (e != cudaSuccess) return cuda_fail(e, "K2 launch");
-    return IMGCORR_OK;
+    return launched(c, l, e, "K2 launch", "requested K2 variant is not eligible for this dtype / alignment",
+                    "unsupported dtype pair src=%d dst=%d", sdt, ddt);
 }
 
 extern "C" IMGCORR_API int imgcorr_undistort(imgcorr_ctx* c, const void* src_dev, int src_dtype, void* dst_dev, int dst_dtype,
@@ -573,9 +578,7 @@ extern "C" IMGCORR_API int imgcorr_undistort_maps(imgcorr_ctx* c, float* mapx_de
     if (!mapx_dev || !mapy_dev) return fail(IMGCORR_ERR_INVALID, "null map pointer");
     int l = 0;
     cudaError_t e = launch_write_maps(c->lens, mapx_dev, mapy_dev, c->H, c->W, (cudaStream_t)stream, &l);
-    c->launches += l;
-    if (e != cudaSuccess) return cuda_fail(e, "map kernel launch");
-    return IMGCORR_OK;
+    return launched(c, l, e, "map kernel launch");
 }
 
 // ---- K3 -------------------------------------------------------------------------------------
@@ -594,8 +597,10 @@ extern "C" IMGCORR_API int imgcorr_warp_perspective(imgcorr_ctx* c, const void* 
         float h[32 * 8 + 32 * 4];
         warp_lanczos4_table(h);
         warp_cubic_table(h + 32 * 8);
-        CK(cudaMalloc(&c->warp_tab, sizeof(h)));
-        CK(cudaMemcpy(c->warp_tab, h, sizeof(h), cudaMemcpyHostToDevice));
+        DevPtr<float> d;
+        CK(dev_alloc(d, sizeof(h)));
+        CK(cudaMemcpy(d.get(), h, sizeof(h), cudaMemcpyHostToDevice));
+        c->warp_tab = std::move(d);
     }
     const int lz = interpolation == IMGCORR_INTER_LANCZOS4;
     if (dtype == DT_U8 && !c->warp_itab[lz]) {
@@ -605,11 +610,13 @@ extern "C" IMGCORR_API int imgcorr_warp_perspective(imgcorr_ctx* c, const void* 
         if (lz) warp_lanczos4_table(t.data()); else warp_cubic_table(t.data());
         std::vector<int16_t> it((size_t)32 * 32 * nn * nn);
         warp_fixed_table(t.data(), nn, it.data());
-        CK(cudaMalloc(&c->warp_itab[lz], it.size() * sizeof(int16_t)));
-        CK(cudaMemcpy(c->warp_itab[lz], it.data(), it.size() * sizeof(int16_t), cudaMemcpyHostToDevice));
+        DevPtr<int16_t> d;
+        CK(dev_alloc(d, it.size() * sizeof(int16_t)));
+        CK(cudaMemcpy(d.get(), it.data(), it.size() * sizeof(int16_t), cudaMemcpyHostToDevice));
+        c->warp_itab[lz] = std::move(d);
     }
     K3Args a;
-    a.itab = dtype == DT_U8 ? c->warp_itab[lz] : nullptr;
+    a.itab = dtype == DT_U8 ? c->warp_itab[lz].get() : nullptr;
     a.src = src_dev;
     a.dst = dst_dev;
     a.H = src_h;
@@ -619,13 +626,10 @@ extern "C" IMGCORR_API int imgcorr_warp_perspective(imgcorr_ctx* c, const void* 
     a.n_frames = n_frames;
     a.border = border_for_dtype(dtype == DT_U8, dtype == DT_U16, border_value);
     a.wc = make_warp_const(M, inverse_map, dst_w, dst_h);
-    a.tab = interpolation == IMGCORR_INTER_LANCZOS4 ? c->warp_tab : c->warp_tab + 32 * 8;
+    a.tab = interpolation == IMGCORR_INTER_LANCZOS4 ? c->warp_tab.get() : c->warp_tab.get() + 32 * 8;
     int l = 0;
     cudaError_t e = launch_k3(a, dtype, interpolation, c->k3_variant, (cudaStream_t)stream, &l);
-    c->launches += l;
-    if (e == cudaErrorNotSupported) return fail(IMGCORR_ERR_INVALID, "the requested K3 variant is not eligible for this call");
-    if (e != cudaSuccess) return cuda_fail(e, "K3 launch");
-    return IMGCORR_OK;
+    return launched(c, l, e, "K3 launch", "the requested K3 variant is not eligible for this call");
 }
 
 extern "C" IMGCORR_API int imgcorr_divide_f64(imgcorr_ctx* c, const void* src_dev, int src_dtype, const double* divisor_dev,
@@ -637,9 +641,7 @@ extern "C" IMGCORR_API int imgcorr_divide_f64(imgcorr_ctx* c, const void* src_de
     int l = 0;
     cudaError_t e = launch_k3_divide(src_dev, src_dtype, divisor_dev, dst_dev, pixels_per_frame, n_frames, c->sm_count,
                                      (cudaStream_t)stream, &l);
-    c->launches += l;
-    if (e != cudaSuccess) return cuda_fail(e, "divide kernel launch");
-    return IMGCORR_OK;
+    return launched(c, l, e, "divide kernel launch");
 }
 
 // ---- K4 -------------------------------------------------------------------------------------
@@ -666,22 +668,20 @@ static int ste_average_impl(imgcorr_ctx* c, const void* frames_dev, int dtype, i
     if (!frames_dev || !avg_dev || !nlf) return fail(IMGCORR_ERR_INVALID, "null pointer");
     if (dtype < DT_U8 || dtype > DT_F64) return fail(IMGCORR_ERR_INVALID, "bad dtype %d", dtype);
     if (n_frames < 2) return fail(IMGCORR_ERR_INVALID, "single-time-effect removal needs at least 2 images (got %d)", n_frames);
-    const size_t npx = (size_t)c->H * c->W;
-    if (!c->ste_avg) {
-        CK(cudaMalloc(&c->ste_avg, npx * sizeof(double)));
-        CK(cudaMalloc(&c->ste_thr, npx * sizeof(double)));
-        CK(cudaMalloc(&c->ste_n, npx * sizeof(int)));
-    }
+    const size_t npx = (size_t)c->H * c->W, part = round256(npx * sizeof(double));
     cudaStream_t st = (cudaStream_t)stream;
+    CK(c->ste_scratch.acquire(2 * part + npx * sizeof(int), st));    // [running average][thresholds][counts]
+    SharedScratch::Guard release{c->ste_scratch, st};
+    char* const s = c->ste_scratch.buf.get();
     // n_frames - 1 launches; ping-pong so that the last one writes avg_dev
-    double* buf[2] = {avg_dev, c->ste_avg};
+    double* buf[2] = {avg_dev, (double*)s};
     int cur = (n_frames - 2) % 2;                  // buffer the FIRST launch writes
     K4Args a;
     a.H = c->H;
     a.W = c->W;
-    a.thr = c->ste_thr;
+    a.thr = (double*)(s + part);
     a.thr_in = thr_dev;
-    a.n = c->ste_n;
+    a.n = (int*)(s + 2 * part);
     a.mask = mask_dev;
     a.sc.minY = nlf[0];
     a.sc.ax = nlf[1];
@@ -699,9 +699,7 @@ static int ste_average_impl(imgcorr_ctx* c, const void* frames_dev, int dtype, i
         e = launch_k4(a, dtype, st, &l);
         cur ^= 1;
     }
-    c->launches += l;
-    if (e != cudaSuccess) return cuda_fail(e, "K4 launch");
-    return IMGCORR_OK;
+    return launched(c, l, e, "K4 launch");
 }
 
 // one frame (or a group of frames) through K1 -> K2 on `st`
@@ -719,63 +717,53 @@ static int chain_frames(imgcorr_ctx* c, const void* raw, int raw_dtype, void* ou
         if (r) return r;
         int l = 0;
         cudaError_t e = launch_k1(a, raw_dtype, out_dtype, c->k1_variant, c->sm_count, c->k1_seg_rows, st, &l);
-        c->launches += l;
-        if (e != cudaSuccess) return cuda_fail(e, "K1 launch");
-        return IMGCORR_OK;
+        return launched(c, l, e, "K1 launch");
     }
-    // K1 -> K2 in groups of `chain_group` frames: the K1 output of a group stays in two alternating scratch
-    // buffers (L2-resident for small groups); K2 evaluates each pixel's map once per group.
+    // K1 -> K2 in groups of `chain_group` frames: the K1 output of a group stays in two alternating halves of the chain
+    // scratch (L2-resident for small groups); K2 evaluates each pixel's map once per group.
     const int grp = c->chain_group < n ? c->chain_group : (n > 0 ? n : 1);
-    if (c->mid_frames < (size_t)grp) {
-        CK(cudaDeviceSynchronize());                   // calls on other streams (correct_host, other torch streams) may still use mid[]
-        for (int i = 0; i < 2; ++i) {
-            if (c->mid[i]) { CK(cudaFree(c->mid[i])); c->mid[i] = nullptr; }
-            CK(cudaMalloc((void**)&c->mid[i], npx * sizeof(float) * grp));
-        }
-        c->mid_frames = grp;
-    }
-    // mid[] is one pair per context: a call on another stream than the last one first waits until that call's K2 has
-    // read it.  The wait precedes ev_entry, so the overlap stream inherits it.
-    if (!c->ev_mid) CK(cudaEventCreateWithFlags(&c->ev_mid, cudaEventDisableTiming));
-    else if (c->mid_st != st) CK(cudaStreamWaitEvent(st, c->ev_mid, 0));
-    struct MidRelease {                                // every K1 / K2 of this call is ordered before the end of `st`
-        imgcorr_ctx* c; cudaStream_t st;
-        ~MidRelease() { cudaEventRecord(c->ev_mid, st); c->mid_st = st; }
-    } release{c, st};
+    const size_t half = round256(npx * sizeof(float) * grp);
+    // the wait for another stream's last use precedes ev_entry, so the overlap stream inherits it
+    CK(c->chain_scratch.acquire(2 * half, st));
+    SharedScratch::Guard release{c->chain_scratch, st};    // every K1 / K2 of this call is ordered before the end of `st`
+    float* const mids[2] = {(float*)c->chain_scratch.buf.get(), (float*)(c->chain_scratch.buf.get() + half)};
     const size_t out_stride = (size_t)ow * oh * dtype_size(out_dtype);
     // Overlap mode: K1 of group g+1 runs on an internal high-priority stream while K2 of group g runs on the caller's
     // stream, so that K2's blocks fill the SM slots K1's last, partially filled wave leaves idle (and vice versa).  The
-    // two scratch buffers are handed back and forth with events; every K2 stays on the caller's stream, so the call is
-    // stream-ordered as before.  A profiled group (IMGCORR_OPT_PROFILE) runs unoverlapped so that its brackets time the
+    // two halves of the scratch are handed back and forth with events; every K2 stays on the caller's stream, so the call
+    // is stream-ordered as before.  A profiled group (IMGCORR_OPT_PROFILE) runs unoverlapped so that its brackets time the
     // kernel alone.
     const bool overlap = c->chain_overlap && n > grp;
+    imgcorr_ctx::ChainOverlap& ov = c->ov;
     cudaStream_t s1 = st;
     if (overlap) {
-        if (!c->s_chain) {
+        if (!ov.st) {
             int lo = 0, hi = 0;
             CK(cudaDeviceGetStreamPriorityRange(&lo, &hi));
-            CK(cudaStreamCreateWithPriority(&c->s_chain, cudaStreamNonBlocking, hi));
+            imgcorr_ctx::ChainOverlap o;
+            CK(new_stream(o.st, hi));
             for (int i = 0; i < 2; ++i) {
-                CK(cudaEventCreateWithFlags(&c->ev_k1[i], cudaEventDisableTiming));
-                CK(cudaEventCreateWithFlags(&c->ev_k2[i], cudaEventDisableTiming));
+                CK(new_event(o.k1[i]));
+                CK(new_event(o.k2[i]));
             }
-            CK(cudaEventCreateWithFlags(&c->ev_entry, cudaEventDisableTiming));
+            CK(new_event(o.entry));
+            ov = std::move(o);
         }
-        s1 = c->s_chain;
-        CK(cudaEventRecord(c->ev_entry, st));          // K1 must not start before the caller's earlier work on `st`
-        CK(cudaStreamWaitEvent(s1, c->ev_entry, 0));
+        s1 = ov.st.get();
+        CK(cudaEventRecord(ov.entry.get(), st));      // K1 must not start before the caller's earlier work on `st`
+        CK(cudaStreamWaitEvent(s1, ov.entry.get(), 0));
     }
     int gi = 0;
     bool exclusive_next = false;
     for (int f = 0; f < n; f += grp, ++gi) {
         const int nf = n - f < grp ? n - f : grp;
-        float* mid = c->mid[gi & 1];
+        float* mid = mids[gi & 1];
         const bool prof = c->profile > 0 && (c->chain_groups_seen++ % c->profile) == 0;
         if (prof) { c->prof_frames[0] += nf; c->prof_frames[1] += nf; }
         if (overlap) {
-            // this buffer was last read by K2 of group gi-2; a profiled group (or the one after it) also waits for gi-1
-            if (gi >= 2) CK(cudaStreamWaitEvent(s1, c->ev_k2[gi & 1], 0));
-            if ((prof || exclusive_next) && gi >= 1) CK(cudaStreamWaitEvent(s1, c->ev_k2[(gi - 1) & 1], 0));
+            // this half was last read by K2 of group gi-2; a profiled group (or the one after it) also waits for gi-1
+            if (gi >= 2) CK(cudaStreamWaitEvent(s1, ov.k2[gi & 1].get(), 0));
+            if ((prof || exclusive_next) && gi >= 1) CK(cudaStreamWaitEvent(s1, ov.k2[(gi - 1) & 1].get(), 0));
             exclusive_next = prof;
         }
         K1Args a;
@@ -785,17 +773,16 @@ static int chain_frames(imgcorr_ctx* c, const void* raw, int raw_dtype, void* ou
         if (prof) prof_mark(c, 0, s1);
         cudaError_t e = launch_k1(a, raw_dtype, DT_F32, c->k1_variant, c->sm_count, c->k1_seg_rows, s1, &l);
         if (prof) prof_mark(c, 0, s1);
-        c->launches += l;
-        if (e != cudaSuccess) return cuda_fail(e, "K1 launch");
+        if ((r = launched(c, l, e, "K1 launch"))) return r;
         if (overlap) {
-            CK(cudaEventRecord(c->ev_k1[gi & 1], s1));
-            CK(cudaStreamWaitEvent(st, c->ev_k1[gi & 1], 0));
+            CK(cudaEventRecord(ov.k1[gi & 1].get(), s1));
+            CK(cudaStreamWaitEvent(st, ov.k1[gi & 1].get(), 0));
         }
         if (prof) prof_mark(c, 1, st);
         r = run_k2(c, mid, DT_F32, (char*)out + f * out_stride, out_dtype, nf, nullptr, nullptr, border, x0, y0, ow, oh, st);
         if (prof) prof_mark(c, 1, st);
         if (r) return r;
-        if (overlap) CK(cudaEventRecord(c->ev_k2[gi & 1], st));
+        if (overlap) CK(cudaEventRecord(ov.k2[gi & 1].get(), st));
     }
     return IMGCORR_OK;
 }
@@ -820,22 +807,27 @@ static bool is_pinned(const void* p) {
 
 static int ensure_pipeline(imgcorr_ctx* c, size_t raw_bytes, size_t out_bytes) {
     if (!c->s_in) {
-        CK(cudaStreamCreateWithFlags(&c->s_in, cudaStreamNonBlocking));
-        CK(cudaStreamCreateWithFlags(&c->s_k, cudaStreamNonBlocking));
-        CK(cudaStreamCreateWithFlags(&c->s_out, cudaStreamNonBlocking));
+        Stream in, k, out;
+        CK(new_stream(in));
+        CK(new_stream(k));
+        CK(new_stream(out));
+        c->s_in = std::move(in);
+        c->s_k = std::move(k);
+        c->s_out = std::move(out);
     }
     if ((int)c->slots.size() == c->host_slots && c->slot_raw_bytes >= raw_bytes && c->slot_out_bytes >= out_bytes)
         return IMGCORR_OK;
     CK(cudaDeviceSynchronize());
-    free_slots(c);
-    c->slots.resize(c->host_slots);
-    for (auto& s : c->slots) {
-        CK(cudaMalloc(&s.d_raw, raw_bytes));
-        CK(cudaMalloc(&s.d_out, out_bytes));
-        CK(cudaEventCreateWithFlags(&s.ev_in, cudaEventDisableTiming));
-        CK(cudaEventCreateWithFlags(&s.ev_k, cudaEventDisableTiming));
-        CK(cudaEventCreateWithFlags(&s.ev_out, cudaEventDisableTiming));
+    c->slots.clear();                                  // the old ring goes first, so peak memory stays one ring
+    std::vector<HostSlot> ring(c->host_slots);
+    for (auto& s : ring) {
+        CK(dev_alloc(s.d_raw, raw_bytes));
+        CK(dev_alloc(s.d_out, out_bytes));
+        CK(new_event(s.ev_in));
+        CK(new_event(s.ev_k));
+        CK(new_event(s.ev_out));
     }
+    c->slots = std::move(ring);
     c->slot_raw_bytes = raw_bytes;
     c->slot_out_bytes = out_bytes;
     return IMGCORR_OK;
@@ -865,21 +857,22 @@ extern "C" IMGCORR_API int imgcorr_correct_host(imgcorr_ctx* c, const void* raw_
     if (r) return r;
     const bool in_pinned = is_pinned(raw_host), out_pinned = is_pinned(out_host);
     for (auto& s : c->slots) {
-        if (!in_pinned && !s.h_raw) CK(cudaHostAlloc(&s.h_raw, c->slot_raw_bytes, cudaHostAllocDefault));
-        if (!out_pinned && !s.h_out) CK(cudaHostAlloc(&s.h_out, c->slot_out_bytes, cudaHostAllocDefault));
+        if (!in_pinned && !s.h_raw) CK(host_alloc(s.h_raw, c->slot_raw_bytes));
+        if (!out_pinned && !s.h_out) CK(host_alloc(s.h_out, c->slot_out_bytes));
     }
     const int ns = (int)c->slots.size();
     const int chunks = (n_frames + G - 1) / G;
+    cudaStream_t const s_in = c->s_in.get(), s_k = c->s_k.get(), s_out = c->s_out.get();
     // whatever happens below, no copy from / into the caller's buffers may still be in flight when this call returns
     struct Drain {
-        imgcorr_ctx* c; bool armed = true;
-        ~Drain() { if (armed) { cudaStreamSynchronize(c->s_in); cudaStreamSynchronize(c->s_k); cudaStreamSynchronize(c->s_out); } }
-    } drain{c};
+        cudaStream_t s_in, s_k, s_out; bool armed = true;
+        ~Drain() { if (armed) { cudaStreamSynchronize(s_in); cudaStreamSynchronize(s_k); cudaStreamSynchronize(s_out); } }
+    } drain{s_in, s_k, s_out};
     auto frames_of = [&](int k) { return n_frames - k * G < G ? n_frames - k * G : G; };
     auto retire = [&](int k) -> int {          // chunk k's D2H has been enqueued on s_out in slot k % ns
         HostSlot& s = c->slots[k % ns];
-        CK(cudaEventSynchronize(s.ev_out));
-        if (!out_pinned) memcpy((char*)out_host + (size_t)k * out_bytes, s.h_out, frame_out * frames_of(k));
+        CK(cudaEventSynchronize(s.ev_out.get()));
+        if (!out_pinned) memcpy((char*)out_host + (size_t)k * out_bytes, s.h_out.get(), frame_out * frames_of(k));
         return IMGCORR_OK;
     };
     for (int k = 0; k < chunks; ++k) {
@@ -887,18 +880,18 @@ extern "C" IMGCORR_API int imgcorr_correct_host(imgcorr_ctx* c, const void* raw_
         if (k >= ns) { r = retire(k - ns); if (r) return r; }
         const int nf = frames_of(k);
         const char* src = (const char*)raw_host + (size_t)k * raw_bytes;
-        if (!in_pinned) { memcpy(s.h_raw, src, frame_raw * nf); src = (const char*)s.h_raw; }
-        CK(cudaMemcpyAsync(s.d_raw, src, frame_raw * nf, cudaMemcpyHostToDevice, c->s_in));
-        CK(cudaEventRecord(s.ev_in, c->s_in));
-        CK(cudaStreamWaitEvent(c->s_k, s.ev_in, 0));
-        r = chain_frames(c, s.d_raw, raw_dtype, s.d_out, out_dtype, nf, threshold, ksize, flags, lens, border_value, x0, y0,
-                         ow, oh, c->s_k);
+        if (!in_pinned) { memcpy(s.h_raw.get(), src, frame_raw * nf); src = (const char*)s.h_raw.get(); }
+        CK(cudaMemcpyAsync(s.d_raw.get(), src, frame_raw * nf, cudaMemcpyHostToDevice, s_in));
+        CK(cudaEventRecord(s.ev_in.get(), s_in));
+        CK(cudaStreamWaitEvent(s_k, s.ev_in.get(), 0));
+        r = chain_frames(c, s.d_raw.get(), raw_dtype, s.d_out.get(), out_dtype, nf, threshold, ksize, flags, lens, border_value,
+                         x0, y0, ow, oh, s_k);
         if (r) return r;
-        CK(cudaEventRecord(s.ev_k, c->s_k));
-        CK(cudaStreamWaitEvent(c->s_out, s.ev_k, 0));
-        void* dst = out_pinned ? (void*)((char*)out_host + (size_t)k * out_bytes) : s.h_out;
-        CK(cudaMemcpyAsync(dst, s.d_out, frame_out * nf, cudaMemcpyDeviceToHost, c->s_out));
-        CK(cudaEventRecord(s.ev_out, c->s_out));
+        CK(cudaEventRecord(s.ev_k.get(), s_k));
+        CK(cudaStreamWaitEvent(s_out, s.ev_k.get(), 0));
+        void* dst = out_pinned ? (void*)((char*)out_host + (size_t)k * out_bytes) : s.h_out.get();
+        CK(cudaMemcpyAsync(dst, s.d_out.get(), frame_out * nf, cudaMemcpyDeviceToHost, s_out));
+        CK(cudaEventRecord(s.ev_out.get(), s_out));
     }
     for (int k = (chunks > ns ? chunks - ns : 0); k < chunks; ++k) { r = retire(k); if (r) return r; }
     drain.armed = false;                               // every chunk was retired: nothing is in flight
@@ -908,13 +901,12 @@ extern "C" IMGCORR_API int imgcorr_correct_host(imgcorr_ctx* c, const void* raw_
 extern "C" IMGCORR_API int imgcorr_selftest_division(imgcorr_ctx* c, int numerators_per_divisor, unsigned long long seed, double out[2]) {
     GUARD(c);
     if (!out || numerators_per_divisor < 1) return fail(IMGCORR_ERR_INVALID, "bad self-test arguments");
-    unsigned long long* d = nullptr;
+    DevPtr<unsigned long long> d;
     unsigned long long h[2] = {0, 0};
-    CK(cudaMalloc((void**)&d, sizeof h));
-    cudaError_t e = cudaMemset(d, 0, sizeof h);
-    if (e == cudaSuccess) e = launch_selftest_division(numerators_per_divisor, seed, d, nullptr);
-    if (e == cudaSuccess) e = cudaMemcpy(h, d, sizeof h, cudaMemcpyDeviceToHost);
-    cudaFree(d);
+    CK(dev_alloc(d, sizeof h));
+    cudaError_t e = cudaMemset(d.get(), 0, sizeof h);
+    if (e == cudaSuccess) e = launch_selftest_division(numerators_per_divisor, seed, d.get(), nullptr);
+    if (e == cudaSuccess) e = cudaMemcpy(h, d.get(), sizeof h, cudaMemcpyDeviceToHost);
     if (e != cudaSuccess) return cuda_fail(e, "division self-test");
     c->launches += 1;
     out[0] = (double)h[0];
@@ -935,9 +927,7 @@ extern "C" IMGCORR_API int imgcorr_stack_mean(imgcorr_ctx* c, const void* frames
     int l = 0;
     cudaError_t e = launch_k5_stack_mean(frames_dev, dtype, n_frames, elems, minus_dev, minus_scalar, use_scalar, gray3, out_dev, c->sm_count,
                                          (cudaStream_t)stream, &l);
-    c->launches += l;
-    if (e != cudaSuccess) return cuda_fail(e, "stack mean launch");
-    return IMGCORR_OK;
+    return launched(c, l, e, "stack mean launch");
 }
 
 extern "C" IMGCORR_API int imgcorr_scale_f64(imgcorr_ctx* c, double* data_dev, size_t elems, double divisor, void* stream) {
@@ -945,9 +935,7 @@ extern "C" IMGCORR_API int imgcorr_scale_f64(imgcorr_ctx* c, double* data_dev, s
     if (!data_dev) return fail(IMGCORR_ERR_INVALID, "null pointer");
     int l = 0;
     cudaError_t e = launch_k5_scale(data_dev, elems, divisor, c->sm_count, (cudaStream_t)stream, &l);
-    c->launches += l;
-    if (e != cudaSuccess) return cuda_fail(e, "scale launch");
-    return IMGCORR_OK;
+    return launched(c, l, e, "scale launch");
 }
 
 extern "C" IMGCORR_API int imgcorr_subsample_f64(imgcorr_ctx* c, const double* src_dev, int height, int width, int step_y, int step_x,
@@ -957,9 +945,7 @@ extern "C" IMGCORR_API int imgcorr_subsample_f64(imgcorr_ctx* c, const double* s
     if (height <= 0 || width <= 0 || step_y <= 0 || step_x <= 0) return fail(IMGCORR_ERR_INVALID, "bad shape / step");
     int l = 0;
     cudaError_t e = launch_k5_subsample(src_dev, height, width, step_y, step_x, dst_dev, (cudaStream_t)stream, &l);
-    c->launches += l;
-    if (e != cudaSuccess) return cuda_fail(e, "subsample launch");
-    return IMGCORR_OK;
+    return launched(c, l, e, "subsample launch");
 }
 
 extern "C" IMGCORR_API int imgcorr_linear_fit(imgcorr_ctx* c, const void* frames_dev, int dtype, int n_frames, size_t pixels, const double* x_host,
@@ -971,19 +957,16 @@ extern "C" IMGCORR_API int imgcorr_linear_fit(imgcorr_ctx* c, const void* frames
     if (n_frames < 2) return fail(IMGCORR_ERR_INVALID, "a line needs at least 2 exposure times (got %d)", n_frames);
     double mn = x_host[0], mx = x_host[0];
     for (int k = 1; k < n_frames; ++k) { mn = x_host[k] < mn ? x_host[k] : mn; mx = x_host[k] > mx ? x_host[k] : mx; }
-    double* xs = nullptr;
-    CK(cudaMalloc((void**)&xs, n_frames * sizeof(double)));
+    DevPtr<double> xs;
+    CK(dev_alloc(xs, n_frames * sizeof(double)));
     cudaStream_t st = (cudaStream_t)stream;
-    cudaError_t e = cudaMemcpyAsync(xs, x_host, n_frames * sizeof(double), cudaMemcpyHostToDevice, st);
+    cudaError_t e = cudaMemcpyAsync(xs.get(), x_host, n_frames * sizeof(double), cudaMemcpyHostToDevice, st);
     int l = 0;
     if (e == cudaSuccess)
-        e = launch_k5_linear_fit(frames_dev, dtype, n_frames, pixels, xs, max_intensity, min_ascent, 0.5 * (mn + mx), offset_dev, ascent_dev,
-                                 rmse_dev, c->sm_count, st, &l);
-    c->launches += l;
+        e = launch_k5_linear_fit(frames_dev, dtype, n_frames, pixels, xs.get(), max_intensity, min_ascent, 0.5 * (mn + mx), offset_dev,
+                                 ascent_dev, rmse_dev, c->sm_count, st, &l);
     if (e == cudaSuccess) e = cudaStreamSynchronize(st);       // x_host / xs may go away when this returns
-    cudaFree(xs);
-    if (e != cudaSuccess) return cuda_fail(e, "linear fit");
-    return IMGCORR_OK;
+    return launched(c, l, e, "linear fit");
 }
 
 // ---- host-side fingerprint of a calibration array ---------------------------------------------------------

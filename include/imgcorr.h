@@ -193,13 +193,19 @@ IMGCORR_API int imgcorr_divide_f64(imgcorr_ctx* ctx, const void* src_dev, int sr
  *   frames_dev [n][H][W] of `dtype` (any), n >= 2;  avg_dev [H][W] float64 = noSTE;
  *   mask_dev   [H][W] uint8 accumulated STE mask (save_ste_indices=True) or NULL.
  * float64 arithmetic as in the reference; the running mean avg += (x - avg) / n restates fancytools'
- * MaskedMovingAverage (absent from the reference tree: that ingredient's parity is unpinned, see oracle/ste.py). */
+ * MaskedMovingAverage (absent from the reference tree: that ingredient's parity is unpinned, see oracle/ste.py).
+ * Asynchronous on `stream`.  The context's K4 scratch is shared by every K4 call (imgcorr_ste_average_thr included): a call
+ * on another stream than the previous K4 call first waits for that call's work on the scratch, so calls of one context on
+ * several streams are correct and run one after the other on the device. */
 IMGCORR_API int imgcorr_ste_average(imgcorr_ctx* ctx, const void* frames_dev, int dtype, int n_frames, double* avg_dev,
                         uint8_t* mask_dev, const double nlf[3], double n_std, void* stream);
 /* The same with a caller-supplied threshold map  threshold_dev[H][W] = noise_level_function(min(images[0], images[1])) * nStd
  * (float64) for noise level functions that are not boundedFunction: the one correct() ESTIMATES when no 'noise' calibration
  * exists may be a polynomial (oneImageNLF -> smooth, camera/NoiseLevelFunction.py:132-159), and a user may have assigned any
- * Python callable to CameraCalibration.noise_level_function. */
+ * Python callable to CameraCalibration.noise_level_function.
+ * Asynchronous on `stream`.  The context's K4 scratch is shared by every K4 call (imgcorr_ste_average included): a call on
+ * another stream than the previous K4 call first waits for that call's work on the scratch, so calls of one context on
+ * several streams are correct and run one after the other on the device. */
 IMGCORR_API int imgcorr_ste_average_thr(imgcorr_ctx* ctx, const void* frames_dev, int dtype, int n_frames, double* avg_dev,
                             uint8_t* mask_dev, const double* threshold_dev, void* stream);
 

@@ -95,6 +95,38 @@ def test_k4_full_frame_properties(engine):
     assert np.array_equal(avg[1400:1600, 1900:2100].cpu().numpy(), ra)
 
 
+def test_k4_two_streams_share_one_context(engine):
+    """two K4 calls of one context on two torch streams, released together by one event after a spin: the second waits
+    for the first's scratch (running average, thresholds, counts) instead of overwriting it"""
+    H, W, n = 1024, 1024, 6
+    rng = np.random.default_rng(23)
+    nlf = (2.0, 10.0, 0.8)
+    stacks = []
+    for level in (3000, 9000):
+        f = rng.normal(level, 40, (n, H, W))
+        f[rng.random(f.shape) < 0.01] += 2000                   # single pixels and, by chance, clusters
+        f[n - 1, 100:103, 200:204] += 5000                      # a blob: stays an STE
+        stacks.append(np.clip(f, 0, 65535).astype(np.uint16))
+    want = [ste.ste_average(list(f), nlf, 4, True) for f in stacks]
+    e = engine.get_engine(H, W)
+    a, b = _dev(stacks[0]), _dev(stacks[1])
+    e.ste_average(a[:2], nlf, 4)                                 # allocation outside the race
+    sa, sb = torch.cuda.Stream(), torch.cuda.Stream()
+    go = torch.cuda.Event()
+    torch.cuda.synchronize()
+    with torch.cuda.stream(sa):
+        torch.cuda._sleep(600_000_000)                           # about 0.3 s of device time
+        go.record(sa)
+        got_a = e.ste_average(a, nlf, 4, want_mask=True)
+    with torch.cuda.stream(sb):
+        sb.wait_event(go)
+        got_b = e.ste_average(b, nlf, 4, want_mask=True)
+    torch.cuda.synchronize()
+    for tag, (avg, mask), (ra, rm) in zip('ab', (got_a, got_b), want):
+        assert np.array_equal(avg.cpu().numpy(), ra), tag
+        assert np.array_equal(mask.cpu().numpy(), rm), tag
+
+
 def test_correct_with_several_exposures():
     """the Python mirror against the reference's correct() (multi-image branches :385-406, :484-498)"""
     if not torch.cuda.is_available():
