@@ -9,7 +9,7 @@ _LIB = None
 
 U8, U16, F32, F64 = 0, 1, 2, 3
 COND_GT, COND_LT = 0, 1
-DO_DARK, DO_FLAT, DO_NAN_TO_NUM = 1, 2, 4
+DO_DARK, DO_FLAT, DO_NAN_TO_NUM, DO_PERSPECTIVE = 1, 2, 4, 8
 OPT_K1_VARIANT, OPT_K2_VARIANT, OPT_HOST_SLOTS, OPT_K1_SEG_ROWS, OPT_PROFILE, OPT_CHAIN_GROUP = 1, 2, 3, 4, 5, 6
 OPT_RAW_BIG_ENDIAN, OPT_RAW_FRAME_GAP, OPT_K3_VARIANT, OPT_CHAIN_OVERLAP, OPT_K2_COORD_CACHE, OPT_K2_TMA_STORE = 7, 8, 9, 10, 11, 12
 INTER_CUBIC, INTER_LANCZOS4 = 2, 4
@@ -41,6 +41,7 @@ SIGNATURES = {
                                       c_double, c_int, c_int, c_int, c_int, c_void_p]),
     'imgcorr_correct_host': (c_int, [c_void_p, c_void_p, c_int, c_void_p, c_int, c_int, c_double, c_int, c_int, c_int,
                                      c_double, c_int, c_int, c_int, c_int]),
+    'imgcorr_set_perspective': (c_int, [c_void_p, c_void_p, c_int, c_int, c_double, c_void_p, c_int, c_int, c_int]),
     'imgcorr_warp_perspective': (c_int, [c_void_p, c_void_p, c_int, c_int, c_int, c_void_p, c_int, c_int, c_int, c_void_p,
                                          c_int, c_int, c_double, c_void_p]),
     'imgcorr_divide_f64': (c_int, [c_void_p, c_void_p, c_int, c_void_p, c_void_p, c_size_t, c_int, c_void_p]),

@@ -505,8 +505,27 @@ if shapes are transposed, execute self.transpose() once """ % (s, array.shape))
         return _engine.to_numpy(out)
 
     # ------------------------------------------------------------------ batches of independent frames
+    @staticmethod
+    def _perspective_stage(perspective, out, out_dtype):
+        """(homography, dsize, border value, tilt factor) of a PerspectiveCorrection as the chain's last stage, or None"""
+        if perspective is None:
+            return None
+        stage = perspective.correct_params()
+        tt = _engine.torch()
+        dt = out.dtype if out is not None else out_dtype
+        f64 = dt is not None and (dt == tt.float64 if isinstance(dt, tt.dtype) else np.dtype(dt) == np.float64)
+        if stage[3] is not None and not f64:
+            raise ValueError('perspective with do_correctIntensity needs out_dtype=float64: the tilt-factor division and '
+                             'the warp after it are computed in float64 (np.asfarray(img) / tf)')
+        return stage
+
+    @staticmethod
+    def _set_perspective(eng, stage):
+        M, dsize, border_value, tf = stage
+        eng.set_perspective(M, dsize, border_value, tf, token=_map_token('tilt', tf))
+
     def correct_batch(self, frames, bgImages=None, exposure_time=None, light_spectrum=None, threshold=0.1,
-                      keep_size=True, date=None, out=None, out_dtype=None, verbose=False, devices=None):
+                      keep_size=True, date=None, out=None, out_dtype=None, verbose=False, devices=None, perspective=None):
         """correct() for n INDEPENDENT frames with one calibration lookup.
 
         ``frames``: numpy [n,H,W] (uint8 / uint16 / float32, host) -> streamed through pinned buffers with
@@ -516,7 +535,16 @@ if shapes are transposed, execute self.transpose() once """ % (s, array.shape))
         ``devices``: CUDA device indices for host frames, e.g. ``range(8)``: the batch is split contiguously over them
         (sharding.shard_range), each device gets its own context with the calibration uploaded once and its own host
         thread driving the pinned H2D / kernels / D2H pipeline (the C ABI calls release the GIL); the shards land in one
-        output array.  No collective is involved: frames are independent (SURVEY §8e)."""
+        output array.  No collective is involved: frames are independent (SURVEY §8e).
+
+        ``perspective``: a PerspectiveCorrection whose correct() becomes the chain's last stage on the device:
+        ``correct_batch(frames, perspective=pc, out_dtype=np.float64)[i]`` equals ``pc.correct(correct(frames[i],
+        keep_size=keep_size))``, and with float32 output the float32 chain frame is warped in float32.  The homography
+        maps the frame the lens stage returns (the roi crop with keep_size=False).  A tilt factor
+        (do_correctIntensity=True) needs float64 output.  The stage stays on the cached engine of the device and frame
+        shape after the call, its tilt factor included (float64 on the device: 98 MB at 4096x3000), so that the next call
+        with the same PerspectiveCorrection uploads nothing; calls without ``perspective=`` do not use it, and
+        ``engine.get_engine(H, W, device).set_perspective(None, None)`` frees it."""
         import contextlib
         import io
         tt = _engine.torch()
@@ -534,9 +562,10 @@ if shapes are transposed, execute self.transpose() once """ % (s, array.shape))
                 raise ValueError('devices= shards HOST frames; a CUDA tensor is processed on its own device')
             if not devices:
                 raise ValueError('devices is empty')
-            if len(devices) > 1:
-                return self._correct_batch_multi(frames, devices, bgImages, exposure_time, light_spectrum, threshold,
-                                                 keep_size, date, out, out_dtype, verbose)
+        stage = self._perspective_stage(perspective, out, out_dtype)
+        if devices is not None and len(devices) > 1:
+            return self._correct_batch_multi(frames, devices, bgImages, exposure_time, light_spectrum, threshold,
+                                             keep_size, date, out, out_dtype, verbose, stage)
         dev_index = frames.device.index if is_tensor else (devices[0] if devices else None)
         eng = _engine.get_engine(H, W, dev_index)
         sink = contextlib.nullcontext() if verbose else contextlib.redirect_stdout(io.StringIO())
@@ -557,6 +586,9 @@ if shapes are transposed, execute self.transpose() once """ % (s, array.shape))
                 lens = None
         if threshold > 0:
             flags |= _lib.DO_NAN_TO_NUM
+        if stage is not None:
+            self._set_perspective(eng, stage)
+            flags |= _lib.DO_PERSPECTIVE
         window = tuple(int(v) for v in lens.roi) if (lens and not keep_size) else None
         thr = threshold if threshold > 0 else 0.0
         if is_tensor:
@@ -569,7 +601,7 @@ if shapes are transposed, execute self.transpose() once """ % (s, array.shape))
                                 window=window, out_dtype=out_dtype or np.float32)
 
     def _correct_batch_multi(self, frames, devices, bgImages, exposure_time, light_spectrum, threshold, keep_size, date,
-                             out, out_dtype, verbose):
+                             out, out_dtype, verbose, stage):
         """host frames [n,H,W] split over several devices of this process: one engine + one host thread per device"""
         import contextlib
         import io
@@ -608,8 +640,12 @@ if shapes are transposed, execute self.transpose() once """ % (s, array.shape))
                     lens = None
             if threshold > 0:
                 flags |= _lib.DO_NAN_TO_NUM
+            if stage is not None:
+                for e in engines:
+                    self._set_perspective(e, stage)
+                flags |= _lib.DO_PERSPECTIVE
             window = tuple(int(v) for v in lens.roi) if (lens and not keep_size) else None
-            oh, ow = (window[3], window[2]) if window else (H, W)
+            oh, ow = engines[0].chain_shape(flags, bool(lens), window)[2]
             odt = np.dtype(out_dtype or np.float32)
             if out is None:
                 out = np.empty((n, oh, ow), dtype=odt)

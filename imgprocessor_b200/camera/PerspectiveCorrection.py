@@ -167,18 +167,24 @@ class PerspectiveCorrection(object):
         out = eng.warp_perspective(img, self.homography, dsize, interpolation, inverse_map, border_value, divide_by)
         return out if is_tensor else _engine.to_numpy(out)
 
+    def correct_params(self):
+        """(homography, dsize (width, height), border value, tilt factor or None) of correct(): the warp
+        cv2.warpPerspective(img [/ tilt factor], homography, dsize, INTER_LANCZOS4, BORDER_CONSTANT, border value).
+        CameraCalibration.correct_batch(perspective=...) runs the same warp as the chain's last stage."""
+        if not self._homography_is_fixed:
+            self._homography = None
+        M = self.homography
+        if None in tuple(self._newBorders):
+            raise NotImplementedError('new_size must be given')
+        tf = self.tiltFactor() if self.opts['do_correctIntensity'] else None
+        return M, tuple(self._newBorders[::-1]), self._cv2_opts(self.opts['cv2_opts']), tf
+
     def correct(self, img):
         """perspective transformation [after the tilt-factor division] (:380-406)"""
         print("CORRECT PERSPECTIVE ...")
         self.img = imread(img)
-        if not self._homography_is_fixed:
-            self._homography = None
-        self.homography
-        if None in tuple(self._newBorders):
-            raise NotImplementedError('new_size must be given')
-        tf = self.tiltFactor() if self.opts['do_correctIntensity'] else None
-        return self._warp(self.img, tuple(self._newBorders[::-1]), 'lanczos4', False,
-                          self._cv2_opts(self.opts['cv2_opts']), tf)
+        _, dsize, border_value, tf = self.correct_params()
+        return self._warp(self.img, dsize, 'lanczos4', False, border_value, tf)
 
     def uncorrect(self, img):
         """:374-378"""

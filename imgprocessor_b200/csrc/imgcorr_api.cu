@@ -136,7 +136,11 @@ struct imgcorr_ctx {
     DevPtr<float> flat_nz;                    // flat with zeros replaced by 1.0
     double dark_absmax = 0.0, flat_absmin = 1.0;   // over finite entries (flat: non-zero entries)
     long long launches = 0;
-    SharedScratch chain_scratch;              // the chain's K1 output: two halves of `chain_group` float32 frames each
+    // the chain's K1 output (with a lens: two halves of `chain_group` float32 frames each), then the warp source of the
+    // perspective stage (a group of chain frames in the output dtype)
+    SharedScratch chain_scratch;
+    struct Perspective { bool on = false; double M[9]; int dh = 0, dw = 0; double border = 0.0; DevPtr<double> tilt; int th = 0, tw = 0; };
+    Perspective persp;                        // the chain's last stage (imgcorr_set_perspective)
     int chain_overlap = 1;                    // K1 of group g+1 on the internal stream while K2 of group g runs: +2-3.5 % on batches
     struct ChainOverlap { Stream st; Event k1[2], k2[2], entry; };
     ChainOverlap ov;                          // high-priority stream of K1 in overlap mode and its hand-off events
@@ -582,6 +586,9 @@ extern "C" IMGCORR_API int imgcorr_undistort_maps(imgcorr_ctx* c, float* mapx_de
 }
 
 // ---- K3 -------------------------------------------------------------------------------------
+static int run_k3(imgcorr_ctx* c, const void* src_dev, int dtype, int src_h, int src_w, void* dst_dev, int dst_h, int dst_w,
+                  int n_frames, const double M[9], int interpolation, int inverse_map, double border_value, cudaStream_t st);
+
 extern "C" IMGCORR_API int imgcorr_warp_perspective(imgcorr_ctx* c, const void* src_dev, int dtype, int src_h, int src_w,
                                         void* dst_dev, int dst_h, int dst_w, int n_frames, const double M[9],
                                         int interpolation, int inverse_map, double border_value, void* stream) {
@@ -593,6 +600,13 @@ extern "C" IMGCORR_API int imgcorr_warp_perspective(imgcorr_ctx* c, const void* 
     if (src_h <= 0 || src_w <= 0 || dst_h <= 0 || dst_w <= 0 || src_h > 32767 || src_w > 32767 || dst_h > 32767 || dst_w > 32767)
         return fail(IMGCORR_ERR_INVALID, "bad frame shape (%d x %d -> %d x %d)", src_h, src_w, dst_h, dst_w);
     if (n_frames < 0) return fail(IMGCORR_ERR_INVALID, "n_frames < 0");
+    return run_k3(c, src_dev, dtype, src_h, src_w, dst_dev, dst_h, dst_w, n_frames, M, interpolation, inverse_map,
+                  border_value, (cudaStream_t)stream);
+}
+
+// K3 on validated arguments; the coefficient tables are built on first use
+static int run_k3(imgcorr_ctx* c, const void* src_dev, int dtype, int src_h, int src_w, void* dst_dev, int dst_h, int dst_w,
+                  int n_frames, const double M[9], int interpolation, int inverse_map, double border_value, cudaStream_t st) {
     if (!c->warp_tab) {
         float h[32 * 8 + 32 * 4];
         warp_lanczos4_table(h);
@@ -628,7 +642,7 @@ extern "C" IMGCORR_API int imgcorr_warp_perspective(imgcorr_ctx* c, const void* 
     a.wc = make_warp_const(M, inverse_map, dst_w, dst_h);
     a.tab = interpolation == IMGCORR_INTER_LANCZOS4 ? c->warp_tab.get() : c->warp_tab.get() + 32 * 8;
     int l = 0;
-    cudaError_t e = launch_k3(a, dtype, interpolation, c->k3_variant, (cudaStream_t)stream, &l);
+    cudaError_t e = launch_k3(a, dtype, interpolation, c->k3_variant, st, &l);
     return launched(c, l, e, "K3 launch", "the requested K3 variant is not eligible for this call");
 }
 
@@ -702,16 +716,69 @@ static int ste_average_impl(imgcorr_ctx* c, const void* frames_dev, int dtype, i
     return launched(c, l, e, "K4 launch");
 }
 
-// one frame (or a group of frames) through K1 -> K2 on `st`
+// ---- the chain --------------------------------------------------------------------------------
+extern "C" IMGCORR_API int imgcorr_set_perspective(imgcorr_ctx* c, const double M[9], int dst_h, int dst_w, double border_value,
+                                       const double* tilt_factor, int tilt_h, int tilt_w, int on_device) {
+    GUARD(c);
+    imgcorr_ctx::Perspective& p = c->persp;
+    // a failed call leaves no stage behind: a chain call with the bit then fails with IMGCORR_ERR_STATE instead of
+    // writing frames of the previous destination shape into buffers sized for another
+    p.on = false;
+    if (M) {
+        if (dst_h <= 0 || dst_w <= 0 || dst_h > 32767 || dst_w > 32767)
+            return fail(IMGCORR_ERR_INVALID, "bad destination shape %d x %d", dst_h, dst_w);
+        if (tilt_factor && (tilt_h <= 0 || tilt_w <= 0))
+            return fail(IMGCORR_ERR_INVALID, "bad tilt factor shape %d x %d", tilt_h, tilt_w);
+    }
+    const size_t tilt_bytes = (M && tilt_factor) ? (size_t)tilt_h * tilt_w * sizeof(double) : 0;
+    // launches on other (non-blocking) streams may still read the tilt factor being replaced or dropped
+    if (p.tilt) {
+        CK(cudaDeviceSynchronize());
+        if (tilt_bytes != (size_t)p.th * p.tw * sizeof(double)) { p.tilt.reset(); p.th = p.tw = 0; }
+    }
+    if (!M) return IMGCORR_OK;
+    if (tilt_bytes) {
+        if (!p.tilt) CK(dev_alloc(p.tilt, tilt_bytes));
+        p.th = tilt_h;
+        p.tw = tilt_w;
+        CK(cudaMemcpy(p.tilt.get(), tilt_factor, tilt_bytes, on_device ? cudaMemcpyDeviceToDevice : cudaMemcpyHostToDevice));
+    } else {
+        p.tilt.reset();
+        p.th = p.tw = 0;
+    }
+    memcpy(p.M, M, sizeof p.M);
+    p.dh = dst_h;
+    p.dw = dst_w;
+    p.border = border_value;
+    p.on = true;
+    return IMGCORR_OK;
+}
+
+// the refusals of a chain call with IMGCORR_DO_PERSPECTIVE whose chain frame is [oh][ow]
+static int check_perspective(const imgcorr_ctx* c, int out_dtype, int ow, int oh) {
+    const imgcorr_ctx::Perspective& p = c->persp;
+    if (!p.on) return fail(IMGCORR_ERR_STATE, "perspective requested but no perspective set");
+    if (ow > 32767 || oh > 32767) return fail(IMGCORR_ERR_INVALID, "perspective source %d x %d exceeds 32767 per side", oh, ow);
+    if (!p.tilt) return IMGCORR_OK;
+    if (out_dtype != DT_F64)
+        return fail(IMGCORR_ERR_INVALID, "a tilt factor needs out_dtype F64: the division and the warp are computed in float64");
+    if (p.th != oh || p.tw != ow)
+        return fail(IMGCORR_ERR_INVALID, "tilt factor %d x %d does not match the chain frame %d x %d", p.th, p.tw, oh, ow);
+    return IMGCORR_OK;
+}
+
+// one frame (or a group of frames) through K1 -> [K2] -> [tilt division] -> [K3] on `st`; `persp` was checked by
+// check_perspective
 static int chain_frames(imgcorr_ctx* c, const void* raw, int raw_dtype, void* out, int out_dtype, int n, double thr,
-                        int ksize, int flags, bool lens, double border, int x0, int y0, int ow, int oh, cudaStream_t st) {
+                        int ksize, int flags, bool lens, bool persp, double border, int x0, int y0, int ow, int oh,
+                        cudaStream_t st) {
     if (out_dtype != DT_F32 && out_dtype != DT_F64) return fail(IMGCORR_ERR_INVALID, "out_dtype must be F32 or F64");
     if (raw_dtype == DT_F64) return fail(IMGCORR_ERR_INVALID, "float64 frames: convert to float32 first (the chain computes in float32)");
     const size_t npx = (size_t)c->H * c->W;
     const size_t raw_stride = npx * dtype_size(raw_dtype) + (size_t)c->raw_gap;
-    if (!lens) {
-        if (x0 != 0 || y0 != 0 || ow != c->W || oh != c->H)
-            return fail(IMGCORR_ERR_INVALID, "output window without a lens");
+    if (!lens && (x0 != 0 || y0 != 0 || ow != c->W || oh != c->H))
+        return fail(IMGCORR_ERR_INVALID, "output window without a lens");
+    if (!lens && !persp) {                             // K1 alone: one launch for the whole batch, no scratch
         K1Args a;
         int r = fill_k1(c, a, raw, raw_dtype, out, nullptr, n, thr, ksize, IMGCORR_COND_GT, flags);
         if (r) return r;
@@ -719,21 +786,28 @@ static int chain_frames(imgcorr_ctx* c, const void* raw, int raw_dtype, void* ou
         cudaError_t e = launch_k1(a, raw_dtype, out_dtype, c->k1_variant, c->sm_count, c->k1_seg_rows, st, &l);
         return launched(c, l, e, "K1 launch");
     }
-    // K1 -> K2 in groups of `chain_group` frames: the K1 output of a group stays in two alternating halves of the chain
-    // scratch (L2-resident for small groups); K2 evaluates each pixel's map once per group.
+    // K1 -> [K2] -> [tilt division] -> [K3] in groups of `chain_group` frames.  With a lens, the K1 output of a group stays
+    // in two alternating halves of the chain scratch (L2-resident for small groups) and K2 evaluates each pixel's map once
+    // per group.  With the perspective stage, the frames the call returns without it (K2's window, or K1's output) go to a
+    // third part, the warp source, and K3 writes `out`.
     const int grp = c->chain_group < n ? c->chain_group : (n > 0 ? n : 1);
-    const size_t half = round256(npx * sizeof(float) * grp);
+    const size_t half = lens ? round256(npx * sizeof(float) * grp) : 0;
+    const size_t src_px = (size_t)ow * oh;              // pixels of a chain frame, the warp source
+    const size_t src_bytes = persp ? src_px * dtype_size(out_dtype) * grp : 0;
     // the wait for another stream's last use precedes ev_entry, so the overlap stream inherits it
-    CK(c->chain_scratch.acquire(2 * half, st));
-    SharedScratch::Guard release{c->chain_scratch, st};    // every K1 / K2 of this call is ordered before the end of `st`
-    float* const mids[2] = {(float*)c->chain_scratch.buf.get(), (float*)(c->chain_scratch.buf.get() + half)};
-    const size_t out_stride = (size_t)ow * oh * dtype_size(out_dtype);
-    // Overlap mode: K1 of group g+1 runs on an internal high-priority stream while K2 of group g runs on the caller's
-    // stream, so that K2's blocks fill the SM slots K1's last, partially filled wave leaves idle (and vice versa).  The
-    // two halves of the scratch are handed back and forth with events; every K2 stays on the caller's stream, so the call
-    // is stream-ordered as before.  A profiled group (IMGCORR_OPT_PROFILE) runs unoverlapped so that its brackets time the
-    // kernel alone.
-    const bool overlap = c->chain_overlap && n > grp;
+    CK(c->chain_scratch.acquire(2 * half + src_bytes, st));
+    SharedScratch::Guard release{c->chain_scratch, st};    // every launch of this call is ordered before the end of `st`
+    char* const scratch = c->chain_scratch.buf.get();
+    float* const mids[2] = {(float*)scratch, (float*)(scratch + half)};
+    void* const wsrc = scratch + 2 * half;
+    const imgcorr_ctx::Perspective& p = c->persp;
+    const size_t out_stride = (persp ? (size_t)p.dw * p.dh : src_px) * dtype_size(out_dtype);
+    // Overlap mode (with a lens): K1 of group g+1 runs on an internal high-priority stream while K2 of group g runs on the
+    // caller's stream, so that K2's blocks fill the SM slots K1's last, partially filled wave leaves idle (and vice versa).
+    // The two halves of the scratch are handed back and forth with events; every K2, division and K3 stays on the caller's
+    // stream, so the call is stream-ordered as before.  A profiled group (IMGCORR_OPT_PROFILE) runs unoverlapped so that
+    // its brackets time the kernel alone.
+    const bool overlap = lens && c->chain_overlap && n > grp;
     imgcorr_ctx::ChainOverlap& ov = c->ov;
     cudaStream_t s1 = st;
     if (overlap) {
@@ -758,7 +832,8 @@ static int chain_frames(imgcorr_ctx* c, const void* raw, int raw_dtype, void* ou
     for (int f = 0; f < n; f += grp, ++gi) {
         const int nf = n - f < grp ? n - f : grp;
         float* mid = mids[gi & 1];
-        const bool prof = c->profile > 0 && (c->chain_groups_seen++ % c->profile) == 0;
+        void* const frames = persp ? wsrc : (char*)out + f * out_stride;     // what the call returns without the stage
+        const bool prof = lens && c->profile > 0 && (c->chain_groups_seen++ % c->profile) == 0;
         if (prof) { c->prof_frames[0] += nf; c->prof_frames[1] += nf; }
         if (overlap) {
             // this half was last read by K2 of group gi-2; a profiled group (or the one after it) also waits for gi-1
@@ -767,22 +842,34 @@ static int chain_frames(imgcorr_ctx* c, const void* raw, int raw_dtype, void* ou
             exclusive_next = prof;
         }
         K1Args a;
-        int r = fill_k1(c, a, (const char*)raw + f * raw_stride, raw_dtype, mid, nullptr, nf, thr, ksize, IMGCORR_COND_GT, flags);
+        int r = fill_k1(c, a, (const char*)raw + f * raw_stride, raw_dtype, lens ? (void*)mid : frames, nullptr, nf, thr, ksize,
+                        IMGCORR_COND_GT, flags);
         if (r) return r;
         int l = 0;
         if (prof) prof_mark(c, 0, s1);
-        cudaError_t e = launch_k1(a, raw_dtype, DT_F32, c->k1_variant, c->sm_count, c->k1_seg_rows, s1, &l);
+        cudaError_t e = launch_k1(a, raw_dtype, lens ? DT_F32 : out_dtype, c->k1_variant, c->sm_count, c->k1_seg_rows, s1, &l);
         if (prof) prof_mark(c, 0, s1);
         if ((r = launched(c, l, e, "K1 launch"))) return r;
-        if (overlap) {
-            CK(cudaEventRecord(ov.k1[gi & 1].get(), s1));
-            CK(cudaStreamWaitEvent(st, ov.k1[gi & 1].get(), 0));
+        if (lens) {
+            if (overlap) {
+                CK(cudaEventRecord(ov.k1[gi & 1].get(), s1));
+                CK(cudaStreamWaitEvent(st, ov.k1[gi & 1].get(), 0));
+            }
+            if (prof) prof_mark(c, 1, st);
+            r = run_k2(c, mid, DT_F32, frames, out_dtype, nf, nullptr, nullptr, border, x0, y0, ow, oh, st);
+            if (prof) prof_mark(c, 1, st);
+            if (r) return r;
+            if (overlap) CK(cudaEventRecord(ov.k2[gi & 1].get(), st));
         }
-        if (prof) prof_mark(c, 1, st);
-        r = run_k2(c, mid, DT_F32, (char*)out + f * out_stride, out_dtype, nf, nullptr, nullptr, border, x0, y0, ow, oh, st);
-        if (prof) prof_mark(c, 1, st);
+        if (!persp) continue;
+        if (p.tilt) {                                  // float64, in place (launch_k3_divide's in-place kernel)
+            l = 0;
+            e = launch_k3_divide(frames, DT_F64, p.tilt.get(), (double*)frames, src_px, nf, c->sm_count, st, &l);
+            if ((r = launched(c, l, e, "divide kernel launch"))) return r;
+        }
+        r = run_k3(c, frames, out_dtype, oh, ow, (char*)out + f * out_stride, p.dh, p.dw, nf, p.M, IMGCORR_INTER_LANCZOS4, 0,
+                   p.border, st);
         if (r) return r;
-        if (overlap) CK(cudaEventRecord(ov.k2[gi & 1].get(), st));
     }
     return IMGCORR_OK;
 }
@@ -794,8 +881,10 @@ extern "C" IMGCORR_API int imgcorr_correct_batch(imgcorr_ctx* c, const void* raw
     if (!raw_dev || !out_dev) return fail(IMGCORR_ERR_INVALID, "null image pointer");
     const bool lens = use_lens && c->has_lens;
     if (!lens) { x0 = 0; y0 = 0; ow = c->W; oh = c->H; }
-    return chain_frames(c, raw_dev, raw_dtype, out_dev, out_dtype, n_frames, threshold, ksize, flags, lens, border_value,
-                        x0, y0, ow, oh, (cudaStream_t)stream);
+    const bool persp = flags & IMGCORR_DO_PERSPECTIVE;
+    if (persp) { int r = check_perspective(c, out_dtype, ow, oh); if (r) return r; }
+    return chain_frames(c, raw_dev, raw_dtype, out_dev, out_dtype, n_frames, threshold, ksize, flags, lens, persp,
+                        border_value, x0, y0, ow, oh, (cudaStream_t)stream);
 }
 
 // ---- host-buffer pipeline ---------------------------------------------------------------------
@@ -844,8 +933,10 @@ extern "C" IMGCORR_API int imgcorr_correct_host(imgcorr_ctx* c, const void* raw_
     if (out_dtype != DT_F32 && out_dtype != DT_F64) return fail(IMGCORR_ERR_INVALID, "out_dtype must be F32 or F64");
     const bool lens = use_lens && c->has_lens;
     if (!lens) { x0 = 0; y0 = 0; ow = c->W; oh = c->H; }
+    const bool persp = flags & IMGCORR_DO_PERSPECTIVE;
+    if (persp) { int r = check_perspective(c, out_dtype, ow, oh); if (r) return r; }
     const size_t frame_raw = (size_t)c->H * c->W * dtype_size(raw_dtype);
-    const size_t frame_out = (size_t)ow * oh * dtype_size(out_dtype);
+    const size_t frame_out = (persp ? (size_t)c->persp.dw * c->persp.dh : (size_t)ow * oh) * dtype_size(out_dtype);
     // small frames travel in chunks of G frames per ring slot (up to 32 MB of raw data, at most 16 frames): one copy each
     // way and one K1 / K2 launch per chunk instead of per frame; frames above 16 MB (the 4096x3000 workload) keep one
     // frame per slot
@@ -884,8 +975,8 @@ extern "C" IMGCORR_API int imgcorr_correct_host(imgcorr_ctx* c, const void* raw_
         CK(cudaMemcpyAsync(s.d_raw.get(), src, frame_raw * nf, cudaMemcpyHostToDevice, s_in));
         CK(cudaEventRecord(s.ev_in.get(), s_in));
         CK(cudaStreamWaitEvent(s_k, s.ev_in.get(), 0));
-        r = chain_frames(c, s.d_raw.get(), raw_dtype, s.d_out.get(), out_dtype, nf, threshold, ksize, flags, lens, border_value,
-                         x0, y0, ow, oh, s_k);
+        r = chain_frames(c, s.d_raw.get(), raw_dtype, s.d_out.get(), out_dtype, nf, threshold, ksize, flags, lens, persp,
+                         border_value, x0, y0, ow, oh, s_k);
         if (r) return r;
         CK(cudaEventRecord(s.ev_k.get(), s_k));
         CK(cudaStreamWaitEvent(s_out, s.ev_k.get(), 0));

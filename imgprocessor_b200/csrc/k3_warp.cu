@@ -265,6 +265,16 @@ __global__ void __launch_bounds__(256) k3_divide_kernel(const T* __restrict__ sr
     }
 }
 
+// the same division in place on float64 frames (src == dst): the chain divides its warp source this way.  No pointer
+// is __restrict__, and each element is read and then written by the thread that owns it.
+__global__ void __launch_bounds__(256) k3_divide_inplace_kernel(double* data, const double* __restrict__ div, size_t npx,
+                                                                 int n_frames) {
+    for (size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < npx; i += (size_t)gridDim.x * blockDim.x) {
+        const double d = div[i];
+        for (int f = 0; f < n_frames; ++f) data[f * npx + i] = ddiv(data[f * npx + i], d);
+    }
+}
+
 template <typename T, typename AT>
 cudaError_t launch_typed(const K3Args& a, int interp, cudaStream_t st) {
     dim3 block(K3_BX, K3_BY), grid((a.dw + K3_BX - 1) / K3_BX, (a.dh + K3_BY - 1) / K3_BY);
@@ -310,6 +320,11 @@ cudaError_t launch_k3_divide(const void* src, int dtype, const double* div, doub
                              cudaStream_t st, int* launches) {
     if (npx == 0 || n_frames <= 0) return cudaSuccess;
     const int grid = (int)std::min<size_t>((npx + 255) / 256, (size_t)sm_count * 8);
+    if (src == dst && dtype == DT_F64) {
+        k3_divide_inplace_kernel<<<grid, 256, 0, st>>>(dst, div, npx, n_frames);
+        if (launches) ++*launches;
+        return cudaGetLastError();
+    }
     switch (dtype) {
         case DT_U8: k3_divide_kernel<<<grid, 256, 0, st>>>((const uint8_t*)src, div, dst, npx, n_frames); break;
         case DT_U16: k3_divide_kernel<<<grid, 256, 0, st>>>((const uint16_t*)src, div, dst, npx, n_frames); break;

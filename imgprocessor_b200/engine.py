@@ -9,7 +9,7 @@ import os
 import numpy as np
 
 from . import _lib
-from ._lib import DO_DARK, DO_FLAT, DO_NAN_TO_NUM  # noqa: F401  (re-exported)
+from ._lib import DO_DARK, DO_FLAT, DO_NAN_TO_NUM, DO_PERSPECTIVE  # noqa: F401  (re-exported)
 
 _TORCH = None
 
@@ -59,6 +59,7 @@ class Engine(object):
         _lib.check(self.lib.imgcorr_ctx_create(self.device_index, self.H, self.W, ctypes.byref(h)))
         self._h = h
         self.has_dark = self.has_flat = self.has_lens = False
+        self.perspective_dsize = None          # (width, height) of the chain's perspective stage, if one is set
         self._tokens = {}
 
     # -- lifetime ---------------------------------------------------------------------------
@@ -156,6 +157,50 @@ class Engine(object):
         _lib.check(self.lib.imgcorr_set_lens(self._h, vp(K), vp(d), vp(P)))
         self.has_lens = True
 
+    def set_perspective(self, M, dsize, border_value=0.0, tilt_factor=None, token=None):
+        """the chain's perspective stage (imgcorr_set_perspective): chain calls with DO_PERSPECTIVE in their flags warp
+        every frame they would return with cv2.warpPerspective(frame, M, dsize=(width, height), INTER_LANCZOS4,
+        BORDER_CONSTANT, border_value), after dividing it by ``tilt_factor`` (float64, the chain frame's shape; needs
+        float64 output) if one is given.  M None removes the stage.  ``token``: an identity of the tilt factor; a call
+        with the same arguments and token as the last one uploads nothing."""
+        if M is None:
+            _lib.check(self.lib.imgcorr_set_perspective(self._h, None, 0, 0, 0.0, None, 0, 0, 0))
+            self.perspective_dsize = None
+            self._tokens['perspective'] = None
+            return
+        Mh = np.ascontiguousarray(np.asarray(M, np.float64).reshape(3, 3))
+        dw, dh = int(dsize[0]), int(dsize[1])
+        key = (Mh.tobytes(), dw, dh, float(border_value), tilt_factor is None, token)
+        if (tilt_factor is None or token is not None) and self._tokens.get('perspective') == key:
+            return
+        tp, th, tw, dev, keep = None, 0, 0, 0, None
+        if tilt_factor is not None:
+            tt = torch()
+            if isinstance(tilt_factor, tt.Tensor):
+                keep = tilt_factor.to(device=self.device, dtype=tt.float64).contiguous()
+                tp, dev = ctypes.c_void_p(keep.data_ptr()), 1
+            else:
+                keep = np.ascontiguousarray(tilt_factor, dtype=np.float64)
+                tp = keep.ctypes.data_as(ctypes.c_void_p)
+            if keep.ndim != 2:
+                raise ValueError('tilt_factor must be 2-D, got shape %s' % (tuple(keep.shape),))
+            th, tw = (int(v) for v in keep.shape)
+        self._tokens['perspective'] = self.perspective_dsize = None          # a failed call leaves no stage behind
+        _lib.check(self.lib.imgcorr_set_perspective(self._h, Mh.ctypes.data_as(ctypes.c_void_p), dh, dw, float(border_value),
+                                                    tp, th, tw, dev))
+        self.perspective_dsize = (dw, dh)
+        self._tokens['perspective'] = key
+
+    def chain_shape(self, flags, use_lens=True, window=None):
+        """(lens, (x0, y0, ow, oh), (h, w)) of a chain call: whether K2 runs, its output window and the shape of every
+        frame the call returns (the perspective stage's destination with DO_PERSPECTIVE and a stage set; without a stage
+        the library refuses the call)"""
+        lens = bool(use_lens and self.has_lens)
+        x0, y0, ow, oh = self._window(window if lens else None)
+        if int(flags) & DO_PERSPECTIVE and self.perspective_dsize is not None:
+            return lens, (x0, y0, ow, oh), self.perspective_dsize[::-1]
+        return lens, (x0, y0, ow, oh), (oh, ow)
+
     # -- helpers ----------------------------------------------------------------------------
     def _frames(self, t):
         tt = torch()
@@ -209,19 +254,18 @@ class Engine(object):
             raise ValueError('buf must be a uint8 tensor on %s with at least %d bytes' % (self.device, need))
         if offset % esz or gap % esz:
             raise ValueError('offset and gap must be multiples of the sample size')
-        lens = bool(kw.get('use_lens', True) and self.has_lens)
-        x0, y0, ow, oh = self._window(kw.get('window') if lens else None)
+        flags = int(kw.get('flags', DO_DARK | DO_FLAT | DO_NAN_TO_NUM))
+        lens, (x0, y0, ow, oh), (h, w) = self.chain_shape(flags, kw.get('use_lens', True), kw.get('window'))
         out = kw.get('out')
         if out is None:
-            out = tt.empty((n_frames, oh, ow), dtype=kw.get('out_dtype') or tt.float32, device=self.device)
+            out = tt.empty((n_frames, h, w), dtype=kw.get('out_dtype') or tt.float32, device=self.device)
         else:
-            self._check_out(out, (n_frames, oh, ow))
+            self._check_out(out, (n_frames, h, w))
         with self.ingest(big_endian, gap):
             _lib.check(self.lib.imgcorr_correct_batch(
                 self._h, ctypes.c_void_p(buf.data_ptr() + offset), _dtype_code(dtype), ctypes.c_void_p(out.data_ptr()),
                 _dtype_code(out.dtype), n_frames, float(kw.get('threshold', 0.1)), int(kw.get('ksize', 3)),
-                int(kw.get('flags', DO_DARK | DO_FLAT | DO_NAN_TO_NUM)), int(lens), float(kw.get('border_value', 0.0)),
-                x0, y0, ow, oh, self._stream()))
+                flags, int(lens), float(kw.get('border_value', 0.0)), x0, y0, ow, oh, self._stream()))
         return out
 
     # -- kernels ----------------------------------------------------------------------------
@@ -418,17 +462,16 @@ class Engine(object):
 
     def correct_batch(self, raw, threshold=0.1, ksize=3, flags=DO_DARK | DO_FLAT | DO_NAN_TO_NUM, use_lens=True,
                       border_value=0.0, window=None, out_dtype=None, out=None):
-        """K1 -> K2 for every frame of a device-resident batch [n,H,W]."""
+        """K1 -> K2 [-> perspective stage with DO_PERSPECTIVE in flags] for every frame of a device-resident batch [n,H,W]."""
         tt = torch()
         squeeze = raw.dim() == 2
         raw = self._frames(raw)
         n = raw.shape[0]
-        lens = bool(use_lens and self.has_lens)
-        x0, y0, ow, oh = self._window(window if lens else None)
+        lens, (x0, y0, ow, oh), (h, w) = self.chain_shape(flags, use_lens, window)
         if out is None:
-            out = tt.empty((n, oh, ow), dtype=out_dtype or tt.float32, device=self.device)
+            out = tt.empty((n, h, w), dtype=out_dtype or tt.float32, device=self.device)
         else:
-            self._check_out(out, (oh, ow) if squeeze and out.dim() == 2 else (n, oh, ow))
+            self._check_out(out, (h, w) if squeeze and out.dim() == 2 else (n, h, w))
         _lib.check(self.lib.imgcorr_correct_batch(
             self._h, ctypes.c_void_p(raw.data_ptr()), _dtype_code(raw.dtype), ctypes.c_void_p(out.data_ptr()),
             _dtype_code(out.dtype), n, float(threshold), int(ksize), int(flags), int(lens), float(border_value),
@@ -438,7 +481,7 @@ class Engine(object):
     def correct_host(self, raw, out=None, threshold=0.1, ksize=3, flags=DO_DARK | DO_FLAT | DO_NAN_TO_NUM,
                      use_lens=True, border_value=0.0, window=None, out_dtype=np.float32):
         """The chain on HOST numpy frames [n,H,W] (uint8/uint16/float32): pinned staging, H2D, kernels and
-        D2H of consecutive frames overlap inside the library.  Synchronous."""
+        D2H of consecutive frames overlap inside the library.  Synchronous.  flags as correct_batch."""
         squeeze = raw.ndim == 2
         raw = np.ascontiguousarray(raw)
         big_endian = raw.dtype.byteorder == '>' or (raw.dtype.byteorder == '=' and not np.little_endian)
@@ -451,12 +494,11 @@ class Engine(object):
         if raw.shape[1:] != (self.H, self.W):
             raise ValueError('frames of shape %s do not match the engine (%d, %d)' % (raw.shape, self.H, self.W))
         n = raw.shape[0]
-        lens = bool(use_lens and self.has_lens)
-        x0, y0, ow, oh = self._window(window if lens else None)
+        lens, (x0, y0, ow, oh), (h, w) = self.chain_shape(flags, use_lens, window)
         if out is None:
-            out = np.empty((n, oh, ow), dtype=out_dtype)
-        if not out.flags.c_contiguous or out.shape != (n, oh, ow):
-            raise ValueError('out must be C-contiguous of shape %s' % ((n, oh, ow),))
+            out = np.empty((n, h, w), dtype=out_dtype)
+        if not out.flags.c_contiguous or out.shape != (n, h, w):
+            raise ValueError('out must be C-contiguous of shape %s' % ((n, h, w),))
         with self.ingest(big_endian, 0):
             _lib.check(self.lib.imgcorr_correct_host(
                 self._h, raw.ctypes.data_as(ctypes.c_void_p), NP_CODES[raw.dtype], out.ctypes.data_as(ctypes.c_void_p),

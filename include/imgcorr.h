@@ -31,7 +31,8 @@ extern "C" {
 #endif
 
 #define IMGCORR_VERSION 200 /* 0.2.0: round 2 added imgcorr_ste_average_thr, imgcorr_stack_mean, imgcorr_scale_f64, imgcorr_subsample_f64,
-                               imgcorr_linear_fit, imgcorr_host_fingerprint, imgcorr_selftest_division and the K2 options 11, 12 */
+                               imgcorr_linear_fit, imgcorr_host_fingerprint, imgcorr_selftest_division and the K2 options 11, 12;
+                               later added imgcorr_set_perspective and IMGCORR_DO_PERSPECTIVE (the chain's perspective stage) */
 
 #if defined(__GNUC__)
 #define IMGCORR_API __attribute__((visibility("default")))
@@ -58,7 +59,9 @@ typedef enum imgcorr_cond { IMGCORR_COND_GT = 0, IMGCORR_COND_LT = 1 } imgcorr_c
 enum {
     IMGCORR_DO_DARK = 1,       /* image -= bg                           CameraCalibration.py:502      */
     IMGCORR_DO_FLAT = 2,       /* image[flat != 0] /= flat[flat != 0]   CameraCalibration.py:525-526  */
-    IMGCORR_DO_NAN_TO_NUM = 4  /* image = np.nan_to_num(image)          CameraCalibration.py:561      */
+    IMGCORR_DO_NAN_TO_NUM = 4, /* image = np.nan_to_num(image)          CameraCalibration.py:561      */
+    IMGCORR_DO_PERSPECTIVE = 8 /* the context's perspective warp as the chain's last stage (imgcorr_set_perspective);
+                                  read by imgcorr_correct_batch and imgcorr_correct_host only */
 };
 
 /* imgcorr_set_option keys */
@@ -151,9 +154,13 @@ IMGCORR_API int imgcorr_undistort_maps(imgcorr_ctx* ctx, float* mapx_dev, float*
  *   threshold > 0 : median-threshold with ksize (3 in correct(), :556-563) after nan_to_num
  *   use_lens      : apply K2 if a lens is set (missing lens -> frames pass through, :570-575)
  *   out_dtype     : F32 or F64 (float64 is what the reference returns, :459)
- * Asynchronous on `stream`.  The context's K1 scratch is shared by every chain call: a call on another stream than
- * the previous chain call (imgcorr_correct_host included) first waits for that call's work on the scratch, so calls
- * of one context on several streams are correct and run one after the other on the device. */
+ *   flags         : IMGCORR_DO_* ; with IMGCORR_DO_PERSPECTIVE the frame described above (the K2 window [oh][ow], or the
+ *                   K1 output [H][W] without a lens) is warped by the context's perspective stage and out_dev is
+ *                   [n][dst_h][dst_w] (see imgcorr_set_perspective); IMGCORR_ERR_STATE if the context has none
+ * Asynchronous on `stream`.  The context's chain scratch (the K1 output and, with the perspective stage, the warp source)
+ * is shared by every chain call: a call on another stream than the previous chain call (imgcorr_correct_host included)
+ * first waits for that call's work on the scratch, so calls of one context on several streams are correct and run one
+ * after the other on the device. */
 IMGCORR_API int imgcorr_correct_batch(imgcorr_ctx* ctx, const void* raw_dev, int raw_dtype, void* out_dev, int out_dtype,
                           int n_frames, double threshold, int ksize, int flags, int use_lens, double border_value,
                           int x0, int y0, int ow, int oh, void* stream);
@@ -166,6 +173,22 @@ IMGCORR_API int imgcorr_correct_batch(imgcorr_ctx* ctx, const void* raw_dev, int
 IMGCORR_API int imgcorr_correct_host(imgcorr_ctx* ctx, const void* raw_host, int raw_dtype, void* out_host, int out_dtype,
                          int n_frames, double threshold, int ksize, int flags, int use_lens, double border_value,
                          int x0, int y0, int ow, int oh);
+
+/* The chain's perspective stage: PerspectiveCorrection.correct (camera/PerspectiveCorrection.py:380-406) on every frame of
+ * an imgcorr_correct_batch / imgcorr_correct_host call that sets IMGCORR_DO_PERSPECTIVE, without the intermediate frames
+ * leaving the device.  Per frame group: K1 -> [K2] -> [tilt division] -> K3 (Lanczos4, forward map, BORDER_CONSTANT).
+ *   M             3x3 row-major homography from the chain's frame (the K2 window, or the full frame without a lens) to
+ *                 the destination; NULL removes the stage (and the tilt factor)
+ *   dst_h, dst_w  destination frame, 1..32767 per side; border_value fills pixels that map outside the source
+ *   tilt_factor   NULL: no intensity correction.  Otherwise float64 [tilt_h][tilt_w] (device pointer if on_device != 0,
+ *                 host pointer otherwise), copied synchronously into the context; the chain frame is divided by it in
+ *                 float64 before the warp (np.asfarray(img) / tf, :394-400)
+ * Precision: with out_dtype F32 the float32 chain frame is warped in float32 (cv2.warpPerspective of that frame); with F64
+ * the float64 chain frame is warped in float64 (pc.correct(cal.correct(frame)) of the Python mirror).  A tilt factor needs
+ * out_dtype F64 and the shape of the chain frame: either mismatch makes the chain call fail with IMGCORR_ERR_INVALID.
+ * The stage adds one part to the chain scratch: a group of chain frames in out_dtype.  Synchronous. */
+IMGCORR_API int imgcorr_set_perspective(imgcorr_ctx* ctx, const double M[9], int dst_h, int dst_w, double border_value,
+                            const double* tilt_factor, int tilt_h, int tilt_w, int on_device);
 
 /* ---- K3: perspective warp (SURVEY §8 row f3) -----------------------------------------------------
  * Replaces cv2.warpPerspective in PerspectiveCorrection.correct (flags=INTER_LANCZOS4,
@@ -181,7 +204,8 @@ IMGCORR_API int imgcorr_warp_perspective(imgcorr_ctx* ctx, const void* src_dev, 
                              int dst_h, int dst_w, int n_frames, const double M[9], int interpolation, int inverse_map,
                              double border_value, void* stream);
 /* dst[f][i] = (double)src[f][i] / divisor[i]: the tilt-factor division in front of the warp
- * (camera/PerspectiveCorrection.py:394-400, np.asfarray(img) / tf).  src of any dtype, divisor and dst float64. */
+ * (camera/PerspectiveCorrection.py:394-400, np.asfarray(img) / tf).  src of any dtype, divisor and dst float64;
+ * dst_dev may equal src_dev for a float64 src (in place), other overlaps are not allowed. */
 IMGCORR_API int imgcorr_divide_f64(imgcorr_ctx* ctx, const void* src_dev, int src_dtype, const double* divisor_dev, double* dst_dev,
                        size_t pixels_per_frame, int n_frames, void* stream);
 
