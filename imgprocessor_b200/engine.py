@@ -387,21 +387,49 @@ class Engine(object):
     def median3x3(self, img):
         """scipy.ndimage.median_filter(img, 3) (mode='reflect') of a host float64 / float32 image through K1: a median-threshold
         whose threshold is so small that every pixel differing from its median is replaced by it (and a pixel equal to
-        its median already is the median).  Used by the noise-level-function estimation (camera/NoiseLevelFunction.py)."""
-        tt = torch()
+        its median already is the median).  Used by the noise-level-function estimation (camera/NoiseLevelFunction.py)
+        and flatFieldFromCloseDistance.
+
+        Where the median is +inf or -inf, K1's predicate |(img - median) / median| > threshold is NaN for a finite pixel,
+        so K1 keeps the pixel.  Those pixels are found by a second K1 run on the 0/1 image (img == inf): its median is 1
+        exactly where at least 5 of the 9 window values are inf, which is where the true median is inf.  A 0/1 image has
+        no infinite median, so K1 is an exact median on it.  Images without infinities take the single K1 run.
+        Images with NaN are not matched to scipy, whose result next to a NaN depends on the order of its selection."""
         a = np.ascontiguousarray(img)
         if a.dtype not in (np.float64, np.float32):
             a = a.astype(np.float64)
-        dev = tt.from_numpy(a).to(self.device)
+        out = self._median3x3_k1(a)
+        for inf in (np.inf, -np.inf):
+            hit = a == inf
+            if hit.any():
+                out[self._median3x3_k1(hit.astype(a.dtype)) == 1] = inf
+        return out
+
+    def _median3x3_k1(self, a):
+        dev = torch().from_numpy(a).to(self.device)
         out, _ = self.pointwise_median(dev, 1e-300, 3, flags=0, out_dtype=dev.dtype)
         return to_numpy(out)
 
     # -- K5: calibration-map producers (frame sizes are free; the engine only supplies the device) -----------
+    def _k5_tensor(self, t, what, f64=False):
+        """the K5 kernels take free shapes, so _frames() does not apply; they still need a tensor on this engine's device,
+        and the float64-only ones a float64 tensor (anything narrower would be read or written past its end)"""
+        tt = torch()
+        if not isinstance(t, tt.Tensor):
+            raise TypeError('%s must be a torch tensor on %s' % (what, self.device))
+        if t.device != self.device:
+            raise ValueError('%s on %s, engine on %s' % (what, t.device, self.device))
+        if f64 and t.dtype != tt.float64:
+            raise TypeError('%s must be float64 (got %s)' % (what, t.dtype))
+        return t
+
     def stack_mean(self, frames, minus=None, gray3=False):
         """imgAverage(frames) [- minus] [-> toGray]: frames = device tensor [n, ...] (any supported dtype; colour frames
         [n,H,W,3] with gray3) -> float64 tensor of one frame's shape (without the channel axis if gray3)"""
         tt = torch()
-        frames = frames.contiguous()
+        frames = self._k5_tensor(frames, 'frames').contiguous()
+        if gray3 and (frames.dim() < 2 or frames.shape[-1] != 3):
+            raise ValueError('gray3 needs colour frames [n, ..., 3], got %s' % (tuple(frames.shape),))
         n = frames.shape[0]
         elems = int(frames[0].numel())
         shape = tuple(frames.shape[1:-1]) if gray3 else tuple(frames.shape[1:])
@@ -422,13 +450,22 @@ class Engine(object):
         return out
 
     def scale_(self, data, divisor):
-        """data /= divisor in place (float64 device tensor)"""
+        """data /= divisor in place (contiguous float64 device tensor)"""
+        self._k5_tensor(data, 'data', f64=True)
+        if not data.is_contiguous():
+            raise ValueError('scale_ works in place and needs a contiguous tensor')
         _lib.check(self.lib.imgcorr_scale_f64(self._h, ctypes.c_void_p(data.data_ptr()), int(data.numel()), float(divisor), self._stream()))
         return data
 
     def subsample(self, img, step_y, step_x):
         """img[::step_y, ::step_x] of a float64 device image"""
         tt = torch()
+        img = self._k5_tensor(img, 'img', f64=True).contiguous()
+        if img.dim() != 2:
+            raise ValueError('subsample needs a 2-d image, got %s' % (tuple(img.shape),))
+        step_y, step_x = int(step_y), int(step_x)
+        if step_y < 1 or step_x < 1:
+            raise ValueError('steps must be >= 1 (got %d, %d)' % (step_y, step_x))
         h, w = img.shape
         out = tt.empty(((h + step_y - 1) // step_y, (w + step_x - 1) // step_x), dtype=tt.float64, device=self.device)
         _lib.check(self.lib.imgcorr_subsample_f64(self._h, ctypes.c_void_p(img.data_ptr()), h, w, int(step_y), int(step_x),
@@ -439,10 +476,13 @@ class Engine(object):
         """per-pixel line frames[k] = offset + ascent * x[k] (getLinearityFunction): device tensor [n,H,W] -> float64 offset,
         ascent (, rmse)"""
         tt = torch()
-        frames = frames.contiguous()
+        frames = self._k5_tensor(frames, 'frames').contiguous()
         n = frames.shape[0]
         px = int(frames[0].numel())
-        xs = (ctypes.c_double * n)(*[float(v) for v in x])
+        x = [float(v) for v in x]
+        if len(x) != n:
+            raise ValueError('%d exposure times for %d frames' % (len(x), n))
+        xs = (ctypes.c_double * n)(*x)
         offset = tt.empty(tuple(frames.shape[1:]), dtype=tt.float64, device=self.device)
         ascent = tt.empty_like(offset)
         rmse = tt.empty_like(offset) if want_rmse else None

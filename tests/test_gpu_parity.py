@@ -64,30 +64,35 @@ def test_k1_bit_exact_generic(ip, shape, dtype, ksize):
     assert np.array_equal(mask.cpu().numpy().astype(bool), wmask)
 
 
-@pytest.mark.parametrize('shape', [(5, 16), (33, 144), (96, 128), (70, 272), (300, 528), (257, 1024), (64, 4096)])
+@pytest.mark.parametrize('shape', [(1, 16), (2, 16), (3, 32), (4, 16), (5, 16), (33, 144), (96, 128), (70, 272), (300, 528),
+                                   (257, 1024), (64, 4096)])
 @pytest.mark.parametrize('dtype', [np.uint8, np.uint16, np.float32])
 @pytest.mark.parametrize('ksize,variant', [(3, 2), (5, 2), (3, 3)])
 def test_k1_bit_exact_tma(ip, shape, dtype, ksize, variant):
-    """variant 2 = TMA-staged tiles, 3 = TMA streaming pipeline"""
+    """variant 2 = TMA-staged tiles, 3 = TMA streaming pipeline.  Heights 1 - 4 are below the stencil: the TMA tiles
+    rebuild reflect rows from zero-filled boxes, and the 3x3 streaming kernel takes its prime / bottom step at height 1"""
     H, W = shape
     raw, dark, flat = _case(H, W, 4, dtype)
     e = _eng(ip, H, W, variant)
-    e.set_dark(dark)
-    e.set_flat(flat)
-    x = models.pointwise_model(raw, dark, flat, nan_to_num=True)
-    want, wmask = models.median_threshold_model(x, 0.1, ksize)
-    out, mask = e.pointwise_median(_dev(raw), 0.1, ksize, want_mask=True)
-    assert np.array_equal(out.cpu().numpy(), want)
-    assert np.array_equal(mask.cpu().numpy().astype(bool), wmask)
-    # partial calibrations through the TMA path as well
-    e.set_dark(None)
-    out, _ = e.pointwise_median(_dev(raw), 0.1, ksize)
-    want, _ = models.median_threshold_model(models.pointwise_model(raw, None, flat, True), 0.1, ksize)
-    assert np.array_equal(out.cpu().numpy(), want)
-    e.set_flat(None)
-    out, _ = e.pointwise_median(_dev(raw), 0.1, ksize)
-    want, _ = models.median_threshold_model(models.pointwise_model(raw, None, None, True), 0.1, ksize)
-    assert np.array_equal(out.cpu().numpy(), want)
+    try:
+        e.set_dark(dark)
+        e.set_flat(flat)
+        x = models.pointwise_model(raw, dark, flat, nan_to_num=True)
+        want, wmask = models.median_threshold_model(x, 0.1, ksize)
+        out, mask = e.pointwise_median(_dev(raw), 0.1, ksize, want_mask=True)
+        assert np.array_equal(out.cpu().numpy(), want)
+        assert np.array_equal(mask.cpu().numpy().astype(bool), wmask)
+        # partial calibrations through the TMA path as well
+        e.set_dark(None)
+        out, _ = e.pointwise_median(_dev(raw), 0.1, ksize)
+        want, _ = models.median_threshold_model(models.pointwise_model(raw, None, flat, True), 0.1, ksize)
+        assert np.array_equal(out.cpu().numpy(), want)
+        e.set_flat(None)
+        out, _ = e.pointwise_median(_dev(raw), 0.1, ksize)
+        want, _ = models.median_threshold_model(models.pointwise_model(raw, None, None, True), 0.1, ksize)
+        assert np.array_equal(out.cpu().numpy(), want)
+    finally:
+        e.set_option(ip.lib_mod.OPT_K1_VARIANT, 0)
 
 
 def test_k1_tma_refused_when_not_eligible(ip):
