@@ -525,12 +525,19 @@ if shapes are transposed, execute self.transpose() once """ % (s, array.shape))
         eng.set_perspective(M, dsize, border_value, tf, token=_map_token('tilt', tf))
 
     def correct_batch(self, frames, bgImages=None, exposure_time=None, light_spectrum=None, threshold=0.1,
-                      keep_size=True, date=None, out=None, out_dtype=None, verbose=False, devices=None, perspective=None):
+                      keep_size=True, date=None, out=None, out_dtype=None, verbose=False, devices=None, perspective=None,
+                      out_scale=None):
         """correct() for n INDEPENDENT frames with one calibration lookup.
 
         ``frames``: numpy [n,H,W] (uint8 / uint16 / float32, host) -> streamed through pinned buffers with
         H2D / kernels / D2H overlapped, result numpy [n,h,w]; or a CUDA torch tensor [n,H,W] -> result stays
         on the device.  ``out_dtype`` defaults to float32 (pass float64 for the reference's dtype).
+
+        ``out_dtype`` uint16 / uint8 (torch.uint16 / torch.uint8 for tensors) returns the float32 result v of every pixel
+        as an integer image, converted inside the chain's last kernel: t = (float64(v) - offset) * gain with
+        ``out_scale=(offset, gain)`` (default (0, 1)), then 0 for NaN and t <= 0, the dtype's maximum for t >= it, else t
+        rounded half to even (OpenCV's saturate_cast for the default scale).  Host frames then bring 2 (or 1) bytes per
+        pixel back over PCIe instead of 4.
 
         ``devices``: CUDA device indices for host frames, e.g. ``range(8)``: the batch is split contiguously over them
         (sharding.shard_range), each device gets its own context with the calibration uploaded once and its own host
@@ -565,7 +572,7 @@ if shapes are transposed, execute self.transpose() once """ % (s, array.shape))
         stage = self._perspective_stage(perspective, out, out_dtype)
         if devices is not None and len(devices) > 1:
             return self._correct_batch_multi(frames, devices, bgImages, exposure_time, light_spectrum, threshold,
-                                             keep_size, date, out, out_dtype, verbose, stage)
+                                             keep_size, date, out, out_dtype, verbose, stage, out_scale)
         dev_index = frames.device.index if is_tensor else (devices[0] if devices else None)
         eng = _engine.get_engine(H, W, dev_index)
         sink = contextlib.nullcontext() if verbose else contextlib.redirect_stdout(io.StringIO())
@@ -593,15 +600,15 @@ if shapes are transposed, execute self.transpose() once """ % (s, array.shape))
         thr = threshold if threshold > 0 else 0.0
         if is_tensor:
             return eng.correct_batch(frames, threshold=thr, ksize=3, flags=flags, use_lens=bool(lens), window=window,
-                                     out_dtype=out_dtype or tt.float32, out=out)
+                                     out_dtype=out_dtype or tt.float32, out=out, out_scale=out_scale)
         be = frames.dtype.kind == 'u' and frames.dtype.itemsize == 2 and frames.dtype.byteorder == '>'
         if not be and (frames.dtype.type not in (np.uint8, np.uint16, np.float32) or not frames.dtype.isnative):
             frames = frames.astype(np.float32)
         return eng.correct_host(frames, out=out, threshold=thr, ksize=3, flags=flags, use_lens=bool(lens),
-                                window=window, out_dtype=out_dtype or np.float32)
+                                window=window, out_dtype=out_dtype or np.float32, out_scale=out_scale)
 
     def _correct_batch_multi(self, frames, devices, bgImages, exposure_time, light_spectrum, threshold, keep_size, date,
-                             out, out_dtype, verbose, stage):
+                             out, out_dtype, verbose, stage, out_scale=None):
         """host frames [n,H,W] split over several devices of this process: one engine + one host thread per device"""
         import contextlib
         import io
@@ -660,7 +667,7 @@ if shapes are transposed, execute self.transpose() once """ % (s, array.shape))
                     return
                 try:
                     engines[i].correct_host(frames[lo:hi], out=out[lo:hi], threshold=thr, ksize=3, flags=flags,
-                                            use_lens=bool(lens), window=window, out_dtype=out.dtype)
+                                            use_lens=bool(lens), window=window, out_dtype=out.dtype, out_scale=out_scale)
                 except BaseException as e:                    # noqa: BLE001 - re-raised in the caller's thread
                     errors[i] = e
 

@@ -112,6 +112,7 @@ struct imgcorr_ctx {
     int device = 0, H = 0, W = 0, sm_count = 148;
     DevPtr<float> dark, ascent, flat;
     double exposure = 0.0, maxval = 65535.0;
+    OutScale out_scale{0.0, 1.0};             // imgcorr_set_output_scale: read by chain calls with U16 / U8 output
     bool has_lens = false;
     LensConst lens{};
     double lens_in[23] = {0};                 // K, dist, P as last given to imgcorr_set_lens (an identical call is a no-op)
@@ -218,6 +219,14 @@ extern "C" IMGCORR_API int imgcorr_ctx_destroy(imgcorr_ctx* c) {
     DeviceGuard g(c->device);
     cudaDeviceSynchronize();
     delete c;
+    return IMGCORR_OK;
+}
+
+extern "C" IMGCORR_API int imgcorr_set_output_scale(imgcorr_ctx* c, double offset, double gain) {
+    if (!c) return fail(IMGCORR_ERR_INVALID, "null context");
+    if (!std::isfinite(offset)) return fail(IMGCORR_ERR_INVALID, "output offset must be finite");
+    if (!std::isfinite(gain) || !(gain > 0.0)) return fail(IMGCORR_ERR_INVALID, "output gain must be finite and > 0");
+    c->out_scale = OutScale{offset, gain};
     return IMGCORR_OK;
 }
 
@@ -433,6 +442,7 @@ static int fill_k1(imgcorr_ctx* c, K1Args& a, const void* raw, int raw_dtype, vo
     if (cond != IMGCORR_COND_GT && cond != IMGCORR_COND_LT) return fail(IMGCORR_ERR_INVALID, "cond %d", cond);
     a = K1Args{};
     a.raw = raw; a.out = out; a.mask = ksize ? mask : nullptr;
+    a.q = OutScale{0.0, 1.0};                         // saturate_cast; chain calls with integer output set the context's scale
     a.H = c->H; a.W = c->W; a.n_frames = n; a.ksize = ksize;
     a.raw_swap = (c->raw_big_endian && raw_dtype == DT_U16) ? 1 : 0;
     a.raw_gap = c->raw_gap;
@@ -466,6 +476,8 @@ extern "C" IMGCORR_API int imgcorr_pointwise_median(imgcorr_ctx* c, const void* 
                                         uint8_t* mask_dev, int n_frames, double threshold, int ksize, int cond,
                                         int flags, void* stream) {
     GUARD(c);
+    if ((out_dtype == DT_U8 || out_dtype == DT_U16) && out_dtype != raw_dtype)        // integer output keeps the input dtype here
+        return fail(IMGCORR_ERR_INVALID, "unsupported dtype pair raw=%d out=%d", raw_dtype, out_dtype);
     K1Args a;
     int r = fill_k1(c, a, raw_dev, raw_dtype, out_dev, mask_dev, n_frames, threshold, ksize, cond, flags);
     if (r) return r;
@@ -477,7 +489,7 @@ extern "C" IMGCORR_API int imgcorr_pointwise_median(imgcorr_ctx* c, const void* 
 }
 
 static int run_k2(imgcorr_ctx* c, const void* src, int sdt, void* dst, int ddt, int n, const float* mapx,
-                  const float* mapy, double border, int x0, int y0, int ow, int oh, cudaStream_t st) {
+                  const float* mapy, double border, int x0, int y0, int ow, int oh, OutScale q, cudaStream_t st) {
     if (!src || !dst) return fail(IMGCORR_ERR_INVALID, "null image pointer");
     if (n < 0) return fail(IMGCORR_ERR_INVALID, "n_frames %d", n);
     if (!mapx && !c->has_lens) return fail(IMGCORR_ERR_STATE, "no lens set");
@@ -492,6 +504,7 @@ static int run_k2(imgcorr_ctx* c, const void* src, int sdt, void* dst, int ddt, 
     a.lens_dev = c->lens_dev.get();
     a.sm_count = c->sm_count;
     a.tma_store = c->k2_tma_store;
+    a.q = q;
     if (!c->k2_wtab) {
         std::vector<float4> t(32 * 32);
         for (int fy = 0; fy < 32; ++fy)
@@ -563,8 +576,10 @@ static int run_k2(imgcorr_ctx* c, const void* src, int sdt, void* dst, int ddt, 
 extern "C" IMGCORR_API int imgcorr_undistort(imgcorr_ctx* c, const void* src_dev, int src_dtype, void* dst_dev, int dst_dtype,
                                  int n_frames, double border_value, int x0, int y0, int ow, int oh, void* stream) {
     GUARD(c);
+    if (src_dtype == DT_F32 && (dst_dtype == DT_U8 || dst_dtype == DT_U16))
+        return fail(IMGCORR_ERR_INVALID, "unsupported dtype pair src=%d dst=%d", src_dtype, dst_dtype);
     return run_k2(c, src_dev, src_dtype, dst_dev, dst_dtype, n_frames, nullptr, nullptr, border_value, x0, y0, ow, oh,
-                  (cudaStream_t)stream);
+                  OutScale{0.0, 1.0}, (cudaStream_t)stream);
 }
 
 extern "C" IMGCORR_API int imgcorr_remap(imgcorr_ctx* c, const void* src_dev, int src_dtype, void* dst_dev, int dst_dtype,
@@ -572,8 +587,10 @@ extern "C" IMGCORR_API int imgcorr_remap(imgcorr_ctx* c, const void* src_dev, in
                              void* stream) {
     GUARD(c);
     if (!mapx_dev || !mapy_dev) return fail(IMGCORR_ERR_INVALID, "null map pointer");
+    if (src_dtype == DT_F32 && (dst_dtype == DT_U8 || dst_dtype == DT_U16))
+        return fail(IMGCORR_ERR_INVALID, "unsupported dtype pair src=%d dst=%d", src_dtype, dst_dtype);
     return run_k2(c, src_dev, src_dtype, dst_dev, dst_dtype, n_frames, mapx_dev, mapy_dev, border_value, 0, 0, c->W,
-                  c->H, (cudaStream_t)stream);
+                  c->H, OutScale{0.0, 1.0}, (cudaStream_t)stream);
 }
 
 extern "C" IMGCORR_API int imgcorr_undistort_maps(imgcorr_ctx* c, float* mapx_dev, float* mapy_dev, void* stream) {
@@ -586,8 +603,9 @@ extern "C" IMGCORR_API int imgcorr_undistort_maps(imgcorr_ctx* c, float* mapx_de
 }
 
 // ---- K3 -------------------------------------------------------------------------------------
-static int run_k3(imgcorr_ctx* c, const void* src_dev, int dtype, int src_h, int src_w, void* dst_dev, int dst_h, int dst_w,
-                  int n_frames, const double M[9], int interpolation, int inverse_map, double border_value, cudaStream_t st);
+static int run_k3(imgcorr_ctx* c, const void* src_dev, int dtype, int src_h, int src_w, void* dst_dev, int dst_dtype, int dst_h,
+                  int dst_w, int n_frames, const double M[9], int interpolation, int inverse_map, double border_value, OutScale q,
+                  cudaStream_t st);
 
 extern "C" IMGCORR_API int imgcorr_warp_perspective(imgcorr_ctx* c, const void* src_dev, int dtype, int src_h, int src_w,
                                         void* dst_dev, int dst_h, int dst_w, int n_frames, const double M[9],
@@ -600,13 +618,15 @@ extern "C" IMGCORR_API int imgcorr_warp_perspective(imgcorr_ctx* c, const void* 
     if (src_h <= 0 || src_w <= 0 || dst_h <= 0 || dst_w <= 0 || src_h > 32767 || src_w > 32767 || dst_h > 32767 || dst_w > 32767)
         return fail(IMGCORR_ERR_INVALID, "bad frame shape (%d x %d -> %d x %d)", src_h, src_w, dst_h, dst_w);
     if (n_frames < 0) return fail(IMGCORR_ERR_INVALID, "n_frames < 0");
-    return run_k3(c, src_dev, dtype, src_h, src_w, dst_dev, dst_h, dst_w, n_frames, M, interpolation, inverse_map,
-                  border_value, (cudaStream_t)stream);
+    return run_k3(c, src_dev, dtype, src_h, src_w, dst_dev, dtype, dst_h, dst_w, n_frames, M, interpolation, inverse_map,
+                  border_value, OutScale{0.0, 1.0}, (cudaStream_t)stream);
 }
 
-// K3 on validated arguments; the coefficient tables are built on first use
-static int run_k3(imgcorr_ctx* c, const void* src_dev, int dtype, int src_h, int src_w, void* dst_dev, int dst_h, int dst_w,
-                  int n_frames, const double M[9], int interpolation, int inverse_map, double border_value, cudaStream_t st) {
+// K3 on validated arguments; the coefficient tables are built on first use.  dst_dtype is dtype, or U16 / U8 for a float32
+// source (the chain's integer output: float32 warp, then quantise with q)
+static int run_k3(imgcorr_ctx* c, const void* src_dev, int dtype, int src_h, int src_w, void* dst_dev, int dst_dtype, int dst_h,
+                  int dst_w, int n_frames, const double M[9], int interpolation, int inverse_map, double border_value, OutScale q,
+                  cudaStream_t st) {
     if (!c->warp_tab) {
         float h[32 * 8 + 32 * 4];
         warp_lanczos4_table(h);
@@ -638,6 +658,8 @@ static int run_k3(imgcorr_ctx* c, const void* src_dev, int dtype, int src_h, int
     a.dh = dst_h;
     a.dw = dst_w;
     a.n_frames = n_frames;
+    a.dst_dtype = dst_dtype;
+    a.q = q;
     a.border = border_for_dtype(dtype == DT_U8, dtype == DT_U16, border_value);
     a.wc = make_warp_const(M, inverse_map, dst_w, dst_h);
     a.tab = interpolation == IMGCORR_INTER_LANCZOS4 ? c->warp_tab.get() : c->warp_tab.get() + 32 * 8;
@@ -769,10 +791,14 @@ static int check_perspective(const imgcorr_ctx* c, int out_dtype, int ow, int oh
 
 // one frame (or a group of frames) through K1 -> [K2] -> [tilt division] -> [K3] on `st`; `persp` was checked by
 // check_perspective
+// Integer output (U16 / U8) is the float32 chain with the quantiser fused into the last kernel's store: K1 without a lens or
+// perspective stage, K2 with a lens, K3 with the stage (which warps the float32 chain frame).
 static int chain_frames(imgcorr_ctx* c, const void* raw, int raw_dtype, void* out, int out_dtype, int n, double thr,
                         int ksize, int flags, bool lens, bool persp, double border, int x0, int y0, int ow, int oh,
                         cudaStream_t st) {
-    if (out_dtype != DT_F32 && out_dtype != DT_F64) return fail(IMGCORR_ERR_INVALID, "out_dtype must be F32 or F64");
+    if (out_dtype < DT_U8 || out_dtype > DT_F64) return fail(IMGCORR_ERR_INVALID, "out_dtype must be U8, U16, F32 or F64");
+    const bool quant = out_dtype == DT_U8 || out_dtype == DT_U16;
+    const int frame_dtype = quant ? DT_F32 : out_dtype;    // the chain frame: what K2 (or K1) returns before the stage
     if (raw_dtype == DT_F64) return fail(IMGCORR_ERR_INVALID, "float64 frames: convert to float32 first (the chain computes in float32)");
     const size_t npx = (size_t)c->H * c->W;
     const size_t raw_stride = npx * dtype_size(raw_dtype) + (size_t)c->raw_gap;
@@ -782,6 +808,7 @@ static int chain_frames(imgcorr_ctx* c, const void* raw, int raw_dtype, void* ou
         K1Args a;
         int r = fill_k1(c, a, raw, raw_dtype, out, nullptr, n, thr, ksize, IMGCORR_COND_GT, flags);
         if (r) return r;
+        if (quant) a.q = c->out_scale;
         int l = 0;
         cudaError_t e = launch_k1(a, raw_dtype, out_dtype, c->k1_variant, c->sm_count, c->k1_seg_rows, st, &l);
         return launched(c, l, e, "K1 launch");
@@ -793,7 +820,7 @@ static int chain_frames(imgcorr_ctx* c, const void* raw, int raw_dtype, void* ou
     const int grp = c->chain_group < n ? c->chain_group : (n > 0 ? n : 1);
     const size_t half = lens ? round256(npx * sizeof(float) * grp) : 0;
     const size_t src_px = (size_t)ow * oh;              // pixels of a chain frame, the warp source
-    const size_t src_bytes = persp ? src_px * dtype_size(out_dtype) * grp : 0;
+    const size_t src_bytes = persp ? src_px * dtype_size(frame_dtype) * grp : 0;
     // the wait for another stream's last use precedes ev_entry, so the overlap stream inherits it
     CK(c->chain_scratch.acquire(2 * half + src_bytes, st));
     SharedScratch::Guard release{c->chain_scratch, st};    // every launch of this call is ordered before the end of `st`
@@ -847,7 +874,7 @@ static int chain_frames(imgcorr_ctx* c, const void* raw, int raw_dtype, void* ou
         if (r) return r;
         int l = 0;
         if (prof) prof_mark(c, 0, s1);
-        cudaError_t e = launch_k1(a, raw_dtype, lens ? DT_F32 : out_dtype, c->k1_variant, c->sm_count, c->k1_seg_rows, s1, &l);
+        cudaError_t e = launch_k1(a, raw_dtype, lens ? DT_F32 : frame_dtype, c->k1_variant, c->sm_count, c->k1_seg_rows, s1, &l);
         if (prof) prof_mark(c, 0, s1);
         if ((r = launched(c, l, e, "K1 launch"))) return r;
         if (lens) {
@@ -856,7 +883,8 @@ static int chain_frames(imgcorr_ctx* c, const void* raw, int raw_dtype, void* ou
                 CK(cudaStreamWaitEvent(st, ov.k1[gi & 1].get(), 0));
             }
             if (prof) prof_mark(c, 1, st);
-            r = run_k2(c, mid, DT_F32, frames, out_dtype, nf, nullptr, nullptr, border, x0, y0, ow, oh, st);
+            r = run_k2(c, mid, DT_F32, frames, persp ? frame_dtype : out_dtype, nf, nullptr, nullptr, border, x0, y0, ow, oh,
+                       c->out_scale, st);
             if (prof) prof_mark(c, 1, st);
             if (r) return r;
             if (overlap) CK(cudaEventRecord(ov.k2[gi & 1].get(), st));
@@ -867,8 +895,8 @@ static int chain_frames(imgcorr_ctx* c, const void* raw, int raw_dtype, void* ou
             e = launch_k3_divide(frames, DT_F64, p.tilt.get(), (double*)frames, src_px, nf, c->sm_count, st, &l);
             if ((r = launched(c, l, e, "divide kernel launch"))) return r;
         }
-        r = run_k3(c, frames, out_dtype, oh, ow, (char*)out + f * out_stride, p.dh, p.dw, nf, p.M, IMGCORR_INTER_LANCZOS4, 0,
-                   p.border, st);
+        r = run_k3(c, frames, frame_dtype, oh, ow, (char*)out + f * out_stride, out_dtype, p.dh, p.dw, nf, p.M,
+                   IMGCORR_INTER_LANCZOS4, 0, p.border, c->out_scale, st);
         if (r) return r;
     }
     return IMGCORR_OK;
@@ -930,7 +958,7 @@ extern "C" IMGCORR_API int imgcorr_correct_host(imgcorr_ctx* c, const void* raw_
     if (n_frames < 0) return fail(IMGCORR_ERR_INVALID, "n_frames %d", n_frames);
     if (raw_dtype < DT_U8 || raw_dtype > DT_F32) return fail(IMGCORR_ERR_INVALID, "raw_dtype %d (U8, U16 or F32)", raw_dtype);
     if (c->raw_gap) return fail(IMGCORR_ERR_INVALID, "IMGCORR_OPT_RAW_FRAME_GAP is not available for host frames (pass the pixel blocks)");
-    if (out_dtype != DT_F32 && out_dtype != DT_F64) return fail(IMGCORR_ERR_INVALID, "out_dtype must be F32 or F64");
+    if (out_dtype < DT_U8 || out_dtype > DT_F64) return fail(IMGCORR_ERR_INVALID, "out_dtype must be U8, U16, F32 or F64");
     const bool lens = use_lens && c->has_lens;
     if (!lens) { x0 = 0; y0 = 0; ow = c->W; oh = c->H; }
     const bool persp = flags & IMGCORR_DO_PERSPECTIVE;

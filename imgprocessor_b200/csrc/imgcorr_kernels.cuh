@@ -32,6 +32,7 @@ struct K1Args {
     int no_overflow;        // the calibration proves |raw - dark| / |flat| < FLT_MAX for this raw dtype: nan_to_num is the identity
     PointwiseConst pw;
     PredicateConst pred;
+    OutScale q;             // integer output (U16 / U8): quantise<OutT>(float32 result, q); the identity (0, 1) outside the chain
 };
 
 // variant: 0 = pick automatically, 1 = generic tiles (plain coalesced loads), 2 = TMA-staged tiles,
@@ -64,6 +65,8 @@ struct K2Args {
     int2* chdr_w;
     int sm_count;
     int tma_store;           // tiled variant: output tile through shared memory + TMA store instead of predicated stores
+                             // (float destinations only: the F32 -> U16 / U8 pairs always store per pixel)
+    OutScale q;              // F32 -> U16 / U8: the float32 blend, then quantise<DstT>(blend, q)
 };
 void k2_cache_size(int geometry, int ow, int oh, size_t* words, size_t* tiles);
 bool k2_will_tile(const K2Args& a, int src_dtype, int dst_dtype, int variant);    // launch_k2 takes the tiled variant
@@ -80,12 +83,14 @@ cudaError_t launch_write_maps(const LensConst& lens, float* mapx, float* mapy, i
 // K3: perspective warp (cv2.warpPerspective, Lanczos4 / bicubic) ------------------------------
 struct K3Args {
     const void* src;        // [n_frames][H][W]
-    void* dst;              // [n_frames][dh][dw], same dtype
+    void* dst;              // [n_frames][dh][dw] of dst_dtype
     int H, W, dh, dw, n_frames;
     double border;          // already converted to the image dtype's value range
     WarpConst wc;
     const float* tab;       // device coefficient table [32][N] of the interpolation
     const int16_t* itab;    // uint8 images: device fixed-point weights [32][32][N*N] (null otherwise)
+    int dst_dtype;          // dtype of dst: the source dtype, or U16 / U8 for a float32 source (float32 warp, then quantise)
+    OutScale q;             // the scale of that quantisation
 };
 cudaError_t launch_k3(const K3Args& a, int dtype, int interp, int variant, cudaStream_t stream, int* launches);
 cudaError_t launch_k3_divide(const void* src, int dtype, const double* div, double* dst, size_t npx, int n_frames,

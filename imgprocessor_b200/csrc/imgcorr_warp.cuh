@@ -126,12 +126,7 @@ inline void warp_fixed_table(const float* tab, int n, int16_t* out) {
         }
 }
 
-// ---- coordinates --------------------------------------------------------------------------
-#if defined(__CUDA_ARCH__)
-IC_HD int d2i_rn(double v) { return __double2int_rn(v); }
-#else
-IC_HD int d2i_rn(double v) { return (int)nearbyint(v); }   // callers clamp to the int range first
-#endif
+// ---- coordinates (d2i_rn: imgcorr_core.cuh) --------------------------------------------------
 
 // X = cvRound(max(INT_MIN, min(INT_MAX, (X0 + M0*x1) * W))); a NaN ends up as INT_MAX (std::min / std::max
 // argument order in OpenCV, fmin / fmax here).  OpenCV additionally saturates X >> 5 to int16; for sources

@@ -49,12 +49,13 @@ template <> struct RawIO<uint16_t> { using CT = float;  static __device__ __forc
 template <> struct RawIO<float>    { using CT = float;  static __device__ __forceinline__ double ld(float v)    { return (double)v; } };
 template <> struct RawIO<double>   { using CT = double; static __device__ __forceinline__ double ld(double v)   { return v; } };
 
-template <typename OutT, typename CT> __device__ __forceinline__ OutT to_out(CT v);
-template <> __device__ __forceinline__ float    to_out<float, float>(float v)       { return v; }
-template <> __device__ __forceinline__ double   to_out<double, float>(float v)      { return (double)v; }
-template <> __device__ __forceinline__ double   to_out<double, double>(double v)    { return v; }
-template <> __device__ __forceinline__ uint16_t to_out<uint16_t, float>(float v)    { return sat_u16(v); }
-template <> __device__ __forceinline__ uint8_t  to_out<uint8_t, float>(float v)     { return sat_u8(v); }
+// integer outputs go through the quantiser with the launch's scale (identity: saturate_cast, as sat_u16 / sat_u8)
+template <typename OutT, typename CT> __device__ __forceinline__ OutT to_out(const K1Args& a, CT v);
+template <> __device__ __forceinline__ float    to_out<float, float>(const K1Args&, float v)    { return v; }
+template <> __device__ __forceinline__ double   to_out<double, float>(const K1Args&, float v)   { return (double)v; }
+template <> __device__ __forceinline__ double   to_out<double, double>(const K1Args&, double v) { return v; }
+template <> __device__ __forceinline__ uint16_t to_out<uint16_t, float>(const K1Args& a, float v) { return quantise<uint16_t>(v, a.q); }
+template <> __device__ __forceinline__ uint8_t  to_out<uint8_t, float>(const K1Args& a, float v)  { return quantise<uint8_t>(v, a.q); }
 
 template <typename T> struct alignas(2 * sizeof(T)) Pair { T x, y; };
 
@@ -83,7 +84,7 @@ __global__ void __launch_bounds__(256) k1_pointwise_kernel(K1Args a) {
         float d = a.dark ? __ldg(a.dark + p) : 0.0f;
         float s = a.ascent ? __ldg(a.ascent + p) : 0.0f;
         float f = a.flat ? __ldg(a.flat + p) : 0.0f;
-        out[p] = to_out<OutT, CT>(pointwise<CT>(pw, RawIO<RawT>::ld(raw_fix<RawT>(__ldg(raw + p), swap)), d, s, f));
+        out[p] = to_out<OutT, CT>(a, pointwise<CT>(pw, RawIO<RawT>::ld(raw_fix<RawT>(__ldg(raw + p), swap)), d, s, f));
     }
 }
 
@@ -146,7 +147,7 @@ __device__ __forceinline__ void median_phase(const CT* __restrict__ xs, const K1
             sorted_row_pair(p, a2, b2, n0, n1);
             const CT m0 = median9(a0, a1, a2), m1 = median9(b0, b1, b2);
             const bool rep0 = predicate(c0, m0, pred), rep1 = predicate(c1, m1, pred);
-            store_pair<OutT, VEC>(out + (size_t)j * W, to_out<OutT, CT>(rep0 ? m0 : c0), to_out<OutT, CT>(rep1 ? m1 : c1), two);
+            store_pair<OutT, VEC>(out + (size_t)j * W, to_out<OutT, CT>(a, rep0 ? m0 : c0), to_out<OutT, CT>(a, rep1 ? m1 : c1), two);
             if (mask) store_pair<uint8_t, VEC>(mask + (size_t)j * W, (uint8_t)rep0, (uint8_t)rep1, two);
             a0 = a1; a1 = a2; b0 = b1; b1 = b2; c0 = n0; c1 = n1;
         };
@@ -184,7 +185,7 @@ __device__ __forceinline__ void median_phase(const CT* __restrict__ xs, const K1
                         const CT med = median25_sorted_rows(w);
                         const CT centre = ctr[(j - 2) % 5];
                         const bool rep = predicate(centre, med, pred);
-                        out[(size_t)o * W + cc] = to_out<OutT, CT>(rep ? med : centre);
+                        out[(size_t)o * W + cc] = to_out<OutT, CT>(a, rep ? med : centre);
                         if (mask) mask[(size_t)o * W + cc] = rep ? 1 : 0;
                     }
                 }
@@ -372,7 +373,8 @@ k1_tma_kernel(const __grid_constant__ CUtensorMap tm_raw, const __grid_constant_
 bool k1_tma_eligible(const K1Args& a, int raw_dtype, int out_dtype) {
     if (a.ksize != 3 && a.ksize != 5) return false;
     if (raw_dtype != DT_U8 && raw_dtype != DT_U16 && raw_dtype != DT_F32) return false;
-    if (out_dtype != DT_F32 && !(raw_dtype == DT_U16 && out_dtype == DT_U16) && !(raw_dtype == DT_U8 && out_dtype == DT_U8)) return false;
+    if (out_dtype != DT_F32 && out_dtype != DT_U16 && out_dtype != DT_U8) return false;
+    if (a.ksize == 5 && out_dtype != DT_F32 && dtype_size(out_dtype) != dtype_size(raw_dtype)) return false;
     if (a.pw.flags & FLAG_DARK_LINEAR) return false;
     if (a.raw_swap || a.raw_gap) return false;
     const size_t esz = dtype_size(raw_dtype);
@@ -446,7 +448,9 @@ static cudaError_t dispatch_ks(const K1Args& a, bool tma, CUtensorMapDataType rd
         return launch_generic_t<RawT, OutT, 3, 32>(a, st);
     }
     if (a.ksize == 5) {
-        if constexpr (sizeof(RawT) <= 4 && sizeof(OutT) <= 4)
+        // integer output of another width than the raw frames (the chain's quantised output) is not built for the 5x5
+        // TMA tiles: those instantiations spill; they run the generic tiles (k1_tma_eligible says so)
+        if constexpr (sizeof(RawT) <= 4 && sizeof(OutT) <= 4 && (sizeof(OutT) == 4 || sizeof(OutT) == sizeof(RawT)))
             if (tma) {
                 return launch_tma_t<RawT, OutT, 5, 16, 2>(a, rdt, sm_count, st);      // 5x5 is register-heavy: small tiles, 3 CTAs / SM
             }
@@ -476,15 +480,19 @@ cudaError_t launch_k1(const K1Args& a, int raw_dtype, int out_dtype, int variant
         case DT_U8:
             if (out_dtype == DT_F32) return dispatch_ks<uint8_t, float>(a, tma, CU_TENSOR_MAP_DATA_TYPE_UINT8, sm_count, st);
             if (out_dtype == DT_U8) return dispatch_ks<uint8_t, uint8_t>(a, tma, CU_TENSOR_MAP_DATA_TYPE_UINT8, sm_count, st);
+            if (out_dtype == DT_U16) return dispatch_ks<uint8_t, uint16_t>(a, tma, CU_TENSOR_MAP_DATA_TYPE_UINT8, sm_count, st);
             if (out_dtype == DT_F64) return dispatch_ks<uint8_t, double>(a, false, CU_TENSOR_MAP_DATA_TYPE_UINT8, sm_count, st);
             break;
         case DT_U16:
             if (out_dtype == DT_F32) return dispatch_ks<uint16_t, float>(a, tma, CU_TENSOR_MAP_DATA_TYPE_UINT16, sm_count, st);
             if (out_dtype == DT_U16) return dispatch_ks<uint16_t, uint16_t>(a, tma, CU_TENSOR_MAP_DATA_TYPE_UINT16, sm_count, st);
+            if (out_dtype == DT_U8) return dispatch_ks<uint16_t, uint8_t>(a, tma, CU_TENSOR_MAP_DATA_TYPE_UINT16, sm_count, st);
             if (out_dtype == DT_F64) return dispatch_ks<uint16_t, double>(a, false, CU_TENSOR_MAP_DATA_TYPE_UINT16, sm_count, st);
             break;
         case DT_F32:
             if (out_dtype == DT_F32) return dispatch_ks<float, float>(a, tma, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, sm_count, st);
+            if (out_dtype == DT_U16) return dispatch_ks<float, uint16_t>(a, tma, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, sm_count, st);
+            if (out_dtype == DT_U8) return dispatch_ks<float, uint8_t>(a, tma, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, sm_count, st);
             if (out_dtype == DT_F64) return dispatch_ks<float, double>(a, false, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, sm_count, st);
             break;
         case DT_F64:

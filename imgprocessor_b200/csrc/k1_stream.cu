@@ -84,10 +84,10 @@ template <> struct StreamRaw<uint8_t>  { static __device__ __forceinline__ void 
 template <> struct StreamRaw<uint16_t> { static __device__ __forceinline__ void ld(uint16_t v, double& d, float& a) { d = (double)(int)v; a = 0.0f; } };
 template <> struct StreamRaw<float>    { static __device__ __forceinline__ void ld(float v, double& d, float& a)    { d = (double)v; a = fabsf(v); } };
 
-template <typename OutT> __device__ __forceinline__ OutT ks_out(float v);
-template <> __device__ __forceinline__ float    ks_out<float>(float v)    { return v; }
-template <> __device__ __forceinline__ uint16_t ks_out<uint16_t>(float v) { return sat_u16(v); }
-template <> __device__ __forceinline__ uint8_t  ks_out<uint8_t>(float v)  { return sat_u8(v); }
+template <typename OutT> __device__ __forceinline__ OutT ks_out(const K1Args& a, float v);
+template <> __device__ __forceinline__ float    ks_out<float>(const K1Args&, float v)      { return v; }
+template <> __device__ __forceinline__ uint16_t ks_out<uint16_t>(const K1Args& a, float v) { return quantise<uint16_t>(v, a.q); }
+template <> __device__ __forceinline__ uint8_t  ks_out<uint8_t>(const K1Args& a, float v)  { return quantise<uint8_t>(v, a.q); }
 
 // store with an L2 eviction-priority hint (float32 results of the straight-line chunks)
 template <typename OutT> __device__ __forceinline__ void ks_store(OutT* p, OutT v, uint64_t) { *p = v; }
@@ -292,14 +292,14 @@ k1_stream_kernel(const __grid_constant__ CUtensorMap tm_raw, const __grid_consta
         auto emit = [&](int f, const Sorted3<float>& t2, bool on) {
             OutT* op = outp + f * frame_px;
             if (nomed) {
-                if (on) *op = ks_out<OutT>(c1[f]);
+                if (on) *op = ks_out<OutT>(a, c1[f]);
                 return;
             }
             const float med = median9(s0[f], s1[f], t2);
             bool rep;
             const bool sure = predicate_certain(c1[f], med, pred, rep);
             if (on) {
-                *op = ks_out<OutT>(rep ? med : c1[f]);
+                *op = ks_out<OutT>(a, rep ? med : c1[f]);
                 if (has_mask) *maskp = rep ? 1 : 0;
             }
             // ~1e-5 of the pixels fall inside the guard band of the float32 test: those lanes evaluate the reference's
@@ -307,7 +307,7 @@ k1_stream_kernel(const __grid_constant__ CUtensorMap tm_raw, const __grid_consta
             if (__any_sync(0xffffffffu, !sure)) {
                 if (!sure && on) {
                     const bool r2 = ks_exact(c1[f], med, pred.thr, pred.cond);
-                    *op = ks_out<OutT>(r2 ? med : c1[f]);
+                    *op = ks_out<OutT>(a, r2 ? med : c1[f]);
                     if (has_mask) *maskp = r2 ? 1 : 0;
                 }
             }
@@ -382,8 +382,8 @@ k1_stream_kernel(const __grid_constant__ CUtensorMap tm_raw, const __grid_consta
                             d1 = skip1 ? dumpp : d1;
                         }
                         if (nomed) {
-                            ks_store<OutT>(d0, ks_out<OutT>(c1[f]), out_policy);
-                            ks_store<OutT>(d1, ks_out<OutT>(xa), out_policy);
+                            ks_store<OutT>(d0, ks_out<OutT>(a, c1[f]), out_policy);
+                            ks_store<OutT>(d1, ks_out<OutT>(a, xa), out_policy);
                             c1[f] = xb;
                             continue;
                         }
@@ -401,8 +401,8 @@ k1_stream_kernel(const __grid_constant__ CUtensorMap tm_raw, const __grid_consta
                             unsure |= !predicate_certain(c1[f], m1, pred, r1);
                             unsure |= !predicate_certain(xa, m2, pred, r2);
                         }
-                        ks_store<OutT>(d0, ks_out<OutT>(r1 ? m1 : c1[f]), out_policy);
-                        ks_store<OutT>(d1, ks_out<OutT>(r2 ? m2 : xa), out_policy);
+                        ks_store<OutT>(d0, ks_out<OutT>(a, r1 ? m1 : c1[f]), out_policy);
+                        ks_store<OutT>(d1, ks_out<OutT>(a, r2 ? m2 : xa), out_policy);
                         if (has_mask) {
                             *((j == 0 && skip0) ? mdump : mp + j * ostride) = r1 ? 1 : 0;
                             *((j == 0 && skip1) ? mdump : mp + (j + 1) * ostride) = r2 ? 1 : 0;
@@ -443,7 +443,7 @@ bool k1_stream_eligible(const K1Args& a, int raw_dtype, int out_dtype) {
     if (a.ksize != 3 && a.ksize != 0) return false;
     if (a.ksize == 0 && a.H < 4) return false;
     if (raw_dtype != DT_U8 && raw_dtype != DT_U16 && raw_dtype != DT_F32) return false;
-    if (out_dtype != DT_F32 && !(raw_dtype == DT_U16 && out_dtype == DT_U16) && !(raw_dtype == DT_U8 && out_dtype == DT_U8)) return false;
+    if (out_dtype != DT_F32 && out_dtype != DT_U16 && out_dtype != DT_U8) return false;
     if (a.pw.flags & FLAG_DARK_LINEAR) return false;
     if (a.raw_gap) return false;
     const size_t esz = dtype_size(raw_dtype);
@@ -575,13 +575,17 @@ cudaError_t launch_k1_stream(const K1Args& a, int raw_dtype, int out_dtype, int 
         case DT_U8:
             if (out_dtype == DT_F32) return launch_stream_t<uint8_t, float>(a, CU_TENSOR_MAP_DATA_TYPE_UINT8, sm_count, seg_rows, st);
             if (out_dtype == DT_U8) return launch_stream_t<uint8_t, uint8_t>(a, CU_TENSOR_MAP_DATA_TYPE_UINT8, sm_count, seg_rows, st);
+            if (out_dtype == DT_U16) return launch_stream_t<uint8_t, uint16_t>(a, CU_TENSOR_MAP_DATA_TYPE_UINT8, sm_count, seg_rows, st);
             break;
         case DT_U16:
             if (out_dtype == DT_F32) return launch_stream_t<uint16_t, float>(a, CU_TENSOR_MAP_DATA_TYPE_UINT16, sm_count, seg_rows, st);
             if (out_dtype == DT_U16) return launch_stream_t<uint16_t, uint16_t>(a, CU_TENSOR_MAP_DATA_TYPE_UINT16, sm_count, seg_rows, st);
+            if (out_dtype == DT_U8) return launch_stream_t<uint16_t, uint8_t>(a, CU_TENSOR_MAP_DATA_TYPE_UINT16, sm_count, seg_rows, st);
             break;
         case DT_F32:
             if (out_dtype == DT_F32) return launch_stream_t<float, float>(a, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, sm_count, seg_rows, st);
+            if (out_dtype == DT_U16) return launch_stream_t<float, uint16_t>(a, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, sm_count, seg_rows, st);
+            if (out_dtype == DT_U8) return launch_stream_t<float, uint8_t>(a, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, sm_count, seg_rows, st);
             break;
     }
     return cudaErrorInvalidValue;

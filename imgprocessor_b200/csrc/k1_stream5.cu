@@ -69,10 +69,10 @@ template <> struct Raw5<uint8_t>  { static __device__ __forceinline__ void ld(ui
 template <> struct Raw5<uint16_t> { static __device__ __forceinline__ void ld(uint16_t v, double& d, float& a) { d = (double)(int)v; a = 0.0f; } };
 template <> struct Raw5<float>    { static __device__ __forceinline__ void ld(float v, double& d, float& a)    { d = (double)v; a = fabsf(v); } };
 
-template <typename OutT> __device__ __forceinline__ OutT out5(float v);
-template <> __device__ __forceinline__ float    out5<float>(float v)    { return v; }
-template <> __device__ __forceinline__ uint16_t out5<uint16_t>(float v) { return sat_u16(v); }
-template <> __device__ __forceinline__ uint8_t  out5<uint8_t>(float v)  { return sat_u8(v); }
+template <typename OutT> __device__ __forceinline__ OutT out5(const K1Args& a, float v);
+template <> __device__ __forceinline__ float    out5<float>(const K1Args&, float v)      { return v; }
+template <> __device__ __forceinline__ uint16_t out5<uint16_t>(const K1Args& a, float v) { return quantise<uint16_t>(v, a.q); }
+template <> __device__ __forceinline__ uint8_t  out5<uint8_t>(const K1Args& a, float v)  { return quantise<uint8_t>(v, a.q); }
 
 __device__ __noinline__ bool exact5(float x, float b, double thr, int cond) {
     PredicateConst pc;
@@ -262,13 +262,13 @@ k1_stream5_kernel(const __grid_constant__ CUtensorMap tm_raw, const __grid_const
             bool rep;
             const bool sure = predicate_certain(c2, med, pred, rep);
             if (on) {
-                *outp = out5<OutT>(rep ? med : c2);
+                *outp = out5<OutT>(a, rep ? med : c2);
                 if (has_mask) *maskp = rep ? 1 : 0;
             }
             if (__any_sync(0xffffffffu, !sure)) {
                 if (!sure && on) {
                     const bool r2 = exact5(c2, med, pred.thr, pred.cond);
-                    *outp = out5<OutT>(r2 ? med : c2);
+                    *outp = out5<OutT>(a, r2 ? med : c2);
                     if (has_mask) *maskp = r2 ? 1 : 0;
                 }
             }
@@ -318,8 +318,8 @@ k1_stream5_kernel(const __grid_constant__ CUtensorMap tm_raw, const __grid_const
                         if (!sure_a) rep_a = exact5(c2, med_a, pred.thr, pred.cond);
                         if (!sure_b) rep_b = exact5(c1, med_b, pred.thr, pred.cond);
                     }
-                    op[0] = out5<OutT>(rep_a ? med_a : c2);
-                    op[ostride] = out5<OutT>(rep_b ? med_b : c1);
+                    op[0] = out5<OutT>(a, rep_a ? med_a : c2);
+                    op[ostride] = out5<OutT>(a, rep_b ? med_b : c1);
                     if (has_mask) { mp[0] = rep_a ? 1 : 0; mp[ostride] = rep_b ? 1 : 0; mp += 2 * ostride; }
                     op += 2 * ostride;
                     push(qa, xa);
@@ -336,7 +336,7 @@ k1_stream5_kernel(const __grid_constant__ CUtensorMap tm_raw, const __grid_const
                     if (__any_sync(0xffffffffu, !sure)) {
                         if (!sure) rep = exact5(c2, med, pred.thr, pred.cond);
                     }
-                    *op = out5<OutT>(rep ? med : c2);
+                    *op = out5<OutT>(a, rep ? med : c2);
                     if (has_mask) { *mp = rep ? 1 : 0; mp += ostride; }
                     op += ostride;
                     push(q, x);
@@ -427,7 +427,7 @@ cudaError_t launch5_t(const K1Args& a_in, CUtensorMapDataType rdt, int sm_count,
 bool k1_stream5_eligible(const K1Args& a, int raw_dtype, int out_dtype) {
     if (a.ksize != 5 || a.H < 8) return false;
     if (raw_dtype != DT_U8 && raw_dtype != DT_U16 && raw_dtype != DT_F32) return false;
-    if (out_dtype != DT_F32 && !(raw_dtype == DT_U16 && out_dtype == DT_U16) && !(raw_dtype == DT_U8 && out_dtype == DT_U8)) return false;
+    if (out_dtype != DT_F32 && out_dtype != DT_U16 && out_dtype != DT_U8) return false;
     if (a.pw.flags & FLAG_DARK_LINEAR) return false;
     if (a.raw_gap) return false;
     const size_t esz = dtype_size(raw_dtype);
@@ -444,13 +444,17 @@ cudaError_t launch_k1_stream5(const K1Args& a, int raw_dtype, int out_dtype, int
         case DT_U8:
             if (out_dtype == DT_F32) return launch5_t<uint8_t, float>(a, CU_TENSOR_MAP_DATA_TYPE_UINT8, sm_count, seg_rows, st);
             if (out_dtype == DT_U8) return launch5_t<uint8_t, uint8_t>(a, CU_TENSOR_MAP_DATA_TYPE_UINT8, sm_count, seg_rows, st);
+            if (out_dtype == DT_U16) return launch5_t<uint8_t, uint16_t>(a, CU_TENSOR_MAP_DATA_TYPE_UINT8, sm_count, seg_rows, st);
             break;
         case DT_U16:
             if (out_dtype == DT_F32) return launch5_t<uint16_t, float>(a, CU_TENSOR_MAP_DATA_TYPE_UINT16, sm_count, seg_rows, st);
             if (out_dtype == DT_U16) return launch5_t<uint16_t, uint16_t>(a, CU_TENSOR_MAP_DATA_TYPE_UINT16, sm_count, seg_rows, st);
+            if (out_dtype == DT_U8) return launch5_t<uint16_t, uint8_t>(a, CU_TENSOR_MAP_DATA_TYPE_UINT16, sm_count, seg_rows, st);
             break;
         case DT_F32:
             if (out_dtype == DT_F32) return launch5_t<float, float>(a, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, sm_count, seg_rows, st);
+            if (out_dtype == DT_U16) return launch5_t<float, uint16_t>(a, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, sm_count, seg_rows, st);
+            if (out_dtype == DT_U8) return launch5_t<float, uint8_t>(a, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, sm_count, seg_rows, st);
             break;
     }
     return cudaErrorInvalidValue;

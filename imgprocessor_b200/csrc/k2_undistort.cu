@@ -101,6 +101,19 @@ template <> struct Blend<uint8_t, uint8_t> {
     }
 };
 
+// F32 -> U16 / U8 (the batch chain's integer output): the float32 pair's result, then the quantiser.  These pairs read
+// the float32 blend of Blend<float, float>, so their values are quantise(the F32 call's values) by construction.
+template <typename SrcT, typename DstT> struct K2Quant { static constexpr bool value = sizeof(SrcT) == 4 && sizeof(DstT) <= 2; };
+template <typename SrcT, typename DstT>
+__device__ __forceinline__ DstT blend_out(SrcT a, SrcT b, SrcT c, SrcT d, const Weights<SrcT>& w, const OutScale& q) {
+    if constexpr (K2Quant<SrcT, DstT>::value) return quantise<DstT>(Blend<float, float>::run(a, b, c, d, w), q);
+    else return Blend<SrcT, DstT>::run(a, b, c, d, w);
+}
+template <typename SrcT, typename DstT> __device__ __forceinline__ DstT border_out(SrcT b, const OutScale& q) {
+    if constexpr (K2Quant<SrcT, DstT>::value) return quantise<DstT>(b, q);
+    else return (DstT)b;
+}
+
 // rim of the image: any neighbour outside [0,W)x[0,H) is the border value; a window entirely outside is the border
 // value itself (OpenCV does not blend it).  Rare -> kept out of line so the hot path stays small.
 template <typename SrcT, typename DstT>
@@ -114,6 +127,12 @@ __device__ __noinline__ DstT remap_rim(const SrcT* __restrict__ src, int H, int 
     const SrcT v10 = (x0 && y1) ? __ldg(p + W) : bval;
     const SrcT v11 = (x1 && y1) ? __ldg(p + W + 1) : bval;
     return Blend<SrcT, DstT>::run(v00, v01, v10, v11, w);
+}
+template <typename SrcT, typename DstT>
+__device__ __forceinline__ DstT rim_out(const SrcT* __restrict__ src, int H, int W, int ix, int iy, const Weights<SrcT>& w, SrcT bval,
+                                        const OutScale& q) {
+    if constexpr (K2Quant<SrcT, DstT>::value) return quantise<DstT>(remap_rim<float, float>(src, H, W, ix, iy, w, bval), q);
+    else return remap_rim<SrcT, DstT>(src, H, W, ix, iy, w, bval);
 }
 
 // MODE: 0 explicit maps, 1 analytic general P, 2 analytic separable P^-1 (x = x(u), y = y(v))
@@ -195,7 +214,7 @@ __global__ void __launch_bounds__(K2_BX * K2_BY, K2_MINB) k2_remap_kernel(K2Args
             }
 #pragma unroll
             for (int j = 0; j < K2_ROWS; ++j)
-                if (fast & (1u << j)) dst[j * K2_BY * ow] = Blend<SrcT, DstT>::run(v00[j], v01[j], v10[j], v11[j], wt[j]);
+                if (fast & (1u << j)) dst[j * K2_BY * ow] = blend_out<SrcT, DstT>(v00[j], v01[j], v10[j], v11[j], wt[j], a.q);
             src += src_stride;
             dst += dst_stride;
         }
@@ -209,7 +228,7 @@ __global__ void __launch_bounds__(K2_BX * K2_BY, K2_MINB) k2_remap_kernel(K2Args
         for (int f = 0; f < nf; ++f) {
 #pragma unroll
             for (int j = 0; j < K2_ROWS; ++j)
-                if (rim & (1u << j)) dst[j * K2_BY * ow] = remap_rim<SrcT, DstT>(src, H, W, cix[j], ciy[j], wt[j], bval);
+                if (rim & (1u << j)) dst[j * K2_BY * ow] = rim_out<SrcT, DstT>(src, H, W, cix[j], ciy[j], wt[j], bval, a.q);
             src += src_stride;
             dst += dst_stride;
         }
@@ -476,9 +495,9 @@ k2_tiled_kernel(const __grid_constant__ CUtensorMap tm_src, const __grid_constan
         const FixedCoord fc = kt_coord<MODE>(a, L2, u, v, (double)v, sxc, dmul(sxc, sxc));
         Weights<SrcT> w;
         w.set(fc);
-        return remap_rim<SrcT, DstT>(src, H, W, fc.ix, fc.iy, w, border_cast<SrcT>(a.border));
+        return rim_out<SrcT, DstT>(src, H, W, fc.ix, fc.iy, w, border_cast<SrcT>(a.border), a.q);
     };
-    const DstT bout = (DstT)border_cast<SrcT>(a.border);
+    const DstT bout = border_out<SrcT, DstT>(border_cast<SrcT>(a.border), a.q);
 
     const int src_stride = H * W, dst_stride = oh * ow;
     const SrcT* src = (const SrcT*)a.src;
@@ -500,7 +519,7 @@ k2_tiled_kernel(const __grid_constant__ CUtensorMap tm_src, const __grid_constan
 #pragma unroll
                 for (int j = 0; j < KT_PX; ++j) {
                     const SrcT* p = box + so[j];
-                    const DstT r = Blend<SrcT, DstT>::run(p[0], p[1], p[BW], p[BW + 1], wt[j]);
+                    const DstT r = blend_out<SrcT, DstT>(p[0], p[1], p[BW], p[BW + 1], wt[j], a.q);
                     sts_if(ot + j * KT_RSTEP * KT_TW, r, fast & (1u << j));
                 }
             }
@@ -539,7 +558,7 @@ k2_tiled_kernel(const __grid_constant__ CUtensorMap tm_src, const __grid_constan
 #pragma unroll
                     for (int j = 0; j < KT_PX; ++j) {
                         const SrcT* p = box + so[j];
-                        const DstT r = Blend<SrcT, DstT>::run(p[0], p[1], p[BW], p[BW + 1], wt[j]);
+                        const DstT r = blend_out<SrcT, DstT>(p[0], p[1], p[BW], p[BW + 1], wt[j], a.q);
                         st_if(dst + j * dstep, r, fast & (1u << j));            // predicated store, no branch around the gather
                     }
                 }
@@ -643,7 +662,7 @@ k2_cached_kernel(const __grid_constant__ CUtensorMap tm_src, const __grid_consta
     Weights<SrcT> wt[KT_PX];
     unsigned fast = 0, slow = 0, outm = 0, phases = 0;
     int tx0 = 0, ty0 = 0;
-    const DstT bout = (DstT)border_cast<SrcT>(a.border);
+    const DstT bout = border_out<SrcT, DstT>(border_cast<SrcT>(a.border), a.q);
     const int src_stride = H * W, dst_stride = oh * ow;
 
     // "slow" pixels (window on the frame rim, or a tile the box does not cover): coordinates recomputed from the lens, per-
@@ -654,7 +673,7 @@ k2_cached_kernel(const __grid_constant__ CUtensorMap tm_src, const __grid_consta
         const FixedCoord fc = fixed_coord_fast(mx, my);
         Weights<SrcT> w;
         w.set(fc);
-        return remap_rim<SrcT, DstT>(src, H, W, fc.ix, fc.iy, w, border_cast<SrcT>(a.border));
+        return rim_out<SrcT, DstT>(src, H, W, fc.ix, fc.iy, w, border_cast<SrcT>(a.border), a.q);
     };
 
     int tile = blockIdx.x, f = 0, slot = 0;
@@ -696,7 +715,7 @@ k2_cached_kernel(const __grid_constant__ CUtensorMap tm_src, const __grid_consta
 #pragma unroll
                 for (int j = 0; j < KT_PX; ++j) {
                     const SrcT* p = box + so[j];
-                    const DstT r = Blend<SrcT, DstT>::run(p[0], p[1], p[BW], p[BW + 1], wt[j]);
+                    const DstT r = blend_out<SrcT, DstT>(p[0], p[1], p[BW], p[BW + 1], wt[j], a.q);
                     sts_if(ot + j * KT_RSTEP * KT_TW, r, fast & (1u << j));
                 }
             }
@@ -726,7 +745,7 @@ k2_cached_kernel(const __grid_constant__ CUtensorMap tm_src, const __grid_consta
 #pragma unroll
                 for (int j = 0; j < KT_PX; ++j) {
                     const SrcT* p = box + so[j];
-                    const DstT r = Blend<SrcT, DstT>::run(p[0], p[1], p[BW], p[BW + 1], wt[j]);
+                    const DstT r = blend_out<SrcT, DstT>(p[0], p[1], p[BW], p[BW + 1], wt[j], a.q);
                     st_if(dst + j * dstep, r, fast & (1u << j));
                 }
             }
@@ -770,7 +789,7 @@ static cudaError_t launch_cached_g(const K2Args& a, cudaStream_t st) {
 }
 
 static bool k2_tiled_eligible(const K2Args& a, int src_dtype, int dst_dtype) {
-    const bool pair = (src_dtype == DT_F32 && (dst_dtype == DT_F32 || dst_dtype == DT_F64)) || (src_dtype == DT_U16 && dst_dtype == DT_U16) ||
+    const bool pair = (src_dtype == DT_F32 && dst_dtype >= DT_U8 && dst_dtype <= DT_F64) || (src_dtype == DT_U16 && dst_dtype == DT_U16) ||
                       (src_dtype == DT_U8 && dst_dtype == DT_U8);
     if (!pair) return false;
     if (a.W < 2 || a.H < 2) return false;
@@ -789,6 +808,7 @@ static cudaError_t launch_tiled_g(const K2Args& a, cudaStream_t st) {
     void (*kern)(const CUtensorMap, const CUtensorMap, K2Args);
     const bool sep = a.lens.affine && a.lens.ir[1] == 0.0 && a.lens.ir[3] == 0.0;
     if (a.cpack && !a.mapx) return launch_cached_g<SrcT, DstT, G, TSTORE>(a, st);
+    if constexpr (K2Quant<SrcT, DstT>::value) if (a.mapx) return cudaErrorNotSupported;    // the chain remaps with the analytic map only
     if (a.mapx) kern = k2_tiled_kernel<SrcT, DstT, 0, G, TSTORE, 0>;
     else if (a.cpack_w) kern = sep ? k2_tiled_kernel<SrcT, DstT, 2, G, TSTORE, 1> : k2_tiled_kernel<SrcT, DstT, 1, G, TSTORE, 1>;
     else kern = sep ? k2_tiled_kernel<SrcT, DstT, 2, G, TSTORE, 0> : k2_tiled_kernel<SrcT, DstT, 1, G, TSTORE, 0>;
@@ -808,9 +828,10 @@ static cudaError_t launch_tiled_t(const K2Args& a, cudaStream_t st) {
     // (16-byte aligned rows).  Measured on B200 it is SLOWER than the predicated per-pixel stores of the other path (21.0 vs
     // 20.1 us per 4096x3000 frame in batches: the tile costs an STS per pixel, a proxy fence and a longer barrier per frame,
     // while the plain stores are already full 128-byte lines per warp), so it is an option (IMGCORR_OPT_K2_TMA_STORE), off by default.
-    const bool tstore = a.tma_store && ((size_t)a.ow * sizeof(DstT)) % 16 == 0 && ((uintptr_t)a.dst) % 16 == 0;
+    // (the F32 -> U16 / U8 pairs are built without the TMA-store option: they always store per pixel)
+    const bool tstore = !K2Quant<SrcT, DstT>::value && a.tma_store && ((size_t)a.ow * sizeof(DstT)) % 16 == 0 && ((uintptr_t)a.dst) % 16 == 0;
     const int g = a.geometry;
-    if (tstore) {
+    if constexpr (!K2Quant<SrcT, DstT>::value) if (tstore) {
         if (g == 3) return launch_tiled_g<SrcT, DstT, KtG3, true>(a, st);
         if (g == 2) return launch_tiled_g<SrcT, DstT, KtG2, true>(a, st);
         if (g == 1) return launch_tiled_g<SrcT, DstT, KtG1, true>(a, st);
@@ -878,6 +899,7 @@ static bool separable(const LensConst& L) { return L.affine && L.ir[1] == 0.0 &&
 template <typename SrcT, typename DstT>
 static cudaError_t launch_t(const K2Args& a, cudaStream_t st) {
     dim3 grid((a.ow + K2_BX - 1) / K2_BX, (a.oh + K2_BY * K2_ROWS - 1) / (K2_BY * K2_ROWS));
+    if constexpr (K2Quant<SrcT, DstT>::value) if (a.mapx) return cudaErrorNotSupported;
     if (a.mapx) k2_remap_kernel<SrcT, DstT, 0><<<grid, K2_BX * K2_BY, 0, st>>>(a);
     else if (separable(a.lens)) k2_remap_kernel<SrcT, DstT, 2><<<grid, K2_BX * K2_BY, 0, st>>>(a);
     else k2_remap_kernel<SrcT, DstT, 1><<<grid, K2_BX * K2_BY, 0, st>>>(a);
@@ -905,10 +927,14 @@ cudaError_t launch_k2(const K2Args& a, int src_dtype, int dst_dtype, int variant
     if (tiled) {
         if (src_dtype == DT_U16) return launch_tiled_t<uint16_t, uint16_t>(a, st);
         if (src_dtype == DT_U8) return launch_tiled_t<uint8_t, uint8_t>(a, st);
+        if (dst_dtype == DT_U16) return launch_tiled_t<float, uint16_t>(a, st);
+        if (dst_dtype == DT_U8) return launch_tiled_t<float, uint8_t>(a, st);
         return dst_dtype == DT_F32 ? launch_tiled_t<float, float>(a, st) : launch_tiled_t<float, double>(a, st);
     }
     if (src_dtype == DT_F32 && dst_dtype == DT_F32) return launch_t<float, float>(a, st);
     if (src_dtype == DT_F32 && dst_dtype == DT_F64) return launch_t<float, double>(a, st);
+    if (src_dtype == DT_F32 && dst_dtype == DT_U16) return launch_t<float, uint16_t>(a, st);
+    if (src_dtype == DT_F32 && dst_dtype == DT_U8) return launch_t<float, uint8_t>(a, st);
     if (src_dtype == DT_F64 && dst_dtype == DT_F64) return launch_t<double, double>(a, st);
     if (src_dtype == DT_U16 && dst_dtype == DT_U16) return launch_t<uint16_t, uint16_t>(a, st);
     if (src_dtype == DT_U8 && dst_dtype == DT_U8) return launch_t<uint8_t, uint8_t>(a, st);

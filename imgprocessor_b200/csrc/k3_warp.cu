@@ -10,6 +10,7 @@
 // is bound by load/FP32 issue (64 loads + 192 FP32 operations per Lanczos4 pixel), not by HBM; consecutive
 // lanes read consecutive source columns, so the gathers are coalesced L1 hits for any sane homography.
 #include <algorithm>
+#include <type_traits>
 #include "imgcorr_kernels.cuh"
 #include "imgcorr_tma.cuh"
 #include "imgcorr_warp.cuh"
@@ -22,6 +23,11 @@ template <typename T> struct OutCast;
 template <> struct OutCast<float> { static __device__ __forceinline__ float cast(float v) { return v; } };
 template <> struct OutCast<double> { static __device__ __forceinline__ double cast(double v) { return v; } };
 template <> struct OutCast<uint16_t> { static __device__ __forceinline__ uint16_t cast(float v) { return sat_u16(v); } };
+// DT != T: a float32 source warped in float32 and stored through the quantiser (the batch chain's integer output)
+template <typename T, typename DT, typename AT> __device__ __forceinline__ DT k3_out(AT v, const OutScale& q) {
+    if constexpr (std::is_same<T, DT>::value) return OutCast<T>::cast(v);
+    else return quantise<DT>(v, q);
+}
 
 template <typename T> __device__ __forceinline__ T ldg(const T* p) { return __ldg(p); }
 
@@ -35,7 +41,7 @@ template <> struct AccOf<double> { typedef double type; };
 
 constexpr int K3_BX = 32, K3_BY = 8;
 
-template <typename T, typename AT, int N>
+template <typename T, typename AT, int N, typename DT = T>
 __global__ void __launch_bounds__(K3_BX* K3_BY) k3_warp_kernel(const K3Args a) {
     __shared__ float tab[N][32];   // transposed: tab[tap][phase] -> lanes with different phases hit different banks
     for (int i = threadIdx.y * K3_BX + threadIdx.x; i < N * 32; i += K3_BX * K3_BY) tab[i % N][i / N] = a.tab[i];
@@ -57,7 +63,7 @@ __global__ void __launch_bounds__(K3_BX* K3_BY) k3_warp_kernel(const K3Args a) {
     const AT cv = (AT)a.border;
     const size_t spx = (size_t)a.H * a.W, dpx = (size_t)a.dh * a.dw;
     const T* S = (const T*)a.src;
-    T* D = (T*)a.dst + (size_t)y * a.dw + x;
+    DT* D = (DT*)a.dst + (size_t)y * a.dw + x;
     const long long o0 = (long long)sy * a.W + sx;
     for (int f = 0; f < a.n_frames; ++f, S += spx, D += dpx) {
         AT v;
@@ -80,7 +86,7 @@ __global__ void __launch_bounds__(K3_BX* K3_BY) k3_warp_kernel(const K3Args a) {
         } else {
             v = warp_border_ool<T, AT, N>(S, a.H, a.W, sx, sy, wy, wx, cv);
         }
-        *D = OutCast<T>::cast(v);
+        *D = k3_out<T, DT>(v, a.q);
     }
 }
 
@@ -110,7 +116,7 @@ template <typename T> constexpr int k3t_box_bytes() { return K3Box<T>::BW * K3T_
 constexpr int K3T_CVT_BYTES = K3T_PITCH * K3T_BH * 4;
 template <typename T> constexpr int k3t_smem() { return K3T_NBUF * k3t_box_bytes<T>() + (sizeof(T) == 4 ? 0 : 2 * K3T_CVT_BYTES) + 128; }
 
-template <typename T, int N>
+template <typename T, int N, typename DT = T>
 __global__ void __launch_bounds__(K3T_THREADS, K3T_MINB_V) k3_tiled_kernel(const __grid_constant__ CUtensorMap tm_src, const K3Args a) {
     constexpr int BW = K3Box<T>::BW, BOX_BYTES = k3t_box_bytes<T>();
     constexpr bool CVT = sizeof(T) != 4;
@@ -153,7 +159,7 @@ __global__ void __launch_bounds__(K3T_THREADS, K3T_MINB_V) k3_tiled_kernel(const
 
     typedef typename AccOf<T>::type AT;
     const size_t spx = (size_t)H * W, dpx = (size_t)a.dh * a.dw;
-    T* D = (T*)a.dst + ((size_t)(live ? y : 0) * a.dw + (live ? x : 0));
+    DT* D = (DT*)a.dst + ((size_t)(live ? y : 0) * a.dw + (live ? x : 0));
     if (fits) {
         const int so = interior ? (sy - by) * K3T_PITCH + (sx - bx) : 0;
         auto issue = [&](int f) {
@@ -190,7 +196,7 @@ __global__ void __launch_bounds__(K3T_THREADS, K3T_MINB_V) k3_tiled_kernel(const
                 for (int k = 1; k < N; ++k) acc = fadd(acc, fmul(P[r * K3T_PITCH + k], fmul(wy[r], wx[k])));
                 v = fadd(v, acc);
             }
-            if (interior) D[f * dpx] = OutCast<T>::cast(v);
+            if (interior) D[f * dpx] = k3_out<T, DT>(v, a.q);
             if (!CVT) {
                 __syncthreads();                       // everyone is done with this buffer
                 if (tid == 0 && f + K3T_NBUF < nf) issue(f + K3T_NBUF);
@@ -208,14 +214,14 @@ __global__ void __launch_bounds__(K3T_THREADS, K3T_MINB_V) k3_tiled_kernel(const
                 for (int k = 1; k < N; ++k) acc = wadd(acc, wmul((AT)ldg(P + k), (AT)fmul(wy[r], wx[k])));
                 v = wadd(v, acc);
             }
-            D[f * dpx] = OutCast<T>::cast(v);
+            D[f * dpx] = k3_out<T, DT>(v, a.q);
         }
     }
     if (live && !interior) {
         const AT cv = (AT)a.border;
         const T* S = (const T*)a.src;
         for (int f = 0; f < nf; ++f, S += spx)
-            D[f * dpx] = OutCast<T>::cast(outside ? cv : warp_border_ool<T, AT, N>(S, H, W, sx, sy, wy, wx, cv));
+            D[f * dpx] = k3_out<T, DT>(outside ? cv : warp_border_ool<T, AT, N>(S, H, W, sx, sy, wy, wx, cv), a.q);
     }
 }
 
@@ -225,15 +231,17 @@ bool k3_tiled_eligible(const K3Args& a) {
     return tensor_map_encoder() != nullptr;
 }
 
-template <typename T>
+template <typename T, typename DT = T>
 cudaError_t launch_tiled(const K3Args& a, int interp, cudaStream_t st) {
     CUtensorMap tm;
     if (!make_tensor_map(&tm, K3Box<T>::DT, sizeof(T), a.src, a.W, a.H, a.n_frames, K3Box<T>::BW, K3T_BH)) return cudaErrorInvalidValue;
     dim3 grid((a.dw + K3T_TW - 1) / K3T_TW, (a.dh + K3T_TH - 1) / K3T_TH);
     if (interp == WARP_LANCZOS4)
-        k3_tiled_kernel<T, 8><<<grid, K3T_THREADS, k3t_smem<T>(), st>>>(tm, a);
-    else
+        k3_tiled_kernel<T, 8, DT><<<grid, K3T_THREADS, k3t_smem<T>(), st>>>(tm, a);
+    else if constexpr (std::is_same<T, DT>::value)           // the chain warps with Lanczos4 only
         k3_tiled_kernel<T, 4><<<grid, K3T_THREADS, k3t_smem<T>(), st>>>(tm, a);
+    else
+        return cudaErrorNotSupported;
     return cudaGetLastError();
 }
 
@@ -275,13 +283,15 @@ __global__ void __launch_bounds__(256) k3_divide_inplace_kernel(double* data, co
     }
 }
 
-template <typename T, typename AT>
+template <typename T, typename AT, typename DT = T>
 cudaError_t launch_typed(const K3Args& a, int interp, cudaStream_t st) {
     dim3 block(K3_BX, K3_BY), grid((a.dw + K3_BX - 1) / K3_BX, (a.dh + K3_BY - 1) / K3_BY);
     if (interp == WARP_LANCZOS4)
-        k3_warp_kernel<T, AT, 8><<<grid, block, 0, st>>>(a);
-    else
+        k3_warp_kernel<T, AT, 8, DT><<<grid, block, 0, st>>>(a);
+    else if constexpr (std::is_same<T, DT>::value)
         k3_warp_kernel<T, AT, 4><<<grid, block, 0, st>>>(a);
+    else
+        return cudaErrorNotSupported;
     return cudaGetLastError();
 }
 
@@ -298,6 +308,14 @@ cudaError_t launch_k3(const K3Args& a, int dtype, int interp, int variant, cudaS
     const bool tiled = wanted && ((dtype == DT_U16 && k3_tiled_eligible<uint16_t>(a)) || (dtype == DT_F32 && k3_tiled_eligible<float>(a)));
     if (variant == 2 && !tiled) return cudaErrorNotSupported;
     cudaError_t e;
+    if (a.dst_dtype != dtype) {
+        // float32 source, integer destination: the float32 warp of the F32 call, stored through the quantiser
+        if (dtype != DT_F32 || (a.dst_dtype != DT_U16 && a.dst_dtype != DT_U8)) return cudaErrorInvalidValue;
+        if (a.dst_dtype == DT_U16) e = tiled ? launch_tiled<float, uint16_t>(a, interp, st) : launch_typed<float, float, uint16_t>(a, interp, st);
+        else e = tiled ? launch_tiled<float, uint8_t>(a, interp, st) : launch_typed<float, float, uint8_t>(a, interp, st);
+        if (launches) ++*launches;
+        return e;
+    }
     switch (dtype) {
         case DT_U8: {
             if (!a.itab) return cudaErrorInvalidValue;

@@ -241,11 +241,20 @@ class Engine(object):
     def ingest(self, big_endian=False, gap=0):
         return Engine._Ingest(self, big_endian, gap)
 
+    def _set_out_scale(self, code, out_scale):
+        """Integer output (U16 / U8): set the context's output scale (offset, gain) for the call that follows; None is the
+        default (0, 1), OpenCV's saturate_cast of the float32 result.  Float output takes no scale."""
+        if code in (_lib.U8, _lib.U16):
+            offset, gain = (0.0, 1.0) if out_scale is None else out_scale
+            _lib.check(self.lib.imgcorr_set_output_scale(self._h, float(offset), float(gain)))
+        elif out_scale is not None:
+            raise ValueError('out_scale applies to uint8 / uint16 output only')
+
     def correct_file_bytes(self, buf, offset, n_frames, gap=0, big_endian=False, dtype=None, **kw):
         """The chain on frames as they sit in a file image: ``buf`` is a uint8 CUDA tensor holding the file bytes,
         the first frame's pixels start at byte ``offset`` and consecutive frames are ``gap`` bytes apart
         (reader/elbin.py: 20-byte per-frame headers; reader/RAW.py: dense, big-endian by default).  No host-side
-        byte swap or de-interleave: K1 does both in its load.  kw as correct_batch."""
+        byte swap or de-interleave: K1 does both in its load.  kw as correct_batch (out_scale included)."""
         tt = torch()
         dtype = dtype or tt.uint16
         esz = {tt.uint8: 1, tt.uint16: 2, tt.float32: 4}[dtype]
@@ -261,6 +270,7 @@ class Engine(object):
             out = tt.empty((n_frames, h, w), dtype=kw.get('out_dtype') or tt.float32, device=self.device)
         else:
             self._check_out(out, (n_frames, h, w))
+        self._set_out_scale(_dtype_code(out.dtype), kw.get('out_scale'))
         with self.ingest(big_endian, gap):
             _lib.check(self.lib.imgcorr_correct_batch(
                 self._h, ctypes.c_void_p(buf.data_ptr() + offset), _dtype_code(dtype), ctypes.c_void_p(out.data_ptr()),
@@ -501,8 +511,10 @@ class Engine(object):
         return mapx, mapy
 
     def correct_batch(self, raw, threshold=0.1, ksize=3, flags=DO_DARK | DO_FLAT | DO_NAN_TO_NUM, use_lens=True,
-                      border_value=0.0, window=None, out_dtype=None, out=None):
-        """K1 -> K2 [-> perspective stage with DO_PERSPECTIVE in flags] for every frame of a device-resident batch [n,H,W]."""
+                      border_value=0.0, window=None, out_dtype=None, out=None, out_scale=None):
+        """K1 -> K2 [-> perspective stage with DO_PERSPECTIVE in flags] for every frame of a device-resident batch [n,H,W].
+        uint16 / uint8 output stores the float32 result v as round_half_even(clip((v - offset) * gain)) with
+        ``out_scale=(offset, gain)`` (default (0, 1)), inside the chain's last kernel."""
         tt = torch()
         squeeze = raw.dim() == 2
         raw = self._frames(raw)
@@ -512,6 +524,7 @@ class Engine(object):
             out = tt.empty((n, h, w), dtype=out_dtype or tt.float32, device=self.device)
         else:
             self._check_out(out, (h, w) if squeeze and out.dim() == 2 else (n, h, w))
+        self._set_out_scale(_dtype_code(out.dtype), out_scale)
         _lib.check(self.lib.imgcorr_correct_batch(
             self._h, ctypes.c_void_p(raw.data_ptr()), _dtype_code(raw.dtype), ctypes.c_void_p(out.data_ptr()),
             _dtype_code(out.dtype), n, float(threshold), int(ksize), int(flags), int(lens), float(border_value),
@@ -519,9 +532,9 @@ class Engine(object):
         return out[0] if squeeze else out
 
     def correct_host(self, raw, out=None, threshold=0.1, ksize=3, flags=DO_DARK | DO_FLAT | DO_NAN_TO_NUM,
-                     use_lens=True, border_value=0.0, window=None, out_dtype=np.float32):
+                     use_lens=True, border_value=0.0, window=None, out_dtype=np.float32, out_scale=None):
         """The chain on HOST numpy frames [n,H,W] (uint8/uint16/float32): pinned staging, H2D, kernels and
-        D2H of consecutive frames overlap inside the library.  Synchronous.  flags as correct_batch."""
+        D2H of consecutive frames overlap inside the library.  Synchronous.  flags, out_scale as correct_batch."""
         squeeze = raw.ndim == 2
         raw = np.ascontiguousarray(raw)
         big_endian = raw.dtype.byteorder == '>' or (raw.dtype.byteorder == '=' and not np.little_endian)
@@ -539,6 +552,9 @@ class Engine(object):
             out = np.empty((n, h, w), dtype=out_dtype)
         if not out.flags.c_contiguous or out.shape != (n, h, w):
             raise ValueError('out must be C-contiguous of shape %s' % ((n, h, w),))
+        if out.dtype not in NP_CODES:
+            raise TypeError('unsupported output dtype %s (uint8, uint16, float32, float64)' % out.dtype)
+        self._set_out_scale(NP_CODES[out.dtype], out_scale)
         with self.ingest(big_endian, 0):
             _lib.check(self.lib.imgcorr_correct_host(
                 self._h, raw.ctypes.data_as(ctypes.c_void_p), NP_CODES[raw.dtype], out.ctypes.data_as(ctypes.c_void_p),

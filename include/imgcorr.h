@@ -32,7 +32,8 @@ extern "C" {
 
 #define IMGCORR_VERSION 200 /* 0.2.0: round 2 added imgcorr_ste_average_thr, imgcorr_stack_mean, imgcorr_scale_f64, imgcorr_subsample_f64,
                                imgcorr_linear_fit, imgcorr_host_fingerprint, imgcorr_selftest_division and the K2 options 11, 12;
-                               later added imgcorr_set_perspective and IMGCORR_DO_PERSPECTIVE (the chain's perspective stage) */
+                               later added imgcorr_set_perspective and IMGCORR_DO_PERSPECTIVE (the chain's perspective stage),
+                               and U16 / U8 output of the chain with imgcorr_set_output_scale */
 
 #if defined(__GNUC__)
 #define IMGCORR_API __attribute__((visibility("default")))
@@ -153,7 +154,11 @@ IMGCORR_API int imgcorr_undistort_maps(imgcorr_ctx* ctx, float* mapx_dev, float*
  * image branch; a stack of frames is a batch here, not the STE average of :385-406).
  *   threshold > 0 : median-threshold with ksize (3 in correct(), :556-563) after nan_to_num
  *   use_lens      : apply K2 if a lens is set (missing lens -> frames pass through, :570-575)
- *   out_dtype     : F32 or F64 (float64 is what the reference returns, :459)
+ *   out_dtype     : F32 or F64 (float64 is what the reference returns, :459), or U16 / U8: the F32 result v of every pixel
+ *                   stored as an integer through the context's output scale (imgcorr_set_output_scale), fused into the
+ *                   chain's last kernel (no extra pass):  t = ((double)v - offset) * gain (two roundings, no FMA);
+ *                   0 if t is NaN or t <= 0, 65535 / 255 if t >= that, else t rounded half to even.  The default scale
+ *                   (0, 1) is OpenCV's saturate_cast of the F32 result.
  *   flags         : IMGCORR_DO_* ; with IMGCORR_DO_PERSPECTIVE the frame described above (the K2 window [oh][ow], or the
  *                   K1 output [H][W] without a lens) is warped by the context's perspective stage and out_dev is
  *                   [n][dst_h][dst_w] (see imgcorr_set_perspective); IMGCORR_ERR_STATE if the context has none
@@ -174,6 +179,12 @@ IMGCORR_API int imgcorr_correct_host(imgcorr_ctx* ctx, const void* raw_host, int
                          int n_frames, double threshold, int ksize, int flags, int use_lens, double border_value,
                          int x0, int y0, int ow, int oh);
 
+/* Scale of the chain's integer output (out_dtype U16 / U8 of imgcorr_correct_batch / imgcorr_correct_host):
+ * stored = quantise((F32 result - offset) * gain), see imgcorr_correct_batch.  Context state, read when a chain call is
+ * enqueued; defaults offset 0, gain 1.  IMGCORR_ERR_INVALID for a non-finite offset or a gain that is not finite and > 0.
+ * Other entry points (imgcorr_pointwise_median's integer output included) do not read it. */
+IMGCORR_API int imgcorr_set_output_scale(imgcorr_ctx* ctx, double offset, double gain);
+
 /* The chain's perspective stage: PerspectiveCorrection.correct (camera/PerspectiveCorrection.py:380-406) on every frame of
  * an imgcorr_correct_batch / imgcorr_correct_host call that sets IMGCORR_DO_PERSPECTIVE, without the intermediate frames
  * leaving the device.  Per frame group: K1 -> [K2] -> [tilt division] -> K3 (Lanczos4, forward map, BORDER_CONSTANT).
@@ -183,10 +194,11 @@ IMGCORR_API int imgcorr_correct_host(imgcorr_ctx* ctx, const void* raw_host, int
  *   tilt_factor   NULL: no intensity correction.  Otherwise float64 [tilt_h][tilt_w] (device pointer if on_device != 0,
  *                 host pointer otherwise), copied synchronously into the context; the chain frame is divided by it in
  *                 float64 before the warp (np.asfarray(img) / tf, :394-400)
- * Precision: with out_dtype F32 the float32 chain frame is warped in float32 (cv2.warpPerspective of that frame); with F64
+ * Precision: with out_dtype F32 the float32 chain frame is warped in float32 (cv2.warpPerspective of that frame), with U16 / U8
+ * that same float32 warp is quantised on store (imgcorr_set_output_scale); with F64
  * the float64 chain frame is warped in float64 (pc.correct(cal.correct(frame)) of the Python mirror).  A tilt factor needs
  * out_dtype F64 and the shape of the chain frame: either mismatch makes the chain call fail with IMGCORR_ERR_INVALID.
- * The stage adds one part to the chain scratch: a group of chain frames in out_dtype.  Synchronous. */
+ * The stage adds one part to the chain scratch: a group of chain frames in out_dtype (float32 for U16 / U8).  Synchronous. */
 IMGCORR_API int imgcorr_set_perspective(imgcorr_ctx* ctx, const double M[9], int dst_h, int dst_w, double border_value,
                             const double* tilt_factor, int tilt_h, int tilt_w, int on_device);
 
