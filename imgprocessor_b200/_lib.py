@@ -43,6 +43,7 @@ SIGNATURES = {
                                      c_double, c_int, c_int, c_int, c_int]),
     'imgcorr_set_output_scale': (c_int, [c_void_p, c_double, c_double]),
     'imgcorr_set_perspective': (c_int, [c_void_p, c_void_p, c_int, c_int, c_double, c_void_p, c_int, c_int, c_int]),
+    'imgcorr_set_perspective_frames': (c_int, [c_void_p, c_void_p, c_int, c_int, c_int, c_double]),
     'imgcorr_warp_perspective': (c_int, [c_void_p, c_void_p, c_int, c_int, c_int, c_void_p, c_int, c_int, c_int, c_void_p,
                                          c_int, c_int, c_double, c_void_p]),
     'imgcorr_divide_f64': (c_int, [c_void_p, c_void_p, c_int, c_void_p, c_void_p, c_size_t, c_int, c_void_p]),

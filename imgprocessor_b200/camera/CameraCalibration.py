@@ -506,10 +506,29 @@ if shapes are transposed, execute self.transpose() once """ % (s, array.shape))
 
     # ------------------------------------------------------------------ batches of independent frames
     @staticmethod
-    def _perspective_stage(perspective, out, out_dtype):
-        """(homography, dsize, border value, tilt factor) of a PerspectiveCorrection as the chain's last stage, or None"""
+    def _perspective_stage(perspective, out, out_dtype, n):
+        """(homography, dsize, border value, tilt factor) of a PerspectiveCorrection as the chain's last stage, or None.
+        A sequence of n PerspectiveCorrection objects, one per frame, gives the homographies stacked to (n, 3, 3) and no
+        tilt factor; they must agree on dsize and border value."""
         if perspective is None:
             return None
+        if isinstance(perspective, (list, tuple)):
+            if len(perspective) != n:
+                raise ValueError('perspective: %d PerspectiveCorrection objects for %d frames' % (len(perspective), n))
+            if n == 0:
+                raise ValueError('perspective: an empty sequence')
+            for i, pc in enumerate(perspective):
+                if pc.opts['do_correctIntensity']:
+                    raise ValueError('perspective[%d] has do_correctIntensity: per-frame tilt factors are not supported '
+                                     'in the batch chain' % i)
+            stages = [pc.correct_params() for pc in perspective]
+            for i, s in enumerate(stages):
+                if tuple(s[1]) != tuple(stages[0][1]) or s[2] != stages[0][2]:
+                    raise ValueError('perspective[%d] has dsize %s and border value %r, perspective[0] %s and %r: the '
+                                     'frames of one batch share both' % (i, tuple(s[1]), s[2], tuple(stages[0][1]),
+                                                                         stages[0][2]))
+            M = np.stack([np.asarray(s[0], np.float64).reshape(3, 3) for s in stages])
+            return M, tuple(stages[0][1]), stages[0][2], None
         stage = perspective.correct_params()
         tt = _engine.torch()
         dt = out.dtype if out is not None else out_dtype
@@ -551,7 +570,13 @@ if shapes are transposed, execute self.transpose() once """ % (s, array.shape))
         (do_correctIntensity=True) needs float64 output.  The stage stays on the cached engine of the device and frame
         shape after the call, its tilt factor included (float64 on the device: 98 MB at 4096x3000), so that the next call
         with the same PerspectiveCorrection uploads nothing; calls without ``perspective=`` do not use it, and
-        ``engine.get_engine(H, W, device).set_perspective(None, None)`` frees it."""
+        ``engine.get_engine(H, W, device).set_perspective(None, None)`` frees it.
+
+        ``perspective`` may also be a list of n PerspectiveCorrection objects, one per frame (each module found at its own
+        place, ``pc_i.setReference(quad_i)``): frame i is warped with ``perspective[i]``'s homography, so that
+        ``correct_batch(frames, perspective=pcs)[i]`` equals ``pcs[i].correct(correct(frames[i]))``.  They must share the
+        destination size and border value, and none may have do_correctIntensity; otherwise ValueError.  With
+        ``devices=``, every device gets the matrices of its own shard."""
         import contextlib
         import io
         tt = _engine.torch()
@@ -569,7 +594,7 @@ if shapes are transposed, execute self.transpose() once """ % (s, array.shape))
                 raise ValueError('devices= shards HOST frames; a CUDA tensor is processed on its own device')
             if not devices:
                 raise ValueError('devices is empty')
-        stage = self._perspective_stage(perspective, out, out_dtype)
+        stage = self._perspective_stage(perspective, out, out_dtype, n)
         if devices is not None and len(devices) > 1:
             return self._correct_batch_multi(frames, devices, bgImages, exposure_time, light_spectrum, threshold,
                                              keep_size, date, out, out_dtype, verbose, stage, out_scale)
@@ -648,8 +673,14 @@ if shapes are transposed, execute self.transpose() once """ % (s, array.shape))
             if threshold > 0:
                 flags |= _lib.DO_NAN_TO_NUM
             if stage is not None:
-                for e in engines:
-                    self._set_perspective(e, stage)
+                for i, e in enumerate(engines):
+                    lo, hi = sharding.shard_range(n, len(engines), i)
+                    if np.ndim(stage[0]) == 3:                # a per-frame table: the matrices of this engine's shard
+                        if hi <= lo:
+                            continue
+                        self._set_perspective(e, (stage[0][lo:hi],) + tuple(stage[1:]))
+                    else:
+                        self._set_perspective(e, stage)
                 flags |= _lib.DO_PERSPECTIVE
             window = tuple(int(v) for v in lens.roi) if (lens and not keep_size) else None
             oh, ow = engines[0].chain_shape(flags, bool(lens), window)[2]

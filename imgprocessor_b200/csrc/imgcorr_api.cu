@@ -140,8 +140,12 @@ struct imgcorr_ctx {
     // the chain's K1 output (with a lens: two halves of `chain_group` float32 frames each), then the warp source of the
     // perspective stage (a group of chain frames in the output dtype)
     SharedScratch chain_scratch;
-    struct Perspective { bool on = false; double M[9]; int dh = 0, dw = 0; double border = 0.0; DevPtr<double> tilt; int th = 0, tw = 0; };
-    Perspective persp;                        // the chain's last stage (imgcorr_set_perspective)
+    // one matrix M (imgcorr_set_perspective), or a device table of one inverted matrix per frame (imgcorr_set_perspective_frames)
+    struct Perspective {
+        bool on = false; double M[9]; int dh = 0, dw = 0; double border = 0.0; DevPtr<double> tilt; int th = 0, tw = 0;
+        DevPtr<WarpConst> table; int n_table = 0;
+    };
+    Perspective persp;                        // the chain's last stage
     int chain_overlap = 1;                    // K1 of group g+1 on the internal stream while K2 of group g runs: +2-3.5 % on batches
     struct ChainOverlap { Stream st; Event k1[2], k2[2], entry; };
     ChainOverlap ov;                          // high-priority stream of K1 in overlap mode and its hand-off events
@@ -604,8 +608,8 @@ extern "C" IMGCORR_API int imgcorr_undistort_maps(imgcorr_ctx* c, float* mapx_de
 
 // ---- K3 -------------------------------------------------------------------------------------
 static int run_k3(imgcorr_ctx* c, const void* src_dev, int dtype, int src_h, int src_w, void* dst_dev, int dst_dtype, int dst_h,
-                  int dst_w, int n_frames, const double M[9], int interpolation, int inverse_map, double border_value, OutScale q,
-                  cudaStream_t st);
+                  int dst_w, int n_frames, const double M[9], const WarpConst* wcs, int interpolation, int inverse_map,
+                  double border_value, OutScale q, cudaStream_t st);
 
 extern "C" IMGCORR_API int imgcorr_warp_perspective(imgcorr_ctx* c, const void* src_dev, int dtype, int src_h, int src_w,
                                         void* dst_dev, int dst_h, int dst_w, int n_frames, const double M[9],
@@ -618,15 +622,16 @@ extern "C" IMGCORR_API int imgcorr_warp_perspective(imgcorr_ctx* c, const void* 
     if (src_h <= 0 || src_w <= 0 || dst_h <= 0 || dst_w <= 0 || src_h > 32767 || src_w > 32767 || dst_h > 32767 || dst_w > 32767)
         return fail(IMGCORR_ERR_INVALID, "bad frame shape (%d x %d -> %d x %d)", src_h, src_w, dst_h, dst_w);
     if (n_frames < 0) return fail(IMGCORR_ERR_INVALID, "n_frames < 0");
-    return run_k3(c, src_dev, dtype, src_h, src_w, dst_dev, dtype, dst_h, dst_w, n_frames, M, interpolation, inverse_map,
+    return run_k3(c, src_dev, dtype, src_h, src_w, dst_dev, dtype, dst_h, dst_w, n_frames, M, nullptr, interpolation, inverse_map,
                   border_value, OutScale{0.0, 1.0}, (cudaStream_t)stream);
 }
 
 // K3 on validated arguments; the coefficient tables are built on first use.  dst_dtype is dtype, or U16 / U8 for a float32
-// source (the chain's integer output: float32 warp, then quantise with q)
+// source (the chain's integer output: float32 warp, then quantise with q).  wcs: a device table of n_frames inverted
+// matrices (the chain's per-frame stage), used instead of M
 static int run_k3(imgcorr_ctx* c, const void* src_dev, int dtype, int src_h, int src_w, void* dst_dev, int dst_dtype, int dst_h,
-                  int dst_w, int n_frames, const double M[9], int interpolation, int inverse_map, double border_value, OutScale q,
-                  cudaStream_t st) {
+                  int dst_w, int n_frames, const double M[9], const WarpConst* wcs, int interpolation, int inverse_map,
+                  double border_value, OutScale q, cudaStream_t st) {
     if (!c->warp_tab) {
         float h[32 * 8 + 32 * 4];
         warp_lanczos4_table(h);
@@ -661,7 +666,8 @@ static int run_k3(imgcorr_ctx* c, const void* src_dev, int dtype, int src_h, int
     a.dst_dtype = dst_dtype;
     a.q = q;
     a.border = border_for_dtype(dtype == DT_U8, dtype == DT_U16, border_value);
-    a.wc = make_warp_const(M, inverse_map, dst_w, dst_h);
+    a.wc = wcs ? WarpConst{} : make_warp_const(M, inverse_map, dst_w, dst_h);
+    a.wcs = wcs;
     a.tab = interpolation == IMGCORR_INTER_LANCZOS4 ? c->warp_tab.get() : c->warp_tab.get() + 32 * 8;
     int l = 0;
     cudaError_t e = launch_k3(a, dtype, interpolation, c->k3_variant, st, &l);
@@ -753,10 +759,12 @@ extern "C" IMGCORR_API int imgcorr_set_perspective(imgcorr_ctx* c, const double 
             return fail(IMGCORR_ERR_INVALID, "bad tilt factor shape %d x %d", tilt_h, tilt_w);
     }
     const size_t tilt_bytes = (M && tilt_factor) ? (size_t)tilt_h * tilt_w * sizeof(double) : 0;
-    // launches on other (non-blocking) streams may still read the tilt factor being replaced or dropped
-    if (p.tilt) {
+    // launches on other (non-blocking) streams may still read the tilt factor or the per-frame table being replaced or dropped
+    if (p.tilt || p.table) {
         CK(cudaDeviceSynchronize());
         if (tilt_bytes != (size_t)p.th * p.tw * sizeof(double)) { p.tilt.reset(); p.th = p.tw = 0; }
+        p.table.reset();
+        p.n_table = 0;
     }
     if (!M) return IMGCORR_OK;
     if (tilt_bytes) {
@@ -776,11 +784,45 @@ extern "C" IMGCORR_API int imgcorr_set_perspective(imgcorr_ctx* c, const double 
     return IMGCORR_OK;
 }
 
-// the refusals of a chain call with IMGCORR_DO_PERSPECTIVE whose chain frame is [oh][ow]
-static int check_perspective(const imgcorr_ctx* c, int out_dtype, int ow, int oh) {
+extern "C" IMGCORR_API int imgcorr_set_perspective_frames(imgcorr_ctx* c, const double* M, int n_matrices, int dst_h, int dst_w,
+                                              double border_value) {
+    GUARD(c);
+    imgcorr_ctx::Perspective& p = c->persp;
+    p.on = false;                                      // as imgcorr_set_perspective: a failed call leaves no stage behind
+    if (M) {
+        if (n_matrices <= 0) return fail(IMGCORR_ERR_INVALID, "n_matrices %d", n_matrices);
+        if (dst_h <= 0 || dst_w <= 0 || dst_h > 32767 || dst_w > 32767)
+            return fail(IMGCORR_ERR_INVALID, "bad destination shape %d x %d", dst_h, dst_w);
+    }
+    // launches on other (non-blocking) streams may still read the tilt factor or the table being replaced or dropped
+    if (p.tilt || p.table) {
+        CK(cudaDeviceSynchronize());
+        p.tilt.reset();
+        p.th = p.tw = 0;
+        if (!M || p.n_table != n_matrices) { p.table.reset(); p.n_table = 0; }
+    }
+    if (!M) return IMGCORR_OK;
+    std::vector<WarpConst> h((size_t)n_matrices);
+    for (int i = 0; i < n_matrices; ++i) h[i] = make_warp_const(M + 9 * (size_t)i, 0, dst_w, dst_h);
+    if (!p.table) {
+        CK(dev_alloc(p.table, h.size() * sizeof(WarpConst)));
+        p.n_table = n_matrices;
+    }
+    CK(cudaMemcpy(p.table.get(), h.data(), h.size() * sizeof(WarpConst), cudaMemcpyHostToDevice));
+    p.dh = dst_h;
+    p.dw = dst_w;
+    p.border = border_value;
+    p.on = true;
+    return IMGCORR_OK;
+}
+
+// the refusals of a chain call with IMGCORR_DO_PERSPECTIVE whose chain frame is [oh][ow], before anything is enqueued
+static int check_perspective(const imgcorr_ctx* c, int out_dtype, int ow, int oh, int n_frames) {
     const imgcorr_ctx::Perspective& p = c->persp;
     if (!p.on) return fail(IMGCORR_ERR_STATE, "perspective requested but no perspective set");
     if (ow > 32767 || oh > 32767) return fail(IMGCORR_ERR_INVALID, "perspective source %d x %d exceeds 32767 per side", oh, ow);
+    if (p.table && n_frames > p.n_table)
+        return fail(IMGCORR_ERR_INVALID, "%d frames but the perspective stage holds %d matrices", n_frames, p.n_table);
     if (!p.tilt) return IMGCORR_OK;
     if (out_dtype != DT_F64)
         return fail(IMGCORR_ERR_INVALID, "a tilt factor needs out_dtype F64: the division and the warp are computed in float64");
@@ -790,12 +832,13 @@ static int check_perspective(const imgcorr_ctx* c, int out_dtype, int ow, int oh
 }
 
 // one frame (or a group of frames) through K1 -> [K2] -> [tilt division] -> [K3] on `st`; `persp` was checked by
-// check_perspective
+// check_perspective.  `first`: the index of raw's first frame in the caller's call (chunks of the host pipeline start
+// later), which picks the matrices of a per-frame perspective table.
 // Integer output (U16 / U8) is the float32 chain with the quantiser fused into the last kernel's store: K1 without a lens or
 // perspective stage, K2 with a lens, K3 with the stage (which warps the float32 chain frame).
 static int chain_frames(imgcorr_ctx* c, const void* raw, int raw_dtype, void* out, int out_dtype, int n, double thr,
                         int ksize, int flags, bool lens, bool persp, double border, int x0, int y0, int ow, int oh,
-                        cudaStream_t st) {
+                        cudaStream_t st, int first) {
     if (out_dtype < DT_U8 || out_dtype > DT_F64) return fail(IMGCORR_ERR_INVALID, "out_dtype must be U8, U16, F32 or F64");
     const bool quant = out_dtype == DT_U8 || out_dtype == DT_U16;
     const int frame_dtype = quant ? DT_F32 : out_dtype;    // the chain frame: what K2 (or K1) returns before the stage
@@ -896,7 +939,7 @@ static int chain_frames(imgcorr_ctx* c, const void* raw, int raw_dtype, void* ou
             if ((r = launched(c, l, e, "divide kernel launch"))) return r;
         }
         r = run_k3(c, frames, frame_dtype, oh, ow, (char*)out + f * out_stride, out_dtype, p.dh, p.dw, nf, p.M,
-                   IMGCORR_INTER_LANCZOS4, 0, p.border, c->out_scale, st);
+                   p.table ? p.table.get() + first + f : nullptr, IMGCORR_INTER_LANCZOS4, 0, p.border, c->out_scale, st);
         if (r) return r;
     }
     return IMGCORR_OK;
@@ -910,9 +953,9 @@ extern "C" IMGCORR_API int imgcorr_correct_batch(imgcorr_ctx* c, const void* raw
     const bool lens = use_lens && c->has_lens;
     if (!lens) { x0 = 0; y0 = 0; ow = c->W; oh = c->H; }
     const bool persp = flags & IMGCORR_DO_PERSPECTIVE;
-    if (persp) { int r = check_perspective(c, out_dtype, ow, oh); if (r) return r; }
+    if (persp) { int r = check_perspective(c, out_dtype, ow, oh, n_frames); if (r) return r; }
     return chain_frames(c, raw_dev, raw_dtype, out_dev, out_dtype, n_frames, threshold, ksize, flags, lens, persp,
-                        border_value, x0, y0, ow, oh, (cudaStream_t)stream);
+                        border_value, x0, y0, ow, oh, (cudaStream_t)stream, 0);
 }
 
 // ---- host-buffer pipeline ---------------------------------------------------------------------
@@ -962,7 +1005,7 @@ extern "C" IMGCORR_API int imgcorr_correct_host(imgcorr_ctx* c, const void* raw_
     const bool lens = use_lens && c->has_lens;
     if (!lens) { x0 = 0; y0 = 0; ow = c->W; oh = c->H; }
     const bool persp = flags & IMGCORR_DO_PERSPECTIVE;
-    if (persp) { int r = check_perspective(c, out_dtype, ow, oh); if (r) return r; }
+    if (persp) { int r = check_perspective(c, out_dtype, ow, oh, n_frames); if (r) return r; }
     const size_t frame_raw = (size_t)c->H * c->W * dtype_size(raw_dtype);
     const size_t frame_out = (persp ? (size_t)c->persp.dw * c->persp.dh : (size_t)ow * oh) * dtype_size(out_dtype);
     // small frames travel in chunks of G frames per ring slot (up to 32 MB of raw data, at most 16 frames): one copy each
@@ -1004,7 +1047,7 @@ extern "C" IMGCORR_API int imgcorr_correct_host(imgcorr_ctx* c, const void* raw_
         CK(cudaEventRecord(s.ev_in.get(), s_in));
         CK(cudaStreamWaitEvent(s_k, s.ev_in.get(), 0));
         r = chain_frames(c, s.d_raw.get(), raw_dtype, s.d_out.get(), out_dtype, nf, threshold, ksize, flags, lens, persp,
-                         border_value, x0, y0, ow, oh, s_k);
+                         border_value, x0, y0, ow, oh, s_k, k * G);
         if (r) return r;
         CK(cudaEventRecord(s.ev_k.get(), s_k));
         CK(cudaStreamWaitEvent(s_out, s.ev_k.get(), 0));

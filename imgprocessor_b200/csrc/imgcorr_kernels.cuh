@@ -91,6 +91,8 @@ struct K3Args {
     const int16_t* itab;    // uint8 images: device fixed-point weights [32][32][N*N] (null otherwise)
     int dst_dtype;          // dtype of dst: the source dtype, or U16 / U8 for a float32 source (float32 warp, then quantise)
     OutScale q;             // the scale of that quantisation
+    const WarpConst* wcs;   // device table [n_frames]: frame f of the launch is warped with wcs[f] (Lanczos4, float32 /
+                            // float64 sources); null: every frame with wc
 };
 cudaError_t launch_k3(const K3Args& a, int dtype, int interp, int variant, cudaStream_t stream, int* launches);
 cudaError_t launch_k3_divide(const void* src, int dtype, const double* div, double* dst, size_t npx, int n_frames,

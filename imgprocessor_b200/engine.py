@@ -162,14 +162,33 @@ class Engine(object):
         every frame they would return with cv2.warpPerspective(frame, M, dsize=(width, height), INTER_LANCZOS4,
         BORDER_CONSTANT, border_value), after dividing it by ``tilt_factor`` (float64, the chain frame's shape; needs
         float64 output) if one is given.  M None removes the stage.  ``token``: an identity of the tilt factor; a call
-        with the same arguments and token as the last one uploads nothing."""
+        with the same arguments and token as the last one uploads nothing.
+
+        M of shape (n, 3, 3) is one matrix per frame (imgcorr_set_perspective_frames): frame i of every chain call is
+        warped with M[i], and a call with more than n frames is refused.  Such a table takes no tilt factor."""
         if M is None:
             _lib.check(self.lib.imgcorr_set_perspective(self._h, None, 0, 0, 0.0, None, 0, 0, 0))
             self.perspective_dsize = None
             self._tokens['perspective'] = None
             return
-        Mh = np.ascontiguousarray(np.asarray(M, np.float64).reshape(3, 3))
         dw, dh = int(dsize[0]), int(dsize[1])
+        Ma = np.asarray(M, np.float64)
+        if Ma.ndim == 3:
+            if Ma.shape[0] < 1 or Ma.shape[1:] != (3, 3):
+                raise ValueError('a per-frame table has shape (n, 3, 3), got %s' % (Ma.shape,))
+            if tilt_factor is not None:
+                raise ValueError('a tilt factor needs a single matrix: the per-frame table has no tilt factor')
+            Mt = np.ascontiguousarray(Ma)
+            key = ('frames', Mt.tobytes(), dw, dh, float(border_value))
+            if self._tokens.get('perspective') == key:
+                return
+            self._tokens['perspective'] = self.perspective_dsize = None      # a failed call leaves no stage behind
+            _lib.check(self.lib.imgcorr_set_perspective_frames(self._h, Mt.ctypes.data_as(ctypes.c_void_p), Mt.shape[0], dh,
+                                                               dw, float(border_value)))
+            self.perspective_dsize = (dw, dh)
+            self._tokens['perspective'] = key
+            return
+        Mh = np.ascontiguousarray(Ma.reshape(3, 3))
         key = (Mh.tobytes(), dw, dh, float(border_value), tilt_factor is None, token)
         if (tilt_factor is None or token is not None) and self._tokens.get('perspective') == key:
             return

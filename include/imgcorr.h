@@ -33,7 +33,8 @@ extern "C" {
 #define IMGCORR_VERSION 200 /* 0.2.0: round 2 added imgcorr_ste_average_thr, imgcorr_stack_mean, imgcorr_scale_f64, imgcorr_subsample_f64,
                                imgcorr_linear_fit, imgcorr_host_fingerprint, imgcorr_selftest_division and the K2 options 11, 12;
                                later added imgcorr_set_perspective and IMGCORR_DO_PERSPECTIVE (the chain's perspective stage),
-                               and U16 / U8 output of the chain with imgcorr_set_output_scale */
+                               U16 / U8 output of the chain with imgcorr_set_output_scale, and imgcorr_set_perspective_frames
+                               (one homography per frame in the perspective stage) */
 
 #if defined(__GNUC__)
 #define IMGCORR_API __attribute__((visibility("default")))
@@ -61,8 +62,9 @@ enum {
     IMGCORR_DO_DARK = 1,       /* image -= bg                           CameraCalibration.py:502      */
     IMGCORR_DO_FLAT = 2,       /* image[flat != 0] /= flat[flat != 0]   CameraCalibration.py:525-526  */
     IMGCORR_DO_NAN_TO_NUM = 4, /* image = np.nan_to_num(image)          CameraCalibration.py:561      */
-    IMGCORR_DO_PERSPECTIVE = 8 /* the context's perspective warp as the chain's last stage (imgcorr_set_perspective);
-                                  read by imgcorr_correct_batch and imgcorr_correct_host only */
+    IMGCORR_DO_PERSPECTIVE = 8 /* the context's perspective warp as the chain's last stage (imgcorr_set_perspective: one
+                                  matrix for every frame, or imgcorr_set_perspective_frames: matrix i for frame i of the
+                                  call); read by imgcorr_correct_batch and imgcorr_correct_host only */
 };
 
 /* imgcorr_set_option keys */
@@ -201,6 +203,18 @@ IMGCORR_API int imgcorr_set_output_scale(imgcorr_ctx* ctx, double offset, double
  * The stage adds one part to the chain scratch: a group of chain frames in out_dtype (float32 for U16 / U8).  Synchronous. */
 IMGCORR_API int imgcorr_set_perspective(imgcorr_ctx* ctx, const double M[9], int dst_h, int dst_w, double border_value,
                             const double* tilt_factor, int tilt_h, int tilt_w, int on_device);
+/* The same stage with one homography per frame: frame i of a chain call (raw_dev[i], raw_host[i]; i counts from the call's
+ * first frame) is warped with matrix i.  Everything else is as imgcorr_set_perspective without a tilt factor: Lanczos4,
+ * forward map, BORDER_CONSTANT, one destination size and border value, the same dtype rules.
+ *   M             host array [n_matrices][9], row-major, each matrix mapping the chain frame to the destination; inverted
+ *                 here with cv::invert's cofactor formula (a singular matrix becomes zeros) and uploaded synchronously.
+ *                 NULL removes the stage.
+ * A chain call with IMGCORR_DO_PERSPECTIVE and more than n_matrices frames fails with IMGCORR_ERR_INVALID before it
+ * enqueues anything.  The two setters replace each other: imgcorr_set_perspective drops the table, this call drops a
+ * single matrix and its tilt factor.  Replacing or removing a table first synchronises the device, since queued chain
+ * calls may still read it.  A failed call leaves no stage.  Synchronous. */
+IMGCORR_API int imgcorr_set_perspective_frames(imgcorr_ctx* ctx, const double* M, int n_matrices, int dst_h, int dst_w,
+                                   double border_value);
 
 /* ---- K3: perspective warp (SURVEY §8 row f3) -----------------------------------------------------
  * Replaces cv2.warpPerspective in PerspectiveCorrection.correct (flags=INTER_LANCZOS4,
