@@ -41,6 +41,10 @@ SIGNATURES = {
                                       c_double, c_int, c_int, c_int, c_int, c_void_p]),
     'imgcorr_correct_host': (c_int, [c_void_p, c_void_p, c_int, c_void_p, c_int, c_int, c_double, c_int, c_int, c_int,
                                      c_double, c_int, c_int, c_int, c_int]),
+    'imgcorr_correct_batch_bg': (c_int, [c_void_p, c_void_p, c_int, c_void_p, c_int, c_void_p, c_int, c_int, c_double, c_int,
+                                         c_int, c_int, c_double, c_int, c_int, c_int, c_int, c_void_p]),
+    'imgcorr_correct_host_bg': (c_int, [c_void_p, c_void_p, c_int, c_void_p, c_int, c_void_p, c_int, c_int, c_double, c_int,
+                                        c_int, c_int, c_double, c_int, c_int, c_int, c_int]),
     'imgcorr_set_output_scale': (c_int, [c_void_p, c_double, c_double]),
     'imgcorr_set_perspective': (c_int, [c_void_p, c_void_p, c_int, c_int, c_double, c_void_p, c_int, c_int, c_int]),
     'imgcorr_set_perspective_frames': (c_int, [c_void_p, c_void_p, c_int, c_int, c_int, c_double]),

@@ -345,18 +345,25 @@ if shapes are transposed, execute self.transpose() once """ % (s, array.shape))
         return dict(dark=bg, ascent=None, exposure=0.0, token=_map_token('dark', bg))
 
     def _configure_engine(self, eng, shape, bgImages, exposure_time, light_spectrum, date, use_dark=True):
-        """upload whatever calibration applies; returns (flags, lens-or-None)"""
+        """upload whatever calibration applies; returns (flags, lens-or-None).  use_dark=False: the call brings one background
+        image per frame (correct_batch(bg_frames=...)), which takes the dark stage's place like bgImages does in correct():
+        the calibrated dark entry is not resolved and the engine's dark map is left as it is."""
         flags = 0
-        try:
-            d = self._resolve_dark(shape, exposure_time, bgImages, date['dark current'])
-            eng.set_dark(d['dark'], d['ascent'], d['exposure'], self.coeffs['depth'], token=d['token'])
+        if not use_dark:
+            print('... remove dark current')
             flags |= _lib.DO_DARK
-            self._last_bg = d
-        except _lib.ImgcorrError:
-            raise
-        except Exception as errm:
-            print('Error: %s' % errm)
             self._last_bg = None
+        else:
+            try:
+                d = self._resolve_dark(shape, exposure_time, bgImages, date['dark current'])
+                eng.set_dark(d['dark'], d['ascent'], d['exposure'], self.coeffs['depth'], token=d['token'])
+                flags |= _lib.DO_DARK
+                self._last_bg = d
+            except _lib.ImgcorrError:
+                raise
+            except Exception as errm:
+                print('Error: %s' % errm)
+                self._last_bg = None
         self._last_flat = None
         try:
             f = self.getCoeff('flat field', light_spectrum, date['flat field'])
@@ -545,7 +552,7 @@ if shapes are transposed, execute self.transpose() once """ % (s, array.shape))
 
     def correct_batch(self, frames, bgImages=None, exposure_time=None, light_spectrum=None, threshold=0.1,
                       keep_size=True, date=None, out=None, out_dtype=None, verbose=False, devices=None, perspective=None,
-                      out_scale=None):
+                      out_scale=None, bg_frames=None):
         """correct() for n INDEPENDENT frames with one calibration lookup.
 
         ``frames``: numpy [n,H,W] (uint8 / uint16 / float32, host) -> streamed through pinned buffers with
@@ -576,7 +583,18 @@ if shapes are transposed, execute self.transpose() once """ % (s, array.shape))
         place, ``pc_i.setReference(quad_i)``): frame i is warped with ``perspective[i]``'s homography, so that
         ``correct_batch(frames, perspective=pcs)[i]`` equals ``pcs[i].correct(correct(frames[i]))``.  They must share the
         destination size and border value, and none may have do_correctIntensity; otherwise ValueError.  With
-        ``devices=``, every device gets the matrices of its own shard."""
+        ``devices=``, every device gets the matrices of its own shard.
+
+        ``bg_frames``: one background image per frame (the same exposure with the module's current off), of the shape of
+        ``frames``: a numpy array for host frames, a CUDA tensor on the frames' device for tensor frames.  Frame i is
+        corrected as ``correct(frames[i], bgImages=bg_frames[i])``: ``bg_frames[i]`` takes the calibrated dark current's
+        place (which is then not looked up), subtracted in float64 inside K1, so that
+        ``correct_batch(frames, bg_frames=bgs, out_dtype=np.float64)[i]`` equals ``correct(frames[i], bgImages=bgs[i])``.
+        Backgrounds of the frames' dtype or float32 go to the device as they are (a big-endian uint16 array is swapped on
+        the host); any other dtype, float64 included, is rounded to float32 once, as correct() does with float64
+        calibration maps.  It combines with ``devices=`` (every device gets its shard's backgrounds), ``perspective=``,
+        ``out_dtype`` / ``out_scale`` and ``keep_size``.  ValueError, before any engine is created, for another shape, for
+        ``bgImages`` given as well, for a numpy / tensor mismatch with ``frames`` and for a tensor on another device."""
         import contextlib
         import io
         tt = _engine.torch()
@@ -595,14 +613,17 @@ if shapes are transposed, execute self.transpose() once """ % (s, array.shape))
             if not devices:
                 raise ValueError('devices is empty')
         stage = self._perspective_stage(perspective, out, out_dtype, n)
+        if bg_frames is not None:
+            bg_frames = self._bg_frames(frames, bg_frames, bgImages)
         if devices is not None and len(devices) > 1:
             return self._correct_batch_multi(frames, devices, bgImages, exposure_time, light_spectrum, threshold,
-                                             keep_size, date, out, out_dtype, verbose, stage, out_scale)
+                                             keep_size, date, out, out_dtype, verbose, stage, out_scale, bg_frames)
         dev_index = frames.device.index if is_tensor else (devices[0] if devices else None)
         eng = _engine.get_engine(H, W, dev_index)
         sink = contextlib.nullcontext() if verbose else contextlib.redirect_stdout(io.StringIO())
         with sink:
-            flags = self._configure_engine(eng, (H, W), bgImages, exposure_time, light_spectrum, date)
+            flags = self._configure_engine(eng, (H, W), bgImages, exposure_time, light_spectrum, date,
+                                           use_dark=bg_frames is None)
             lens = None
             try:
                 lens = self.getLens(light_spectrum, date['lens'])
@@ -624,16 +645,47 @@ if shapes are transposed, execute self.transpose() once """ % (s, array.shape))
         window = tuple(int(v) for v in lens.roi) if (lens and not keep_size) else None
         thr = threshold if threshold > 0 else 0.0
         if is_tensor:
+            if bg_frames is not None:
+                bg_frames = self._bg_dtype(bg_frames, frames.dtype)
             return eng.correct_batch(frames, threshold=thr, ksize=3, flags=flags, use_lens=bool(lens), window=window,
-                                     out_dtype=out_dtype or tt.float32, out=out, out_scale=out_scale)
+                                     out_dtype=out_dtype or tt.float32, out=out, out_scale=out_scale, bg=bg_frames)
         be = frames.dtype.kind == 'u' and frames.dtype.itemsize == 2 and frames.dtype.byteorder == '>'
         if not be and (frames.dtype.type not in (np.uint8, np.uint16, np.float32) or not frames.dtype.isnative):
             frames = frames.astype(np.float32)
+        if bg_frames is not None:
+            bg_frames = self._bg_dtype(bg_frames, frames.dtype.newbyteorder('='))
         return eng.correct_host(frames, out=out, threshold=thr, ksize=3, flags=flags, use_lens=bool(lens),
-                                window=window, out_dtype=out_dtype or np.float32, out_scale=out_scale)
+                                window=window, out_dtype=out_dtype or np.float32, out_scale=out_scale, bg=bg_frames)
+
+    @staticmethod
+    def _bg_frames(frames, bg_frames, bgImages):
+        """the refusals of correct_batch(bg_frames=...), before any engine is created"""
+        tt = _engine.torch()
+        if bgImages is not None:
+            raise ValueError('bg_frames and bgImages exclude each other: bg_frames gives every frame its own background')
+        if isinstance(frames, tt.Tensor) != isinstance(bg_frames, tt.Tensor):
+            raise ValueError('bg_frames must be a CUDA tensor for tensor frames and a numpy array for host frames')
+        if not isinstance(bg_frames, tt.Tensor):
+            bg_frames = np.asarray(bg_frames)
+        elif not bg_frames.is_cuda or bg_frames.device != frames.device:
+            raise ValueError('bg_frames on %s, frames on %s' % (bg_frames.device, frames.device))
+        if tuple(bg_frames.shape) != tuple(frames.shape):
+            raise ValueError('bg_frames of shape %s for frames of shape %s' % (tuple(bg_frames.shape), tuple(frames.shape)))
+        return bg_frames
+
+    @staticmethod
+    def _bg_dtype(bg, frame_dtype):
+        """backgrounds of the frames' dtype or float32 as they are (native byte order); anything else rounded to float32"""
+        tt = _engine.torch()
+        if isinstance(bg, tt.Tensor):
+            return bg if bg.dtype in (frame_dtype, tt.float32) else bg.to(tt.float32)
+        dt = bg.dtype.newbyteorder('=')
+        if dt in (np.dtype(frame_dtype), np.dtype(np.float32)):
+            return bg.astype(dt, copy=False)
+        return bg.astype(np.float32)
 
     def _correct_batch_multi(self, frames, devices, bgImages, exposure_time, light_spectrum, threshold, keep_size, date,
-                             out, out_dtype, verbose, stage, out_scale=None):
+                             out, out_dtype, verbose, stage, out_scale=None, bg_frames=None):
         """host frames [n,H,W] split over several devices of this process: one engine + one host thread per device"""
         import contextlib
         import io
@@ -643,6 +695,8 @@ if shapes are transposed, execute self.transpose() once """ % (s, array.shape))
         be = frames.dtype.kind == 'u' and frames.dtype.itemsize == 2 and frames.dtype.byteorder == '>'
         if not be and (frames.dtype.type not in (np.uint8, np.uint16, np.float32) or not frames.dtype.isnative):
             frames = frames.astype(np.float32)
+        if bg_frames is not None:
+            bg_frames = self._bg_dtype(bg_frames, frames.dtype.newbyteorder('='))
         engines, own = [], []
         sink = contextlib.nullcontext() if verbose else contextlib.redirect_stdout(io.StringIO())
         lens = None
@@ -658,7 +712,8 @@ if shapes are transposed, execute self.transpose() once """ % (s, array.shape))
                 flags = 0
                 for i, e in enumerate(engines):               # calibration goes to every device once
                     with contextlib.nullcontext() if (verbose and i == 0) else contextlib.redirect_stdout(io.StringIO()):
-                        flags = self._configure_engine(e, (H, W), bgImages, exposure_time, light_spectrum, date)
+                        flags = self._configure_engine(e, (H, W), bgImages, exposure_time, light_spectrum, date,
+                                                       use_dark=bg_frames is None)
                 try:
                     lens = self.getLens(light_spectrum, date['lens'])
                     if lens:
@@ -698,7 +753,8 @@ if shapes are transposed, execute self.transpose() once """ % (s, array.shape))
                     return
                 try:
                     engines[i].correct_host(frames[lo:hi], out=out[lo:hi], threshold=thr, ksize=3, flags=flags,
-                                            use_lens=bool(lens), window=window, out_dtype=out.dtype, out_scale=out_scale)
+                                            use_lens=bool(lens), window=window, out_dtype=out.dtype, out_scale=out_scale,
+                                            bg=None if bg_frames is None else bg_frames[lo:hi])
                 except BaseException as e:                    # noqa: BLE001 - re-raised in the caller's thread
                     errors[i] = e
 

@@ -105,6 +105,8 @@ struct SharedScratch {
 struct HostSlot {
     DevPtr<void> d_raw, d_out;
     PinnedPtr h_raw, h_out;
+    DevPtr<void> d_bg;                        // per-frame backgrounds of the slot's chunk (imgcorr_correct_host_bg only)
+    PinnedPtr h_bg;                           // their staging for pageable input
     Event ev_in, ev_k, ev_out;
 };
 
@@ -155,7 +157,7 @@ struct imgcorr_ctx {
     // host pipeline
     Stream s_in, s_k, s_out;
     std::vector<HostSlot> slots;
-    size_t slot_raw_bytes = 0, slot_out_bytes = 0;
+    size_t slot_raw_bytes = 0, slot_out_bytes = 0, slot_bg_bytes = 0;
 };
 
 // The end of every launch: count the kernels the launch helper issued and map its error to a status.  K1, K2 and K3 name
@@ -437,8 +439,9 @@ extern "C" IMGCORR_API int imgcorr_set_lens(imgcorr_ctx* c, const double K[9], c
     return IMGCORR_OK;
 }
 
+// bg: per-frame backgrounds [n][H][W] of bg_dtype in place of the dark map (checked by check_bg), or null
 static int fill_k1(imgcorr_ctx* c, K1Args& a, const void* raw, int raw_dtype, void* out, uint8_t* mask, int n, double thr,
-                   int ksize, int cond, int flags) {
+                   int ksize, int cond, int flags, const void* bg = nullptr, int bg_dtype = DT_F32) {
     if (!raw || !out) return fail(IMGCORR_ERR_INVALID, "null image pointer");
     if (n < 0) return fail(IMGCORR_ERR_INVALID, "n_frames %d", n);
     if (!(thr > 0.0)) ksize = 0;                      // also NaN
@@ -454,7 +457,9 @@ static int fill_k1(imgcorr_ctx* c, K1Args& a, const void* raw, int raw_dtype, vo
         return fail(IMGCORR_ERR_INVALID, "big-endian ingest is implemented for uint16 frames");
     if (c->raw_gap % (long long)dtype_size(raw_dtype)) return fail(IMGCORR_ERR_INVALID, "frame gap must be a multiple of the sample size");
     int f = 0;
-    if ((flags & IMGCORR_DO_DARK) && c->dark) {
+    if (bg) {
+        f |= FLAG_DARK; a.bg = bg; a.bg_dtype = bg_dtype;
+    } else if ((flags & IMGCORR_DO_DARK) && c->dark) {
         f |= FLAG_DARK; a.dark = c->dark.get();
         if (c->ascent) { f |= FLAG_DARK_LINEAR; a.ascent = c->ascent.get(); }
     }
@@ -465,9 +470,10 @@ static int fill_k1(imgcorr_ctx* c, K1Args& a, const void* raw, int raw_dtype, vo
     a.flat_nz = a.flat ? c->flat_nz.get() : nullptr;
     if (!c->dump) CK(dev_alloc(c->dump, (size_t)4 << 20));
     a.dump = c->dump.get();
-    // integer frames: |raw - dark| <= raw_max + max|dark|; divided by min|flat| it must stay below FLT_MAX
+    // integer frames: |raw - dark| <= raw_max + max|dark|; divided by min|flat| it must stay below FLT_MAX.  Backgrounds of
+    // the raw integer dtype: |raw - bg| <= raw_max.  Float32 backgrounds are not checked at upload: no proof
     a.no_overflow = 0;
-    if (a.maps_finite && (raw_dtype == DT_U8 || raw_dtype == DT_U16)) {
+    if (a.maps_finite && (raw_dtype == DT_U8 || raw_dtype == DT_U16) && (!bg || bg_dtype == raw_dtype)) {
         const double num = (raw_dtype == DT_U8 ? 255.0 : 65535.0) + (a.dark ? c->dark_absmax : 0.0);
         const double den = a.flat ? c->flat_absmin : 1.0;
         a.no_overflow = (num / den < 3.0e38) ? 1 : 0;
@@ -836,9 +842,10 @@ static int check_perspective(const imgcorr_ctx* c, int out_dtype, int ow, int oh
 // later), which picks the matrices of a per-frame perspective table.
 // Integer output (U16 / U8) is the float32 chain with the quantiser fused into the last kernel's store: K1 without a lens or
 // perspective stage, K2 with a lens, K3 with the stage (which warps the float32 chain frame).
+// `bg`: the call's per-frame backgrounds from raw's first frame on (dense, bg_dtype; checked by check_bg), or null.
 static int chain_frames(imgcorr_ctx* c, const void* raw, int raw_dtype, void* out, int out_dtype, int n, double thr,
                         int ksize, int flags, bool lens, bool persp, double border, int x0, int y0, int ow, int oh,
-                        cudaStream_t st, int first) {
+                        cudaStream_t st, int first, const void* bg, int bg_dtype) {
     if (out_dtype < DT_U8 || out_dtype > DT_F64) return fail(IMGCORR_ERR_INVALID, "out_dtype must be U8, U16, F32 or F64");
     const bool quant = out_dtype == DT_U8 || out_dtype == DT_U16;
     const int frame_dtype = quant ? DT_F32 : out_dtype;    // the chain frame: what K2 (or K1) returns before the stage
@@ -849,7 +856,7 @@ static int chain_frames(imgcorr_ctx* c, const void* raw, int raw_dtype, void* ou
         return fail(IMGCORR_ERR_INVALID, "output window without a lens");
     if (!lens && !persp) {                             // K1 alone: one launch for the whole batch, no scratch
         K1Args a;
-        int r = fill_k1(c, a, raw, raw_dtype, out, nullptr, n, thr, ksize, IMGCORR_COND_GT, flags);
+        int r = fill_k1(c, a, raw, raw_dtype, out, nullptr, n, thr, ksize, IMGCORR_COND_GT, flags, bg, bg_dtype);
         if (r) return r;
         if (quant) a.q = c->out_scale;
         int l = 0;
@@ -913,7 +920,7 @@ static int chain_frames(imgcorr_ctx* c, const void* raw, int raw_dtype, void* ou
         }
         K1Args a;
         int r = fill_k1(c, a, (const char*)raw + f * raw_stride, raw_dtype, lens ? (void*)mid : frames, nullptr, nf, thr, ksize,
-                        IMGCORR_COND_GT, flags);
+                        IMGCORR_COND_GT, flags, bg ? (const char*)bg + f * npx * dtype_size(bg_dtype) : nullptr, bg_dtype);
         if (r) return r;
         int l = 0;
         if (prof) prof_mark(c, 0, s1);
@@ -945,17 +952,43 @@ static int chain_frames(imgcorr_ctx* c, const void* raw, int raw_dtype, void* ou
     return IMGCORR_OK;
 }
 
-extern "C" IMGCORR_API int imgcorr_correct_batch(imgcorr_ctx* c, const void* raw_dev, int raw_dtype, void* out_dev, int out_dtype,
-                                     int n_frames, double threshold, int ksize, int flags, int use_lens,
-                                     double border_value, int x0, int y0, int ow, int oh, void* stream) {
-    GUARD(c);
+// the refusals of a chain call with per-frame backgrounds, before anything is enqueued
+static int check_bg(int raw_dtype, const void* bg, int bg_dtype, int flags) {
+    if (!bg) return IMGCORR_OK;
+    if (!(flags & IMGCORR_DO_DARK)) return fail(IMGCORR_ERR_INVALID, "per-frame backgrounds need IMGCORR_DO_DARK");
+    if (raw_dtype < DT_U8 || raw_dtype > DT_F32) return fail(IMGCORR_ERR_INVALID, "raw_dtype %d (U8, U16 or F32)", raw_dtype);
+    if (bg_dtype != raw_dtype && bg_dtype != DT_F32)
+        return fail(IMGCORR_ERR_INVALID, "bg_dtype %d: the raw dtype (%d) or F32", bg_dtype, raw_dtype);
+    return IMGCORR_OK;
+}
+
+static int correct_batch(imgcorr_ctx* c, const void* raw_dev, int raw_dtype, const void* bg_dev, int bg_dtype, void* out_dev,
+                         int out_dtype, int n_frames, double threshold, int ksize, int flags, int use_lens,
+                         double border_value, int x0, int y0, int ow, int oh, void* stream) {
     if (!raw_dev || !out_dev) return fail(IMGCORR_ERR_INVALID, "null image pointer");
+    if (int r = check_bg(raw_dtype, bg_dev, bg_dtype, flags)) return r;
     const bool lens = use_lens && c->has_lens;
     if (!lens) { x0 = 0; y0 = 0; ow = c->W; oh = c->H; }
     const bool persp = flags & IMGCORR_DO_PERSPECTIVE;
     if (persp) { int r = check_perspective(c, out_dtype, ow, oh, n_frames); if (r) return r; }
     return chain_frames(c, raw_dev, raw_dtype, out_dev, out_dtype, n_frames, threshold, ksize, flags, lens, persp,
-                        border_value, x0, y0, ow, oh, (cudaStream_t)stream, 0);
+                        border_value, x0, y0, ow, oh, (cudaStream_t)stream, 0, bg_dev, bg_dtype);
+}
+
+extern "C" IMGCORR_API int imgcorr_correct_batch(imgcorr_ctx* c, const void* raw_dev, int raw_dtype, void* out_dev, int out_dtype,
+                                     int n_frames, double threshold, int ksize, int flags, int use_lens,
+                                     double border_value, int x0, int y0, int ow, int oh, void* stream) {
+    GUARD(c);
+    return correct_batch(c, raw_dev, raw_dtype, nullptr, DT_F32, out_dev, out_dtype, n_frames, threshold, ksize, flags, use_lens,
+                         border_value, x0, y0, ow, oh, stream);
+}
+
+extern "C" IMGCORR_API int imgcorr_correct_batch_bg(imgcorr_ctx* c, const void* raw_dev, int raw_dtype, const void* bg_dev, int bg_dtype,
+                                        void* out_dev, int out_dtype, int n_frames, double threshold, int ksize, int flags,
+                                        int use_lens, double border_value, int x0, int y0, int ow, int oh, void* stream) {
+    GUARD(c);
+    return correct_batch(c, raw_dev, raw_dtype, bg_dev, bg_dtype, out_dev, out_dtype, n_frames, threshold, ksize, flags, use_lens,
+                         border_value, x0, y0, ow, oh, stream);
 }
 
 // ---- host-buffer pipeline ---------------------------------------------------------------------
@@ -965,7 +998,8 @@ static bool is_pinned(const void* p) {
     return at.type == cudaMemoryTypeHost;
 }
 
-static int ensure_pipeline(imgcorr_ctx* c, size_t raw_bytes, size_t out_bytes) {
+// bg_bytes: the per-slot background buffer of a call with backgrounds (0: none needed, none allocated)
+static int ensure_pipeline(imgcorr_ctx* c, size_t raw_bytes, size_t out_bytes, size_t bg_bytes) {
     if (!c->s_in) {
         Stream in, k, out;
         CK(new_stream(in));
@@ -975,14 +1009,25 @@ static int ensure_pipeline(imgcorr_ctx* c, size_t raw_bytes, size_t out_bytes) {
         c->s_k = std::move(k);
         c->s_out = std::move(out);
     }
-    if ((int)c->slots.size() == c->host_slots && c->slot_raw_bytes >= raw_bytes && c->slot_out_bytes >= out_bytes)
+    if ((int)c->slots.size() == c->host_slots && c->slot_raw_bytes >= raw_bytes && c->slot_out_bytes >= out_bytes) {
+        if (c->slot_bg_bytes >= bg_bytes) return IMGCORR_OK;
+        // the ring stays; its slots get (larger) background buffers.  Every earlier host call has drained the ring.
+        for (auto& s : c->slots) {
+            s.d_bg.reset();
+            s.h_bg.reset();
+        }
+        c->slot_bg_bytes = 0;
+        for (auto& s : c->slots) CK(dev_alloc(s.d_bg, bg_bytes));
+        c->slot_bg_bytes = bg_bytes;
         return IMGCORR_OK;
+    }
     CK(cudaDeviceSynchronize());
     c->slots.clear();                                  // the old ring goes first, so peak memory stays one ring
     std::vector<HostSlot> ring(c->host_slots);
     for (auto& s : ring) {
         CK(dev_alloc(s.d_raw, raw_bytes));
         CK(dev_alloc(s.d_out, out_bytes));
+        if (bg_bytes) CK(dev_alloc(s.d_bg, bg_bytes));
         CK(new_event(s.ev_in));
         CK(new_event(s.ev_k));
         CK(new_event(s.ev_out));
@@ -990,14 +1035,15 @@ static int ensure_pipeline(imgcorr_ctx* c, size_t raw_bytes, size_t out_bytes) {
     c->slots = std::move(ring);
     c->slot_raw_bytes = raw_bytes;
     c->slot_out_bytes = out_bytes;
+    c->slot_bg_bytes = bg_bytes;
     return IMGCORR_OK;
 }
 
-extern "C" IMGCORR_API int imgcorr_correct_host(imgcorr_ctx* c, const void* raw_host, int raw_dtype, void* out_host, int out_dtype,
-                                    int n_frames, double threshold, int ksize, int flags, int use_lens,
-                                    double border_value, int x0, int y0, int ow, int oh) {
-    GUARD(c);
+static int correct_host(imgcorr_ctx* c, const void* raw_host, int raw_dtype, const void* bg_host, int bg_dtype, void* out_host,
+                        int out_dtype, int n_frames, double threshold, int ksize, int flags, int use_lens,
+                        double border_value, int x0, int y0, int ow, int oh) {
     if (!raw_host || !out_host) return fail(IMGCORR_ERR_INVALID, "null image pointer");
+    if (int r = check_bg(raw_dtype, bg_host, bg_dtype, flags)) return r;
     if (n_frames < 0) return fail(IMGCORR_ERR_INVALID, "n_frames %d", n_frames);
     if (raw_dtype < DT_U8 || raw_dtype > DT_F32) return fail(IMGCORR_ERR_INVALID, "raw_dtype %d (U8, U16 or F32)", raw_dtype);
     if (c->raw_gap) return fail(IMGCORR_ERR_INVALID, "IMGCORR_OPT_RAW_FRAME_GAP is not available for host frames (pass the pixel blocks)");
@@ -1007,20 +1053,24 @@ extern "C" IMGCORR_API int imgcorr_correct_host(imgcorr_ctx* c, const void* raw_
     const bool persp = flags & IMGCORR_DO_PERSPECTIVE;
     if (persp) { int r = check_perspective(c, out_dtype, ow, oh, n_frames); if (r) return r; }
     const size_t frame_raw = (size_t)c->H * c->W * dtype_size(raw_dtype);
+    const size_t frame_bg = bg_host ? (size_t)c->H * c->W * dtype_size(bg_dtype) : 0;
     const size_t frame_out = (persp ? (size_t)c->persp.dw * c->persp.dh : (size_t)ow * oh) * dtype_size(out_dtype);
-    // small frames travel in chunks of G frames per ring slot (up to 32 MB of raw data, at most 16 frames): one copy each
-    // way and one K1 / K2 launch per chunk instead of per frame; frames above 16 MB (the 4096x3000 workload) keep one
-    // frame per slot
+    // small frames travel in chunks of G frames per ring slot (up to 32 MB of raw data and backgrounds, at most 16 frames):
+    // one copy each way and one K1 / K2 launch per chunk instead of per frame; frames above 16 MB (the 4096x3000 workload)
+    // keep one frame per slot
+    const size_t frame_in = frame_raw + frame_bg;
     int G = 1;
-    if (frame_raw <= ((size_t)16 << 20)) G = (int)std::min<size_t>(16, ((size_t)32 << 20) / frame_raw);
+    if (frame_in <= ((size_t)16 << 20)) G = (int)std::min<size_t>(16, ((size_t)32 << 20) / frame_in);
     if (G > n_frames) G = n_frames > 0 ? n_frames : 1;
-    const size_t raw_bytes = frame_raw * G, out_bytes = frame_out * G;
-    int r = ensure_pipeline(c, raw_bytes, out_bytes);
+    const size_t raw_bytes = frame_raw * G, out_bytes = frame_out * G, bg_bytes = frame_bg * G;
+    int r = ensure_pipeline(c, raw_bytes, out_bytes, bg_bytes);
     if (r) return r;
     const bool in_pinned = is_pinned(raw_host), out_pinned = is_pinned(out_host);
+    const bool bg_pinned = bg_host && is_pinned(bg_host);
     for (auto& s : c->slots) {
         if (!in_pinned && !s.h_raw) CK(host_alloc(s.h_raw, c->slot_raw_bytes));
         if (!out_pinned && !s.h_out) CK(host_alloc(s.h_out, c->slot_out_bytes));
+        if (bg_host && !bg_pinned && !s.h_bg) CK(host_alloc(s.h_bg, c->slot_bg_bytes));
     }
     const int ns = (int)c->slots.size();
     const int chunks = (n_frames + G - 1) / G;
@@ -1044,10 +1094,15 @@ extern "C" IMGCORR_API int imgcorr_correct_host(imgcorr_ctx* c, const void* raw_
         const char* src = (const char*)raw_host + (size_t)k * raw_bytes;
         if (!in_pinned) { memcpy(s.h_raw.get(), src, frame_raw * nf); src = (const char*)s.h_raw.get(); }
         CK(cudaMemcpyAsync(s.d_raw.get(), src, frame_raw * nf, cudaMemcpyHostToDevice, s_in));
+        if (bg_host) {
+            const char* bsrc = (const char*)bg_host + (size_t)k * bg_bytes;
+            if (!bg_pinned) { memcpy(s.h_bg.get(), bsrc, frame_bg * nf); bsrc = (const char*)s.h_bg.get(); }
+            CK(cudaMemcpyAsync(s.d_bg.get(), bsrc, frame_bg * nf, cudaMemcpyHostToDevice, s_in));
+        }
         CK(cudaEventRecord(s.ev_in.get(), s_in));
         CK(cudaStreamWaitEvent(s_k, s.ev_in.get(), 0));
         r = chain_frames(c, s.d_raw.get(), raw_dtype, s.d_out.get(), out_dtype, nf, threshold, ksize, flags, lens, persp,
-                         border_value, x0, y0, ow, oh, s_k, k * G);
+                         border_value, x0, y0, ow, oh, s_k, k * G, bg_host ? s.d_bg.get() : nullptr, bg_dtype);
         if (r) return r;
         CK(cudaEventRecord(s.ev_k.get(), s_k));
         CK(cudaStreamWaitEvent(s_out, s.ev_k.get(), 0));
@@ -1058,6 +1113,22 @@ extern "C" IMGCORR_API int imgcorr_correct_host(imgcorr_ctx* c, const void* raw_
     for (int k = (chunks > ns ? chunks - ns : 0); k < chunks; ++k) { r = retire(k); if (r) return r; }
     drain.armed = false;                               // every chunk was retired: nothing is in flight
     return IMGCORR_OK;
+}
+
+extern "C" IMGCORR_API int imgcorr_correct_host(imgcorr_ctx* c, const void* raw_host, int raw_dtype, void* out_host, int out_dtype,
+                                    int n_frames, double threshold, int ksize, int flags, int use_lens,
+                                    double border_value, int x0, int y0, int ow, int oh) {
+    GUARD(c);
+    return correct_host(c, raw_host, raw_dtype, nullptr, DT_F32, out_host, out_dtype, n_frames, threshold, ksize, flags, use_lens,
+                        border_value, x0, y0, ow, oh);
+}
+
+extern "C" IMGCORR_API int imgcorr_correct_host_bg(imgcorr_ctx* c, const void* raw_host, int raw_dtype, const void* bg_host, int bg_dtype,
+                                       void* out_host, int out_dtype, int n_frames, double threshold, int ksize, int flags,
+                                       int use_lens, double border_value, int x0, int y0, int ow, int oh) {
+    GUARD(c);
+    return correct_host(c, raw_host, raw_dtype, bg_host, bg_dtype, out_host, out_dtype, n_frames, threshold, ksize, flags, use_lens,
+                        border_value, x0, y0, ow, oh);
 }
 
 extern "C" IMGCORR_API int imgcorr_selftest_division(imgcorr_ctx* c, int numerators_per_divisor, unsigned long long seed, double out[2]) {

@@ -33,6 +33,9 @@ struct K1Args {
     PointwiseConst pw;
     PredicateConst pred;
     OutScale q;             // integer output (U16 / U8): quantise<OutT>(float32 result, q); the identity (0, 1) outside the chain
+    const void* bg;         // [n_frames][H][W] of bg_dtype, dense and native-endian, or null: frame f subtracts float32(bg[f])
+                            // in place of the dark map (FLAG_DARK set, dark / ascent null)
+    int bg_dtype;           // the raw dtype or DT_F32
 };
 
 // variant: 0 = pick automatically, 1 = generic tiles (plain coalesced loads), 2 = TMA-staged tiles,

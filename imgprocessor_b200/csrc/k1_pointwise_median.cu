@@ -72,8 +72,17 @@ template <typename RawT> __device__ __forceinline__ const RawT* raw_frame(const 
 // ------------------------------------------------------------------------------------------
 // pointwise only (ksize == 0): pure streaming kernel; frames in grid.y, no per-pixel modulo
 // ------------------------------------------------------------------------------------------
-template <typename RawT, typename OutT>
-__global__ void __launch_bounds__(256) k1_pointwise_kernel(K1Args a) {
+// per-frame background (K1Args::bg): sample i of the dense [n][H][W] block as the float32 dark value of its pixel.  The
+// dtype is read at run time: the generic kernels are the fall-back of every allowed pair, and one instantiation serves
+// all of them
+__device__ __forceinline__ float bg_sample(const K1Args& a, size_t i) {
+    if (a.bg_dtype == DT_U8) return (float)__ldg((const uint8_t*)a.bg + i);
+    if (a.bg_dtype == DT_U16) return (float)__ldg((const uint16_t*)a.bg + i);
+    return __ldg((const float*)a.bg + i);
+}
+
+template <typename RawT, typename OutT, bool BG>
+__device__ __forceinline__ void k1_pointwise_body(const K1Args& a) {
     using CT = typename RawIO<RawT>::CT;
     const size_t npx = (size_t)a.H * a.W;
     const RawT* raw = raw_frame<RawT>(a, blockIdx.y);
@@ -81,12 +90,16 @@ __global__ void __launch_bounds__(256) k1_pointwise_kernel(K1Args a) {
     const PointwiseConst pw = a.pw;
     const int swap = a.raw_swap;
     for (size_t p = (size_t)blockIdx.x * blockDim.x + threadIdx.x; p < npx; p += (size_t)gridDim.x * blockDim.x) {
-        float d = a.dark ? __ldg(a.dark + p) : 0.0f;
+        float d = BG ? bg_sample(a, (size_t)blockIdx.y * npx + p) : (a.dark ? __ldg(a.dark + p) : 0.0f);
         float s = a.ascent ? __ldg(a.ascent + p) : 0.0f;
         float f = a.flat ? __ldg(a.flat + p) : 0.0f;
         out[p] = to_out<OutT, CT>(a, pointwise<CT>(pw, RawIO<RawT>::ld(raw_fix<RawT>(__ldg(raw + p), swap)), d, s, f));
     }
 }
+template <typename RawT, typename OutT>
+__global__ void __launch_bounds__(256) k1_pointwise_kernel(K1Args a) { k1_pointwise_body<RawT, OutT, false>(a); }
+template <typename RawT, typename OutT>
+__global__ void __launch_bounds__(256) k1_pointwise_bg_kernel(K1Args a) { k1_pointwise_body<RawT, OutT, true>(a); }
 
 // ------------------------------------------------------------------------------------------
 // phase B: median-threshold of one tile from the shared pointwise tile xs[TH+2h][K1_BOXW]
@@ -197,8 +210,8 @@ __device__ __forceinline__ void median_phase(const CT* __restrict__ xs, const K1
 // ------------------------------------------------------------------------------------------
 // generic variant: one tile per CTA, reflect indexing on global loads
 // ------------------------------------------------------------------------------------------
-template <typename RawT, typename OutT, int KS, int TH, bool VEC>
-__global__ void __launch_bounds__(K1_THREADS) k1_generic_kernel(K1Args a, int tiles_x, int tiles_y) {
+template <typename RawT, typename OutT, int KS, int TH, bool VEC, bool BG>
+__device__ __forceinline__ void k1_generic_body(const K1Args& a, int tiles_x, int tiles_y) {
     using CT = typename RawIO<RawT>::CT;
     constexpr int HALO = KS / 2;
     constexpr int LH = TH + 2 * HALO;
@@ -220,7 +233,7 @@ __global__ void __launch_bounds__(K1_THREADS) k1_generic_kernel(K1Args a, int ti
         CT* xrow = xs + ly * K1_BOXW + (K1_XOFF - HALO);
         for (int lx = lane; lx < LW; lx += 32) {
             const size_t g = grow + reflect_index(tx0 - HALO + lx, a.W);
-            float d = a.dark ? __ldg(a.dark + g) : 0.0f;
+            float d = BG ? bg_sample(a, (size_t)frame * a.H * a.W + g) : (a.dark ? __ldg(a.dark + g) : 0.0f);
             float s = a.ascent ? __ldg(a.ascent + g) : 0.0f;
             float f = a.flat ? __ldg(a.flat + g) : 0.0f;
             xrow[lx] = pointwise<CT>(pw, RawIO<RawT>::ld(raw_fix<RawT>(__ldg(raw + g), swap)), d, s, f);
@@ -229,6 +242,16 @@ __global__ void __launch_bounds__(K1_THREADS) k1_generic_kernel(K1Args a, int ti
     __syncthreads();
     const PredicateConst pred = a.pred;
     median_phase<CT, OutT, KS, TH, VEC>(xs, a, pred, frame, tx0, ty0);
+}
+
+template <typename RawT, typename OutT, int KS, int TH, bool VEC>
+__global__ void __launch_bounds__(K1_THREADS) k1_generic_kernel(K1Args a, int tiles_x, int tiles_y) {
+    k1_generic_body<RawT, OutT, KS, TH, VEC, false>(a, tiles_x, tiles_y);
+}
+// per-frame backgrounds: scalar stores only (any alignment), one instantiation per dtype pair and window size
+template <typename RawT, typename OutT, int KS, int TH>
+__global__ void __launch_bounds__(K1_THREADS) k1_generic_bg_kernel(K1Args a, int tiles_x, int tiles_y) {
+    k1_generic_body<RawT, OutT, KS, TH, false, true>(a, tiles_x, tiles_y);
 }
 
 // ------------------------------------------------------------------------------------------
@@ -377,6 +400,7 @@ bool k1_tma_eligible(const K1Args& a, int raw_dtype, int out_dtype) {
     if (a.ksize == 5 && out_dtype != DT_F32 && dtype_size(out_dtype) != dtype_size(raw_dtype)) return false;
     if (a.pw.flags & FLAG_DARK_LINEAR) return false;
     if (a.raw_swap || a.raw_gap) return false;
+    if (a.bg) return false;                              // per-frame backgrounds: the streaming pipeline or the generic tiles
     const size_t esz = dtype_size(raw_dtype);
     if (((size_t)a.W * esz) % 16 || ((size_t)a.W * 4) % 16) return false;
     if (((size_t)a.H * a.W * esz) % 16) return false;
@@ -414,6 +438,12 @@ template <typename RawT, typename OutT, int KS, int TH>
 static cudaError_t launch_generic_t(const K1Args& a, cudaStream_t st) {
     const int tiles_x = (a.W + K1_TW - 1) / K1_TW, tiles_y = (a.H + TH - 1) / TH;
     const long long total = (long long)tiles_x * tiles_y * a.n_frames;
+    if constexpr (sizeof(RawT) <= 4) {
+        if (a.bg) {
+            k1_generic_bg_kernel<RawT, OutT, KS, TH><<<(unsigned)total, K1_THREADS, 0, st>>>(a, tiles_x, tiles_y);
+            return cudaGetLastError();
+        }
+    }
     const bool vec = (a.W % 2 == 0) && ((uintptr_t)a.out % (2 * sizeof(OutT)) == 0) && (!a.mask || (uintptr_t)a.mask % 2 == 0);
     if (vec) k1_generic_kernel<RawT, OutT, KS, TH, true><<<(unsigned)total, K1_THREADS, 0, st>>>(a, tiles_x, tiles_y);
     else k1_generic_kernel<RawT, OutT, KS, TH, false><<<(unsigned)total, K1_THREADS, 0, st>>>(a, tiles_x, tiles_y);
@@ -431,6 +461,13 @@ static cudaError_t launch_pointwise_t(const K1Args& a, int sm_count, cudaStream_
         const int nf = a.n_frames - f0 < 65535 ? a.n_frames - f0 : 65535;
         b.raw = (const char*)a.raw + (size_t)f0 * (npx * sizeof(RawT) + (size_t)a.raw_gap);
         b.out = (char*)a.out + (size_t)f0 * npx * sizeof(OutT);
+        if constexpr (sizeof(RawT) <= 4) {
+            if (a.bg) {
+                b.bg = (const char*)a.bg + (size_t)f0 * npx * dtype_size(a.bg_dtype);
+                k1_pointwise_bg_kernel<RawT, OutT><<<dim3((unsigned)bx, (unsigned)nf), 256, 0, st>>>(b);
+                continue;
+            }
+        }
         k1_pointwise_kernel<RawT, OutT><<<dim3((unsigned)bx, (unsigned)nf), 256, 0, st>>>(b);
     }
     return cudaGetLastError();

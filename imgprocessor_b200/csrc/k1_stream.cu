@@ -19,6 +19,7 @@
 //   * vertical 'reflect' needs no halo rows: the first / last row's sorted triple is used twice.
 //
 // Same arithmetic as the tile kernels (imgcorr_core.cuh) — results are bit-identical.
+#include <type_traits>
 #include "imgcorr_kernels.cuh"
 #include "imgcorr_tma.cuh"
 
@@ -62,18 +63,29 @@ typedef KsShape<KS_WIDE_R, KS_WIDE_NSTAGE, KS_WIDE_MINB, 1> KsWide;
 #define KS_PAIR_MINB 3
 #endif
 typedef KsShape<KS_PAIR_R, KS_PAIR_NSTAGE, KS_PAIR_MINB, 2> KsPair;
+// frame pairs with per-frame backgrounds: a background box per frame replaces the dark box.  Three stages of the pair
+// shape would need 25.6 KB (uint16) / 40 KB (float32) each, just above what 3 (uint16) / 2 (float32) CTAs per SM can
+// hold, so these shapes keep two stages.  Float32 frames fit 2 CTAs per SM (80 KB each) and get their registers:
+// with the cap of 3 CTAs the checked arithmetic spills
+#ifndef KS_PAIRBG_R
+#define KS_PAIRBG_R 16
+#define KS_PAIRBG_NSTAGE 2
+#endif
+typedef KsShape<KS_PAIRBG_R, KS_PAIRBG_NSTAGE, 3, 2> KsPairBg;         // uint16 frames, finite flat field
+typedef KsShape<KS_PAIRBG_R, KS_PAIRBG_NSTAGE, 2, 2> KsPairBgF32;      // float32 frames
 constexpr int KS_MAPW = 128;                // float32 box: tx0-4 .. tx0+123
 constexpr int KS_MAPX = 4;
 constexpr int KS_THREADS = (KS_CW + 1) * 32;
 
-template <typename RawT, typename C> struct StreamBox {
+template <typename RawT, typename C, bool BG = false> struct StreamBox {
     static constexpr int XOFF = 16 / (int)sizeof(RawT);                        // u8 16, u16 8, f32 4
     static constexpr int GRAN = 16 / (int)sizeof(RawT);
     // the box starts at the 16-byte boundary at or left of tx0, minus XOFF: columns tx0-1 .. tx0+120 are inside
     static constexpr int BOXW = ((KS_TW + 2 * XOFF + GRAN - 1) / GRAN) * GRAN;  // u8 160, u16 136, f32 128
     static constexpr size_t raw_bytes = (size_t)C::R * BOXW * sizeof(RawT);     // multiples of 128
     static constexpr size_t map_bytes = (size_t)C::R * KS_MAPW * sizeof(float);
-    static constexpr size_t stage_bytes = C::NF * raw_bytes + 2 * map_bytes;    // raw[NF] | dark | flat
+    static constexpr size_t dark_bytes = BG ? C::NF * raw_bytes : map_bytes;     // the dark box, or a background box per frame
+    static constexpr size_t stage_bytes = C::NF * raw_bytes + dark_bytes + map_bytes;    // raw[NF] | dark or bg[NF] | flat
     static_assert(raw_bytes % 128 == 0 && map_bytes % 128 == 0, "TMA destinations must be 128-byte aligned: rows per stage must be a multiple of 8");
     static constexpr size_t bar_off = C::NSTAGE * stage_bytes;
     static constexpr size_t total = bar_off + 2 * C::NSTAGE * sizeof(uint64_t) + 64;
@@ -134,7 +146,11 @@ __device__ __forceinline__ UnitGeom ks_unit(int unit, int strips, int seg_rows, 
 
 // CFG >= 0 bakes the per-launch switches into the instruction stream (the kernel is issue bound: every
 // per-row flag test costs); CFG < 0 reads them from the arguments.
-enum : int { KS_DARK = 1, KS_FLAT = 2, KS_N2N = 4, KS_MASK = 8, KS_CHECK = 16, KS_LT = 32, KS_NZ = 64, KS_SWAP = 128, KS_NOMED = 256 };
+enum : int { KS_DARK = 1, KS_FLAT = 2, KS_N2N = 4, KS_MASK = 8, KS_CHECK = 16, KS_LT = 32, KS_NZ = 64, KS_SWAP = 128, KS_NOMED = 256,
+             KS_BG = 512 };
+// KS_BG: per-frame backgrounds (K1Args::bg, of the raw dtype) in place of the dark map.  The producer loads one background
+// box per frame next to the raw box (evict first: each is read once); the flat value's float64 reciprocal stays shared by
+// the frames of the unit, and each frame subtracts float64(float32(its own background sample))
 // KS_NOMED: ksize 0 (threshold <= 0, CameraCalibration.py:556-557 skips the artefact step): the pointwise value itself is
 // stored, through the same pipeline (one row late, like the median's centre pixel)
 // KS_SWAP: big-endian uint16 samples (reader/RAW.py default) — one PRMT per pixel after the shared-memory load
@@ -166,12 +182,14 @@ template <typename RawT, typename OutT, int CFG, typename C>
 __global__ void __launch_bounds__(KS_THREADS, C::MINB)
 k1_stream_kernel(const __grid_constant__ CUtensorMap tm_raw, const __grid_constant__ CUtensorMap tm_dark,
                  const __grid_constant__ CUtensorMap tm_flat, K1Args a, int strips, int seg_rows, int total_units) {
-    using B = StreamBox<RawT, C>;
+    constexpr bool BG = CFG >= 0 && (CFG & KS_BG);
+    using B = StreamBox<RawT, C, BG>;
     constexpr int KS_R = C::R, KS_NSTAGE = C::NSTAGE, NF = C::NF;
     static_assert(KS_R % 2 == 0, "rows per stage must be even (outputs are produced in vertical pairs)");
     static_assert(NF == 1 || (CFG >= 0 && !(CFG & KS_MASK)), "multi-frame units: specialised configurations without a mask only");
     // the frame-independent half of the division is hoisted whenever the flat value is known to be non-zero
     constexpr bool FASTDIV = CFG >= 0 && (CFG & KS_NZ) && (CFG & KS_DARK) && (CFG & KS_FLAT);
+    static_assert(!BG || FASTDIV, "per-frame backgrounds: the specialised dark + zero-free flat configurations only");
     extern __shared__ __align__(128) uint8_t smem[];
     uint64_t* full = (uint64_t*)(smem + B::bar_off);
     uint64_t* empty = full + KS_NSTAGE;
@@ -199,7 +217,7 @@ k1_stream_kernel(const __grid_constant__ CUtensorMap tm_raw, const __grid_consta
     if (warp == KS_CW) {
         // ------------------------------------------------------------------ producer
         if (lane != 0) return;
-        const uint32_t tx_bytes = (uint32_t)(NF * B::raw_bytes + (has_dark ? B::map_bytes : 0) + (has_flat ? B::map_bytes : 0));
+        const uint32_t tx_bytes = (uint32_t)(NF * B::raw_bytes + (has_dark ? B::dark_bytes : 0) + (has_flat ? B::map_bytes : 0));
         uint32_t g = 0;
         for (int unit = blockIdx.x; unit < total_units; unit += gridDim.x) {
             const UnitGeom u = ks_unit<KS_R, NF>(unit, strips, seg_rows, H, n_groups);
@@ -216,9 +234,17 @@ k1_stream_kernel(const __grid_constant__ CUtensorMap tm_raw, const __grid_consta
                 for (int f = 0; f < NF; ++f)
                     tma_load_3d_hint(base + f * B::raw_bytes, &tm_raw, &full[stage], (u.tx0 / B::GRAN) * B::GRAN - B::XOFF, y, u.frame + f,
                                      KS_L2_HINTS ? L2_EVICT_FIRST : L2_EVICT_NORMAL);
-                if (has_dark) tma_load_2d_hint(base + NF * B::raw_bytes, &tm_dark, &full[stage], u.tx0 - KS_MAPX, y,
-                                               KS_L2_HINTS ? L2_EVICT_LAST : L2_EVICT_NORMAL);
-                if (has_flat) tma_load_2d_hint(base + NF * B::raw_bytes + B::map_bytes, &tm_flat, &full[stage], u.tx0 - KS_MAPX, y,
+                if (BG) {
+                    // tm_dark holds the backgrounds [n][H][W]: the same box as the raw samples, streamed once as well
+#pragma unroll
+                    for (int f = 0; f < NF; ++f)
+                        tma_load_3d_hint(base + (NF + f) * B::raw_bytes, &tm_dark, &full[stage], (u.tx0 / B::GRAN) * B::GRAN - B::XOFF, y,
+                                         u.frame + f, KS_L2_HINTS ? L2_EVICT_FIRST : L2_EVICT_NORMAL);
+                } else if (has_dark) {
+                    tma_load_2d_hint(base + NF * B::raw_bytes, &tm_dark, &full[stage], u.tx0 - KS_MAPX, y,
+                                     KS_L2_HINTS ? L2_EVICT_LAST : L2_EVICT_NORMAL);
+                }
+                if (has_flat) tma_load_2d_hint(base + NF * B::raw_bytes + B::dark_bytes, &tm_flat, &full[stage], u.tx0 - KS_MAPX, y,
                                                KS_L2_HINTS ? L2_EVICT_LAST : L2_EVICT_NORMAL);
             }
         }
@@ -258,8 +284,8 @@ k1_stream_kernel(const __grid_constant__ CUtensorMap tm_raw, const __grid_consta
         int i = 0;
 
         auto maps = [&](const uint8_t* base, int j, RowMaps& m) {
-            m.d = has_dark ? ((const float*)(base + NF * B::raw_bytes))[j * KS_MAPW + mcol] : 0.0f;
-            m.f = has_flat ? ((const float*)(base + NF * B::raw_bytes + B::map_bytes))[j * KS_MAPW + mcol] : 0.0f;
+            m.d = has_dark && !BG ? ((const float*)(base + NF * B::raw_bytes))[j * KS_MAPW + mcol] : 0.0f;
+            m.f = has_flat ? ((const float*)(base + NF * B::raw_bytes + B::dark_bytes))[j * KS_MAPW + mcol] : 0.0f;
             if (FASTDIV) {
                 m.dd = (double)m.d;
                 m.fd = (double)m.f;
@@ -271,16 +297,22 @@ k1_stream_kernel(const __grid_constant__ CUtensorMap tm_raw, const __grid_consta
             if (sizeof(RawT) == 2 && swap) rv = (RawT)__byte_perm((unsigned)rv, 0u, 0x0001);
             double rd; float ra;
             StreamRaw<RawT>::ld(rv, rd, ra);
+            float d = m.d;
+            double dd = m.dd;
+            if constexpr (BG) {
+                d = (float)((const RawT*)(base + (NF + f) * B::raw_bytes))[j * B::BOXW + rcol];      // exact for integer samples
+                dd = (double)d;
+            }
             float x;
             bool ok;
             if (FASTDIV) {
-                x = (float)ddiv_rcp(dsub(rd, m.dd), m.fd, m.y);
+                x = (float)ddiv_rcp(dsub(rd, dd), m.fd, m.y);
                 if (flags & FLAG_NAN_TO_NUM) x = fminf(fmaxf(x, -FLT_MAX), FLT_MAX);
-                if (check) ok = (fabsf(m.d) + fabsf(m.f) + ra) <= FLT_MAX;
+                if (check) ok = (fabsf(d) + fabsf(m.f) + ra) <= FLT_MAX;
             } else {
-                x = (CFG >= 0 && (CFG & KS_NZ)) ? pointwise_fast_nz(flags, rd, ra, m.d, m.f, ok) : pointwise_fast(flags, rd, ra, m.d, m.f, ok);
+                x = (CFG >= 0 && (CFG & KS_NZ)) ? pointwise_fast_nz(flags, rd, ra, d, m.f, ok) : pointwise_fast(flags, rd, ra, d, m.f, ok);
             }
-            if (check) { if (!ok) x = pointwise<float>(pw, rd, m.d, 0.0f, m.f); }
+            if (check) { if (!ok) x = pointwise<float>(pw, rd, d, 0.0f, m.f); }
             return x;
         };
         auto triple = [&](float x) -> Sorted3<float> {
@@ -439,6 +471,29 @@ k1_stream_kernel(const __grid_constant__ CUtensorMap tm_raw, const __grid_consta
 }
 
 // ------------------------------------------------------------------------------------------ host
+// per-frame backgrounds stream in these configurations only (the dtype pairs and options the instantiations below cover):
+// a background of the raw dtype, uint16 or float32 frames, native byte order, the chain's dark + flat (+ nan_to_num) with
+// the 3x3 median, or dark + flat alone with threshold <= 0.  Returns the configuration, or -1 (the generic tiles).
+static int ks_bg_cfg(const K1Args& a, int raw_dtype) {
+    if (!a.bg || a.bg_dtype != raw_dtype || (raw_dtype != DT_U16 && raw_dtype != DT_F32)) return -1;
+    const int f = a.pw.flags;
+    if (a.raw_swap || a.mask || a.dark || !a.flat || !a.flat_nz || !(f & FLAG_DARK) || !(f & FLAG_FLAT) || (f & FLAG_DARK_LINEAR))
+        return -1;
+    // float32 backgrounds can hold NaN / inf / FLT_MAX: the checked arithmetic, as for float32 frames
+    const bool check = !a.maps_finite || raw_dtype == DT_F32;
+    const int base = KS_BG | KS_DARK | KS_FLAT | KS_NZ;
+    if (a.ksize == 3) {
+        if (!(f & FLAG_NAN_TO_NUM) || a.pred.cond != COND_GT || (KS_PRED_MID && !a.pred.mid_ok)) return -1;
+        return check ? base | KS_N2N | KS_CHECK : a.no_overflow ? base : base | KS_N2N;
+    }
+    if (a.ksize == 0 && a.H >= 4) {
+        const int n2n = (f & FLAG_NAN_TO_NUM) && !a.no_overflow ? KS_N2N : 0;
+        if (raw_dtype == DT_F32) return base | KS_NOMED | KS_CHECK | n2n;
+        return check ? -1 : base | KS_NOMED | n2n;
+    }
+    return -1;
+}
+
 bool k1_stream_eligible(const K1Args& a, int raw_dtype, int out_dtype) {
     if (a.ksize != 3 && a.ksize != 0) return false;
     if (a.ksize == 0 && a.H < 4) return false;
@@ -452,10 +507,90 @@ bool k1_stream_eligible(const K1Args& a, int raw_dtype, int out_dtype) {
     if (((uintptr_t)a.raw) % 16) return false;
     if (a.dark && ((uintptr_t)a.dark) % 16) return false;
     if (a.flat && ((uintptr_t)a.flat) % 16) return false;
+    if (a.bg && (ks_bg_cfg(a, raw_dtype) < 0 || ((uintptr_t)a.bg) % 16)) return false;
     return tensor_map_encoder() != nullptr;
 }
 
 typedef void (*ks_kern_t)(const CUtensorMap, const CUtensorMap, const CUtensorMap, K1Args, int, int, int);
+
+// the per-frame-background instantiations of one raw dtype (uint16: finite flat maps, with and without the overflow proof,
+// and the checked chain; float32: checked only), or null
+template <typename RawT, typename OutT, typename C>
+static ks_kern_t ks_bg_kernel(int cfg) {
+    constexpr int B0 = KS_BG | KS_DARK | KS_FLAT | KS_NZ;
+    if constexpr (sizeof(RawT) == 2) {
+        if (cfg == B0) return k1_stream_kernel<RawT, OutT, B0, C>;
+        if (cfg == (B0 | KS_N2N)) return k1_stream_kernel<RawT, OutT, B0 | KS_N2N, C>;
+        if constexpr (C::NF == 1) {
+            if (cfg == (B0 | KS_N2N | KS_CHECK)) return k1_stream_kernel<RawT, OutT, B0 | KS_N2N | KS_CHECK, C>;
+            if (cfg == (B0 | KS_NOMED)) return k1_stream_kernel<RawT, OutT, B0 | KS_NOMED, C>;
+            if (cfg == (B0 | KS_NOMED | KS_N2N)) return k1_stream_kernel<RawT, OutT, B0 | KS_NOMED | KS_N2N, C>;
+        }
+    } else if constexpr (sizeof(RawT) == 4) {
+        if (cfg == (B0 | KS_N2N | KS_CHECK)) return k1_stream_kernel<RawT, OutT, B0 | KS_N2N | KS_CHECK, C>;
+        if constexpr (C::NF == 1) {
+            if (cfg == (B0 | KS_NOMED | KS_CHECK)) return k1_stream_kernel<RawT, OutT, B0 | KS_NOMED | KS_CHECK, C>;
+            if (cfg == (B0 | KS_NOMED | KS_CHECK | KS_N2N)) return k1_stream_kernel<RawT, OutT, B0 | KS_NOMED | KS_CHECK | KS_N2N, C>;
+        }
+    }
+    return nullptr;
+}
+
+// grid, segment height and launch of a streaming instantiation with stage layout B
+template <typename B, typename C>
+static cudaError_t ks_run(ks_kern_t kern, const K1Args& a, const CUtensorMap& tr, const CUtensorMap& td, const CUtensorMap& tf,
+                          int sm_count, int seg_rows, cudaStream_t st) {
+    constexpr int KS_R = C::R, NF = C::NF;
+    cudaError_t e = cudaSuccess;
+    const int per_sm = blocks_per_sm_cached((const void*)kern, KS_THREADS, B::total, &e);
+    if (e != cudaSuccess) return e;
+    const int strips = (a.W + KS_TW - 1) / KS_TW;
+    const int n_groups = a.n_frames / NF;
+    const long long slots = (long long)sm_count * per_sm;
+    if (seg_rows <= 0) {
+        // all units cost the same: pick the segment height whose unit count fills whole waves of the resident CTAs best,
+        // counting the two re-read halo rows per segment against it.  (Searching beyond 8 waves finds better fills on
+        // paper — 231-row segments for 32 frames — but measured slower, 36.1 vs 33.6 us/frame: every unit start refills
+        // the pipeline and runs its first chunk row by row.)
+        double best = -1.0;
+        for (int waves = 1; waves <= 8; ++waves) {
+            long long segs_try = slots * waves / ((long long)strips * n_groups);
+            if (segs_try < 1) continue;
+            int rows = (int)((a.H + segs_try - 1) / segs_try);
+            if (rows < 2 * KS_R) rows = 2 * KS_R;
+            const long long units = (long long)strips * ((a.H + rows - 1) / rows) * n_groups;
+            const double util = (double)units / (double)(((units + slots - 1) / slots) * slots) * rows / (rows + 2.0);
+            if (util > best) { best = util; seg_rows = rows; }
+        }
+        if (seg_rows <= 0) seg_rows = a.H;
+    }
+    if (seg_rows < 4) seg_rows = 4;
+    const int segs = (a.H + seg_rows - 1) / seg_rows;
+    const long long total = (long long)strips * segs * n_groups;
+    if (total > 0x7fffffffLL) return cudaErrorInvalidValue;
+    long long grid = slots;
+    if (grid > total) grid = total;
+    kern<<<(unsigned)grid, KS_THREADS, B::total, st>>>(tr, td, tf, a, strips, seg_rows, (int)total);
+    return cudaGetLastError();
+}
+
+// per-frame backgrounds (ks_bg_cfg): the background block is a second 3-D map with the raw samples' box
+template <typename RawT, typename OutT, typename C>
+static cudaError_t launch_stream_bg(const K1Args& a_in, CUtensorMapDataType rdt, int sm_count, int seg_rows, cudaStream_t st) {
+    using B = StreamBox<RawT, C, true>;
+    constexpr int RDT = sizeof(RawT) == 1 ? DT_U8 : sizeof(RawT) == 2 ? DT_U16 : DT_F32;
+    K1Args a = a_in;
+    const int cfg = ks_bg_cfg(a, RDT);
+    if (cfg < 0 || a.n_frames % C::NF) return cudaErrorInvalidValue;
+    ks_kern_t kern = ks_bg_kernel<RawT, OutT, C>(cfg);
+    if (!kern) return cudaErrorInvalidValue;
+    a.flat = a.flat_nz;                                  // zero-free copy: an unconditional division
+    CUtensorMap tr, tb, tf;
+    if (!make_tensor_map(&tr, rdt, sizeof(RawT), a.raw, a.W, a.H, a.n_frames, B::BOXW, C::R)) return cudaErrorInvalidValue;
+    if (!make_tensor_map(&tb, rdt, sizeof(RawT), a.bg, a.W, a.H, a.n_frames, B::BOXW, C::R)) return cudaErrorInvalidValue;
+    if (!make_tensor_map(&tf, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 4, a.flat, a.W, a.H, 0, KS_MAPW, C::R)) return cudaErrorInvalidValue;
+    return ks_run<B, C>(kern, a, tr, tb, tf, sm_count, seg_rows, st);
+}
 
 template <typename RawT, typename OutT, typename C>
 static cudaError_t launch_stream_c(const K1Args& a_in, CUtensorMapDataType rdt, int sm_count, int seg_rows, cudaStream_t st) {
@@ -509,45 +644,33 @@ static cudaError_t launch_stream_c(const K1Args& a_in, CUtensorMapDataType rdt, 
         return cudaErrorInvalidValue;
     if (!make_tensor_map(&tf, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 4, a.flat ? (const void*)a.flat : a.raw, a.W, a.H, 0, KS_MAPW, KS_R) && a.flat)
         return cudaErrorInvalidValue;
-    cudaError_t e = cudaSuccess;
-    const int per_sm = blocks_per_sm_cached((const void*)kern, KS_THREADS, B::total, &e);
-    if (e != cudaSuccess) return e;
-    const int strips = (a.W + KS_TW - 1) / KS_TW;
-    const int n_groups = a.n_frames / NF;
-    const long long slots = (long long)sm_count * per_sm;
-    if (seg_rows <= 0) {
-        // all units cost the same: pick the segment height whose unit count fills whole waves of the resident CTAs best,
-        // counting the two re-read halo rows per segment against it.  (Searching beyond 8 waves finds better fills on
-        // paper — 231-row segments for 32 frames — but measured slower, 36.1 vs 33.6 us/frame: every unit start refills
-        // the pipeline and runs its first chunk row by row.)
-        double best = -1.0;
-        for (int waves = 1; waves <= 8; ++waves) {
-            long long segs_try = slots * waves / ((long long)strips * n_groups);
-            if (segs_try < 1) continue;
-            int rows = (int)((a.H + segs_try - 1) / segs_try);
-            if (rows < 2 * KS_R) rows = 2 * KS_R;
-            const long long units = (long long)strips * ((a.H + rows - 1) / rows) * n_groups;
-            const double util = (double)units / (double)(((units + slots - 1) / slots) * slots) * rows / (rows + 2.0);
-            if (util > best) { best = util; seg_rows = rows; }
-        }
-        if (seg_rows <= 0) seg_rows = a.H;
-    }
-    if (seg_rows < 4) seg_rows = 4;
-    const int segs = (a.H + seg_rows - 1) / seg_rows;
-    const long long total = (long long)strips * segs * n_groups;
-    if (total > 0x7fffffffLL) return cudaErrorInvalidValue;
-    long long grid = slots;
-    if (grid > total) grid = total;
-    kern<<<(unsigned)grid, KS_THREADS, B::total, st>>>(tr, td, tf, a, strips, seg_rows, (int)total);
-    return cudaGetLastError();
+    return ks_run<B, C>(kern, a, tr, td, tf, sm_count, seg_rows, st);
 }
 
 template <typename RawT, typename OutT>
 static cudaError_t launch_stream_t(const K1Args& a, CUtensorMapDataType rdt, int sm_count, int seg_rows, cudaStream_t st) {
     if constexpr (sizeof(OutT) == 4) {
         const int f = a.pw.flags;
-        const bool chain = a.ksize == 3 && a.dark && a.flat && a.flat_nz && (f & FLAG_DARK) && (f & FLAG_FLAT) && (f & FLAG_NAN_TO_NUM) && !a.mask &&
-                           a.pred.cond == COND_GT && !a.raw_swap;
+        const bool chain = a.ksize == 3 && (a.dark || a.bg) && a.flat && a.flat_nz && (f & FLAG_DARK) && (f & FLAG_FLAT) &&
+                           (f & FLAG_NAN_TO_NUM) && !a.mask && a.pred.cond == COND_GT && !a.raw_swap;
+        if (a.bg) {
+            // per-frame backgrounds: frame pairs of the chain (uint16 frames with a finite flat field, float32 frames),
+            // everything else and an odd last frame one frame per unit in the narrow shape
+            using P = typename std::conditional<sizeof(RawT) == 4, KsPairBgF32, KsPairBg>::type;
+            if (!chain || a.n_frames < 4 || (sizeof(RawT) != 4 && !a.maps_finite))
+                return launch_stream_bg<RawT, OutT, KsNarrow>(a, rdt, sm_count, seg_rows, st);
+            const int even = a.n_frames & ~1;
+            K1Args b = a;
+            b.n_frames = even;
+            cudaError_t e = launch_stream_bg<RawT, OutT, P>(b, rdt, sm_count, seg_rows, st);
+            if (e != cudaSuccess || even == a.n_frames) return e;
+            b = a;
+            b.n_frames = 1;
+            b.raw = (const char*)a.raw + (size_t)even * a.H * a.W * sizeof(RawT);
+            b.bg = (const char*)a.bg + (size_t)even * a.H * a.W * sizeof(RawT);
+            b.out = (char*)a.out + (size_t)even * a.H * a.W * sizeof(OutT);
+            return launch_stream_bg<RawT, OutT, KsNarrow>(b, rdt, sm_count, seg_rows, st);
+        }
         // batches of the chain configuration: two frames per work unit share the dark / flat half of the arithmetic;
         // an odd last frame goes through the one-frame kernel
 #ifndef KS_NO_PAIR
@@ -567,6 +690,7 @@ static cudaError_t launch_stream_t(const K1Args& a, CUtensorMapDataType rdt, int
         // the wide shape pays with float32 output and a few frames per launch (see KsShape)
         if (a.n_frames >= 4) return launch_stream_c<RawT, OutT, KsWide>(a, rdt, sm_count, seg_rows, st);
     }
+    if (a.bg) return launch_stream_bg<RawT, OutT, KsNarrow>(a, rdt, sm_count, seg_rows, st);
     return launch_stream_c<RawT, OutT, KsNarrow>(a, rdt, sm_count, seg_rows, st);
 }
 

@@ -430,6 +430,7 @@ bool k1_stream5_eligible(const K1Args& a, int raw_dtype, int out_dtype) {
     if (out_dtype != DT_F32 && out_dtype != DT_U16 && out_dtype != DT_U8) return false;
     if (a.pw.flags & FLAG_DARK_LINEAR) return false;
     if (a.raw_gap) return false;
+    if (a.bg) return false;                              // per-frame backgrounds with 5x5: the generic tiles
     const size_t esz = dtype_size(raw_dtype);
     if (((size_t)a.W * esz) % 16 || ((size_t)a.W * 4) % 16) return false;
     if (((size_t)a.H * a.W * esz) % 16) return false;

@@ -529,21 +529,50 @@ class Engine(object):
                                                    ctypes.c_void_p(mapy.data_ptr()), self._stream()))
         return mapx, mapy
 
+    @staticmethod
+    def _bg_code(bg_dtype, raw_code):
+        """library dtype code of per-frame backgrounds: the frames' dtype or float32"""
+        tt = torch()
+        if isinstance(bg_dtype, tt.dtype):
+            code = {tt.uint8: _lib.U8, tt.uint16: _lib.U16, tt.float32: _lib.F32}.get(bg_dtype)
+        else:
+            code = NP_CODES.get(np.dtype(bg_dtype))
+        if code is None or code not in (raw_code, _lib.F32):
+            raise ValueError("bg of dtype %s: the frames' dtype or float32" % (bg_dtype,))
+        return code
+
     def correct_batch(self, raw, threshold=0.1, ksize=3, flags=DO_DARK | DO_FLAT | DO_NAN_TO_NUM, use_lens=True,
-                      border_value=0.0, window=None, out_dtype=None, out=None, out_scale=None):
+                      border_value=0.0, window=None, out_dtype=None, out=None, out_scale=None, bg=None):
         """K1 -> K2 [-> perspective stage with DO_PERSPECTIVE in flags] for every frame of a device-resident batch [n,H,W].
         uint16 / uint8 output stores the float32 result v as round_half_even(clip((v - offset) * gain)) with
-        ``out_scale=(offset, gain)`` (default (0, 1)), inside the chain's last kernel."""
+        ``out_scale=(offset, gain)`` (default (0, 1)), inside the chain's last kernel.
+        ``bg``: one background image per frame, a CUDA tensor [n,H,W] on this engine's device of the frames' dtype or
+        float32: frame i subtracts bg[i] in place of the dark map (imgcorr_correct_batch_bg; flags must hold DO_DARK)."""
         tt = torch()
         squeeze = raw.dim() == 2
         raw = self._frames(raw)
         n = raw.shape[0]
+        if bg is not None:
+            if not isinstance(bg, tt.Tensor) or not bg.is_cuda or bg.device != self.device:
+                raise ValueError('bg must be a CUDA tensor on %s' % self.device)
+            if squeeze and bg.dim() == 2:
+                bg = bg.unsqueeze(0)
+            if tuple(bg.shape) != tuple(raw.shape):
+                raise ValueError('bg has shape %s, frames %s' % (tuple(bg.shape), tuple(raw.shape)))
+            bg_code = self._bg_code(bg.dtype, _dtype_code(raw.dtype))
+            bg = bg.contiguous()
         lens, (x0, y0, ow, oh), (h, w) = self.chain_shape(flags, use_lens, window)
         if out is None:
             out = tt.empty((n, h, w), dtype=out_dtype or tt.float32, device=self.device)
         else:
             self._check_out(out, (h, w) if squeeze and out.dim() == 2 else (n, h, w))
         self._set_out_scale(_dtype_code(out.dtype), out_scale)
+        if bg is not None:
+            _lib.check(self.lib.imgcorr_correct_batch_bg(
+                self._h, ctypes.c_void_p(raw.data_ptr()), _dtype_code(raw.dtype), ctypes.c_void_p(bg.data_ptr()), bg_code,
+                ctypes.c_void_p(out.data_ptr()), _dtype_code(out.dtype), n, float(threshold), int(ksize), int(flags),
+                int(lens), float(border_value), x0, y0, ow, oh, self._stream()))
+            return out[0] if squeeze else out
         _lib.check(self.lib.imgcorr_correct_batch(
             self._h, ctypes.c_void_p(raw.data_ptr()), _dtype_code(raw.dtype), ctypes.c_void_p(out.data_ptr()),
             _dtype_code(out.dtype), n, float(threshold), int(ksize), int(flags), int(lens), float(border_value),
@@ -551,9 +580,11 @@ class Engine(object):
         return out[0] if squeeze else out
 
     def correct_host(self, raw, out=None, threshold=0.1, ksize=3, flags=DO_DARK | DO_FLAT | DO_NAN_TO_NUM,
-                     use_lens=True, border_value=0.0, window=None, out_dtype=np.float32, out_scale=None):
+                     use_lens=True, border_value=0.0, window=None, out_dtype=np.float32, out_scale=None, bg=None):
         """The chain on HOST numpy frames [n,H,W] (uint8/uint16/float32): pinned staging, H2D, kernels and
-        D2H of consecutive frames overlap inside the library.  Synchronous.  flags, out_scale as correct_batch."""
+        D2H of consecutive frames overlap inside the library.  Synchronous.  flags, out_scale as correct_batch.
+        ``bg``: one background image per frame, a numpy array [n,H,W] of the frames' dtype or float32, native byte order
+        (imgcorr_correct_host_bg)."""
         squeeze = raw.ndim == 2
         raw = np.ascontiguousarray(raw)
         big_endian = raw.dtype.byteorder == '>' or (raw.dtype.byteorder == '=' and not np.little_endian)
@@ -566,6 +597,17 @@ class Engine(object):
         if raw.shape[1:] != (self.H, self.W):
             raise ValueError('frames of shape %s do not match the engine (%d, %d)' % (raw.shape, self.H, self.W))
         n = raw.shape[0]
+        if bg is not None:
+            if not isinstance(bg, np.ndarray):
+                raise ValueError('bg must be a numpy array for host frames')
+            if squeeze and bg.ndim == 2:
+                bg = bg[None]
+            if bg.shape != raw.shape:
+                raise ValueError('bg has shape %s, frames %s' % (bg.shape, raw.shape))
+            if not bg.dtype.isnative:
+                raise ValueError('bg must be in native byte order')
+            bg_code = self._bg_code(bg.dtype, NP_CODES.get(raw.dtype))
+            bg = np.ascontiguousarray(bg)
         lens, (x0, y0, ow, oh), (h, w) = self.chain_shape(flags, use_lens, window)
         if out is None:
             out = np.empty((n, h, w), dtype=out_dtype)
@@ -575,10 +617,16 @@ class Engine(object):
             raise TypeError('unsupported output dtype %s (uint8, uint16, float32, float64)' % out.dtype)
         self._set_out_scale(NP_CODES[out.dtype], out_scale)
         with self.ingest(big_endian, 0):
-            _lib.check(self.lib.imgcorr_correct_host(
-                self._h, raw.ctypes.data_as(ctypes.c_void_p), NP_CODES[raw.dtype], out.ctypes.data_as(ctypes.c_void_p),
-                NP_CODES[out.dtype], n, float(threshold), int(ksize), int(flags), int(lens), float(border_value),
-                x0, y0, ow, oh))
+            if bg is not None:
+                _lib.check(self.lib.imgcorr_correct_host_bg(
+                    self._h, raw.ctypes.data_as(ctypes.c_void_p), NP_CODES[raw.dtype], bg.ctypes.data_as(ctypes.c_void_p),
+                    bg_code, out.ctypes.data_as(ctypes.c_void_p), NP_CODES[out.dtype], n, float(threshold), int(ksize),
+                    int(flags), int(lens), float(border_value), x0, y0, ow, oh))
+            else:
+                _lib.check(self.lib.imgcorr_correct_host(
+                    self._h, raw.ctypes.data_as(ctypes.c_void_p), NP_CODES[raw.dtype], out.ctypes.data_as(ctypes.c_void_p),
+                    NP_CODES[out.dtype], n, float(threshold), int(ksize), int(flags), int(lens), float(border_value),
+                    x0, y0, ow, oh))
         return out[0] if squeeze else out
 
 

@@ -33,8 +33,9 @@ extern "C" {
 #define IMGCORR_VERSION 200 /* 0.2.0: round 2 added imgcorr_ste_average_thr, imgcorr_stack_mean, imgcorr_scale_f64, imgcorr_subsample_f64,
                                imgcorr_linear_fit, imgcorr_host_fingerprint, imgcorr_selftest_division and the K2 options 11, 12;
                                later added imgcorr_set_perspective and IMGCORR_DO_PERSPECTIVE (the chain's perspective stage),
-                               U16 / U8 output of the chain with imgcorr_set_output_scale, and imgcorr_set_perspective_frames
-                               (one homography per frame in the perspective stage) */
+                               U16 / U8 output of the chain with imgcorr_set_output_scale, imgcorr_set_perspective_frames
+                               (one homography per frame in the perspective stage), and imgcorr_correct_batch_bg /
+                               imgcorr_correct_host_bg (one background image per frame in place of the dark map) */
 
 #if defined(__GNUC__)
 #define IMGCORR_API __attribute__((visibility("default")))
@@ -180,6 +181,27 @@ IMGCORR_API int imgcorr_correct_batch(imgcorr_ctx* ctx, const void* raw_dev, int
 IMGCORR_API int imgcorr_correct_host(imgcorr_ctx* ctx, const void* raw_host, int raw_dtype, void* out_host, int out_dtype,
                          int n_frames, double threshold, int ksize, int flags, int use_lens, double border_value,
                          int x0, int y0, int ow, int oh);
+
+/* The chain with one background image per frame: correct(image, bgImages=bg) of the reference
+ * (camera/CameraCalibration.py:484-502) for n (image, background) pairs.  Frame i of the call subtracts background i in
+ * float64 (image -= bg) in place of the context's dark map, then the flat division rounds once to float32 and the rest of
+ * the chain is unchanged; for U8 / U16 / F32 backgrounds the result equals imgcorr_correct_batch with the dark map set to
+ * float32(bg[i]).
+ *   bg_dev / bg_host  dense [n][H][W] of bg_dtype, native byte order; i counts from the call's first frame.  The ingest
+ *                     options (IMGCORR_OPT_RAW_BIG_ENDIAN, IMGCORR_OPT_RAW_FRAME_GAP) apply to the raw frames only.
+ *   bg_dtype          raw_dtype or F32; anything else, or flags without IMGCORR_DO_DARK, fails with IMGCORR_ERR_INVALID
+ *                     before anything is enqueued
+ * The context's dark map and linear dark model are neither read nor modified: a later call without backgrounds uses them
+ * as before.  bg == NULL is imgcorr_correct_batch / imgcorr_correct_host.  Float32 backgrounds may hold NaN / inf; they
+ * take the checked arithmetic of float32 frames.  The host call stages the backgrounds through its ring next to the raw
+ * frames (a device buffer per slot, pinned staging for pageable input) and counts both against its chunk size.
+ * Everything else (stream order, scratch, perspective stage, output scale) is as the calls without backgrounds. */
+IMGCORR_API int imgcorr_correct_batch_bg(imgcorr_ctx* ctx, const void* raw_dev, int raw_dtype, const void* bg_dev, int bg_dtype,
+                             void* out_dev, int out_dtype, int n_frames, double threshold, int ksize, int flags,
+                             int use_lens, double border_value, int x0, int y0, int ow, int oh, void* stream);
+IMGCORR_API int imgcorr_correct_host_bg(imgcorr_ctx* ctx, const void* raw_host, int raw_dtype, const void* bg_host, int bg_dtype,
+                            void* out_host, int out_dtype, int n_frames, double threshold, int ksize, int flags,
+                            int use_lens, double border_value, int x0, int y0, int ow, int oh);
 
 /* Scale of the chain's integer output (out_dtype U16 / U8 of imgcorr_correct_batch / imgcorr_correct_host):
  * stored = quantise((F32 result - offset) * gain), see imgcorr_correct_batch.  Context state, read when a chain call is
