@@ -11,7 +11,7 @@ U8, U16, F32, F64 = 0, 1, 2, 3
 COND_GT, COND_LT = 0, 1
 DO_DARK, DO_FLAT, DO_NAN_TO_NUM, DO_PERSPECTIVE = 1, 2, 4, 8
 OPT_K1_VARIANT, OPT_K2_VARIANT, OPT_HOST_SLOTS, OPT_K1_SEG_ROWS, OPT_PROFILE, OPT_CHAIN_GROUP = 1, 2, 3, 4, 5, 6
-OPT_RAW_BIG_ENDIAN, OPT_RAW_FRAME_GAP, OPT_K3_VARIANT, OPT_CHAIN_OVERLAP, OPT_K2_COORD_CACHE, OPT_K2_TMA_STORE = 7, 8, 9, 10, 11, 12
+OPT_RAW_BIG_ENDIAN, OPT_RAW_FRAME_GAP, OPT_K3_VARIANT, OPT_CHAIN_OVERLAP, OPT_K2_COORD_CACHE = 7, 8, 9, 10, 11
 INTER_CUBIC, INTER_LANCZOS4 = 2, 4
 OK, ERR_INVALID, ERR_CUDA, ERR_STATE, ERR_NOMEM = 0, -1, -2, -3, -4
 

@@ -126,7 +126,7 @@ struct imgcorr_ctx {
     // written by the first tiled launch, read by the following ones; dropped by set_lens
     struct K2Cache { int x0, y0, ow, oh, g, esz; DevPtr<unsigned> pack; DevPtr<int2> hdr; Event ev; cudaStream_t st; unsigned long long stamp; };
     std::vector<K2Cache> k2_cache;
-    int k2_cache_on = 1, k2_tma_store = 0;
+    int k2_cache_on = 1;
     unsigned long long k2_stamp = 0;
     DevPtr<void> dump;                        // scratch for stores of lanes that own no output pixel
     int raw_big_endian = 0;
@@ -249,9 +249,6 @@ extern "C" IMGCORR_API int imgcorr_set_option(imgcorr_ctx* c, int key, int value
             return IMGCORR_OK;
         case IMGCORR_OPT_CHAIN_OVERLAP:
             c->chain_overlap = value ? 1 : 0;
-            return IMGCORR_OK;
-        case IMGCORR_OPT_K2_TMA_STORE:
-            c->k2_tma_store = value ? 1 : 0;
             return IMGCORR_OK;
         case IMGCORR_OPT_K2_COORD_CACHE:
             c->k2_cache_on = value ? 1 : 0;
@@ -513,7 +510,6 @@ static int run_k2(imgcorr_ctx* c, const void* src, int sdt, void* dst, int ddt, 
     a.lens = c->lens;
     a.lens_dev = c->lens_dev.get();
     a.sm_count = c->sm_count;
-    a.tma_store = c->k2_tma_store;
     a.q = q;
     if (!c->k2_wtab) {
         std::vector<float4> t(32 * 32);

@@ -67,9 +67,7 @@ struct K2Args {
     unsigned* cpack_w;       // write the cache while computing (first launch for this lens / window / geometry)
     int2* chdr_w;
     int sm_count;
-    int tma_store;           // tiled variant: output tile through shared memory + TMA store instead of predicated stores
-                             // (float destinations only: the F32 -> U16 / U8 pairs always store per pixel)
-    OutScale q;              // F32 -> U16 / U8: the float32 blend, then quantise<DstT>(blend, q)
+    OutScale q;             // F32 -> U16 / U8: the float32 blend, then quantise<DstT>(blend, q)
 };
 void k2_cache_size(int geometry, int ow, int oh, size_t* words, size_t* tiles);
 bool k2_will_tile(const K2Args& a, int src_dtype, int dst_dtype, int variant);    // launch_k2 takes the tiled variant

@@ -68,16 +68,6 @@ __device__ __forceinline__ void bulk_load_1d(void* dst, const void* src, uint32_
     asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];"
                  ::"r"(smem_u32(dst)), "l"(src), "r"(bytes), "r"(smem_u32(bar)) : "memory");
 }
-// tiled bulk tensor store shared -> global (bulk async-group completion); parts of the box outside the tensor are
-// not written.  Sequence: write the tile with ordinary stores, fence_proxy_async_smem() in every writing thread,
-// barrier, one thread issues the store + commit, and waits for `.read` before the tile is overwritten.
-__device__ __forceinline__ void tma_store_3d(const CUtensorMap* tm, const void* src, int x, int y, int z) {
-    asm volatile("cp.async.bulk.tensor.3d.global.shared::cta.bulk_group [%0, {%2, %3, %4}], [%1];"
-                 ::"l"(tm), "r"(smem_u32(src)), "r"(x), "r"(y), "r"(z) : "memory");
-}
-__device__ __forceinline__ void tma_store_commit() { asm volatile("cp.async.bulk.commit_group;" ::: "memory"); }
-template <int N> __device__ __forceinline__ void tma_store_wait_read() { asm volatile("cp.async.bulk.wait_group.read %0;" ::"n"(N) : "memory"); }
-__device__ __forceinline__ void fence_proxy_async_smem() { asm volatile("fence.proxy.async.shared::cta;" ::: "memory"); }
 
 // ---- host ---------------------------------------------------------------------------------------------------
 typedef CUresult (*PFN_tensorMapEncodeTiled)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*,

@@ -45,18 +45,6 @@ typedef KsShape<KS_NARROW_R, KS_NARROW_NSTAGE, KS_NARROW_MINB, 1> KsNarrow;
 #define KS_WIDE_MINB 3
 #endif
 typedef KsShape<KS_WIDE_R, KS_WIDE_NSTAGE, KS_WIDE_MINB, 1> KsWide;
-// KS_PRED_MID 1: the straight-line chunks decide with the one-sided predicate_mid and count certain decisions with an
-// IMAD.HI on the FMA pipe (18.1 instead of 19.4 ALU operations per lane-row, 40.1 instead of 38.4 instructions).  Measured
-// SLOWER on B200 (25.95 vs 24.61 us per 4096x3000 frame in batches, 43.0 vs 41.0 for one frame): off.
-#ifndef KS_PRED_MID
-#define KS_PRED_MID 0
-#endif
-#ifndef KS_L2_HINTS
-#define KS_L2_HINTS 1
-#endif
-#ifndef KS_FIRST_FAST
-#define KS_FIRST_FAST 1
-#endif
 #ifndef KS_PAIR_R
 #define KS_PAIR_R 16
 #define KS_PAIR_NSTAGE 3
@@ -105,15 +93,6 @@ template <> __device__ __forceinline__ uint8_t  ks_out<uint8_t>(const K1Args& a,
 template <typename OutT> __device__ __forceinline__ void ks_store(OutT* p, OutT v, uint64_t) { *p = v; }
 template <> __device__ __forceinline__ void ks_store<float>(float* p, float v, uint64_t policy) {
     asm volatile("st.global.L2::cache_hint.f32 [%0], %1, %2;" ::"l"(p), "f"(v), "l"(policy) : "memory");
-}
-
-// acc += sign bit of w, as one IMAD.HI on the FMA pipe (the multiplier 2 lives in constant memory: with an immediate
-// ptxas turns the multiply into a shift + add on the ALU pipe, which is the pipe this is meant to relieve)
-__constant__ unsigned ks_two = 2u;
-__device__ __forceinline__ unsigned ks_count_sign(float w, unsigned acc) {
-    unsigned r;
-    asm("mad.hi.u32 %0, %1, %2, %3;" : "=r"(r) : "r"(__float_as_uint(w)), "r"(ks_two), "r"(acc));
-    return r;
 }
 
 __device__ __noinline__ bool ks_exact(float x, float b, double thr, int cond) {
@@ -209,7 +188,6 @@ k1_stream_kernel(const __grid_constant__ CUtensorMap tm_raw, const __grid_consta
     if (threadIdx.x == 0) {
         for (int s = 0; s < KS_NSTAGE; ++s) { mbar_init(&full[s], 1); mbar_init(&empty[s], KS_CW); }
         sconst[0] = a.pred.lo; sconst[1] = a.pred.hi; *(double*)(sconst + 2) = a.pred.thr;
-        sconst[4] = a.pred.thr32; sconst[5] = a.pred.gw;
         mbar_init_fence();
     }
     __syncthreads();
@@ -233,19 +211,18 @@ k1_stream_kernel(const __grid_constant__ CUtensorMap tm_raw, const __grid_consta
 #pragma unroll
                 for (int f = 0; f < NF; ++f)
                     tma_load_3d_hint(base + f * B::raw_bytes, &tm_raw, &full[stage], (u.tx0 / B::GRAN) * B::GRAN - B::XOFF, y, u.frame + f,
-                                     KS_L2_HINTS ? L2_EVICT_FIRST : L2_EVICT_NORMAL);
+                                     L2_EVICT_FIRST);
                 if (BG) {
                     // tm_dark holds the backgrounds [n][H][W]: the same box as the raw samples, streamed once as well
 #pragma unroll
                     for (int f = 0; f < NF; ++f)
                         tma_load_3d_hint(base + (NF + f) * B::raw_bytes, &tm_dark, &full[stage], (u.tx0 / B::GRAN) * B::GRAN - B::XOFF, y,
-                                         u.frame + f, KS_L2_HINTS ? L2_EVICT_FIRST : L2_EVICT_NORMAL);
+                                         u.frame + f, L2_EVICT_FIRST);
                 } else if (has_dark) {
-                    tma_load_2d_hint(base + NF * B::raw_bytes, &tm_dark, &full[stage], u.tx0 - KS_MAPX, y,
-                                     KS_L2_HINTS ? L2_EVICT_LAST : L2_EVICT_NORMAL);
+                    tma_load_2d_hint(base + NF * B::raw_bytes, &tm_dark, &full[stage], u.tx0 - KS_MAPX, y, L2_EVICT_LAST);
                 }
                 if (has_flat) tma_load_2d_hint(base + NF * B::raw_bytes + B::dark_bytes, &tm_flat, &full[stage], u.tx0 - KS_MAPX, y,
-                                               KS_L2_HINTS ? L2_EVICT_LAST : L2_EVICT_NORMAL);
+                                               L2_EVICT_LAST);
             }
         }
         return;
@@ -256,12 +233,11 @@ k1_stream_kernel(const __grid_constant__ CUtensorMap tm_raw, const __grid_consta
     // per-launch constants come from shared memory: ptxas would re-read kernel parameters at every use
     PredicateConst pred = a.pred;
     pred.lo = sconst[0]; pred.hi = sconst[1]; pred.thr = *(const double*)(sconst + 2);
-    pred.thr32 = sconst[4]; pred.gw = sconst[5];
     if (CFG >= 0) pred.cond = (CFG & KS_LT) ? COND_LT : COND_GT;
     const int lc = warp * KS_SW - 1 + lane;            // strip-local column of this lane: -1 .. 120
     // results that nobody reads back soon (a K1-only call) leave L2 first, so that the calibration maps stay; inside the
     // chain K2 reads them right away and they keep the normal priority
-    const uint64_t out_policy = (KS_L2_HINTS && a.out_streaming) ? L2_EVICT_FIRST : L2_EVICT_NORMAL;
+    const uint64_t out_policy = a.out_streaming ? L2_EVICT_FIRST : L2_EVICT_NORMAL;
     const ptrdiff_t frame_px = (ptrdiff_t)H * W;
     uint32_t g = 0;
 
@@ -376,7 +352,7 @@ k1_stream_kernel(const __grid_constant__ CUtensorMap tm_raw, const __grid_consta
                 }
             }
             const int rows = u.n_in - k * KS_R;
-            if ((KS_FIRST_FAST || k > 0) && rows >= KS_R) {
+            if (rows >= KS_R) {
                 // straight-line chunk: every row emits; the store is unconditional (lanes without an output pixel write to
                 // a private scratch slot) and the guard-band test is only accumulated — if any lane of the warp hit the
                 // band in this chunk (rare), the chunk is redone below with the exact predicate.  A unit's FIRST chunk goes
@@ -396,7 +372,6 @@ k1_stream_kernel(const __grid_constant__ CUtensorMap tm_raw, const __grid_consta
                 const int ostride = valid ? W : 0;       // element index j * ostride stays below 2^31 (R * 32767)
                 const bool skip0 = k == 0, skip1 = k == 0 && i_first == 2;      // steps of this chunk that emit nothing
                 bool unsure = false;
-                unsigned n_sure = 0;                     // predicate_mid: decisions of this chunk that were certain
 #pragma unroll
                 for (int j = 0; j < KS_R; j += 2) {
                     RowMaps ma, mb;
@@ -423,16 +398,8 @@ k1_stream_kernel(const __grid_constant__ CUtensorMap tm_raw, const __grid_consta
                         float m1, m2;
                         median9_pair(s0[f], s1[f], ta, tb, m1, m2);
                         bool r1, r2;
-                        if (KS_PRED_MID && CFG >= 0) {
-                            float w1, w2;
-                            r1 = predicate_mid(c1[f], m1, pred, w1);
-                            r2 = predicate_mid(xa, m2, pred, w2);
-                            n_sure = ks_count_sign(w1, n_sure);
-                            n_sure = ks_count_sign(w2, n_sure);
-                        } else {
-                            unsure |= !predicate_certain(c1[f], m1, pred, r1);
-                            unsure |= !predicate_certain(xa, m2, pred, r2);
-                        }
+                        unsure |= !predicate_certain(c1[f], m1, pred, r1);
+                        unsure |= !predicate_certain(xa, m2, pred, r2);
                         ks_store<OutT>(d0, ks_out<OutT>(a, r1 ? m1 : c1[f]), out_policy);
                         ks_store<OutT>(d1, ks_out<OutT>(a, r2 ? m2 : xa), out_policy);
                         if (has_mask) {
@@ -442,7 +409,6 @@ k1_stream_kernel(const __grid_constant__ CUtensorMap tm_raw, const __grid_consta
                         s0[f] = ta; s1[f] = tb; c1[f] = xb;
                     }
                 }
-                if (KS_PRED_MID && CFG >= 0 && !nomed) unsure = n_sure != (unsigned)(KS_R * NF);
                 if (__any_sync(0xffffffffu, unsure)) {
 #pragma unroll
                     for (int f = 0; f < NF; ++f) { s0[f] = k0[f]; s1[f] = k1[f]; c1[f] = kc[f]; }
@@ -483,7 +449,7 @@ static int ks_bg_cfg(const K1Args& a, int raw_dtype) {
     const bool check = !a.maps_finite || raw_dtype == DT_F32;
     const int base = KS_BG | KS_DARK | KS_FLAT | KS_NZ;
     if (a.ksize == 3) {
-        if (!(f & FLAG_NAN_TO_NUM) || a.pred.cond != COND_GT || (KS_PRED_MID && !a.pred.mid_ok)) return -1;
+        if (!(f & FLAG_NAN_TO_NUM) || a.pred.cond != COND_GT) return -1;
         return check ? base | KS_N2N | KS_CHECK : a.no_overflow ? base : base | KS_N2N;
     }
     if (a.ksize == 0 && a.H >= 4) {
@@ -627,17 +593,6 @@ static cudaError_t launch_stream_c(const K1Args& a_in, CUtensorMapDataType rdt, 
         else if (plain) kern = k1_stream_kernel<RawT, OutT, KS_MASK, C>;
         else kern = k1_stream_kernel<RawT, OutT, -1, C>;
     }
-
-    if (KS_PRED_MID && !a.pred.mid_ok && a.ksize != 0) {
-        // the specialised instantiations decide with predicate_mid (thresholds in [1e-6, 0.5)); anything else runs the
-        // run-time-flag instantiation with the two-sided test
-        if constexpr (NF > 1) {
-            return cudaErrorNotSupported;
-        } else {
-            kern = k1_stream_kernel<RawT, OutT, -1, C>;
-            a.flat = a_in.flat;
-        }
-    }
     CUtensorMap tr, td, tf;
     if (!make_tensor_map(&tr, rdt, sizeof(RawT), a.raw, a.W, a.H, a.n_frames, B::BOXW, KS_R)) return cudaErrorInvalidValue;
     if (!make_tensor_map(&td, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 4, a.dark ? (const void*)a.dark : a.raw, a.W, a.H, 0, KS_MAPW, KS_R) && a.dark)
@@ -673,8 +628,7 @@ static cudaError_t launch_stream_t(const K1Args& a, CUtensorMapDataType rdt, int
         }
         // batches of the chain configuration: two frames per work unit share the dark / flat half of the arithmetic;
         // an odd last frame goes through the one-frame kernel
-#ifndef KS_NO_PAIR
-        if (chain && a.n_frames >= 4 && (!KS_PRED_MID || a.pred.mid_ok)) {
+        if (chain && a.n_frames >= 4) {
             const int even = a.n_frames & ~1;
             K1Args b = a;
             b.n_frames = even;
@@ -686,7 +640,6 @@ static cudaError_t launch_stream_t(const K1Args& a, CUtensorMapDataType rdt, int
             b.out = (char*)a.out + (size_t)even * a.H * a.W * sizeof(OutT);
             return launch_stream_c<RawT, OutT, KsNarrow>(b, rdt, sm_count, seg_rows, st);
         }
-#endif
         // the wide shape pays with float32 output and a few frames per launch (see KsShape)
         if (a.n_frames >= 4) return launch_stream_c<RawT, OutT, KsWide>(a, rdt, sm_count, seg_rows, st);
     }

@@ -19,7 +19,6 @@
 
 namespace imgcorr {
 
-#if !defined(K5_INTKEYS) || K5_INTKEYS
 __constant__ int k5_one = 1, k5_minus_one = -1;   // run-time values for ptxas: keeps the two IMADs from folding into IADD3
 template <> __device__ __forceinline__ void cswap<OrdKey>(OrdKey& a, OrdKey& b) {
     const int lo = a.k < b.k ? a.k : b.k;
@@ -29,7 +28,6 @@ template <> __device__ __forceinline__ void cswap<OrdKey>(OrdKey& a, OrdKey& b) 
     b.k = hi;
     a.k = lo;
 }
-#endif
 
 namespace {
 
@@ -80,25 +78,11 @@ __device__ __noinline__ bool exact5(float x, float b, double thr, int cond) {
     return predicate_exact((double)x, (double)b, pc);
 }
 
-#ifndef K5_INTKEYS
-#define K5_INTKEYS 1
-#endif
-#ifndef K5_PAIR
-#define K5_PAIR 1
-#endif
-#if K5_INTKEYS
 typedef OrdKey K5T;                         // the window holds order-preserving integer keys (see imgcorr_core.cuh)
 __device__ __forceinline__ K5T k5_in(float x) { return to_key(x); }
 __device__ __forceinline__ float k5_out(K5T q) { return from_key(q); }
 __device__ __forceinline__ K5T k5_shfl_up(K5T c, int d) { K5T r; r.k = __shfl_up_sync(0xffffffffu, c.k, d); return r; }
 __device__ __forceinline__ K5T k5_shfl_down(K5T c, int d) { K5T r; r.k = __shfl_down_sync(0xffffffffu, c.k, d); return r; }
-#else
-typedef float K5T;
-__device__ __forceinline__ K5T k5_in(float x) { return x; }
-__device__ __forceinline__ float k5_out(K5T q) { return q; }
-__device__ __forceinline__ K5T k5_shfl_up(K5T c, int d) { return __shfl_up_sync(0xffffffffu, c, d); }
-__device__ __forceinline__ K5T k5_shfl_down(K5T c, int d) { return __shfl_down_sync(0xffffffffu, c, d); }
-#endif
 struct Q5 { K5T v[5]; };                    // sorted horizontal quintuple of one row
 
 // Row-pair scheme (median25_pair_net.inc, tools/gen_median25_pair.py): two vertically adjacent windows share four of their
@@ -301,7 +285,6 @@ k1_stream5_kernel(const __grid_constant__ CUtensorMap tm_raw, const __grid_const
                 OutT* op = valid ? outp : (OutT*)a.dump + (size_t)blockIdx.x * K5_THREADS + threadIdx.x;
                 uint8_t* mp = has_mask ? (valid ? maskp : (uint8_t*)a.dump + (size_t)(gridDim.x + blockIdx.x) * K5_THREADS * sizeof(OutT) + threadIdx.x) : nullptr;
                 const int ostride = valid ? W : 0;
-#if K5_PAIR
                 static_assert(K5_R % 2 == 0, "rows per stage must be even (outputs are produced in vertical pairs)");
 #pragma unroll
                 for (int j = 0; j < K5_R; j += 2) {
@@ -325,23 +308,6 @@ k1_stream5_kernel(const __grid_constant__ CUtensorMap tm_raw, const __grid_const
                     push(qa, xa);
                     push(qb, xb);
                 }
-#else
-#pragma unroll
-                for (int j = 0; j < K5_R; ++j) {
-                    const float x = pixel(base, j);
-                    const Q5 q = quint(x);
-                    const float med = median(q);
-                    bool rep;
-                    const bool sure = predicate_certain(c2, med, pred, rep);
-                    if (__any_sync(0xffffffffu, !sure)) {
-                        if (!sure) rep = exact5(c2, med, pred.thr, pred.cond);
-                    }
-                    *op = out5<OutT>(a, rep ? med : c2);
-                    if (has_mask) { *mp = rep ? 1 : 0; mp += ostride; }
-                    op += ostride;
-                    push(q, x);
-                }
-#endif
                 outp += (size_t)K5_R * W;
                 if (has_mask) maskp += (size_t)K5_R * W;
                 i += K5_R;

@@ -249,8 +249,7 @@ __global__ void __launch_bounds__(K2_BX * K2_BY, K2_MINB) k2_remap_kernel(K2Args
 //     the border value (written once per frame, no reads); anything else (frame rim, or outside the box: a fraction of a
 //     percent) -> "slow": gathered from global memory with per-neighbour border handling.  A tile whose window does not fit
 //     a box at all (stronger distortion than the launch geometry was chosen for) is all "slow": correct for any map;
-//   * results leave by predicated per-pixel stores (full 128-byte lines per warp) or, optionally, through a shared output
-//     tile and one TMA store per frame (cp.async.bulk.tensor, bounds-clipped by the hardware; measured slower).
+//   * results leave by predicated per-pixel stores (full 128-byte lines per warp).
 template <int TW_, int TH_, int BW_, int BH_, int NBUF_, int MINB_> struct KtGeom {
     static constexpr int TW = TW_, TH = TH_, BW = BW_, BH = BH_, NBUF = NBUF_, MINB = MINB_;
 };
@@ -259,9 +258,6 @@ template <int TW_, int TH_, int BW_, int BH_, int NBUF_, int MINB_> struct KtGeo
 #endif
 #ifndef KT_MINB_V
 #define KT_MINB_V 4
-#endif
-#ifndef KT_FPB
-#define KT_FPB 1
 #endif
 // 28 rows x 5 boxes in flight instead of 32 x 4 (same shared memory): the moderate 4096x3000 lens needs 27 rows, and the kernel
 // waits on box arrival (19.6 vs 20.1 us per frame); lenses that need 29-32 rows take the 96x32 geometry
@@ -278,9 +274,7 @@ constexpr int KT_MARGIN = 3;                                     // pixels added
 template <typename SrcT, typename G> struct KtBox {
     static constexpr int BW = sizeof(SrcT) == 1 ? G::BW + 16 : G::BW, GRAN = 16 / (int)sizeof(SrcT), BYTES = BW * G::BH * (int)sizeof(SrcT);
 };
-template <typename SrcT, typename DstT, typename G, bool TSTORE> constexpr int kt_smem() {
-    return G::NBUF * KtBox<SrcT, G>::BYTES + 128 + (TSTORE ? 2 * G::TW * G::TH * (int)sizeof(DstT) : 0);
-}
+template <typename SrcT, typename G> constexpr int kt_smem() { return G::NBUF * KtBox<SrcT, G>::BYTES + 128; }
 
 // predicated global store: a plain `if (flag) *p = v` lets ptxas wrap the whole gather of that pixel in a branch.
 // No "memory" clobber: these stores write output pixels that nothing in the kernel reads back, and a clobber would stop
@@ -296,20 +290,6 @@ __device__ __forceinline__ void st_if(uint16_t* p, uint16_t v, unsigned flag) {
 }
 __device__ __forceinline__ void st_if(uint8_t* p, uint8_t v, unsigned flag) {
     asm volatile("{\n\t.reg .pred q;\n\tsetp.ne.u32 q, %2, 0;\n\t@q st.global.u8 [%0], %1;\n\t}" ::"l"(p), "r"((unsigned)v), "r"(flag));
-}
-
-// predicated shared-memory store (same reason)
-__device__ __forceinline__ void sts_if(float* p, float v, unsigned flag) {
-    asm volatile("{\n\t.reg .pred q;\n\tsetp.ne.u32 q, %2, 0;\n\t@q st.shared.f32 [%0], %1;\n\t}" ::"r"(smem_u32(p)), "f"(v), "r"(flag));
-}
-__device__ __forceinline__ void sts_if(double* p, double v, unsigned flag) {
-    asm volatile("{\n\t.reg .pred q;\n\tsetp.ne.u32 q, %2, 0;\n\t@q st.shared.f64 [%0], %1;\n\t}" ::"r"(smem_u32(p)), "d"(v), "r"(flag));
-}
-__device__ __forceinline__ void sts_if(uint16_t* p, uint16_t v, unsigned flag) {
-    asm volatile("{\n\t.reg .pred q;\n\tsetp.ne.u32 q, %2, 0;\n\t@q st.shared.u16 [%0], %1;\n\t}" ::"r"(smem_u32(p)), "h"(v), "r"(flag));
-}
-__device__ __forceinline__ void sts_if(uint8_t* p, uint8_t v, unsigned flag) {
-    asm volatile("{\n\t.reg .pred q;\n\tsetp.ne.u32 q, %2, 0;\n\t@q st.shared.u8 [%0], %1;\n\t}" ::"r"(smem_u32(p)), "r"((unsigned)v), "r"(flag));
 }
 struct KtLens { LensConst L; };
 template <int MODE> __device__ __forceinline__ void kt_load_lens(const K2Args& a, LensConst& L) {
@@ -352,9 +332,8 @@ constexpr unsigned KP_OUTSIDE = 0x80000000u, KP_SLOW = 0x40000000u;
 //       2: coordinates read from the cache: 4 bytes per pixel instead of ~45 float64 operations and ~90 instructions.
 // The lens is constant per context, so the analytic evaluation — what bounds a ONE-frame launch (119 instructions per pixel,
 // 65 us per 4096x3000 frame, issue bound: profiles/r2_k2_single_analytic_ncu_full.txt) — is paid once, not once per call.
-template <typename SrcT, typename DstT, int MODE, typename G, bool TSTORE, int CMODE>
-__global__ void __launch_bounds__(KT_THREADS, G::MINB)
-k2_tiled_kernel(const __grid_constant__ CUtensorMap tm_src, const __grid_constant__ CUtensorMap tm_dst, K2Args a) {
+template <typename SrcT, typename DstT, int MODE, typename G, int CMODE>
+__global__ void __launch_bounds__(KT_THREADS, G::MINB) k2_tiled_kernel(const __grid_constant__ CUtensorMap tm_src, K2Args a) {
     constexpr int KT_TW = G::TW, KT_TH = G::TH, KT_BH = G::BH, KT_NBUF = G::NBUF;
     constexpr int KT_PX = KT_TW * KT_TH / KT_THREADS, KT_RSTEP = KT_THREADS / KT_TW;
     constexpr int BW = KtBox<SrcT, G>::BW, KT_BOX_BYTES = KtBox<SrcT, G>::BYTES, GRAN = KtBox<SrcT, G>::GRAN;
@@ -362,7 +341,6 @@ k2_tiled_kernel(const __grid_constant__ CUtensorMap tm_src, const __grid_constan
     extern __shared__ __align__(128) uint8_t smem[];
     uint64_t* full = (uint64_t*)(smem + KT_NBUF * KT_BOX_BYTES);
     int* est = (int*)(smem + KT_NBUF * KT_BOX_BYTES + 64);      // bx, by (bx < 0: no box)
-    DstT* otile = (DstT*)(smem + KT_NBUF * KT_BOX_BYTES + 128); // [2][TH][TW] when TSTORE
     const int tid = threadIdx.x;
     const int c = tid % KT_TW, r0 = tid / KT_TW;               // rows r0 + RSTEP * j
     const int tx0 = blockIdx.x * KT_TW, ty0 = blockIdx.y * KT_TH;
@@ -501,86 +479,35 @@ k2_tiled_kernel(const __grid_constant__ CUtensorMap tm_src, const __grid_constan
 
     const int src_stride = H * W, dst_stride = oh * ow;
     const SrcT* src = (const SrcT*)a.src;
-    if (TSTORE) {
-        // every pixel of the tile goes through the shared output tile and leaves in one TMA store per frame
-        const int oo = r0 * KT_TW + c;
-        // pixels whose window lies outside the frame hold the border value in both output tiles for the whole launch
+    DstT* dst = (DstT*)a.dst + (oy0 * ow + ox);
+    const int dstep = KT_RSTEP * ow;
+#pragma unroll 1
+    for (int f = 0; f < nf; ++f) {
+        if (have_box) {
+            mbar_wait(&full[f % KT_NBUF], (f / KT_NBUF) & 1);
+            const SrcT* box = (const SrcT*)(smem + (f % KT_NBUF) * KT_BOX_BYTES);
+#pragma unroll
+            for (int j = 0; j < KT_PX; ++j) {
+                const SrcT* p = box + so[j];
+                const DstT r = blend_out<SrcT, DstT>(p[0], p[1], p[BW], p[BW + 1], wt[j], a.q);
+                st_if(dst + j * dstep, r, fast & (1u << j));            // predicated store, no branch around the gather
+            }
+        }
         if (outm) {
 #pragma unroll
             for (int j = 0; j < KT_PX; ++j)
-                if (outm & (1u << j)) { otile[oo + j * KT_RSTEP * KT_TW] = bout; otile[KT_TW * KT_TH + oo + j * KT_RSTEP * KT_TW] = bout; }
+                if (outm & (1u << j)) dst[j * dstep] = bout;
         }
+        if (slow) {
 #pragma unroll 1
-        for (int f = 0; f < nf; ++f) {
-            DstT* ot = otile + (f & 1) * (KT_TW * KT_TH) + oo;
-            if (have_box) {
-                mbar_wait(&full[f % KT_NBUF], (f / KT_NBUF) & 1);
-                const SrcT* box = (const SrcT*)(smem + (f % KT_NBUF) * KT_BOX_BYTES);
-#pragma unroll
-                for (int j = 0; j < KT_PX; ++j) {
-                    const SrcT* p = box + so[j];
-                    const DstT r = blend_out<SrcT, DstT>(p[0], p[1], p[BW], p[BW + 1], wt[j], a.q);
-                    sts_if(ot + j * KT_RSTEP * KT_TW, r, fast & (1u << j));
-                }
-            }
-            if (slow) {
-#pragma unroll 1
-                for (int j = 0; j < KT_PX; ++j)
-                    if (slow & (1u << j)) ot[j * KT_RSTEP * KT_TW] = slow_pixel(src, j);
-            }
-            fence_proxy_async_smem();                  // generic-proxy writes of the tile -> visible to the TMA store
-            if (tid == 0) tma_store_wait_read<0>();    // the store of frame f-1 has read its tile: the other buffer is free again
-            __syncthreads();                           // tile complete; everyone is done with this source box
-            if (tid == 0) {
-                tma_store_3d(&tm_dst, otile + (f & 1) * (KT_TW * KT_TH), tx0, ty0, f);
-                tma_store_commit();
-                if (have_box && f + KT_NBUF < nf) issue(f + KT_NBUF, bx, by);
-            }
-            src += src_stride;
+            for (int j = 0; j < KT_PX; ++j)
+                if (slow & (1u << j)) dst[j * dstep] = slow_pixel(src, j);
         }
-        if (tid == 0) tma_store_wait_read<0>();
-        return;
-    }
-    DstT* dst = (DstT*)a.dst + (oy0 * ow + ox);
-    const int dstep = KT_RSTEP * ow;
-    // KT_FPB frames per CTA barrier: the ring holds KT_NBUF boxes, KT_FPB of them are blended between two barriers and
-    // refilled together (one barrier per frame cost 0.85-2.9 stall cycles per issued instruction in the profiles)
-    constexpr int FPB = (KT_NBUF % KT_FPB == 0 && KT_NBUF >= 2 * KT_FPB) ? KT_FPB : 1;
-#pragma unroll 1
-    for (int f0 = 0; f0 < nf; f0 += FPB) {
-#pragma unroll
-        for (int g = 0; g < FPB; ++g) {
-            const int f = f0 + g;
-            if (f < nf) {
-                if (have_box) {
-                    mbar_wait(&full[f % KT_NBUF], (f / KT_NBUF) & 1);
-                    const SrcT* box = (const SrcT*)(smem + (f % KT_NBUF) * KT_BOX_BYTES);
-#pragma unroll
-                    for (int j = 0; j < KT_PX; ++j) {
-                        const SrcT* p = box + so[j];
-                        const DstT r = blend_out<SrcT, DstT>(p[0], p[1], p[BW], p[BW + 1], wt[j], a.q);
-                        st_if(dst + j * dstep, r, fast & (1u << j));            // predicated store, no branch around the gather
-                    }
-                }
-                if (outm) {
-#pragma unroll
-                    for (int j = 0; j < KT_PX; ++j)
-                        if (outm & (1u << j)) dst[j * dstep] = bout;
-                }
-                if (slow) {
-#pragma unroll 1
-                    for (int j = 0; j < KT_PX; ++j)
-                        if (slow & (1u << j)) dst[j * dstep] = slow_pixel(src, j);
-                }
-                src += src_stride;
-                dst += dst_stride;
-            }
-        }
+        src += src_stride;
+        dst += dst_stride;
         if (have_box) {
-            __syncthreads();                           // everyone is done with these buffers
-            if (tid == 0)
-                for (int g = 0; g < FPB; ++g)
-                    if (f0 + g + KT_NBUF < nf) issue(f0 + g + KT_NBUF, bx, by);
+            __syncthreads();                           // everyone is done with this buffer
+            if (tid == 0 && f + KT_NBUF < nf) issue(f + KT_NBUF, bx, by);
         }
     }
 }
@@ -597,7 +524,7 @@ template <typename T> static CUtensorMapDataType kt_dtype() {
 // mbarrier — so DRAM latency is covered across tiles as well as across frames: a ONE-frame launch streams like a batch
 // (the analytic kernel above serialises box latency -> blend -> store per CTA and is issue bound on top of that).
 // Per item: wait, (new tile: unpack offsets, weights from OpenCV's table, pixel classes), four shared-memory gathers and
-// the blend per pixel, output tile to shared memory, one TMA store.  No lens arithmetic except for "slow" pixels.
+// the blend per pixel, predicated per-pixel stores.  No lens arithmetic except for "slow" pixels.
 #ifndef KC_NBUF
 #define KC_NBUF 3
 #endif
@@ -607,10 +534,9 @@ constexpr int KC_MAXT = 256;
 #ifndef KC_MINB
 #define KC_MINB 3           // 85 registers: 46 vs 51 us for one 4096x3000 frame with 4 CTAs of 64 registers
 #endif
-template <typename SrcT, typename DstT, typename G, bool TSTORE>
+template <typename SrcT, typename DstT, typename G>
 __global__ void __launch_bounds__(KT_THREADS, KC_MINB)
-k2_cached_kernel(const __grid_constant__ CUtensorMap tm_src, const __grid_constant__ CUtensorMap tm_dst, K2Args a, int tiles_x,
-                 long long n_items) {
+k2_cached_kernel(const __grid_constant__ CUtensorMap tm_src, K2Args a, int tiles_x, long long n_items) {
     constexpr int KT_TW = G::TW, KT_TH = G::TH, KT_BH = G::BH, NBUF = KcGeom<G>::NBUF;
     constexpr int KT_PX = KT_TW * KT_TH / KT_THREADS, KT_RSTEP = KT_THREADS / KT_TW;
     constexpr int BW = KtBox<SrcT, G>::BW, BOX_BYTES = KtBox<SrcT, G>::BYTES;
@@ -619,7 +545,6 @@ k2_cached_kernel(const __grid_constant__ CUtensorMap tm_src, const __grid_consta
     uint64_t* full = (uint64_t*)(smem + NBUF * SLOT);
     int* meta = (int*)(smem + NBUF * SLOT + 64);               // per slot: the item's tile has a box
     int2* hdrs = (int2*)(smem + NBUF * SLOT + 128);             // box origins of this CTA's tiles (KC_MAXT of them)
-    DstT* otile = (DstT*)(smem + NBUF * SLOT + 128 + KC_MAXT * 8); // [2][TH][TW] when TSTORE
     const int tid = threadIdx.x;
     const int c = tid % KT_TW, r0 = tid / KT_TW;
     const int H = a.H, W = a.W, nf = a.n_frames, ow = a.ow, oh = a.oh;
@@ -708,83 +633,49 @@ k2_cached_kernel(const __grid_constant__ CUtensorMap tm_src, const __grid_consta
             }
         }
         const SrcT* src = (const SrcT*)a.src + (size_t)f * src_stride;
-        if (TSTORE) {
-            DstT* ot = otile + (k & 1) * (KT_TW * KT_TH) + r0 * KT_TW + c;
-            if (have_box) {
-                const SrcT* box = (const SrcT*)base;
+        DstT* dst = (DstT*)a.dst + (size_t)f * dst_stride + ((ty0 + r0) * ow + tx0 + c);
+        const int dstep = KT_RSTEP * ow;
+        if (have_box) {
+            const SrcT* box = (const SrcT*)base;
 #pragma unroll
-                for (int j = 0; j < KT_PX; ++j) {
-                    const SrcT* p = box + so[j];
-                    const DstT r = blend_out<SrcT, DstT>(p[0], p[1], p[BW], p[BW + 1], wt[j], a.q);
-                    sts_if(ot + j * KT_RSTEP * KT_TW, r, fast & (1u << j));
-                }
+            for (int j = 0; j < KT_PX; ++j) {
+                const SrcT* p = box + so[j];
+                const DstT r = blend_out<SrcT, DstT>(p[0], p[1], p[BW], p[BW + 1], wt[j], a.q);
+                st_if(dst + j * dstep, r, fast & (1u << j));
             }
-            if (outm) {
-#pragma unroll
-                for (int j = 0; j < KT_PX; ++j)
-                    if (outm & (1u << j)) ot[j * KT_RSTEP * KT_TW] = bout;
-            }
-            if (slow) {
-#pragma unroll 1
-                for (int j = 0; j < KT_PX; ++j)
-                    if (slow & (1u << j)) ot[j * KT_RSTEP * KT_TW] = slow_pixel(src, j);
-            }
-            fence_proxy_async_smem();                  // generic-proxy writes of the tile -> visible to the TMA store
-            if (tid == 0) tma_store_wait_read<0>();    // the previous store has read its tile: the other buffer is free again
-            __syncthreads();                           // tile complete; everyone is done with this slot
-            if (tid == 0) {
-                tma_store_3d(&tm_dst, otile + (k & 1) * (KT_TW * KT_TH), tx0, ty0, f);
-                tma_store_commit();
-                if (p_k < n_mine) issue();
-            }
-        } else {
-            DstT* dst = (DstT*)a.dst + (size_t)f * dst_stride + ((ty0 + r0) * ow + tx0 + c);
-            const int dstep = KT_RSTEP * ow;
-            if (have_box) {
-                const SrcT* box = (const SrcT*)base;
-#pragma unroll
-                for (int j = 0; j < KT_PX; ++j) {
-                    const SrcT* p = box + so[j];
-                    const DstT r = blend_out<SrcT, DstT>(p[0], p[1], p[BW], p[BW + 1], wt[j], a.q);
-                    st_if(dst + j * dstep, r, fast & (1u << j));
-                }
-            }
-            if (outm) {
-#pragma unroll
-                for (int j = 0; j < KT_PX; ++j)
-                    if (outm & (1u << j)) dst[j * dstep] = bout;
-            }
-            if (slow) {
-#pragma unroll 1
-                for (int j = 0; j < KT_PX; ++j)
-                    if (slow & (1u << j)) dst[j * dstep] = slow_pixel(src, j);
-            }
-            __syncthreads();                           // everyone is done with this slot
-            if (tid == 0 && p_k < n_mine) issue();
         }
+        if (outm) {
+#pragma unroll
+            for (int j = 0; j < KT_PX; ++j)
+                if (outm & (1u << j)) dst[j * dstep] = bout;
+        }
+        if (slow) {
+#pragma unroll 1
+            for (int j = 0; j < KT_PX; ++j)
+                if (slow & (1u << j)) dst[j * dstep] = slow_pixel(src, j);
+        }
+        __syncthreads();                               // everyone is done with this slot
+        if (tid == 0 && p_k < n_mine) issue();
         if (++f == nf) { f = 0; tile += gridDim.x; }
         if (++slot == NBUF) slot = 0;
     }
-    if (TSTORE && tid == 0) tma_store_wait_read<0>();
 }
 
-template <typename SrcT, typename DstT, typename G, bool TSTORE>
+template <typename SrcT, typename DstT, typename G>
 static cudaError_t launch_cached_g(const K2Args& a, cudaStream_t st) {
-    CUtensorMap tm, td;
+    CUtensorMap tm;
     if (!make_tensor_map(&tm, kt_dtype<SrcT>(), sizeof(SrcT), a.src, a.W, a.H, a.n_frames, KtBox<SrcT, G>::BW, G::BH)) return cudaErrorInvalidValue;
-    td = tm;
-    if (TSTORE && !make_tensor_map(&td, kt_dtype<DstT>(), sizeof(DstT), a.dst, a.ow, a.oh, a.n_frames, G::TW, G::TH)) return cudaErrorInvalidValue;
     const int tiles_x = (a.ow + G::TW - 1) / G::TW, tiles_y = (a.oh + G::TH - 1) / G::TH;
     const long long n_items = (long long)tiles_x * tiles_y * a.n_frames;
     if (n_items > 0x7fffffffLL) return cudaErrorInvalidValue;
-    constexpr int SMEM = KcGeom<G>::NBUF * (KtBox<SrcT, G>::BYTES + G::TW * G::TH * 4) + 128 + KC_MAXT * 8 + (TSTORE ? 2 * G::TW * G::TH * (int)sizeof(DstT) : 0);
-    auto kern = k2_cached_kernel<SrcT, DstT, G, TSTORE>;
+    constexpr int SMEM = KcGeom<G>::NBUF * (KtBox<SrcT, G>::BYTES + G::TW * G::TH * 4) + 128 + KC_MAXT * 8;
+    auto kern = k2_cached_kernel<SrcT, DstT, G>;
     cudaError_t e = cudaSuccess;
     const int per_sm = blocks_per_sm_cached((const void*)kern, KT_THREADS, SMEM, &e);
     if (e != cudaSuccess) return e;
     long long grid = (long long)(a.sm_count > 0 ? a.sm_count : 148) * per_sm;
     if (grid > (long long)tiles_x * tiles_y) grid = (long long)tiles_x * tiles_y;
-    kern<<<(unsigned)grid, KT_THREADS, SMEM, st>>>(tm, td, a, tiles_x, n_items);
+    kern<<<(unsigned)grid, KT_THREADS, SMEM, st>>>(tm, a, tiles_x, n_items);
     return cudaGetLastError();
 }
 
@@ -797,50 +688,35 @@ static bool k2_tiled_eligible(const K2Args& a, int src_dtype, int dst_dtype) {
     return tensor_map_encoder() != nullptr;
 }
 
-template <typename SrcT, typename DstT, typename G, bool TSTORE>
+template <typename SrcT, typename DstT, typename G>
 static cudaError_t launch_tiled_g(const K2Args& a, cudaStream_t st) {
-    CUtensorMap tm, td;
+    CUtensorMap tm;
     if (!make_tensor_map(&tm, kt_dtype<SrcT>(), sizeof(SrcT), a.src, a.W, a.H, a.n_frames, KtBox<SrcT, G>::BW, G::BH)) return cudaErrorInvalidValue;
-    td = tm;
-    if (TSTORE && !make_tensor_map(&td, kt_dtype<DstT>(), sizeof(DstT), a.dst, a.ow, a.oh, a.n_frames, G::TW, G::TH)) return cudaErrorInvalidValue;
     dim3 grid((a.ow + G::TW - 1) / G::TW, (a.oh + G::TH - 1) / G::TH);
-    constexpr int SMEM = kt_smem<SrcT, DstT, G, TSTORE>();
-    void (*kern)(const CUtensorMap, const CUtensorMap, K2Args);
+    constexpr int SMEM = kt_smem<SrcT, G>();
+    void (*kern)(const CUtensorMap, K2Args);
     const bool sep = a.lens.affine && a.lens.ir[1] == 0.0 && a.lens.ir[3] == 0.0;
-    if (a.cpack && !a.mapx) return launch_cached_g<SrcT, DstT, G, TSTORE>(a, st);
+    if (a.cpack && !a.mapx) return launch_cached_g<SrcT, DstT, G>(a, st);
     if constexpr (K2Quant<SrcT, DstT>::value) if (a.mapx) return cudaErrorNotSupported;    // the chain remaps with the analytic map only
-    if (a.mapx) kern = k2_tiled_kernel<SrcT, DstT, 0, G, TSTORE, 0>;
-    else if (a.cpack_w) kern = sep ? k2_tiled_kernel<SrcT, DstT, 2, G, TSTORE, 1> : k2_tiled_kernel<SrcT, DstT, 1, G, TSTORE, 1>;
-    else kern = sep ? k2_tiled_kernel<SrcT, DstT, 2, G, TSTORE, 0> : k2_tiled_kernel<SrcT, DstT, 1, G, TSTORE, 0>;
+    if (a.mapx) kern = k2_tiled_kernel<SrcT, DstT, 0, G, 0>;
+    else if (a.cpack_w) kern = sep ? k2_tiled_kernel<SrcT, DstT, 2, G, 1> : k2_tiled_kernel<SrcT, DstT, 1, G, 1>;
+    else kern = sep ? k2_tiled_kernel<SrcT, DstT, 2, G, 0> : k2_tiled_kernel<SrcT, DstT, 1, G, 0>;
     if (SMEM > 48 * 1024) {
         cudaError_t e = cudaSuccess;
         blocks_per_sm_cached((const void*)kern, KT_THREADS, SMEM, &e);       // opt-in to > 48 KB, once per (device, kernel)
         if (e != cudaSuccess) return e;
     }
-    kern<<<grid, KT_THREADS, SMEM, st>>>(tm, td, a);
+    kern<<<grid, KT_THREADS, SMEM, st>>>(tm, a);
     return cudaGetLastError();
 }
 
 template <typename SrcT, typename DstT>
 static cudaError_t launch_tiled_t(const K2Args& a, cudaStream_t st) {
-    // the output tile leaves by TMA when the destination qualifies (16-byte aligned rows), else by predicated stores
-    // The output tile can leave through shared memory as one TMA store per frame (UTMASTG) when the destination qualifies
-    // (16-byte aligned rows).  Measured on B200 it is SLOWER than the predicated per-pixel stores of the other path (21.0 vs
-    // 20.1 us per 4096x3000 frame in batches: the tile costs an STS per pixel, a proxy fence and a longer barrier per frame,
-    // while the plain stores are already full 128-byte lines per warp), so it is an option (IMGCORR_OPT_K2_TMA_STORE), off by default.
-    // (the F32 -> U16 / U8 pairs are built without the TMA-store option: they always store per pixel)
-    const bool tstore = !K2Quant<SrcT, DstT>::value && a.tma_store && ((size_t)a.ow * sizeof(DstT)) % 16 == 0 && ((uintptr_t)a.dst) % 16 == 0;
     const int g = a.geometry;
-    if constexpr (!K2Quant<SrcT, DstT>::value) if (tstore) {
-        if (g == 3) return launch_tiled_g<SrcT, DstT, KtG3, true>(a, st);
-        if (g == 2) return launch_tiled_g<SrcT, DstT, KtG2, true>(a, st);
-        if (g == 1) return launch_tiled_g<SrcT, DstT, KtG1, true>(a, st);
-        return launch_tiled_g<SrcT, DstT, KtG0, true>(a, st);
-    }
-    if (g == 3) return launch_tiled_g<SrcT, DstT, KtG3, false>(a, st);
-    if (g == 2) return launch_tiled_g<SrcT, DstT, KtG2, false>(a, st);
-    if (g == 1) return launch_tiled_g<SrcT, DstT, KtG1, false>(a, st);
-    return launch_tiled_g<SrcT, DstT, KtG0, false>(a, st);
+    if (g == 3) return launch_tiled_g<SrcT, DstT, KtG3>(a, st);
+    if (g == 2) return launch_tiled_g<SrcT, DstT, KtG2>(a, st);
+    if (g == 1) return launch_tiled_g<SrcT, DstT, KtG1>(a, st);
+    return launch_tiled_g<SrcT, DstT, KtG0>(a, st);
 }
 
 // words of the coordinate cache for an output window under geometry g (whole tiles) and the number of tiles

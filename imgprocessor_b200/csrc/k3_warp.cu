@@ -264,131 +264,6 @@ __global__ void __launch_bounds__(K3T_THREADS, K3T_MINB_V) k3_tiled_kernel(const
     }
 }
 
-// The same tiles with one matrix per frame (a.wcs, float32 sources): the TMA box, and whether the tile's windows fit it,
-// are per-frame quantities, and the producer issues frame f's box K3T_NBUF frames ahead.  So iteration f computes every
-// pixel's coordinate of frame f + NBUF, reduces it into that frame's box (REDUX + shared atomics, double-buffered over
-// 2 * NBUF frames so that a box is never reset while it is still read), and keeps the coordinate in shared memory for
-// the iteration that uses it; the per-frame barrier publishes the box before thread 0 issues the load.  A frame whose
-// windows do not fit takes the global gathers for this tile only; `fits` is read from shared memory, so it is CTA-uniform.
-constexpr int K3T_RED_BYTES = 2 * K3T_NBUF * 4 * (int)sizeof(int);
-constexpr int K3T_COORD_BYTES = K3T_NBUF * K3T_THREADS * (int)sizeof(int2);
-constexpr int k3t_frames_smem() { return K3T_NBUF * k3t_box_bytes<float>() + K3T_COORD_BYTES + 64 + K3T_RED_BYTES; }
-
-template <int N, typename DT>
-__global__ void __launch_bounds__(K3T_THREADS, K3T_MINB_V) k3_tiled_frames_kernel(const __grid_constant__ CUtensorMap tm_src, const K3Args a) {
-    constexpr int BW = K3Box<float>::BW, BOX_BYTES = k3t_box_bytes<float>(), RING = K3T_NBUF * BOX_BYTES;
-    constexpr int OFF = N / 2 - 1, NRED = 2 * K3T_NBUF;
-    extern __shared__ __align__(128) uint8_t smem[];
-    __shared__ float tab[N][32];
-    int2* coords = (int2*)(smem + RING);                       // [NBUF][threads]: (X, Y) of frame k in slot k % NBUF
-    uint64_t* full = (uint64_t*)(smem + RING + K3T_COORD_BYTES);
-    int* red = (int*)(smem + RING + K3T_COORD_BYTES + 64);     // [2 * NBUF][min sx, max sx + N - 1, min sy, max sy + N - 1]
-    const int tid = threadIdx.x;
-    if (tid == 0) {
-        for (int b = 0; b < K3T_NBUF; ++b) mbar_init(&full[b], 1);
-        for (int k = 0; k < NRED; ++k) { red[4 * k] = 0x7fffffff; red[4 * k + 1] = -1; red[4 * k + 2] = 0x7fffffff; red[4 * k + 3] = -1; }
-        mbar_init_fence();
-    }
-    for (int i = tid; i < N * 32; i += K3T_THREADS) tab[i % N][i / N] = a.tab[i];
-    const int x = blockIdx.x * K3T_TW + (tid % K3T_TW), y = blockIdx.y * K3T_TH + (tid / K3T_TW);
-    const bool live = x < a.dw && y < a.dh;
-    const int H = a.H, W = a.W, nf = a.n_frames;
-    const int w1 = max(W - (N - 1), 0), h1 = max(H - (N - 1), 0);
-    __syncthreads();                                   // red[], the barriers and the table are ready
-
-    // frame k: this pixel's coordinate into coords[k % NBUF], its window into the box of frame k
-    auto stage = [&](int k) {
-        const FixedCoord c = warp_coord(a.wcs[k], live ? x : 0, live ? y : 0);
-        coords[(k % K3T_NBUF) * K3T_THREADS + tid] = make_int2((int)(((unsigned)c.ix << 5) | c.fx), (int)(((unsigned)c.iy << 5) | c.fy));
-        const int sx = c.ix - OFF, sy = c.iy - OFF;
-        const bool interior = live && (unsigned)sx < (unsigned)w1 && (unsigned)sy < (unsigned)h1;
-        const int mnx = __reduce_min_sync(0xffffffffu, interior ? sx : 0x7fffffff);
-        const int mxx = __reduce_max_sync(0xffffffffu, interior ? sx + N - 1 : -1);
-        const int mny = __reduce_min_sync(0xffffffffu, interior ? sy : 0x7fffffff);
-        const int mxy = __reduce_max_sync(0xffffffffu, interior ? sy + N - 1 : -1);
-        int* r = red + 4 * (k % NRED);
-        if ((tid & 31) == 0) { atomicMin(&r[0], mnx); atomicMax(&r[1], mxx); atomicMin(&r[2], mny); atomicMax(&r[3], mxy); }
-    };
-    struct Box { int bx, by; bool fits; };
-    auto box = [&](int k) {
-        const int* r = red + 4 * (k % NRED);
-        Box b;
-        b.bx = r[0] & ~(K3Box<float>::GRAN - 1);
-        b.by = r[2];
-        b.fits = r[1] >= 0 && (r[1] + 1 - b.bx) <= BW && (r[3] + 1 - b.by) <= K3T_BH;
-        return b;
-    };
-    auto issue = [&](int k) {                          // thread 0, after a barrier that follows frame k's stage()
-        const Box b = box(k);
-        if (!b.fits) return;
-        uint64_t* bar = &full[k % K3T_NBUF];
-        mbar_expect_tx(bar, BOX_BYTES);
-        tma_load_3d(smem + (k % K3T_NBUF) * BOX_BYTES, &tm_src, bar, b.bx, b.by, k);
-    };
-    for (int k = 0; k < K3T_NBUF && k < nf; ++k) stage(k);
-    __syncthreads();
-    if (tid == 0) for (int k = 0; k < K3T_NBUF && k < nf; ++k) issue(k);
-
-    const size_t spx = (size_t)H * W, dpx = (size_t)a.dh * a.dw;
-    DT* D = (DT*)a.dst + ((size_t)(live ? y : 0) * a.dw + (live ? x : 0));
-    const float cv = (float)a.border;
-    uint32_t phase = 0;                                // bit b: parity of the next wait on full[b] (only fitting frames load)
-#pragma unroll 1
-    for (int f = 0; f < nf; ++f) {
-        const Box b = box(f);
-        const int2 xy = coords[(f % K3T_NBUF) * K3T_THREADS + tid];
-        if (f + K3T_NBUF < nf) stage(f + K3T_NBUF);     // into the coordinate slot just read; its latency hides behind the wait
-        const int sx = (xy.x >> 5) - OFF, sy = (xy.y >> 5) - OFF;
-        float wy[N], wx[N];
-#pragma unroll
-        for (int i = 0; i < N; ++i) {
-            wy[i] = tab[i][xy.y & 31];
-            wx[i] = tab[i][xy.x & 31];
-        }
-        const bool interior = live && (unsigned)sx < (unsigned)w1 && (unsigned)sy < (unsigned)h1;
-        const float* S = (const float*)a.src + f * spx;
-        if (b.fits) {
-            const int slot = f % K3T_NBUF;
-            mbar_wait(&full[slot], (phase >> slot) & 1);
-            phase ^= 1u << slot;
-            if (interior) {
-                const float* P = (const float*)(smem + slot * BOX_BYTES) + ((sy - b.by) * K3T_PITCH + (sx - b.bx));
-                float v = 0.0f;
-#pragma unroll
-                for (int r = 0; r < N; ++r) {
-                    float acc = fmul(P[r * K3T_PITCH], fmul(wy[r], wx[0]));
-#pragma unroll
-                    for (int k = 1; k < N; ++k) acc = fadd(acc, fmul(P[r * K3T_PITCH + k], fmul(wy[r], wx[k])));
-                    v = fadd(v, acc);
-                }
-                D[f * dpx] = k3_out<float, DT>(v, a.q);
-            }
-        } else if (interior) {
-            const float* P = S + ((long long)sy * W + sx);
-            float v = 0.0f;
-#pragma unroll
-            for (int r = 0; r < N; ++r) {
-                float acc = fmul(ldg(P), fmul(wy[r], wx[0]));
-#pragma unroll
-                for (int k = 1; k < N; ++k) acc = fadd(acc, fmul(ldg(P + k), fmul(wy[r], wx[k])));
-                v = fadd(v, acc);
-                P += W;
-            }
-            D[f * dpx] = k3_out<float, DT>(v, a.q);
-        }
-        if (live && !interior) {
-            const bool outside = sx >= W || sx + N <= 0 || sy >= H || sy + N <= 0;
-            D[f * dpx] = k3_out<float, DT>(outside ? cv : warp_border_ool<float, float, N>(S, H, W, sx, sy, wy, wx, cv), a.q);
-        }
-        __syncthreads();                               // the ring buffer is free, box f + NBUF is complete, box f is read
-        if (tid == 0) {
-            int* r = red + 4 * (f % NRED);              // next filled for frame f + 2 * NBUF, after at least one more barrier
-            r[0] = 0x7fffffff; r[1] = -1; r[2] = 0x7fffffff; r[3] = -1;
-            if (f + K3T_NBUF < nf) issue(f + K3T_NBUF);
-        }
-    }
-}
-
 template <typename T>
 bool k3_tiled_eligible(const K3Args& a) {
     if (((size_t)a.W * sizeof(T)) % 16 || ((uintptr_t)a.src) % 16) return false;
@@ -459,19 +334,9 @@ cudaError_t launch_typed(const K3Args& a, int interp, cudaStream_t st) {
     return cudaGetLastError();
 }
 
-// one matrix per frame (a.wcs), Lanczos4: T = float (staged tiles or L1 gathers) to float / U16 / U8, or double to double
+// one matrix per frame (a.wcs), Lanczos4 through L1: float to float / U16 / U8, or double to double
 template <typename T, typename DT>
-cudaError_t launch_frames(const K3Args& a, bool tiled, cudaStream_t st) {
-    if constexpr (std::is_same<T, float>::value) {
-        if (tiled) {
-            CUtensorMap tm;
-            if (!make_tensor_map(&tm, K3Box<float>::DT, sizeof(float), a.src, a.W, a.H, a.n_frames, K3Box<float>::BW, K3T_BH))
-                return cudaErrorInvalidValue;
-            dim3 grid((a.dw + K3T_TW - 1) / K3T_TW, (a.dh + K3T_TH - 1) / K3T_TH);
-            k3_tiled_frames_kernel<8, DT><<<grid, K3T_THREADS, k3t_frames_smem(), st>>>(tm, a);
-            return cudaGetLastError();
-        }
-    }
+cudaError_t launch_frames(const K3Args& a, cudaStream_t st) {
     dim3 block(K3_BX, K3_BY), grid((a.dw + K3_BX - 1) / K3_BX, (a.dh + K3_BY - 1) / K3_BY);
     k3_warp_kernel<T, T, 8, DT, true><<<grid, block, 0, st>>>(a);
     return cudaGetLastError();
@@ -479,29 +344,32 @@ cudaError_t launch_frames(const K3Args& a, bool tiled, cudaStream_t st) {
 
 }  // namespace
 
-// variant: 0 auto, 1 gathers through L1, 2 shared-memory staged tiles (uint16 / float32; fails if not eligible)
+// variant: 0 auto, 1 gathers through L1, 2 shared-memory staged tiles (uint16 / float32, one matrix per launch; fails if
+// not eligible)
 cudaError_t launch_k3(const K3Args& a, int dtype, int interp, int variant, cudaStream_t st, int* launches) {
     if (a.n_frames <= 0 || a.dw <= 0 || a.dh <= 0) return cudaSuccess;
     if (interp != WARP_LANCZOS4 && interp != WARP_CUBIC) return cudaErrorInvalidValue;
-    // measured (4096x3000, B200): the staged tiles win for Lanczos4 once a launch carries a few frames (float32 138 vs
-    // 160 us/frame, uint16 174 vs 224); a single frame and the 4x4 bicubic window are faster straight through L1, and so
-    // is a launch with a per-frame table (tools/perframe_warp.py, DESIGN §4 "Chain, host pipeline, batches")
-    const bool wanted = variant == 2 || (variant == 0 && interp == WARP_LANCZOS4 && a.n_frames >= 4 && !a.wcs);
-    if (variant == 2 && dtype == DT_U8) return cudaErrorNotSupported;
-    const bool tiled = wanted && ((dtype == DT_U16 && k3_tiled_eligible<uint16_t>(a)) || (dtype == DT_F32 && k3_tiled_eligible<float>(a)));
-    if (variant == 2 && !tiled) return cudaErrorNotSupported;
     cudaError_t e;
     if (a.wcs) {
-        // the chain's per-frame table: float32 frames to float32 / U16 / U8, float64 frames to float64
+        // the chain's per-frame table: float32 frames to float32 / U16 / U8, float64 frames to float64.  Measured (4096x3000,
+        // B200) it is faster through L1 than through staged tiles (tools/perframe_warp.py, DESIGN §4 "Chain, host pipeline,
+        // batches"), so it has no tiled kernel
+        if (variant == 2) return cudaErrorNotSupported;
         if (interp != WARP_LANCZOS4) return cudaErrorInvalidValue;
-        if (dtype == DT_F64 && a.dst_dtype == DT_F64) e = launch_frames<double, double>(a, false, st);
-        else if (dtype == DT_F32 && a.dst_dtype == DT_F32) e = launch_frames<float, float>(a, tiled, st);
-        else if (dtype == DT_F32 && a.dst_dtype == DT_U16) e = launch_frames<float, uint16_t>(a, tiled, st);
-        else if (dtype == DT_F32 && a.dst_dtype == DT_U8) e = launch_frames<float, uint8_t>(a, tiled, st);
+        if (dtype == DT_F64 && a.dst_dtype == DT_F64) e = launch_frames<double, double>(a, st);
+        else if (dtype == DT_F32 && a.dst_dtype == DT_F32) e = launch_frames<float, float>(a, st);
+        else if (dtype == DT_F32 && a.dst_dtype == DT_U16) e = launch_frames<float, uint16_t>(a, st);
+        else if (dtype == DT_F32 && a.dst_dtype == DT_U8) e = launch_frames<float, uint8_t>(a, st);
         else return cudaErrorInvalidValue;
         if (launches) ++*launches;
         return e;
     }
+    // measured (4096x3000, B200): the staged tiles win for Lanczos4 once a launch carries a few frames (float32 138 vs
+    // 160 us/frame, uint16 174 vs 224); a single frame and the 4x4 bicubic window are faster straight through L1
+    const bool wanted = variant == 2 || (variant == 0 && interp == WARP_LANCZOS4 && a.n_frames >= 4);
+    if (variant == 2 && dtype == DT_U8) return cudaErrorNotSupported;
+    const bool tiled = wanted && ((dtype == DT_U16 && k3_tiled_eligible<uint16_t>(a)) || (dtype == DT_F32 && k3_tiled_eligible<float>(a)));
+    if (variant == 2 && !tiled) return cudaErrorNotSupported;
     if (a.dst_dtype != dtype) {
         // float32 source, integer destination: the float32 warp of the F32 call, stored through the quantiser
         if (dtype != DT_F32 || (a.dst_dtype != DT_U16 && a.dst_dtype != DT_U8)) return cudaErrorInvalidValue;

@@ -86,9 +86,9 @@ enum {
     IMGCORR_OPT_K2_COORD_CACHE = 11, /* 1 (default): the first tiled K2 launch for a lens / output window stores the packed fixed-point source
                                        coordinates it computed (4 bytes per pixel of device memory, at most two windows), later launches read them
                                        instead of re-evaluating the float64 lens model; 0: evaluate on every launch */
-    IMGCORR_OPT_K2_TMA_STORE = 12,  /* 1: the tiled K2 writes its output tile through shared memory and one TMA store per frame (destination rows must be
-                                       16-byte multiples); 0 (default): predicated per-pixel stores, measured faster on B200 */
-    IMGCORR_OPT_K3_VARIANT = 9      /* 0 auto, 1 gathers through L1/L2, 2 shared-memory staged tiles (uint16 / float32 sources; fails if not eligible) */
+    /* key 12 is retired and not reused */
+    IMGCORR_OPT_K3_VARIANT = 9      /* 0 auto, 1 gathers through L1/L2, 2 shared-memory staged tiles (uint16 / float32 sources; fails if not eligible;
+                                       a launch with a per-frame table, as imgcorr_correct_batch's per-frame homographies, is never eligible) */
 };
 
 IMGCORR_API const char* imgcorr_last_error(void);

@@ -439,7 +439,7 @@ def test_k2_coordinate_cache(ip, shape, lens_kind):
     the following ones (IMGCORR_OPT_K2_COORD_CACHE): first launch, cached launches, cache switched off and the oracle all
     agree bit for bit — whole frame and roi window, float32 / float64 / uint16 outputs, any box geometry (the strong and
     the extreme lens need the larger staged boxes; tiles the box cannot cover fall back to gathers), border values;
-    a new lens drops the cache"""
+    a new lens drops the cache.  Option key 12 (retired) is refused."""
     H, W = shape
     p = {'moderate': synth.lens_moderate(H, W), 'strong': synth.lens_strong(H, W),
          'extreme': (0.45 * W, 0.45 * W, W / 2.0 + 3, H / 2.0 - 2, -0.3, 0.12, -0.02, 4e-3, -3e-3)}[lens_kind]
@@ -449,10 +449,12 @@ def test_k2_coordinate_cache(ip, shape, lens_kind):
     rng = np.random.default_rng(11)
     src = (rng.random((5, H, W)) * 4000).astype(np.float32)
     x0, y0, ww, hh = (int(v) for v in roi)
+    with pytest.raises(ip.lib_mod.ImgcorrError) as err:
+        e.set_option(12, 1)
+    assert err.value.status == ip.lib_mod.ERR_INVALID
     try:
-        for cache in (1, 0, 2):                                    # 2: cache on + output tile through TMA stores
-            e.set_option(ip.lib_mod.OPT_K2_COORD_CACHE, 1 if cache else 0)
-            e.set_option(ip.lib_mod.OPT_K2_TMA_STORE, 1 if cache == 2 else 0)
+        for cache in (1, 0):
+            e.set_option(ip.lib_mod.OPT_K2_COORD_CACHE, cache)
             e.set_lens(K, d, P)                                    # drops any cache of an earlier test
             for rep in range(3):                                   # 1st: computes (and writes), 2nd / 3rd: read
                 for border in (0.0, 7.5):
@@ -469,7 +471,7 @@ def test_k2_coordinate_cache(ip, shape, lens_kind):
             if cache == 1:
                 cached = a
             else:
-                assert np.array_equal(a, cached)                   # cache on == cache off == TMA stores, bit for bit
+                assert np.array_equal(a, cached)                   # cache on == cache off, bit for bit
             wide = e.undistort(_dev(src[0]), out_dtype=torch.float64).cpu().numpy()
             assert np.array_equal(wide, a[0].astype(np.float64))
         e.set_option(ip.lib_mod.OPT_K2_COORD_CACHE, 1)
@@ -493,7 +495,6 @@ def test_k2_coordinate_cache(ip, shape, lens_kind):
         assert (got != models.remap_model(src[0], mapx2, mapy2, 0)).mean() < 1e-5
     finally:
         e.set_option(ip.lib_mod.OPT_K2_COORD_CACHE, 1)
-        e.set_option(ip.lib_mod.OPT_K2_TMA_STORE, 0)
         e.set_lens(None, None, None)
 
 

@@ -75,7 +75,7 @@ def test_device_frames_vs_oracle(ip, shape, dtype):
     a zoom-out whose windows do not fit K3's staged box, next to frames whose windows fit.  Base: lens on, full frame,
     float32 out, K3 variant auto (its L1 gathers for a table).  Then the lens off, the roi window, float64 out (with and
     without the roi), uint16 out (quantise of the float32 result), and K3 forced to its L1 gathers (1) and to its staged
-    tiles (2; refused where the chain frame's float32 rows are not 16-byte multiples)."""
+    tiles (2: refused, a table is never eligible for them)."""
     H, W = shape
     n = 6
     L = ip.lib_mod
@@ -96,7 +96,7 @@ def test_device_frames_vs_oracle(ip, shape, dtype):
                 e.set_perspective(Ms, dsize, 2.5)
                 tdt = {np.float32: torch.float32, np.float64: torch.float64, np.uint16: torch.uint16}[c['odt']]
                 call = lambda: e.correct_batch(dev, flags=fl, use_lens=c['lens'], window=c['window'], out_dtype=tdt)  # noqa: E731
-                if c['variant'] == 2 and _src_shape(e, c['window'], c['lens'])[1] % 4:   # rows not 16-byte multiples
+                if c['variant'] == 2:
                     with pytest.raises(L.ImgcorrError) as err:
                         call()
                     assert err.value.status == L.ERR_INVALID
@@ -116,9 +116,8 @@ def test_device_frames_vs_oracle(ip, shape, dtype):
 
 # ---------------------------------------------------------------------------------------------- 2. group seams
 def test_group_seams_vs_oracle(ip):
-    """11 frames in groups of 4 (4 + 4 + 3), overlap on and off: with the lens and the roi in float32 (K3's L1 gathers),
-    with the lens on the full frame in float32 and K3 forced to its staged tiles, and without a lens in float64.  Frame i
-    of the call takes matrix i across every seam."""
+    """11 frames in groups of 4 (4 + 4 + 3), overlap on and off: with the lens and the roi in float32, with the lens on
+    the full frame in float32, and without a lens in float64.  Frame i of the call takes matrix i across every seam."""
     H, W, n = 96, 256, 11
     L = ip.lib_mod
     e, dark, flat, roi, maps = _setup(ip, H, W, 5)
@@ -128,10 +127,8 @@ def test_group_seams_vs_oracle(ip):
     try:
         with _Options(ip, e) as o:
             o.set(L.OPT_CHAIN_GROUP, 4)
-            for lens, window, tdt, odt, variant in ((True, roi, torch.float32, np.float32, 0),
-                                                    (True, None, torch.float32, np.float32, 2),
-                                                    (False, None, torch.float64, np.float64, 0)):
-                o.set(L.OPT_K3_VARIANT, variant)
+            for lens, window, tdt, odt in ((True, roi, torch.float32, np.float32), (True, None, torch.float32, np.float32),
+                                           (False, None, torch.float64, np.float64)):
                 Ms, dsize = _table(*_src_shape(e, window, lens), n, ['strong', 'mild', 'outside'], dsize='larger')
                 e.set_perspective(Ms, dsize, 0.0)
                 for overlap in (1, 0):
@@ -139,9 +136,8 @@ def test_group_seams_vs_oracle(ip):
                     got = _host(e.correct_batch(dev, flags=_flags(L, 0.1) | L.DO_PERSPECTIVE, use_lens=lens, window=window,
                                                 out_dtype=tdt))
                     for i in range(n):
-                        assert _same(got[i], want(i, Ms[i], dsize, 0.0, window, odt, lens)), (lens, variant, overlap, i)
+                        assert _same(got[i], want(i, Ms[i], dsize, 0.0, window, odt, lens)), (lens, window, overlap, i)
     finally:
-        e.set_option(L.OPT_K3_VARIANT, 0)
         e.set_perspective(None, None)
 
 
@@ -149,7 +145,8 @@ def test_group_seams_vs_oracle(ip):
 @pytest.mark.parametrize('variant', [0, 1, 2])
 def test_equal_table_is_the_single_matrix_stage(ip, variant):
     """a table whose n matrices are all M gives the output of imgcorr_set_perspective(M), for float32, float64 and uint16
-    output; and the two setters replace each other in both directions"""
+    output; and the two setters replace each other in both directions.  With K3 forced to its staged tiles (2) the single
+    matrix runs them and the table is refused."""
     H, W, n = 96, 256, 9
     L = ip.lib_mod
     e, dark, flat, roi, maps = _setup(ip, H, W, 23)
@@ -166,7 +163,13 @@ def test_equal_table_is_the_single_matrix_stage(ip, variant):
                 e.set_perspective(M, dsize, 1.25)
                 one = e.correct_batch(dev, flags=fl, out_dtype=tdt)
                 e.set_perspective(np.stack([M] * n), dsize, 1.25)
-                table = e.correct_batch(dev, flags=fl, out_dtype=tdt)
+                if variant == 2:
+                    with pytest.raises(L.ImgcorrError) as err:
+                        e.correct_batch(dev, flags=fl, out_dtype=tdt)
+                    assert err.value.status == L.ERR_INVALID, tdt
+                    table = one
+                else:
+                    table = e.correct_batch(dev, flags=fl, out_dtype=tdt)
                 e.set_perspective(M, dsize, 1.25)
                 again = e.correct_batch(dev, flags=fl, out_dtype=tdt)
                 assert torch.equal(one, table) and torch.equal(one, again), tdt
@@ -393,7 +396,7 @@ def test_replacing_the_table_while_a_call_is_queued(ip):
 def test_full_size_against_the_two_step_composition(ip):
     """17 uint16 4096x3000 frames with the moderate lens (groups of 16 + 1) through a table of jittered mild homographies
     onto 4000x2900, against correct_batch followed by Engine.warp_perspective of each frame with its own matrix: the full
-    frame with K3 forced to its staged tiles, and the roi window with K3's default (its L1 gathers)"""
+    frame and the roi window"""
     H, W, n = 3000, 4096, 17
     L = ip.lib_mod
     e = ip.engine_mod.get_engine(H, W)
@@ -403,21 +406,18 @@ def test_full_size_against_the_two_step_composition(ip):
     src = synth.scene_torch(n, H, W, 7, torch.device('cuda', torch.cuda.current_device()))
     dsize = (4000, 2900)
     try:
-        for window, variant in ((None, 2), (roi, 0)):
-            e.set_option(L.OPT_K3_VARIANT, variant)
+        for window in (None, roi):
             sh = _src_shape(e, window)
             M = _homography([(fx * sh[1], fy * sh[0]) for fx, fy in QUADS['mild']],
                             [(0, 0), (4000, 0), (4000, 2900), (0, 2900)])
             Ms = np.stack([_jitter(M, i, 2900, 4000) for i in range(n)])
             e.set_perspective(Ms, dsize, 0.0)
             got = e.correct_batch(src, flags=_flags(L, 0.1) | L.DO_PERSPECTIVE, window=window)
-            e.set_option(L.OPT_K3_VARIANT, 0)
             mid = e.correct_batch(src, window=window)
             assert tuple(got.shape) == (n, 2900, 4000)
             bad = [i for i in range(n) if not torch.equal(got[i], e.warp_perspective(mid[i], Ms[i], dsize))]
             assert not bad, (window, bad)
             del got, mid
     finally:
-        e.set_option(L.OPT_K3_VARIANT, 0)
         e.set_perspective(None, None)
         e.set_lens(None, None, None)

@@ -7,14 +7,13 @@ module sits at a slightly different place in each image, and pc_i.setReference(q
 Frame i's homography maps a mild quad, jittered by a few pixels and a fraction of a degree per frame, onto a 4000x2900
 destination.  Every path is warmed up first:
   a   device frames, the per-frame stage:  cal.correct_batch(frames_dev, perspective=[pc_0, ..., pc_n-1])
-  a2  the same with K3 forced to its staged tiles (IMGCORR_OPT_K3_VARIANT = 2) instead of the L1 gathers it picks
   b   device frames, the stage with one shared matrix (pc_0 for every frame): the cost of per-frame coordinates is a - b
   c   device frames, two steps:  cal.correct_batch(frames_dev), then Engine.warp_perspective of each frame with its matrix
   d   pinned host frames, the per-frame stage:  cal.correct_batch(frames_host, perspective=[pc_0, ..., pc_n-1])
   e   pinned host frames, two steps:  cal.correct_batch(frames_host), then pc_i.correct(frame_i) for every frame
 Prints one JSON line: the GPU's name and power limit, and per path the median over --reps of the call's wall time divided
-by the frame count (each call ends in a device synchronise or returns host arrays).  Asserts a == c, a2 == a and d == e
-bit for bit."""
+by the frame count (each call ends in a device synchronise or returns host arrays).  Asserts a == c and d == e bit for
+bit."""
 import argparse
 import contextlib
 import io
@@ -65,7 +64,7 @@ def main():
     ap.add_argument('--device', type=int, default=0)
     args = ap.parse_args()
     import torch
-    from imgprocessor_b200 import _lib, engine, synth
+    from imgprocessor_b200 import engine, synth
     from imgprocessor_b200.camera import CameraCalibration, LensDistortion, PerspectiveCorrection
     if not torch.cuda.is_available():
         raise SystemExit('perframe_warp.py measures on a CUDA device; none found')
@@ -101,13 +100,6 @@ def main():
         torch.cuda.synchronize()
         return r
 
-    def path_a2():
-        eng.set_option(_lib.OPT_K3_VARIANT, 2)
-        try:
-            return path_a()
-        finally:
-            eng.set_option(_lib.OPT_K3_VARIANT, 0)
-
     def path_b():
         r = cal.correct_batch(frames_dev, perspective=pcs[0])
         torch.cuda.synchronize()
@@ -127,8 +119,7 @@ def main():
         with contextlib.redirect_stdout(io.StringIO()):
             return [pcs[i].correct(mid[i]) for i in range(n)]
 
-    paths = {'a_device_per_frame_stage': path_a, 'a2_device_per_frame_stage_k3_tiles': path_a2,
-             'b_device_shared_matrix_stage': path_b, 'c_device_two_steps': path_c, 'd_host_per_frame_stage': path_d,
+    paths = {'a_device_per_frame_stage': path_a, 'b_device_shared_matrix_stage': path_b, 'c_device_two_steps': path_c, 'd_host_per_frame_stage': path_d,
              'e_host_two_steps': path_e}
     per_frame_ms, checks = {}, {}
     for name, fn in paths.items():
@@ -141,8 +132,6 @@ def main():
         per_frame_ms[name] = round(1e3 * float(np.median(times)) / n, 3)
         if name == 'a_device_per_frame_stage':
             a = first.clone()
-        elif name == 'a2_device_per_frame_stage_k3_tiles':
-            checks['a2_equals_a'] = bool(torch.equal(first, a))
         elif name == 'c_device_two_steps':
             checks['a_equals_c'] = bool(first.shape == (n, dh, dw) and torch.equal(a, first))
         elif name == 'd_host_per_frame_stage':
