@@ -28,6 +28,7 @@ SIGNATURES = {
     'imgcorr_launch_count': (ctypes.c_longlong, [c_void_p]),
     'imgcorr_profile_read': (c_int, [c_void_p, ctypes.POINTER(c_double)]),
     'imgcorr_set_dark': (c_int, [c_void_p, c_void_p, c_void_p, c_double, c_int, c_int]),
+    'imgcorr_set_dark_exposures': (c_int, [c_void_p, c_void_p, c_int]),
     'imgcorr_set_flat': (c_int, [c_void_p, c_void_p, c_int]),
     'imgcorr_set_lens': (c_int, [c_void_p, c_void_p, c_void_p, c_void_p]),
     'imgcorr_pointwise_median': (c_int, [c_void_p, c_void_p, c_int, c_void_p, c_int, c_void_p, c_int, c_double,

@@ -594,7 +594,17 @@ if shapes are transposed, execute self.transpose() once """ % (s, array.shape))
         the host); any other dtype, float64 included, is rounded to float32 once, as correct() does with float64
         calibration maps.  It combines with ``devices=`` (every device gets its shard's backgrounds), ``perspective=``,
         ``out_dtype`` / ``out_scale`` and ``keep_size``.  ValueError, before any engine is created, for another shape, for
-        ``bgImages`` given as well, for a numpy / tensor mismatch with ``frames`` and for a tensor on another device."""
+        ``bgImages`` given as well, for a numpy / tensor mismatch with ``frames`` and for a tensor on another device.
+
+        ``exposure_time`` may be a 1-D sequence of n exposure times, one per frame (an .elbin stack's labels, frames taken
+        at several exposures).  With a tuple dark-current entry (offset, ascent) frame i evaluates the line model with its
+        own time, bit for bit as ``correct_batch(frames[i:i+1], exposure_time=t_i)``, inside K1: with float64 output
+        ``correct_batch(frames, exposure_time=ts, out_dtype=np.float64)[i]`` equals ``correct(frames[i],
+        exposure_time=ts[i])``.  With an array entry, ``bg_frames`` or ``bgImages`` the times are checked and then unused,
+        as correct() does with its scalar.  It combines with host frames, CUDA tensors, ``devices=`` (every device gets
+        its shard's times), ``perspective=``, ``keep_size``, ``out_dtype`` / ``out_scale`` and big-endian frames.
+        ValueError, before any engine is created, for a length other than n, a sequence that is not 1-D, a non-numeric
+        value or NaN."""
         import contextlib
         import io
         tt = _engine.torch()
@@ -615,15 +625,19 @@ if shapes are transposed, execute self.transpose() once """ % (s, array.shape))
         stage = self._perspective_stage(perspective, out, out_dtype, n)
         if bg_frames is not None:
             bg_frames = self._bg_frames(frames, bg_frames, bgImages)
+        times = self._exposure_times(exposure_time, n)
+        if times is not None:
+            exposure_time = float(times[0]) if n else 0.0       # resolves the dark entry; the table replaces it per frame
         if devices is not None and len(devices) > 1:
             return self._correct_batch_multi(frames, devices, bgImages, exposure_time, light_spectrum, threshold,
-                                             keep_size, date, out, out_dtype, verbose, stage, out_scale, bg_frames)
+                                             keep_size, date, out, out_dtype, verbose, stage, out_scale, bg_frames, times)
         dev_index = frames.device.index if is_tensor else (devices[0] if devices else None)
         eng = _engine.get_engine(H, W, dev_index)
         sink = contextlib.nullcontext() if verbose else contextlib.redirect_stdout(io.StringIO())
         with sink:
             flags = self._configure_engine(eng, (H, W), bgImages, exposure_time, light_spectrum, date,
                                            use_dark=bg_frames is None)
+            self._set_exposures(eng, times)
             lens = None
             try:
                 lens = self.getLens(light_spectrum, date['lens'])
@@ -658,6 +672,35 @@ if shapes are transposed, execute self.transpose() once """ % (s, array.shape))
                                 window=window, out_dtype=out_dtype or np.float32, out_scale=out_scale, bg=bg_frames)
 
     @staticmethod
+    def _exposure_times(exposure_time, n):
+        """correct_batch's per-frame exposure times as a float64 array of n, or None for a scalar / None (used as
+        today); ValueError for anything else that is not n numbers"""
+        if np.ndim(exposure_time) == 0 and not isinstance(exposure_time, (list, tuple)):
+            return None
+        tt = _engine.torch()
+        if isinstance(exposure_time, tt.Tensor):
+            exposure_time = exposure_time.detach().cpu().numpy()
+        t = np.asarray(exposure_time)
+        if t.ndim != 1:
+            raise ValueError('exposure_time: a scalar or a 1-D sequence of one time per frame, got shape %s' % (t.shape,))
+        if t.size and t.dtype.kind not in 'iuf':
+            raise ValueError('exposure_time: numbers expected, got %s' % t.dtype)
+        if t.size != n:
+            raise ValueError('exposure_time: %d times for %d frames' % (t.size, n))
+        t = t.astype(np.float64)
+        if np.isnan(t).any():
+            raise ValueError('exposure_time[%d] is NaN' % int(np.flatnonzero(np.isnan(t))[0]))
+        return t
+
+    def _set_exposures(self, eng, times):
+        """per-frame exposure times on the engine when the line model is in use (a tuple dark entry); otherwise no table"""
+        linear = self._last_bg is not None and self._last_bg.get('ascent') is not None
+        if times is not None and linear and times.size:
+            eng.set_dark_exposures(times)
+        elif eng.has_exposures:
+            eng.set_dark_exposures(None)
+
+    @staticmethod
     def _bg_frames(frames, bg_frames, bgImages):
         """the refusals of correct_batch(bg_frames=...), before any engine is created"""
         tt = _engine.torch()
@@ -685,7 +728,7 @@ if shapes are transposed, execute self.transpose() once """ % (s, array.shape))
         return bg.astype(np.float32)
 
     def _correct_batch_multi(self, frames, devices, bgImages, exposure_time, light_spectrum, threshold, keep_size, date,
-                             out, out_dtype, verbose, stage, out_scale=None, bg_frames=None):
+                             out, out_dtype, verbose, stage, out_scale=None, bg_frames=None, times=None):
         """host frames [n,H,W] split over several devices of this process: one engine + one host thread per device"""
         import contextlib
         import io
@@ -714,6 +757,8 @@ if shapes are transposed, execute self.transpose() once """ % (s, array.shape))
                     with contextlib.nullcontext() if (verbose and i == 0) else contextlib.redirect_stdout(io.StringIO()):
                         flags = self._configure_engine(e, (H, W), bgImages, exposure_time, light_spectrum, date,
                                                        use_dark=bg_frames is None)
+                    lo, hi = sharding.shard_range(n, len(engines), i)
+                    self._set_exposures(e, None if times is None else times[lo:hi])
                 try:
                     lens = self.getLens(light_spectrum, date['lens'])
                     if lens:

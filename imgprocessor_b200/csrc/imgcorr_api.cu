@@ -112,8 +112,12 @@ struct HostSlot {
 
 struct imgcorr_ctx {
     int device = 0, H = 0, W = 0, sm_count = 148;
-    DevPtr<float> dark, ascent, flat;
+    DevPtr<float> dark, flat;                 // dark: [H][W], or [2][H][W] = offset, ascent with the line model (`linear`)
+    bool linear = false;
     double exposure = 0.0, maxval = 65535.0;
+    DevPtr<double> exposures;                 // imgcorr_set_dark_exposures: one time per frame of a call, or empty
+    int n_exposures = 0;
+    double exposures_absmax = 0.0;            // max |t| over the table
     OutScale out_scale{0.0, 1.0};             // imgcorr_set_output_scale: read by chain calls with U16 / U8 output
     bool has_lens = false;
     LensConst lens{};
@@ -135,9 +139,9 @@ struct imgcorr_ctx {
     long long chain_groups_seen = 0;
     double prof_frames[2] = {0.0, 0.0};
     std::vector<Event> prof_ev[2];            // [kernel] start/stop pairs (timing events)
-    bool dark_finite = true, flat_finite = true;
+    bool dark_finite = true, flat_finite = true, ascent_finite = true;
     DevPtr<float> flat_nz;                    // flat with zeros replaced by 1.0
-    double dark_absmax = 0.0, flat_absmin = 1.0;   // over finite entries (flat: non-zero entries)
+    double dark_absmax = 0.0, ascent_absmax = 0.0, flat_absmin = 1.0;   // over finite entries (flat: non-zero entries)
     long long launches = 0;
     // the chain's K1 output (with a lens: two halves of `chain_group` float32 frames each), then the warp source of the
     // perspective stage (a group of chain frames in the output dtype)
@@ -355,23 +359,103 @@ static int upload_map(imgcorr_ctx* c, DevPtr<float>& slot, const float* src, int
     return IMGCORR_OK;
 }
 
+// finiteness and the largest finite magnitude of a host map, read in place
+static void scan_map(const float* h, size_t n, bool* finite, double* absmax) {
+    bool ok = true;
+    float mx = 0.0f;
+    for (size_t i = 0; i < n; ++i) {
+        const float av = fabsf(h[i]);
+        ok &= av <= 3.402823466e+38f;
+        if (av <= 3.402823466e+38f && av > mx) mx = av;
+    }
+    *finite = ok;
+    *absmax = mx;
+}
+
 extern "C" IMGCORR_API int imgcorr_set_dark(imgcorr_ctx* c, const float* dark, const float* ascent, double exposure_time,
                                 int depth_bits, int on_device) {
     GUARD(c);
+    if (c->exposures) {                                // the times belong to the model being replaced; queued calls may read them
+        CK(cudaDeviceSynchronize());
+        c->exposures.reset();
+        c->n_exposures = 0;
+    }
     if (!dark && ascent) return fail(IMGCORR_ERR_INVALID, "ascent given without offset map");
     if (ascent && (depth_bits < 1 || depth_bits > 62)) return fail(IMGCORR_ERR_INVALID, "depth_bits %d", depth_bits);
     if (ascent && !(exposure_time == exposure_time)) return fail(IMGCORR_ERR_INVALID, "exposure_time is NaN");
-    bool fin2 = true;
-    std::vector<float> h;
-    int r = upload_map(c, c->dark, dark, on_device, &c->dark_finite, &h);
-    if (r) return r;
-    c->dark_absmax = 0.0;
-    for (float v : h) { const float av = fabsf(v); if (av <= 3.402823466e+38f && av > c->dark_absmax) c->dark_absmax = av; }
-    r = upload_map(c, c->ascent, ascent, on_device, &fin2);
-    if (r) return r;
+    if (!ascent) {
+        if (c->linear) {                               // the [2][H][W] block goes; upload_map allocates [H][W]
+            CK(cudaDeviceSynchronize());
+            c->dark.reset();
+            c->linear = false;
+        }
+        std::vector<float> h;
+        int r = upload_map(c, c->dark, dark, on_device, &c->dark_finite, &h);
+        if (r) return r;
+        c->dark_absmax = 0.0;
+        for (float v : h) { const float av = fabsf(v); if (av <= 3.402823466e+38f && av > c->dark_absmax) c->dark_absmax = av; }
+        c->exposure = exposure_time;
+        c->maxval = 65535.0;
+        return IMGCORR_OK;
+    }
+    // The line model keeps offset and ascent in one [2][H][W] block: the streaming kernel loads both boxes of a stage with
+    // one 3-D copy.  A failed upload leaves no dark map.
+    const size_t n = (size_t)c->H * c->W, bytes = n * sizeof(float);
+    if (c->dark) CK(cudaDeviceSynchronize());          // launches on other streams may still read the map being replaced
+    c->dark.reset();
+    c->linear = false;
+    DevPtr<float> blk;
+    CK(dev_alloc(blk, 2 * bytes));
+    const cudaMemcpyKind kind = on_device ? cudaMemcpyDeviceToDevice : cudaMemcpyHostToDevice;
+    CK(cudaMemcpy(blk.get(), dark, bytes, kind));
+    CK(cudaMemcpy(blk.get() + n, ascent, bytes, kind));
+    if (on_device) {
+        std::vector<float> h(2 * n);
+        CK(cudaMemcpy(h.data(), blk.get(), 2 * bytes, cudaMemcpyDeviceToHost));
+        scan_map(h.data(), n, &c->dark_finite, &c->dark_absmax);
+        scan_map(h.data() + n, n, &c->ascent_finite, &c->ascent_absmax);
+    } else {
+        scan_map(dark, n, &c->dark_finite, &c->dark_absmax);
+        scan_map(ascent, n, &c->ascent_finite, &c->ascent_absmax);
+    }
+    c->dark = std::move(blk);
+    c->linear = true;
     c->exposure = exposure_time;
-    c->maxval = ascent ? ldexp(1.0, depth_bits) - 1.0 : 65535.0;
+    c->maxval = ldexp(1.0, depth_bits) - 1.0;
     return IMGCORR_OK;
+}
+
+extern "C" IMGCORR_API int imgcorr_set_dark_exposures(imgcorr_ctx* c, const double* t, int n) {
+    GUARD(c);
+    // launches on other (non-blocking) streams may still read the table being replaced or dropped; a failed call leaves
+    // no table behind
+    if (c->exposures) {
+        CK(cudaDeviceSynchronize());
+        c->exposures.reset();
+        c->n_exposures = 0;
+    }
+    if (!t) return IMGCORR_OK;
+    if (!c->linear) return fail(IMGCORR_ERR_STATE, "per-frame exposure times need the linear dark model (imgcorr_set_dark with ascent)");
+    if (n <= 0) return fail(IMGCORR_ERR_INVALID, "n %d", n);
+    double mx = 0.0;
+    for (int i = 0; i < n; ++i) {
+        if (!(t[i] == t[i])) return fail(IMGCORR_ERR_INVALID, "exposure time %d is NaN", i);
+        if (fabs(t[i]) > mx) mx = fabs(t[i]);
+    }
+    DevPtr<double> d;
+    CK(dev_alloc(d, (size_t)n * sizeof(double)));
+    CK(cudaMemcpy(d.get(), t, (size_t)n * sizeof(double), cudaMemcpyHostToDevice));
+    c->exposures = std::move(d);
+    c->n_exposures = n;
+    c->exposures_absmax = mx;
+    return IMGCORR_OK;
+}
+
+// the refusal of a call that evaluates the line model over more frames than the per-frame exposure table holds, before
+// anything is enqueued
+static int check_exposures(const imgcorr_ctx* c, int flags, const void* bg, int n_frames) {
+    if (!c->exposures || bg || !(flags & IMGCORR_DO_DARK) || n_frames <= c->n_exposures) return IMGCORR_OK;
+    return fail(IMGCORR_ERR_INVALID, "%d frames but the exposure table holds %d times", n_frames, c->n_exposures);
 }
 
 extern "C" IMGCORR_API int imgcorr_set_flat(imgcorr_ctx* c, const float* flat, int on_device) {
@@ -436,9 +520,10 @@ extern "C" IMGCORR_API int imgcorr_set_lens(imgcorr_ctx* c, const double K[9], c
     return IMGCORR_OK;
 }
 
-// bg: per-frame backgrounds [n][H][W] of bg_dtype in place of the dark map (checked by check_bg), or null
+// bg: per-frame backgrounds [n][H][W] of bg_dtype in place of the dark map (checked by check_bg), or null.  first: the
+// index of raw's first frame in the caller's call, which picks its per-frame exposure times (checked by check_exposures)
 static int fill_k1(imgcorr_ctx* c, K1Args& a, const void* raw, int raw_dtype, void* out, uint8_t* mask, int n, double thr,
-                   int ksize, int cond, int flags, const void* bg = nullptr, int bg_dtype = DT_F32) {
+                   int ksize, int cond, int flags, const void* bg = nullptr, int bg_dtype = DT_F32, int first = 0) {
     if (!raw || !out) return fail(IMGCORR_ERR_INVALID, "null image pointer");
     if (n < 0) return fail(IMGCORR_ERR_INVALID, "n_frames %d", n);
     if (!(thr > 0.0)) ksize = 0;                      // also NaN
@@ -458,20 +543,32 @@ static int fill_k1(imgcorr_ctx* c, K1Args& a, const void* raw, int raw_dtype, vo
         f |= FLAG_DARK; a.bg = bg; a.bg_dtype = bg_dtype;
     } else if ((flags & IMGCORR_DO_DARK) && c->dark) {
         f |= FLAG_DARK; a.dark = c->dark.get();
-        if (c->ascent) { f |= FLAG_DARK_LINEAR; a.ascent = c->ascent.get(); }
+        if (c->linear) {
+            f |= FLAG_DARK_LINEAR; a.ascent = c->dark.get() + (size_t)c->H * c->W;
+            if (c->exposures) a.exposures = c->exposures.get() + first;
+        }
     }
     if ((flags & IMGCORR_DO_FLAT) && c->flat) { f |= FLAG_FLAT; a.flat = c->flat.get(); }
     if (flags & IMGCORR_DO_NAN_TO_NUM) f |= FLAG_NAN_TO_NUM;
     a.pw.flags = f; a.pw.exposure_time = c->exposure; a.pw.max_value = c->maxval;
-    a.maps_finite = ((!a.dark || c->dark_finite) && (!a.flat || c->flat_finite)) ? 1 : 0;
+    a.maps_finite = ((!a.dark || c->dark_finite) && (!a.ascent || c->ascent_finite) && (!a.flat || c->flat_finite)) ? 1 : 0;
     a.flat_nz = a.flat ? c->flat_nz.get() : nullptr;
     if (!c->dump) CK(dev_alloc(c->dump, (size_t)4 << 20));
     a.dump = c->dump.get();
     // integer frames: |raw - dark| <= raw_max + max|dark|; divided by min|flat| it must stay below FLT_MAX.  Backgrounds of
     // the raw integer dtype: |raw - bg| <= raw_max.  Float32 backgrounds are not checked at upload: no proof
+    // The line model: |bg| <= max|offset| + max|ascent| * max|t| over the scalar or the table in use, a finite bound or none.
     a.no_overflow = 0;
+    double bg_max = a.dark ? c->dark_absmax : 0.0;
+    if (a.ascent) {
+        const double tmax = a.exposures ? c->exposures_absmax : fabs(c->exposure);
+        bg_max = bg_max + c->ascent_absmax * tmax;
+        // the streaming kernel's unchecked division needs |raw - bg| well inside float64's range: |bg| <= FLT_MAX.  A larger
+        // bound (an infinite time, inf * 0) is no proof: the checked arithmetic
+        if (!(bg_max <= 3.0e38)) a.maps_finite = 0;
+    }
     if (a.maps_finite && (raw_dtype == DT_U8 || raw_dtype == DT_U16) && (!bg || bg_dtype == raw_dtype)) {
-        const double num = (raw_dtype == DT_U8 ? 255.0 : 65535.0) + (a.dark ? c->dark_absmax : 0.0);
+        const double num = (raw_dtype == DT_U8 ? 255.0 : 65535.0) + bg_max;
         const double den = a.flat ? c->flat_absmin : 1.0;
         a.no_overflow = (num / den < 3.0e38) ? 1 : 0;
     }
@@ -486,6 +583,7 @@ extern "C" IMGCORR_API int imgcorr_pointwise_median(imgcorr_ctx* c, const void* 
     if ((out_dtype == DT_U8 || out_dtype == DT_U16) && out_dtype != raw_dtype)        // integer output keeps the input dtype here
         return fail(IMGCORR_ERR_INVALID, "unsupported dtype pair raw=%d out=%d", raw_dtype, out_dtype);
     K1Args a;
+    if (int r = check_exposures(c, flags, nullptr, n_frames)) return r;
     int r = fill_k1(c, a, raw_dev, raw_dtype, out_dev, mask_dev, n_frames, threshold, ksize, cond, flags);
     if (r) return r;
     a.out_streaming = 1;
@@ -839,6 +937,7 @@ static int check_perspective(const imgcorr_ctx* c, int out_dtype, int ow, int oh
 // Integer output (U16 / U8) is the float32 chain with the quantiser fused into the last kernel's store: K1 without a lens or
 // perspective stage, K2 with a lens, K3 with the stage (which warps the float32 chain frame).
 // `bg`: the call's per-frame backgrounds from raw's first frame on (dense, bg_dtype; checked by check_bg), or null.
+// `first` also picks the frames' entries of a per-frame exposure table (checked by check_exposures).
 static int chain_frames(imgcorr_ctx* c, const void* raw, int raw_dtype, void* out, int out_dtype, int n, double thr,
                         int ksize, int flags, bool lens, bool persp, double border, int x0, int y0, int ow, int oh,
                         cudaStream_t st, int first, const void* bg, int bg_dtype) {
@@ -852,7 +951,7 @@ static int chain_frames(imgcorr_ctx* c, const void* raw, int raw_dtype, void* ou
         return fail(IMGCORR_ERR_INVALID, "output window without a lens");
     if (!lens && !persp) {                             // K1 alone: one launch for the whole batch, no scratch
         K1Args a;
-        int r = fill_k1(c, a, raw, raw_dtype, out, nullptr, n, thr, ksize, IMGCORR_COND_GT, flags, bg, bg_dtype);
+        int r = fill_k1(c, a, raw, raw_dtype, out, nullptr, n, thr, ksize, IMGCORR_COND_GT, flags, bg, bg_dtype, first);
         if (r) return r;
         if (quant) a.q = c->out_scale;
         int l = 0;
@@ -916,7 +1015,7 @@ static int chain_frames(imgcorr_ctx* c, const void* raw, int raw_dtype, void* ou
         }
         K1Args a;
         int r = fill_k1(c, a, (const char*)raw + f * raw_stride, raw_dtype, lens ? (void*)mid : frames, nullptr, nf, thr, ksize,
-                        IMGCORR_COND_GT, flags, bg ? (const char*)bg + f * npx * dtype_size(bg_dtype) : nullptr, bg_dtype);
+                        IMGCORR_COND_GT, flags, bg ? (const char*)bg + f * npx * dtype_size(bg_dtype) : nullptr, bg_dtype, first + f);
         if (r) return r;
         int l = 0;
         if (prof) prof_mark(c, 0, s1);
@@ -963,6 +1062,7 @@ static int correct_batch(imgcorr_ctx* c, const void* raw_dev, int raw_dtype, con
                          double border_value, int x0, int y0, int ow, int oh, void* stream) {
     if (!raw_dev || !out_dev) return fail(IMGCORR_ERR_INVALID, "null image pointer");
     if (int r = check_bg(raw_dtype, bg_dev, bg_dtype, flags)) return r;
+    if (int r = check_exposures(c, flags, bg_dev, n_frames)) return r;
     const bool lens = use_lens && c->has_lens;
     if (!lens) { x0 = 0; y0 = 0; ow = c->W; oh = c->H; }
     const bool persp = flags & IMGCORR_DO_PERSPECTIVE;
@@ -1041,6 +1141,7 @@ static int correct_host(imgcorr_ctx* c, const void* raw_host, int raw_dtype, con
     if (!raw_host || !out_host) return fail(IMGCORR_ERR_INVALID, "null image pointer");
     if (int r = check_bg(raw_dtype, bg_host, bg_dtype, flags)) return r;
     if (n_frames < 0) return fail(IMGCORR_ERR_INVALID, "n_frames %d", n_frames);
+    if (int r = check_exposures(c, flags, bg_host, n_frames)) return r;
     if (raw_dtype < DT_U8 || raw_dtype > DT_F32) return fail(IMGCORR_ERR_INVALID, "raw_dtype %d (U8, U16 or F32)", raw_dtype);
     if (c->raw_gap) return fail(IMGCORR_ERR_INVALID, "IMGCORR_OPT_RAW_FRAME_GAP is not available for host frames (pass the pixel blocks)");
     if (out_dtype < DT_U8 || out_dtype > DT_F64) return fail(IMGCORR_ERR_INVALID, "out_dtype must be U8, U16, F32 or F64");

@@ -36,6 +36,8 @@ struct K1Args {
     const void* bg;         // [n_frames][H][W] of bg_dtype, dense and native-endian, or null: frame f subtracts float32(bg[f])
                             // in place of the dark map (FLAG_DARK set, dark / ascent null)
     int bg_dtype;           // the raw dtype or DT_F32
+    const double* exposures;    // [n_frames] or null (FLAG_DARK_LINEAR only): frame f evaluates the line model with
+                                // exposures[f] instead of pw.exposure_time
 };
 
 // variant: 0 = pick automatically, 1 = generic tiles (plain coalesced loads), 2 = TMA-staged tiles,

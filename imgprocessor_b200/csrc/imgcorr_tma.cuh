@@ -116,12 +116,12 @@ inline int blocks_per_sm_cached(const void* kern, int threads, size_t smem, cuda
 
 // dense row-major [N][H][W] (N == 0: [H][W], rank 2) of `esz`-byte elements, box = boxw x boxh (x 1)
 inline bool make_tensor_map(CUtensorMap* tm, CUtensorMapDataType dt, size_t esz, const void* ptr, int W, int H, int N,
-                            int boxw, int boxh) {
+                            int boxw, int boxh, int boxd = 1) {
     PFN_tensorMapEncodeTiled enc = tensor_map_encoder();
     if (!enc) return false;
     cuuint64_t dims[3] = {(cuuint64_t)W, (cuuint64_t)H, (cuuint64_t)(N > 0 ? N : 1)};
     cuuint64_t strides[2] = {(cuuint64_t)W * esz, (cuuint64_t)W * H * esz};
-    cuuint32_t box[3] = {(cuuint32_t)boxw, (cuuint32_t)boxh, 1};
+    cuuint32_t box[3] = {(cuuint32_t)boxw, (cuuint32_t)boxh, (cuuint32_t)boxd};
     cuuint32_t estr[3] = {1, 1, 1};
     const int rank = N > 0 ? 3 : 2;
     return enc(tm, dt, rank, const_cast<void*>(ptr), dims, strides, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,

@@ -9,7 +9,8 @@
 //
 // This file holds the tile kernels and the dispatcher (launch_k1).  The default paths are the streaming pipelines in
 // k1_stream.cu (3x3, and threshold <= 0) and k1_stream5.cu (5x5); the tiles below serve the shapes / dtypes / options
-// those do not take (odd widths, float64 frames, the legacy linear dark model, framed file images).
+// those do not take (odd widths, float64 frames, framed file images, the linear dark model outside the streaming
+// configurations).
 //
 // Two staging variants share the same compute phases:
 //   generic : coalesced ld.global.nc with reflect indexing (any W, any alignment, any dtype)
@@ -81,13 +82,15 @@ __device__ __forceinline__ float bg_sample(const K1Args& a, size_t i) {
     return __ldg((const float*)a.bg + i);
 }
 
-template <typename RawT, typename OutT, bool BG>
+// TT: per-frame exposure times (K1Args::exposures) for the line model: the frame's time replaces pw.exposure_time
+template <typename RawT, typename OutT, bool BG, bool TT = false>
 __device__ __forceinline__ void k1_pointwise_body(const K1Args& a) {
     using CT = typename RawIO<RawT>::CT;
     const size_t npx = (size_t)a.H * a.W;
     const RawT* raw = raw_frame<RawT>(a, blockIdx.y);
     OutT* out = (OutT*)a.out + (size_t)blockIdx.y * npx;
-    const PointwiseConst pw = a.pw;
+    PointwiseConst pw = a.pw;
+    if (TT) pw.exposure_time = __ldg(a.exposures + blockIdx.y);
     const int swap = a.raw_swap;
     for (size_t p = (size_t)blockIdx.x * blockDim.x + threadIdx.x; p < npx; p += (size_t)gridDim.x * blockDim.x) {
         float d = BG ? bg_sample(a, (size_t)blockIdx.y * npx + p) : (a.dark ? __ldg(a.dark + p) : 0.0f);
@@ -100,6 +103,8 @@ template <typename RawT, typename OutT>
 __global__ void __launch_bounds__(256) k1_pointwise_kernel(K1Args a) { k1_pointwise_body<RawT, OutT, false>(a); }
 template <typename RawT, typename OutT>
 __global__ void __launch_bounds__(256) k1_pointwise_bg_kernel(K1Args a) { k1_pointwise_body<RawT, OutT, true>(a); }
+template <typename RawT, typename OutT>
+__global__ void __launch_bounds__(256) k1_pointwise_tt_kernel(K1Args a) { k1_pointwise_body<RawT, OutT, false, true>(a); }
 
 // ------------------------------------------------------------------------------------------
 // phase B: median-threshold of one tile from the shared pointwise tile xs[TH+2h][K1_BOXW]
@@ -210,7 +215,7 @@ __device__ __forceinline__ void median_phase(const CT* __restrict__ xs, const K1
 // ------------------------------------------------------------------------------------------
 // generic variant: one tile per CTA, reflect indexing on global loads
 // ------------------------------------------------------------------------------------------
-template <typename RawT, typename OutT, int KS, int TH, bool VEC, bool BG>
+template <typename RawT, typename OutT, int KS, int TH, bool VEC, bool BG, bool TT = false>
 __device__ __forceinline__ void k1_generic_body(const K1Args& a, int tiles_x, int tiles_y) {
     using CT = typename RawIO<RawT>::CT;
     constexpr int HALO = KS / 2;
@@ -224,7 +229,8 @@ __device__ __forceinline__ void k1_generic_body(const K1Args& a, int tiles_x, in
     const int frame = t / tiles_y;
     const int tx0 = txi * K1_TW, ty0 = tyi * TH;
     const RawT* raw = raw_frame<RawT>(a, frame);
-    const PointwiseConst pw = a.pw;
+    PointwiseConst pw = a.pw;
+    if (TT) pw.exposure_time = __ldg(a.exposures + frame);
     const int swap = a.raw_swap;
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
 
@@ -252,6 +258,11 @@ __global__ void __launch_bounds__(K1_THREADS) k1_generic_kernel(K1Args a, int ti
 template <typename RawT, typename OutT, int KS, int TH>
 __global__ void __launch_bounds__(K1_THREADS) k1_generic_bg_kernel(K1Args a, int tiles_x, int tiles_y) {
     k1_generic_body<RawT, OutT, KS, TH, false, true>(a, tiles_x, tiles_y);
+}
+// per-frame exposure times of the line model (K1Args::exposures)
+template <typename RawT, typename OutT, int KS, int TH, bool VEC>
+__global__ void __launch_bounds__(K1_THREADS) k1_generic_tt_kernel(K1Args a, int tiles_x, int tiles_y) {
+    k1_generic_body<RawT, OutT, KS, TH, VEC, false, true>(a, tiles_x, tiles_y);
 }
 
 // ------------------------------------------------------------------------------------------
@@ -445,6 +456,11 @@ static cudaError_t launch_generic_t(const K1Args& a, cudaStream_t st) {
         }
     }
     const bool vec = (a.W % 2 == 0) && ((uintptr_t)a.out % (2 * sizeof(OutT)) == 0) && (!a.mask || (uintptr_t)a.mask % 2 == 0);
+    if (a.exposures) {
+        if (vec) k1_generic_tt_kernel<RawT, OutT, KS, TH, true><<<(unsigned)total, K1_THREADS, 0, st>>>(a, tiles_x, tiles_y);
+        else k1_generic_tt_kernel<RawT, OutT, KS, TH, false><<<(unsigned)total, K1_THREADS, 0, st>>>(a, tiles_x, tiles_y);
+        return cudaGetLastError();
+    }
     if (vec) k1_generic_kernel<RawT, OutT, KS, TH, true><<<(unsigned)total, K1_THREADS, 0, st>>>(a, tiles_x, tiles_y);
     else k1_generic_kernel<RawT, OutT, KS, TH, false><<<(unsigned)total, K1_THREADS, 0, st>>>(a, tiles_x, tiles_y);
     return cudaGetLastError();
@@ -467,6 +483,11 @@ static cudaError_t launch_pointwise_t(const K1Args& a, int sm_count, cudaStream_
                 k1_pointwise_bg_kernel<RawT, OutT><<<dim3((unsigned)bx, (unsigned)nf), 256, 0, st>>>(b);
                 continue;
             }
+        }
+        if (a.exposures) {
+            b.exposures = a.exposures + f0;
+            k1_pointwise_tt_kernel<RawT, OutT><<<dim3((unsigned)bx, (unsigned)nf), 256, 0, st>>>(b);
+            continue;
         }
         k1_pointwise_kernel<RawT, OutT><<<dim3((unsigned)bx, (unsigned)nf), 256, 0, st>>>(b);
     }

@@ -61,18 +61,29 @@ typedef KsShape<KS_PAIR_R, KS_PAIR_NSTAGE, KS_PAIR_MINB, 2> KsPair;
 #endif
 typedef KsShape<KS_PAIRBG_R, KS_PAIRBG_NSTAGE, 3, 2> KsPairBg;         // uint16 frames, finite flat field
 typedef KsShape<KS_PAIRBG_R, KS_PAIRBG_NSTAGE, 2, 2> KsPairBgF32;      // float32 frames
+// the line model (KS_LIN): an offset box and an ascent box per stage in place of the dark box.  A 16-row uint16 pair stage
+// is 33.3 KB (float32: 40 KB), a 24-row one-frame stage 42.4 KB (float32: 48 KB).  uint16 pairs take 3 stages x 2 CTAs per
+// SM: at 2 stages x 3 CTAs the register cap makes the chain configurations spill (4 and 16 bytes)
+#ifndef KS_PAIRLIN_NSTAGE
+#define KS_PAIRLIN_NSTAGE 3
+#define KS_PAIRLIN_MINB 2
+#endif
+typedef KsShape<16, KS_PAIRLIN_NSTAGE, KS_PAIRLIN_MINB, 2> KsPairLin;  // uint16 frames
+typedef KsShape<16, 2, 2, 2> KsPairLinF32;                             // float32 frames
+typedef KsShape<24, 2, 2, 1> KsNarrowLin;                              // one frame per unit
 constexpr int KS_MAPW = 128;                // float32 box: tx0-4 .. tx0+123
 constexpr int KS_MAPX = 4;
 constexpr int KS_THREADS = (KS_CW + 1) * 32;
 
-template <typename RawT, typename C, bool BG = false> struct StreamBox {
+template <typename RawT, typename C, bool BG = false, bool LIN = false> struct StreamBox {
     static constexpr int XOFF = 16 / (int)sizeof(RawT);                        // u8 16, u16 8, f32 4
     static constexpr int GRAN = 16 / (int)sizeof(RawT);
     // the box starts at the 16-byte boundary at or left of tx0, minus XOFF: columns tx0-1 .. tx0+120 are inside
     static constexpr int BOXW = ((KS_TW + 2 * XOFF + GRAN - 1) / GRAN) * GRAN;  // u8 160, u16 136, f32 128
     static constexpr size_t raw_bytes = (size_t)C::R * BOXW * sizeof(RawT);     // multiples of 128
     static constexpr size_t map_bytes = (size_t)C::R * KS_MAPW * sizeof(float);
-    static constexpr size_t dark_bytes = BG ? C::NF * raw_bytes : map_bytes;     // the dark box, or a background box per frame
+    // the dark box, a background box per frame, or the offset and ascent boxes of the line model
+    static constexpr size_t dark_bytes = BG ? C::NF * raw_bytes : LIN ? 2 * map_bytes : map_bytes;
     static constexpr size_t stage_bytes = C::NF * raw_bytes + dark_bytes + map_bytes;    // raw[NF] | dark or bg[NF] | flat
     static_assert(raw_bytes % 128 == 0 && map_bytes % 128 == 0, "TMA destinations must be 128-byte aligned: rows per stage must be a multiple of 8");
     static constexpr size_t bar_off = C::NSTAGE * stage_bytes;
@@ -126,7 +137,13 @@ __device__ __forceinline__ UnitGeom ks_unit(int unit, int strips, int seg_rows, 
 // CFG >= 0 bakes the per-launch switches into the instruction stream (the kernel is issue bound: every
 // per-row flag test costs); CFG < 0 reads them from the arguments.
 enum : int { KS_DARK = 1, KS_FLAT = 2, KS_N2N = 4, KS_MASK = 8, KS_CHECK = 16, KS_LT = 32, KS_NZ = 64, KS_SWAP = 128, KS_NOMED = 256,
-             KS_BG = 512 };
+             KS_BG = 512, KS_LIN = 1024 };
+// KS_LIN: the line model (FLAG_DARK_LINEAR).  tm_dark maps the context's [2][H][W] offset / ascent block and the producer
+// loads a box two maps deep (offset rows, then ascent rows) where the dark box was.  Consumers convert both values to
+// float64 once per pixel position and, per frame, evaluate bg = offset + ascent * t (DMUL, DADD, the clip to max_value:
+// dark_value()'s arithmetic) with the frame's time (K1Args::exposures, or pw.exposure_time); the flat value's float64
+// reciprocal stays shared by the frames of the unit.  The checked arithmetic falls back to pointwise() where |bg| is above
+// FLT_MAX or NaN
 // KS_BG: per-frame backgrounds (K1Args::bg, of the raw dtype) in place of the dark map.  The producer loads one background
 // box per frame next to the raw box (evict first: each is read once); the flat value's float64 reciprocal stays shared by
 // the frames of the unit, and each frame subtracts float64(float32(its own background sample))
@@ -138,8 +155,8 @@ enum : int { KS_DARK = 1, KS_FLAT = 2, KS_N2N = 4, KS_MASK = 8, KS_CHECK = 16, K
 
 // dark / flat of one pixel position, prepared once for all frames of the unit
 struct RowMaps {
-    float d, f;
-    double dd, fd, y;       // float64 copies and the refined reciprocal of the (zero-free) flat value
+    float d, f, s;          // s: the ascent (KS_LIN)
+    double dd, fd, y, sd;   // float64 copies and the refined reciprocal of the (zero-free) flat value
 };
 
 // medians of two vertically adjacent 3x3 windows from the sorted horizontal triples of four consecutive rows a, b, c, e:
@@ -162,13 +179,15 @@ __global__ void __launch_bounds__(KS_THREADS, C::MINB)
 k1_stream_kernel(const __grid_constant__ CUtensorMap tm_raw, const __grid_constant__ CUtensorMap tm_dark,
                  const __grid_constant__ CUtensorMap tm_flat, K1Args a, int strips, int seg_rows, int total_units) {
     constexpr bool BG = CFG >= 0 && (CFG & KS_BG);
-    using B = StreamBox<RawT, C, BG>;
+    constexpr bool LIN = CFG >= 0 && (CFG & KS_LIN);
+    using B = StreamBox<RawT, C, BG, LIN>;
     constexpr int KS_R = C::R, KS_NSTAGE = C::NSTAGE, NF = C::NF;
     static_assert(KS_R % 2 == 0, "rows per stage must be even (outputs are produced in vertical pairs)");
     static_assert(NF == 1 || (CFG >= 0 && !(CFG & KS_MASK)), "multi-frame units: specialised configurations without a mask only");
     // the frame-independent half of the division is hoisted whenever the flat value is known to be non-zero
     constexpr bool FASTDIV = CFG >= 0 && (CFG & KS_NZ) && (CFG & KS_DARK) && (CFG & KS_FLAT);
     static_assert(!BG || FASTDIV, "per-frame backgrounds: the specialised dark + zero-free flat configurations only");
+    static_assert(!LIN || FASTDIV, "the line model: the specialised dark + zero-free flat configurations only");
     extern __shared__ __align__(128) uint8_t smem[];
     uint64_t* full = (uint64_t*)(smem + B::bar_off);
     uint64_t* empty = full + KS_NSTAGE;
@@ -218,6 +237,8 @@ k1_stream_kernel(const __grid_constant__ CUtensorMap tm_raw, const __grid_consta
                     for (int f = 0; f < NF; ++f)
                         tma_load_3d_hint(base + (NF + f) * B::raw_bytes, &tm_dark, &full[stage], (u.tx0 / B::GRAN) * B::GRAN - B::XOFF, y,
                                          u.frame + f, L2_EVICT_FIRST);
+                } else if (LIN) {
+                    tma_load_3d_hint(base + NF * B::raw_bytes, &tm_dark, &full[stage], u.tx0 - KS_MAPX, y, 0, L2_EVICT_LAST);
                 } else if (has_dark) {
                     tma_load_2d_hint(base + NF * B::raw_bytes, &tm_dark, &full[stage], u.tx0 - KS_MAPX, y, L2_EVICT_LAST);
                 }
@@ -258,6 +279,11 @@ k1_stream_kernel(const __grid_constant__ CUtensorMap tm_raw, const __grid_consta
         Sorted3<float> s0[NF], s1[NF];
         float c1[NF];
         int i = 0;
+        double tf[NF];                                   // KS_LIN: the exposure time of each frame of the unit
+        if constexpr (LIN) {
+#pragma unroll
+            for (int f = 0; f < NF; ++f) tf[f] = a.exposures ? __ldg(a.exposures + u.frame + f) : pw.exposure_time;
+        }
 
         auto maps = [&](const uint8_t* base, int j, RowMaps& m) {
             m.d = has_dark && !BG ? ((const float*)(base + NF * B::raw_bytes))[j * KS_MAPW + mcol] : 0.0f;
@@ -266,6 +292,10 @@ k1_stream_kernel(const __grid_constant__ CUtensorMap tm_raw, const __grid_consta
                 m.dd = (double)m.d;
                 m.fd = (double)m.f;
                 m.y = rcp_f32range(m.fd);
+            }
+            if constexpr (LIN) {
+                m.s = ((const float*)(base + NF * B::raw_bytes + B::map_bytes))[j * KS_MAPW + mcol];
+                m.sd = (double)m.s;
             }
         };
         auto pixel = [&](const uint8_t* base, int j, int f, const RowMaps& m) -> float {
@@ -279,16 +309,30 @@ k1_stream_kernel(const __grid_constant__ CUtensorMap tm_raw, const __grid_consta
                 d = (float)((const RawT*)(base + (NF + f) * B::raw_bytes))[j * B::BOXW + rcol];      // exact for integer samples
                 dd = (double)d;
             }
+            if constexpr (LIN) {
+                dd = dadd(m.dd, dmul(m.sd, tf[f]));
+                dd = dd > pw.max_value ? pw.max_value : dd;     // NaN stays NaN
+            }
             float x;
             bool ok;
             if (FASTDIV) {
                 x = (float)ddiv_rcp(dsub(rd, dd), m.fd, m.y);
                 if (flags & FLAG_NAN_TO_NUM) x = fminf(fmaxf(x, -FLT_MAX), FLT_MAX);
-                if (check) ok = (fabsf(d) + fabsf(m.f) + ra) <= FLT_MAX;
+                if (check) ok = ((LIN ? (float)fabs(dd) : fabsf(d)) + fabsf(m.f) + ra) <= FLT_MAX;
             } else {
                 x = (CFG >= 0 && (CFG & KS_NZ)) ? pointwise_fast_nz(flags, rd, ra, d, m.f, ok) : pointwise_fast(flags, rd, ra, d, m.f, ok);
             }
-            if (check) { if (!ok) x = pointwise<float>(pw, rd, d, 0.0f, m.f); }
+            if (check) {
+                if (!ok) {
+                    if constexpr (LIN) {
+                        PointwiseConst pf = pw;
+                        pf.exposure_time = tf[f];
+                        x = pointwise<float>(pf, rd, m.d, m.s, m.f);
+                    } else {
+                        x = pointwise<float>(pw, rd, d, 0.0f, m.f);
+                    }
+                }
+            }
             return x;
         };
         auto triple = [&](float x) -> Sorted3<float> {
@@ -460,12 +504,34 @@ static int ks_bg_cfg(const K1Args& a, int raw_dtype) {
     return -1;
 }
 
+// the line model streams in the same configurations as per-frame backgrounds (uint16 and float32 frames, the chain's 3x3
+// and threshold <= 0), with the context's [2][H][W] offset / ascent block.  Returns the configuration, or -1
+static int ks_lin_cfg(const K1Args& a, int raw_dtype) {
+    const int f = a.pw.flags;
+    if (!(f & FLAG_DARK_LINEAR) || a.bg || (raw_dtype != DT_U16 && raw_dtype != DT_F32)) return -1;
+    if (a.raw_swap || a.mask || !a.dark || a.ascent != a.dark + (size_t)a.H * a.W || !a.flat || !a.flat_nz || !(f & FLAG_DARK) ||
+        !(f & FLAG_FLAT))
+        return -1;
+    const bool check = !a.maps_finite || raw_dtype == DT_F32;
+    const int base = KS_LIN | KS_DARK | KS_FLAT | KS_NZ;
+    if (a.ksize == 3) {
+        if (!(f & FLAG_NAN_TO_NUM) || a.pred.cond != COND_GT) return -1;
+        return check ? base | KS_N2N | KS_CHECK : a.no_overflow ? base : base | KS_N2N;
+    }
+    if (a.ksize == 0 && a.H >= 4) {
+        const int n2n = (f & FLAG_NAN_TO_NUM) && !a.no_overflow ? KS_N2N : 0;
+        if (raw_dtype == DT_F32) return base | KS_NOMED | KS_CHECK | n2n;
+        return check ? -1 : base | KS_NOMED | n2n;
+    }
+    return -1;
+}
+
 bool k1_stream_eligible(const K1Args& a, int raw_dtype, int out_dtype) {
     if (a.ksize != 3 && a.ksize != 0) return false;
     if (a.ksize == 0 && a.H < 4) return false;
     if (raw_dtype != DT_U8 && raw_dtype != DT_U16 && raw_dtype != DT_F32) return false;
     if (out_dtype != DT_F32 && out_dtype != DT_U16 && out_dtype != DT_U8) return false;
-    if (a.pw.flags & FLAG_DARK_LINEAR) return false;
+    if ((a.pw.flags & FLAG_DARK_LINEAR) && ks_lin_cfg(a, raw_dtype) < 0) return false;
     if (a.raw_gap) return false;
     const size_t esz = dtype_size(raw_dtype);
     if (((size_t)a.W * esz) % 16 || ((size_t)a.W * 4) % 16) return false;
@@ -484,6 +550,29 @@ typedef void (*ks_kern_t)(const CUtensorMap, const CUtensorMap, const CUtensorMa
 template <typename RawT, typename OutT, typename C>
 static ks_kern_t ks_bg_kernel(int cfg) {
     constexpr int B0 = KS_BG | KS_DARK | KS_FLAT | KS_NZ;
+    if constexpr (sizeof(RawT) == 2) {
+        if (cfg == B0) return k1_stream_kernel<RawT, OutT, B0, C>;
+        if (cfg == (B0 | KS_N2N)) return k1_stream_kernel<RawT, OutT, B0 | KS_N2N, C>;
+        if constexpr (C::NF == 1) {
+            if (cfg == (B0 | KS_N2N | KS_CHECK)) return k1_stream_kernel<RawT, OutT, B0 | KS_N2N | KS_CHECK, C>;
+            if (cfg == (B0 | KS_NOMED)) return k1_stream_kernel<RawT, OutT, B0 | KS_NOMED, C>;
+            if (cfg == (B0 | KS_NOMED | KS_N2N)) return k1_stream_kernel<RawT, OutT, B0 | KS_NOMED | KS_N2N, C>;
+        }
+    } else if constexpr (sizeof(RawT) == 4) {
+        if (cfg == (B0 | KS_N2N | KS_CHECK)) return k1_stream_kernel<RawT, OutT, B0 | KS_N2N | KS_CHECK, C>;
+        if constexpr (C::NF == 1) {
+            if (cfg == (B0 | KS_NOMED | KS_CHECK)) return k1_stream_kernel<RawT, OutT, B0 | KS_NOMED | KS_CHECK, C>;
+            if (cfg == (B0 | KS_NOMED | KS_CHECK | KS_N2N)) return k1_stream_kernel<RawT, OutT, B0 | KS_NOMED | KS_CHECK | KS_N2N, C>;
+        }
+    }
+    return nullptr;
+}
+
+// the line-model instantiations, the same set as ks_bg_kernel's (uint16: finite maps with and without the overflow proof,
+// and the checked chain; float32: checked only), or null
+template <typename RawT, typename OutT, typename C>
+static ks_kern_t ks_lin_kernel(int cfg) {
+    constexpr int B0 = KS_LIN | KS_DARK | KS_FLAT | KS_NZ;
     if constexpr (sizeof(RawT) == 2) {
         if (cfg == B0) return k1_stream_kernel<RawT, OutT, B0, C>;
         if (cfg == (B0 | KS_N2N)) return k1_stream_kernel<RawT, OutT, B0 | KS_N2N, C>;
@@ -558,6 +647,24 @@ static cudaError_t launch_stream_bg(const K1Args& a_in, CUtensorMapDataType rdt,
     return ks_run<B, C>(kern, a, tr, tb, tf, sm_count, seg_rows, st);
 }
 
+// the line model (ks_lin_cfg): the offset / ascent block is a 3-D map two deep, loaded as one box
+template <typename RawT, typename OutT, typename C>
+static cudaError_t launch_stream_lin(const K1Args& a_in, CUtensorMapDataType rdt, int sm_count, int seg_rows, cudaStream_t st) {
+    using B = StreamBox<RawT, C, false, true>;
+    constexpr int RDT = sizeof(RawT) == 1 ? DT_U8 : sizeof(RawT) == 2 ? DT_U16 : DT_F32;
+    K1Args a = a_in;
+    const int cfg = ks_lin_cfg(a, RDT);
+    if (cfg < 0 || a.n_frames % C::NF) return cudaErrorInvalidValue;
+    ks_kern_t kern = ks_lin_kernel<RawT, OutT, C>(cfg);
+    if (!kern) return cudaErrorInvalidValue;
+    a.flat = a.flat_nz;                                  // zero-free copy: an unconditional division
+    CUtensorMap tr, td, tf;
+    if (!make_tensor_map(&tr, rdt, sizeof(RawT), a.raw, a.W, a.H, a.n_frames, B::BOXW, C::R)) return cudaErrorInvalidValue;
+    if (!make_tensor_map(&td, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 4, a.dark, a.W, a.H, 2, KS_MAPW, C::R, 2)) return cudaErrorInvalidValue;
+    if (!make_tensor_map(&tf, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 4, a.flat, a.W, a.H, 0, KS_MAPW, C::R)) return cudaErrorInvalidValue;
+    return ks_run<B, C>(kern, a, tr, td, tf, sm_count, seg_rows, st);
+}
+
 template <typename RawT, typename OutT, typename C>
 static cudaError_t launch_stream_c(const K1Args& a_in, CUtensorMapDataType rdt, int sm_count, int seg_rows, cudaStream_t st) {
     using B = StreamBox<RawT, C>;
@@ -608,6 +715,24 @@ static cudaError_t launch_stream_t(const K1Args& a, CUtensorMapDataType rdt, int
         const int f = a.pw.flags;
         const bool chain = a.ksize == 3 && (a.dark || a.bg) && a.flat && a.flat_nz && (f & FLAG_DARK) && (f & FLAG_FLAT) &&
                            (f & FLAG_NAN_TO_NUM) && !a.mask && a.pred.cond == COND_GT && !a.raw_swap;
+        if (a.pw.flags & FLAG_DARK_LINEAR) {
+            // the line model: frame pairs of the chain (uint16 frames with finite maps and a bounded |bg|, float32 frames),
+            // everything else and an odd last frame one frame per unit
+            using P = typename std::conditional<sizeof(RawT) == 4, KsPairLinF32, KsPairLin>::type;
+            if (!chain || a.n_frames < 4 || (sizeof(RawT) != 4 && !a.maps_finite))
+                return launch_stream_lin<RawT, OutT, KsNarrowLin>(a, rdt, sm_count, seg_rows, st);
+            const int even = a.n_frames & ~1;
+            K1Args b = a;
+            b.n_frames = even;
+            cudaError_t e = launch_stream_lin<RawT, OutT, P>(b, rdt, sm_count, seg_rows, st);
+            if (e != cudaSuccess || even == a.n_frames) return e;
+            b = a;
+            b.n_frames = 1;
+            b.raw = (const char*)a.raw + (size_t)even * a.H * a.W * sizeof(RawT);
+            b.out = (char*)a.out + (size_t)even * a.H * a.W * sizeof(OutT);
+            if (b.exposures) b.exposures += even;
+            return launch_stream_lin<RawT, OutT, KsNarrowLin>(b, rdt, sm_count, seg_rows, st);
+        }
         if (a.bg) {
             // per-frame backgrounds: frame pairs of the chain (uint16 frames with a finite flat field, float32 frames),
             // everything else and an odd last frame one frame per unit in the narrow shape
@@ -643,6 +768,7 @@ static cudaError_t launch_stream_t(const K1Args& a, CUtensorMapDataType rdt, int
         // the wide shape pays with float32 output and a few frames per launch (see KsShape)
         if (a.n_frames >= 4) return launch_stream_c<RawT, OutT, KsWide>(a, rdt, sm_count, seg_rows, st);
     }
+    if (a.pw.flags & FLAG_DARK_LINEAR) return launch_stream_lin<RawT, OutT, KsNarrowLin>(a, rdt, sm_count, seg_rows, st);
     if (a.bg) return launch_stream_bg<RawT, OutT, KsNarrow>(a, rdt, sm_count, seg_rows, st);
     return launch_stream_c<RawT, OutT, KsNarrow>(a, rdt, sm_count, seg_rows, st);
 }

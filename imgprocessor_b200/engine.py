@@ -58,7 +58,7 @@ class Engine(object):
         h = ctypes.c_void_p()
         _lib.check(self.lib.imgcorr_ctx_create(self.device_index, self.H, self.W, ctypes.byref(h)))
         self._h = h
-        self.has_dark = self.has_flat = self.has_lens = False
+        self.has_dark = self.has_flat = self.has_lens = self.has_exposures = False
         self.perspective_dsize = None          # (width, height) of the chain's perspective stage, if one is set
         self._tokens = {}
 
@@ -131,9 +131,25 @@ class Engine(object):
         p2, dev2, keep2 = self._map_arg(ascent)
         if keep is not None and keep2 is not None and dev != dev2:
             raise ValueError('dark and ascent must both be host arrays or both device tensors')
+        self.has_exposures = False                       # imgcorr_set_dark drops the per-frame exposure times
         _lib.check(self.lib.imgcorr_set_dark(self._h, p, p2, float(exposure_time), int(depth_bits), dev))
         self.has_dark = dark is not None
         self._tokens['dark'] = token
+
+    def set_dark_exposures(self, times):
+        """One exposure time per frame for the linear dark model of set_dark(dark, ascent, ...)
+        (imgcorr_set_dark_exposures): frame i of every later call evaluates dark + ascent * times[i], clipped, exactly as
+        the same call with exposure_time=times[i]; a call with more frames than times is refused.  Calls with per-frame
+        backgrounds ignore the table.  None removes it; set_dark removes it too."""
+        self.has_exposures = False                       # a failed call leaves no table behind
+        if times is None:
+            _lib.check(self.lib.imgcorr_set_dark_exposures(self._h, None, 0))
+            return
+        t = np.ascontiguousarray(np.asarray(times, dtype=np.float64))
+        if t.ndim != 1:
+            raise ValueError('exposure times must be 1-D, got shape %s' % (t.shape,))
+        _lib.check(self.lib.imgcorr_set_dark_exposures(self._h, t.ctypes.data_as(ctypes.c_void_p), int(t.size)))
+        self.has_exposures = True
 
     def set_flat(self, flat, token=None):
         if token is not None and self._tokens.get('flat') == token:

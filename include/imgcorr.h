@@ -35,7 +35,8 @@ extern "C" {
                                later added imgcorr_set_perspective and IMGCORR_DO_PERSPECTIVE (the chain's perspective stage),
                                U16 / U8 output of the chain with imgcorr_set_output_scale, imgcorr_set_perspective_frames
                                (one homography per frame in the perspective stage), and imgcorr_correct_batch_bg /
-                               imgcorr_correct_host_bg (one background image per frame in place of the dark map) */
+                               imgcorr_correct_host_bg (one background image per frame in place of the dark map), and
+                               imgcorr_set_dark_exposures (one exposure time per frame for the linear dark model) */
 
 #if defined(__GNUC__)
 #define IMGCORR_API __attribute__((visibility("default")))
@@ -117,6 +118,16 @@ IMGCORR_API int imgcorr_profile_read(imgcorr_ctx* ctx, double out[4]);
  * otherwise host pointers.  dark == NULL removes the calibration. Synchronous. */
 IMGCORR_API int imgcorr_set_dark(imgcorr_ctx* ctx, const float* dark, const float* ascent, double exposure_time,
                      int depth_bits, int on_device);
+/* One exposure time per frame for the linear dark model of imgcorr_set_dark: frame i of a call (i counts from the call's
+ * first frame: raw_dev[i], raw_host[i], frame i of a framed file image) evaluates bg = dark + ascent * t[i], clipped to
+ * 2**depth_bits - 1, bit for bit as the same call with exposure_time = t[i].  Read by imgcorr_pointwise_median,
+ * imgcorr_correct_batch and imgcorr_correct_host; the _bg forms ignore it (their backgrounds replace the dark stage).
+ *   t      host array [n] of exposure times, copied synchronously; NULL removes the table (n is ignored then)
+ * IMGCORR_ERR_STATE if the context has no linear model (ascent), IMGCORR_ERR_INVALID for n <= 0 or a NaN entry.  A call
+ * that evaluates the model (IMGCORR_DO_DARK, no per-frame backgrounds) over more frames than the table holds fails with
+ * IMGCORR_ERR_INVALID before it enqueues anything.  imgcorr_set_dark drops the table.  Replacing or removing a table first
+ * synchronises the device, since queued calls may still read it; a failed call leaves no table.  Synchronous. */
+IMGCORR_API int imgcorr_set_dark_exposures(imgcorr_ctx* ctx, const double* t, int n);
 /* Flat field (camera/CameraCalibration.py:520-526).  flat == NULL removes it. Synchronous. */
 IMGCORR_API int imgcorr_set_flat(imgcorr_ctx* ctx, const float* flat, int on_device);
 /* Lens (camera/LensDistortion.py:342-358): K = cameraMatrix (3x3 row-major), dist = [k1,k2,p1,p2,k3]
