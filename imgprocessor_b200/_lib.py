@@ -31,6 +31,7 @@ SIGNATURES = {
     'imgcorr_set_dark_exposures': (c_int, [c_void_p, c_void_p, c_int]),
     'imgcorr_set_flat': (c_int, [c_void_p, c_void_p, c_int]),
     'imgcorr_set_lens': (c_int, [c_void_p, c_void_p, c_void_p, c_void_p]),
+    'imgcorr_set_lens_model': (c_int, [c_void_p, c_void_p, c_void_p, c_int, c_void_p]),
     'imgcorr_pointwise_median': (c_int, [c_void_p, c_void_p, c_int, c_void_p, c_int, c_void_p, c_int, c_double,
                                          c_int, c_int, c_int, c_void_p]),
     'imgcorr_undistort': (c_int, [c_void_p, c_void_p, c_int, c_void_p, c_int, c_int, c_double, c_int, c_int, c_int,

@@ -2,7 +2,8 @@
 (camera/LensDistortion.py:16-402).
 
 What moved to the GPU (kernel K2, csrc/k2_undistort.cu):
-  * correct()                  :316-330   analytic Brown-Conrady map + OpenCV fixed-point bilinear remap
+  * correct()                  :316-330   analytic lens map (OpenCV's 4-, 5-, 8-, 12- and 14-coefficient models)
+                                          + OpenCV fixed-point bilinear remap
   * getUndistortRectifyMap()   :342-358   the float32 maps themselves (written by a map kernel)
   * distortImage()             :332-340   remap with explicit maps
 What stays on the host, exactly as in the reference: cv2.getOptimalNewCameraMatrix (a 3x3, :350-353)
@@ -75,11 +76,12 @@ class LensDistortion(object):
     def _lens_setup(self, imgWidth, imgHeight):
         """host part of getUndistortRectifyMap (:347-353): P and roi from OpenCV, then the lens
         constants go to the device context."""
-        import cv2
         cam = np.asarray(self.coeffs['cameraMatrix'], np.float64)
         d = np.asarray(self.coeffs['distortionCoeffs'], np.float64)
-        if d.size != 5:
-            raise ValueError('only the 5-term distortion model [k1,k2,p1,p2,k3] is supported (got %d terms)' % d.size)
+        if d.size not in _engine.LENS_MODEL_SIZES:      # what cv2.initUndistortRectifyMap takes
+            raise ValueError('distortionCoeffs: 4, 5, 8, 12 or 14 terms (k1 k2 p1 p2 k3 k4 k5 k6 s1 s2 s3 s4 tau_x tau_y), '
+                             'got %d' % d.size)
+        import cv2
         P, self.roi = cv2.getOptimalNewCameraMatrix(cam, d, (imgWidth, imgHeight), 1, (imgWidth, imgHeight))
         self._new_camera_matrix = P
         eng = _engine.get_engine(imgHeight, imgWidth)

@@ -121,7 +121,10 @@ struct imgcorr_ctx {
     OutScale out_scale{0.0, 1.0};             // imgcorr_set_output_scale: read by chain calls with U16 / U8 output
     bool has_lens = false;
     LensConst lens{};
-    double lens_in[23] = {0};                 // K, dist, P as last given to imgcorr_set_lens (an identical call is a no-op)
+    LensExt lens_x{};                         // the lens' rational / thin-prism / tilt terms, used when lens_ext is set
+    bool lens_ext = false;                    // some extra term is non-zero: K2 runs its EXT kernels
+    double lens_in[33] = {0};                 // K, dist (14, zero-padded), P and the coefficient count as last given to
+                                              // imgcorr_set_lens_model (an identical call is a no-op)
     DevPtr<double> lens_dev;
     DevPtr<float4> k2_wtab;                   // OpenCV's BilinearTab_f [32][32] (K2 tiles)
     struct GeomKey { int x0, y0, ow, oh, esz, g; };
@@ -481,27 +484,28 @@ extern "C" IMGCORR_API int imgcorr_set_flat(imgcorr_ctx* c, const float* flat, i
     return IMGCORR_OK;
 }
 
-extern "C" IMGCORR_API int imgcorr_set_lens(imgcorr_ctx* c, const double K[9], const double dist[5], const double P[9]) {
+extern "C" IMGCORR_API int imgcorr_set_lens_model(imgcorr_ctx* c, const double K[9], const double* dist, int n_dist, const double P[9]) {
     if (!c) return fail(IMGCORR_ERR_INVALID, "null context");
     if (!K) { c->has_lens = false; return IMGCORR_OK; }
     if (!dist || !P) return fail(IMGCORR_ERR_INVALID, "dist / P is null");
-    {
-        // the Python mirror sets the lens on every correct() call (the reference builds a new LensDistortion per call,
-        // camera/CameraCalibration.py:565-568): the same lens again must not drop K2's geometry choice and coordinate cache
-        double in[23];
-        memcpy(in, K, 9 * sizeof(double)); memcpy(in + 9, dist, 5 * sizeof(double)); memcpy(in + 14, P, 9 * sizeof(double));
-        if (c->has_lens && c->lens_dev && memcmp(in, c->lens_in, sizeof in) == 0) return IMGCORR_OK;
-    }
-    LensConst L{};
-    if (!invert3x3(P, L.ir)) return fail(IMGCORR_ERR_INVALID, "new camera matrix P is singular");
-    L.k1 = dist[0]; L.k2 = dist[1]; L.p1 = dist[2]; L.p2 = dist[3]; L.k3 = dist[4];
-    L.p1x2 = L.p1 + L.p1; L.p2x2 = L.p2 + L.p2;
-    L.fx = K[0]; L.fy = K[4]; L.cx = K[2]; L.cy = K[5];
-    L.affine = (L.ir[6] == 0.0 && L.ir[7] == 0.0 && L.ir[8] == 1.0) ? 1 : 0;
-    double pack[LP_COUNT] = {0};
+    if (n_dist != 4 && n_dist != 5 && n_dist != 8 && n_dist != 12 && n_dist != 14)
+        return fail(IMGCORR_ERR_INVALID, "%d distortion coefficients (4, 5, 8, 12 or 14)", n_dist);
+    // K, the coefficients zero-padded to 14, P and the count: two lenses that differ in any of them differ here
+    double in[33] = {0};
+    memcpy(in, K, 9 * sizeof(double)); memcpy(in + 9, dist, n_dist * sizeof(double)); memcpy(in + 23, P, 9 * sizeof(double));
+    in[32] = n_dist;
+    // the Python mirror sets the lens on every correct() call (the reference builds a new LensDistortion per call,
+    // camera/CameraCalibration.py:565-568): the same lens again must not drop K2's geometry choice and coordinate cache
+    if (c->has_lens && c->lens_dev && memcmp(in, c->lens_in, sizeof in) == 0) return IMGCORR_OK;
+    LensConst L;
+    if (!make_lens_const(K, dist, n_dist, P, L)) return fail(IMGCORR_ERR_INVALID, "new camera matrix P is singular");
+    LensExt X;
+    const bool ext = make_lens_ext(dist, n_dist, X);
+    double pack[LP_EXT_COUNT] = {0};
     pack[LP_K1] = L.k1; pack[LP_K2] = L.k2; pack[LP_K3] = L.k3; pack[LP_P1] = L.p1; pack[LP_P2] = L.p2;
     pack[LP_P1X2] = L.p1x2; pack[LP_P2X2] = L.p2x2; pack[LP_FX] = L.fx; pack[LP_FY] = L.fy; pack[LP_CX] = L.cx;
     pack[LP_CY] = L.cy; pack[LP_IR0] = L.ir[0]; pack[LP_IR2] = L.ir[2]; pack[LP_IR4] = L.ir[4]; pack[LP_IR5] = L.ir[5];
+    memcpy(pack + LP_COUNT, &X, sizeof X);
     {
         DeviceGuard g(c->device);
         if (!g.ok) return cuda_fail(cudaGetLastError(), "cudaSetDevice");
@@ -509,8 +513,10 @@ extern "C" IMGCORR_API int imgcorr_set_lens(imgcorr_ctx* c, const double K[9], c
         CK(cudaMemcpy(c->lens_dev.get(), pack, sizeof pack, cudaMemcpyHostToDevice));
     }
     c->lens = L;
+    c->lens_x = X;
+    c->lens_ext = ext;
     c->has_lens = true;
-    memcpy(c->lens_in, K, 9 * sizeof(double)); memcpy(c->lens_in + 9, dist, 5 * sizeof(double)); memcpy(c->lens_in + 14, P, 9 * sizeof(double));
+    memcpy(c->lens_in, in, sizeof in);
     c->k2_geom.clear();
     if (!c->k2_cache.empty()) {
         DeviceGuard g(c->device);
@@ -518,6 +524,10 @@ extern "C" IMGCORR_API int imgcorr_set_lens(imgcorr_ctx* c, const double K[9], c
         c->k2_cache.clear();
     }
     return IMGCORR_OK;
+}
+
+extern "C" IMGCORR_API int imgcorr_set_lens(imgcorr_ctx* c, const double K[9], const double dist[5], const double P[9]) {
+    return imgcorr_set_lens_model(c, K, dist, 5, P);
 }
 
 // bg: per-frame backgrounds [n][H][W] of bg_dtype in place of the dark map (checked by check_bg), or null.  first: the
@@ -607,6 +617,7 @@ static int run_k2(imgcorr_ctx* c, const void* src, int sdt, void* dst, int ddt, 
     a.border = border_for_dtype(sdt == DT_U8, sdt == DT_U16, border);
     a.lens = c->lens;
     a.lens_dev = c->lens_dev.get();
+    a.lens_ext = c->lens_ext ? 1 : 0;
     a.sm_count = c->sm_count;
     a.q = q;
     if (!c->k2_wtab) {
@@ -630,7 +641,7 @@ static int run_k2(imgcorr_ctx* c, const void* src, int sdt, void* dst, int ddt, 
         for (const auto& k : c->k2_geom)
             if (k.x0 == x0 && k.y0 == y0 && k.ow == ow && k.oh == oh && k.esz == gesz) { a.geometry = k.g; found = true; break; }
         if (!found) {
-            a.geometry = k2_pick_geometry(c->lens, c->H, c->W, x0, y0, ow, oh, gesz);
+            a.geometry = k2_pick_geometry(c->lens, c->lens_ext ? &c->lens_x : nullptr, c->H, c->W, x0, y0, ow, oh, gesz);
             if (c->k2_geom.size() > 64) c->k2_geom.clear();
             c->k2_geom.push_back({x0, y0, ow, oh, gesz, a.geometry});
         }
@@ -702,7 +713,7 @@ extern "C" IMGCORR_API int imgcorr_undistort_maps(imgcorr_ctx* c, float* mapx_de
     if (!c->has_lens) return fail(IMGCORR_ERR_STATE, "no lens set");
     if (!mapx_dev || !mapy_dev) return fail(IMGCORR_ERR_INVALID, "null map pointer");
     int l = 0;
-    cudaError_t e = launch_write_maps(c->lens, mapx_dev, mapy_dev, c->H, c->W, (cudaStream_t)stream, &l);
+    cudaError_t e = launch_write_maps(c->lens, c->lens_ext ? &c->lens_x : nullptr, mapx_dev, mapy_dev, c->H, c->W, (cudaStream_t)stream, &l);
     return launched(c, l, e, "map kernel launch");
 }
 

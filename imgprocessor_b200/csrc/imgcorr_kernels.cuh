@@ -70,17 +70,21 @@ struct K2Args {
     int2* chdr_w;
     int sm_count;
     OutScale q;             // F32 -> U16 / U8: the float32 blend, then quantise<DstT>(blend, q)
+    int lens_ext;           // the lens has rational / thin-prism / tilt terms (LensExt at lens_dev + LP_COUNT): the EXT kernels
 };
 void k2_cache_size(int geometry, int ow, int oh, size_t* words, size_t* tiles);
 bool k2_will_tile(const K2Args& a, int src_dtype, int dst_dtype, int variant);    // launch_k2 takes the tiled variant
-int k2_pick_geometry(const LensConst& lens, int H, int W, int x0, int y0, int ow, int oh, int src_elem_size);
+int k2_pick_geometry(const LensConst& lens, const LensExt* ext, int H, int W, int x0, int y0, int ow, int oh, int src_elem_size);
 
 // order of the doubles in K2Args::lens_dev
 enum LensPack : int { LP_K1, LP_K2, LP_K3, LP_P1, LP_P2, LP_P1X2, LP_P2X2, LP_FX, LP_FY, LP_CX, LP_CY, LP_IR0, LP_IR2, LP_IR4, LP_IR5, LP_PAD, LP_COUNT };
+// followed by the LensExt of the lens (its 16 doubles in declaration order), read by the EXT kernels
+constexpr int LP_EXT_COUNT = LP_COUNT + (int)(sizeof(LensExt) / sizeof(double));
+static_assert(sizeof(LensExt) == 16 * sizeof(double), "LensExt is packed as 16 doubles");
 
 cudaError_t launch_k2(const K2Args& a, int src_dtype, int dst_dtype, int variant, cudaStream_t stream,
                       int* launches);
-cudaError_t launch_write_maps(const LensConst& lens, float* mapx, float* mapy, int H, int W,
+cudaError_t launch_write_maps(const LensConst& lens, const LensExt* ext, float* mapx, float* mapy, int H, int W,
                               cudaStream_t stream, int* launches);
 
 // K3: perspective warp (cv2.warpPerspective, Lanczos4 / bicubic) ------------------------------

@@ -1,4 +1,5 @@
-// K2 — lens undistortion: per output pixel evaluate the Brown-Conrady model analytically
+// K2 — lens undistortion: per output pixel evaluate the lens model analytically (Brown-Conrady; with the EXT flag
+// OpenCV's rational, thin-prism and tilted-sensor terms as well)
 // (float64, one rounding to float32 — no map arrays are read), convert to OpenCV's 5-bit
 // fixed-point coordinates and gather the bilinear blend from the K1 output through L1/L2.
 //
@@ -135,14 +136,30 @@ __device__ __forceinline__ DstT rim_out(const SrcT* __restrict__ src, int H, int
     else return remap_rim<SrcT, DstT>(src, H, W, ix, iy, w, bval);
 }
 
+// the extra terms of a lens (LensExt, packed after the LensPack slots): eight 16-byte loads
+__device__ __forceinline__ void load_lens_ext(const double* lens_dev, LensExt& E) {
+    const double2* lp = reinterpret_cast<const double2*>(lens_dev + LP_COUNT);
+    double2 q;
+    q = __ldg(lp + 0); E.k4 = q.x; E.k5 = q.y;
+    q = __ldg(lp + 1); E.k6 = q.x; E.s1 = q.y;
+    q = __ldg(lp + 2); E.s2 = q.x; E.s3 = q.y;
+    q = __ldg(lp + 3); E.s4 = q.x; E.t[0] = q.y;
+    q = __ldg(lp + 4); E.t[1] = q.x; E.t[2] = q.y;
+    q = __ldg(lp + 5); E.t[3] = q.x; E.t[4] = q.y;
+    q = __ldg(lp + 6); E.t[5] = q.x; E.t[6] = q.y;
+    q = __ldg(lp + 7); E.t[7] = q.x; E.t[8] = q.y;
+}
+
 // MODE: 0 explicit maps, 1 analytic general P, 2 analytic separable P^-1 (x = x(u), y = y(v))
+// EXT: the analytic map with OpenCV's rational, thin-prism and tilt terms (map_distort_ext); only MODE 1 and 2
 //
 // The kernel is bound by the latency of the four-neighbour gathers, not by the float64 map evaluation (with explicit
 // maps it is no faster, see profiles/).  So a thread first computes the coordinates of all its K2_ROWS pixels, then
 // issues all 4*K2_ROWS gathers unconditionally (pixels on the rim gather from offset 0 and are redone out of line),
 // then blends and stores: 4*K2_ROWS loads in flight per thread instead of 4.
-template <typename SrcT, typename DstT, int MODE>
+template <typename SrcT, typename DstT, int MODE, bool EXT>
 __global__ void __launch_bounds__(K2_BX * K2_BY, K2_MINB) k2_remap_kernel(K2Args a) {
+    static_assert(!EXT || MODE != 0, "explicit maps have no lens terms");
     const int ox = blockIdx.x * K2_BX + (threadIdx.x % K2_BX);
     const int ty = threadIdx.x / K2_BX;
     if (ox >= a.ow) return;
@@ -166,6 +183,8 @@ __global__ void __launch_bounds__(K2_BX * K2_BY, K2_MINB) k2_remap_kernel(K2Args
         q = __ldg(lp + 6); L.ir[2] = q.x; L.ir[4] = q.y;
         q = __ldg(lp + 7); L.ir[5] = q.x;
     }
+    LensExt E;
+    if constexpr (EXT) load_lens_ext(a.lens_dev, E);
     double xc = 0.0, xc2 = 0.0;
     if (MODE == 2) {
         xc = fma((double)u, L.ir[0], L.ir[2]);
@@ -184,9 +203,11 @@ __global__ void __launch_bounds__(K2_BX * K2_BY, K2_MINB) k2_remap_kernel(K2Args
         float mx, my;
         if (MODE == 2) {
             const double y = fma((double)v, L.ir[4], L.ir[5]);
-            map_distort(L, xc, y, xc2, dmul(y, y), mx, my);
+            if constexpr (EXT) map_distort_ext(L, E, xc, y, xc2, dmul(y, y), mx, my);
+            else map_distort(L, xc, y, xc2, dmul(y, y), mx, my);
         } else if (MODE == 1) {
-            undistort_map(L, u, v, mx, my);
+            if constexpr (EXT) undistort_map_ext(L, E, u, v, mx, my);
+            else undistort_map(L, u, v, mx, my);
         } else {
             mx = __ldg(a.mapx + v * W + u);
             my = __ldg(a.mapy + v * W + u);
@@ -308,13 +329,17 @@ template <int MODE> __device__ __forceinline__ void kt_load_lens(const K2Args& a
     }
 }
 // fixed-point source coordinate of output pixel (u, v) (full-frame coordinates)
-template <int MODE> __device__ __forceinline__ FixedCoord kt_coord(const K2Args& a, const LensConst& L, int u, int v, double dv, double xc, double xc2) {
+template <int MODE, bool EXT>
+__device__ __forceinline__ FixedCoord kt_coord(const K2Args& a, const LensConst& L, const LensExt& E, int u, int v, double dv, double xc,
+                                               double xc2) {
     float mx, my;
     if (MODE == 2) {
         const double y = fma(dv, L.ir[4], L.ir[5]);                 // dv == (double)v
-        map_distort(L, xc, y, xc2, dmul(y, y), mx, my);
+        if constexpr (EXT) map_distort_ext(L, E, xc, y, xc2, dmul(y, y), mx, my);
+        else map_distort(L, xc, y, xc2, dmul(y, y), mx, my);
     } else if (MODE == 1) {
-        undistort_map(L, u, v, mx, my);
+        if constexpr (EXT) undistort_map_ext(L, E, u, v, mx, my);
+        else undistort_map(L, u, v, mx, my);
     } else {
         mx = __ldg(a.mapx + v * a.W + u);
         my = __ldg(a.mapy + v * a.W + u);
@@ -332,8 +357,9 @@ constexpr unsigned KP_OUTSIDE = 0x80000000u, KP_SLOW = 0x40000000u;
 //       2: coordinates read from the cache: 4 bytes per pixel instead of ~45 float64 operations and ~90 instructions.
 // The lens is constant per context, so the analytic evaluation — what bounds a ONE-frame launch (119 instructions per pixel,
 // 65 us per 4096x3000 frame, issue bound: profiles/r2_k2_single_analytic_ncu_full.txt) — is paid once, not once per call.
-template <typename SrcT, typename DstT, int MODE, typename G, int CMODE>
+template <typename SrcT, typename DstT, int MODE, typename G, int CMODE, bool EXT>
 __global__ void __launch_bounds__(KT_THREADS, G::MINB) k2_tiled_kernel(const __grid_constant__ CUtensorMap tm_src, K2Args a) {
+    static_assert(!EXT || (MODE != 0 && CMODE != 2), "EXT: analytic maps that are evaluated");
     constexpr int KT_TW = G::TW, KT_TH = G::TH, KT_BH = G::BH, KT_NBUF = G::NBUF;
     constexpr int KT_PX = KT_TW * KT_TH / KT_THREADS, KT_RSTEP = KT_THREADS / KT_TW;
     constexpr int BW = KtBox<SrcT, G>::BW, KT_BOX_BYTES = KtBox<SrcT, G>::BYTES, GRAN = KtBox<SrcT, G>::GRAN;
@@ -376,6 +402,8 @@ __global__ void __launch_bounds__(KT_THREADS, G::MINB) k2_tiled_kernel(const __g
         }
         LensConst L;
         kt_load_lens<MODE>(a, L);
+        LensExt E;
+        if constexpr (EXT) load_lens_ext(a.lens_dev, E);
         // ---- the staged box: position ESTIMATED by warp 0 from nine sample pixels of the tile (3 x 3: corners, edge
         // midpoints, centre; exact coordinates, KT_MARGIN pixels added all round) and clamped to the frame, so that
         // "inside the box" implies "all four neighbours exist".  Thread 0 issues the boxes of the first frames at once:
@@ -389,7 +417,7 @@ __global__ void __launch_bounds__(KT_THREADS, G::MINB) k2_tiled_kernel(const __g
             if (tid < 9) {
                 const int su = sx + a.x0, sv = sy + a.y0;
                 const double sxc = MODE == 2 ? fma((double)su, L.ir[0], L.ir[2]) : 0.0;
-                const FixedCoord fc = kt_coord<MODE>(a, L, su, sv, (double)sv, sxc, dmul(sxc, sxc));
+                const FixedCoord fc = kt_coord<MODE, EXT>(a, L, E, su, sv, (double)sv, sxc, dmul(sxc, sxc));
                 if (!(fc.ix < -1 || fc.ix > W - 1 || fc.iy < -1 || fc.iy > H - 1)) {       // outside the frame: nothing to stage
                     const int qx = fc.ix < 0 ? 0 : (fc.ix > W - 2 ? W - 2 : fc.ix), qy = fc.iy < 0 ? 0 : (fc.iy > H - 2 ? H - 2 : fc.iy);
                     ex0 = ex1 = qx; ey0 = ey1 = qy;
@@ -420,7 +448,7 @@ __global__ void __launch_bounds__(KT_THREADS, G::MINB) k2_tiled_kernel(const __g
         for (int j = 0; j < KT_PX; ++j) {
             const int oy = oy0 + j * KT_RSTEP;
             const int v = (MODE == 0 ? (oy < oh ? oy : oh - 1) : oy) + a.y0;
-            const FixedCoord fc = kt_coord<MODE>(a, L, u, v, dadd(dv0, (double)(j * KT_RSTEP)), xc, xc2);
+            const FixedCoord fc = kt_coord<MODE, EXT>(a, L, E, u, v, dadd(dv0, (double)(j * KT_RSTEP)), xc, xc2);
             cix[j] = fc.ix; ciy[j] = fc.iy;
             pk[j] = (unsigned)(fc.fx << 14) | (unsigned)(fc.fy << 19);
         }
@@ -467,10 +495,12 @@ __global__ void __launch_bounds__(KT_THREADS, G::MINB) k2_tiled_kernel(const __g
     auto slow_pixel = [&](const SrcT* src, int j) -> DstT {
         LensConst L2;
         kt_load_lens<MODE>(a, L2);
+        LensExt E2;
+        if constexpr (EXT) load_lens_ext(a.lens_dev, E2);
         const int oy = oy0 + j * KT_RSTEP;
         const int v = (MODE == 0 ? (oy < oh ? oy : oh - 1) : oy) + a.y0;
         const double sxc = MODE == 2 ? fma((double)u, L2.ir[0], L2.ir[2]) : 0.0;
-        const FixedCoord fc = kt_coord<MODE>(a, L2, u, v, (double)v, sxc, dmul(sxc, sxc));
+        const FixedCoord fc = kt_coord<MODE, EXT>(a, L2, E2, u, v, (double)v, sxc, dmul(sxc, sxc));
         Weights<SrcT> w;
         w.set(fc);
         return rim_out<SrcT, DstT>(src, H, W, fc.ix, fc.iy, w, border_cast<SrcT>(a.border), a.q);
@@ -534,7 +564,8 @@ constexpr int KC_MAXT = 256;
 #ifndef KC_MINB
 #define KC_MINB 3           // 85 registers: 46 vs 51 us for one 4096x3000 frame with 4 CTAs of 64 registers
 #endif
-template <typename SrcT, typename DstT, typename G>
+// EXT: the lens has extra terms, which the "slow" pixels' recomputed coordinates need
+template <typename SrcT, typename DstT, typename G, bool EXT>
 __global__ void __launch_bounds__(KT_THREADS, KC_MINB)
 k2_cached_kernel(const __grid_constant__ CUtensorMap tm_src, K2Args a, int tiles_x, long long n_items) {
     constexpr int KT_TW = G::TW, KT_TH = G::TH, KT_BH = G::BH, NBUF = KcGeom<G>::NBUF;
@@ -594,7 +625,13 @@ k2_cached_kernel(const __grid_constant__ CUtensorMap tm_src, K2Args a, int tiles
     // neighbour border handling from global memory — a fraction of a percent of the pixels
     auto slow_pixel = [&](const SrcT* src, int j) -> DstT {
         float mx, my;
-        undistort_map(a.lens, tx0 + c + a.x0, ty0 + r0 + j * KT_RSTEP + a.y0, mx, my);
+        if constexpr (EXT) {
+            LensExt E;
+            load_lens_ext(a.lens_dev, E);
+            undistort_map_ext(a.lens, E, tx0 + c + a.x0, ty0 + r0 + j * KT_RSTEP + a.y0, mx, my);
+        } else {
+            undistort_map(a.lens, tx0 + c + a.x0, ty0 + r0 + j * KT_RSTEP + a.y0, mx, my);
+        }
         const FixedCoord fc = fixed_coord_fast(mx, my);
         Weights<SrcT> w;
         w.set(fc);
@@ -661,7 +698,7 @@ k2_cached_kernel(const __grid_constant__ CUtensorMap tm_src, K2Args a, int tiles
     }
 }
 
-template <typename SrcT, typename DstT, typename G>
+template <typename SrcT, typename DstT, typename G, bool EXT>
 static cudaError_t launch_cached_g(const K2Args& a, cudaStream_t st) {
     CUtensorMap tm;
     if (!make_tensor_map(&tm, kt_dtype<SrcT>(), sizeof(SrcT), a.src, a.W, a.H, a.n_frames, KtBox<SrcT, G>::BW, G::BH)) return cudaErrorInvalidValue;
@@ -669,7 +706,7 @@ static cudaError_t launch_cached_g(const K2Args& a, cudaStream_t st) {
     const long long n_items = (long long)tiles_x * tiles_y * a.n_frames;
     if (n_items > 0x7fffffffLL) return cudaErrorInvalidValue;
     constexpr int SMEM = KcGeom<G>::NBUF * (KtBox<SrcT, G>::BYTES + G::TW * G::TH * 4) + 128 + KC_MAXT * 8;
-    auto kern = k2_cached_kernel<SrcT, DstT, G>;
+    auto kern = k2_cached_kernel<SrcT, DstT, G, EXT>;
     cudaError_t e = cudaSuccess;
     const int per_sm = blocks_per_sm_cached((const void*)kern, KT_THREADS, SMEM, &e);
     if (e != cudaSuccess) return e;
@@ -696,11 +733,13 @@ static cudaError_t launch_tiled_g(const K2Args& a, cudaStream_t st) {
     constexpr int SMEM = kt_smem<SrcT, G>();
     void (*kern)(const CUtensorMap, K2Args);
     const bool sep = a.lens.affine && a.lens.ir[1] == 0.0 && a.lens.ir[3] == 0.0;
-    if (a.cpack && !a.mapx) return launch_cached_g<SrcT, DstT, G>(a, st);
+    if (a.cpack && !a.mapx) return a.lens_ext ? launch_cached_g<SrcT, DstT, G, true>(a, st) : launch_cached_g<SrcT, DstT, G, false>(a, st);
     if constexpr (K2Quant<SrcT, DstT>::value) if (a.mapx) return cudaErrorNotSupported;    // the chain remaps with the analytic map only
-    if (a.mapx) kern = k2_tiled_kernel<SrcT, DstT, 0, G, 0>;
-    else if (a.cpack_w) kern = sep ? k2_tiled_kernel<SrcT, DstT, 2, G, 1> : k2_tiled_kernel<SrcT, DstT, 1, G, 1>;
-    else kern = sep ? k2_tiled_kernel<SrcT, DstT, 2, G, 0> : k2_tiled_kernel<SrcT, DstT, 1, G, 0>;
+    if (a.mapx) kern = k2_tiled_kernel<SrcT, DstT, 0, G, 0, false>;
+    else if (a.lens_ext && a.cpack_w) kern = sep ? k2_tiled_kernel<SrcT, DstT, 2, G, 1, true> : k2_tiled_kernel<SrcT, DstT, 1, G, 1, true>;
+    else if (a.lens_ext) kern = sep ? k2_tiled_kernel<SrcT, DstT, 2, G, 0, true> : k2_tiled_kernel<SrcT, DstT, 1, G, 0, true>;
+    else if (a.cpack_w) kern = sep ? k2_tiled_kernel<SrcT, DstT, 2, G, 1, false> : k2_tiled_kernel<SrcT, DstT, 1, G, 1, false>;
+    else kern = sep ? k2_tiled_kernel<SrcT, DstT, 2, G, 0, false> : k2_tiled_kernel<SrcT, DstT, 1, G, 0, false>;
     if (SMEM > 48 * 1024) {
         cudaError_t e = cudaSuccess;
         blocks_per_sm_cached((const void*)kern, KT_THREADS, SMEM, &e);       // opt-in to > 48 KB, once per (device, kernel)
@@ -730,8 +769,9 @@ void k2_cache_size(int g, int ow, int oh, size_t* words, size_t* tiles) {
 // Host: the staged-box geometry a lens needs for an output window — the largest source window (plus margins) over all
 // 64x16 tiles, from the exact map at the very 3 x 3 sample points the kernel estimates from.
 // 0: 80x32 box, 1: 96x32, 2: 112x48, 3: 32-wide tiles with a 112x64 box.  `src_elem_size` sets the column granularity of the
-// box origin (16 bytes: 4 / 8 / 16 columns).  Cached per window by the caller (imgcorr_api.cu).
-int k2_pick_geometry(const LensConst& L, int H, int W, int x0, int y0, int ow, int oh, int src_elem_size) {
+// box origin (16 bytes: 4 / 8 / 16 columns).  `ext`: the lens' extra terms, or null for the 5-term model.  Cached per window
+// by the caller (imgcorr_api.cu).
+int k2_pick_geometry(const LensConst& L, const LensExt* ext, int H, int W, int x0, int y0, int ow, int oh, int src_elem_size) {
     int need_w = 0, need_h = 0;
     const int TW = 64, TH = 16;
     for (int ty = 0; ty < oh; ty += TH)
@@ -742,7 +782,8 @@ int k2_pick_geometry(const LensConst& L, int H, int W, int x0, int y0, int ow, i
                 const int sx = (k % 3) == 0 ? tx : ((k % 3) == 1 ? x1 : (tx + x1) / 2);
                 const int sy = (k / 3) == 0 ? ty : ((k / 3) == 1 ? y1 : (ty + y1) / 2);
                 float mx, my;
-                undistort_map(L, sx + x0, sy + y0, mx, my);
+                if (ext) undistort_map_ext(L, *ext, sx + x0, sy + y0, mx, my);
+                else undistort_map(L, sx + x0, sy + y0, mx, my);
                 const FixedCoord fc = fixed_coord(mx, my);
                 if (fc.ix < -1 || fc.ix > W - 1 || fc.iy < -1 || fc.iy > H - 1) continue;     // outside: nothing to stage
                 const int qx = fc.ix < 0 ? 0 : (fc.ix > W - 2 ? W - 2 : fc.ix), qy = fc.iy < 0 ? 0 : (fc.iy > H - 2 ? H - 2 : fc.iy);
@@ -760,12 +801,14 @@ int k2_pick_geometry(const LensConst& L, int H, int W, int x0, int y0, int ow, i
     return 3;
 }
 
-__global__ void __launch_bounds__(256) k2_write_maps_kernel(LensConst lens, float* mapx, float* mapy, int H, int W) {
+template <bool EXT>
+__global__ void __launch_bounds__(256) k2_write_maps_kernel(LensConst lens, LensExt ext, float* mapx, float* mapy, int H, int W) {
     const int u = blockIdx.x * 32 + (threadIdx.x % 32);
     const int v = blockIdx.y * 8 + (threadIdx.x / 32);
     if (u >= W || v >= H) return;
     float mx, my;
-    undistort_map(lens, u, v, mx, my);
+    if constexpr (EXT) undistort_map_ext(lens, ext, u, v, mx, my);
+    else undistort_map(lens, u, v, mx, my);
     mapx[(size_t)v * W + u] = mx;
     mapy[(size_t)v * W + u] = my;
 }
@@ -776,9 +819,11 @@ template <typename SrcT, typename DstT>
 static cudaError_t launch_t(const K2Args& a, cudaStream_t st) {
     dim3 grid((a.ow + K2_BX - 1) / K2_BX, (a.oh + K2_BY * K2_ROWS - 1) / (K2_BY * K2_ROWS));
     if constexpr (K2Quant<SrcT, DstT>::value) if (a.mapx) return cudaErrorNotSupported;
-    if (a.mapx) k2_remap_kernel<SrcT, DstT, 0><<<grid, K2_BX * K2_BY, 0, st>>>(a);
-    else if (separable(a.lens)) k2_remap_kernel<SrcT, DstT, 2><<<grid, K2_BX * K2_BY, 0, st>>>(a);
-    else k2_remap_kernel<SrcT, DstT, 1><<<grid, K2_BX * K2_BY, 0, st>>>(a);
+    if (a.mapx) k2_remap_kernel<SrcT, DstT, 0, false><<<grid, K2_BX * K2_BY, 0, st>>>(a);
+    else if (a.lens_ext && separable(a.lens)) k2_remap_kernel<SrcT, DstT, 2, true><<<grid, K2_BX * K2_BY, 0, st>>>(a);
+    else if (a.lens_ext) k2_remap_kernel<SrcT, DstT, 1, true><<<grid, K2_BX * K2_BY, 0, st>>>(a);
+    else if (separable(a.lens)) k2_remap_kernel<SrcT, DstT, 2, false><<<grid, K2_BX * K2_BY, 0, st>>>(a);
+    else k2_remap_kernel<SrcT, DstT, 1, false><<<grid, K2_BX * K2_BY, 0, st>>>(a);
     return cudaGetLastError();
 }
 
@@ -818,11 +863,12 @@ cudaError_t launch_k2(const K2Args& a, int src_dtype, int dst_dtype, int variant
     return cudaErrorInvalidValue;
 }
 
-cudaError_t launch_write_maps(const LensConst& lens, float* mapx, float* mapy, int H, int W, cudaStream_t st,
+cudaError_t launch_write_maps(const LensConst& lens, const LensExt* ext, float* mapx, float* mapy, int H, int W, cudaStream_t st,
                               int* launches) {
     if (H <= 0 || W <= 0) return cudaSuccess;
     dim3 grid((W + 31) / 32, (H + 7) / 8);
-    k2_write_maps_kernel<<<grid, 256, 0, st>>>(lens, mapx, mapy, H, W);
+    if (ext) k2_write_maps_kernel<true><<<grid, 256, 0, st>>>(lens, *ext, mapx, mapy, H, W);
+    else k2_write_maps_kernel<false><<<grid, 256, 0, st>>>(lens, LensExt{}, mapx, mapy, H, W);
     if (launches) ++*launches;
     return cudaGetLastError();
 }

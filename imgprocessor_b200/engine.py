@@ -37,6 +37,8 @@ def _torch_dtype(code):
 
 NP_CODES = {np.dtype(np.uint8): _lib.U8, np.dtype(np.uint16): _lib.U16, np.dtype(np.float32): _lib.F32,
             np.dtype(np.float64): _lib.F64}
+# coefficient counts of the lens models cv2.initUndistortRectifyMap takes (Engine.set_lens)
+LENS_MODEL_SIZES = (4, 5, 8, 12, 14)
 
 
 def require_cuda():
@@ -165,12 +167,13 @@ class Engine(object):
             self.has_lens = False
             return
         K = np.ascontiguousarray(np.asarray(K, np.float64).reshape(3, 3))
-        d = np.ascontiguousarray(np.asarray(dist, np.float64).ravel())
-        if d.size != 5:
-            raise ValueError('only the 5-term distortion model [k1,k2,p1,p2,k3] is supported, got %d terms' % d.size)
+        d = np.ascontiguousarray(np.asarray(dist, np.float64).ravel())     # (1, n), (n,) or (n, 1)
+        if d.size not in LENS_MODEL_SIZES:
+            raise ValueError('distortion coefficients: 4, 5, 8, 12 or 14 terms (OpenCV order k1 k2 p1 p2 k3 k4 k5 k6 '
+                             's1 s2 s3 s4 tau_x tau_y), got %d' % d.size)
         P = np.ascontiguousarray(np.asarray(P, np.float64)[:3, :3])
         vp = lambda a: a.ctypes.data_as(ctypes.c_void_p)
-        _lib.check(self.lib.imgcorr_set_lens(self._h, vp(K), vp(d), vp(P)))
+        _lib.check(self.lib.imgcorr_set_lens_model(self._h, vp(K), vp(d), d.size, vp(P)))
         self.has_lens = True
 
     def set_perspective(self, M, dsize, border_value=0.0, tilt_factor=None, token=None):

@@ -36,7 +36,8 @@ extern "C" {
                                U16 / U8 output of the chain with imgcorr_set_output_scale, imgcorr_set_perspective_frames
                                (one homography per frame in the perspective stage), and imgcorr_correct_batch_bg /
                                imgcorr_correct_host_bg (one background image per frame in place of the dark map), and
-                               imgcorr_set_dark_exposures (one exposure time per frame for the linear dark model) */
+                               imgcorr_set_dark_exposures (one exposure time per frame for the linear dark model), and
+                               imgcorr_set_lens_model (OpenCV's 4-, 8-, 12- and 14-coefficient lens models in K2) */
 
 #if defined(__GNUC__)
 #define IMGCORR_API __attribute__((visibility("default")))
@@ -132,8 +133,17 @@ IMGCORR_API int imgcorr_set_dark_exposures(imgcorr_ctx* ctx, const double* t, in
 IMGCORR_API int imgcorr_set_flat(imgcorr_ctx* ctx, const float* flat, int on_device);
 /* Lens (camera/LensDistortion.py:342-358): K = cameraMatrix (3x3 row-major), dist = [k1,k2,p1,p2,k3]
  * (camera/LensDistortion.py:370,380), P = newCameraMatrix from cv2.getOptimalNewCameraMatrix (:350-353,
- * computed by the host wrapper exactly as the reference does).  K == NULL removes the lens. */
+ * computed by the host wrapper exactly as the reference does).  K == NULL removes the lens.
+ * The same as imgcorr_set_lens_model(ctx, K, dist, 5, P). */
 IMGCORR_API int imgcorr_set_lens(imgcorr_ctx* ctx, const double K[9], const double dist[5], const double P[9]);
+/* Lens with any coefficient vector cv2.initUndistortRectifyMap takes: n_dist = 4, 5, 8, 12 or 14 coefficients in OpenCV's
+ * order k1 k2 p1 p2 [k3 [k4 k5 k6 [s1 s2 s3 s4 [tau_x tau_y]]]] (rational model, thin prism, tilted sensor; missing
+ * terms are zero).  K and P as for imgcorr_set_lens; the rectification is the identity.  K2 and imgcorr_undistort_maps
+ * evaluate OpenCV's full model in float64 with correctly rounded divisions.  When every term after k3 is zero the
+ * lens is the 5-term lens [k1, k2, p1, p2, k3] (k3 = 0 for n_dist = 4) and gives its results bit for bit.
+ * IMGCORR_ERR_INVALID for another count, a null dist or P, or a singular P.  K == NULL removes the lens.
+ * Setting the lens of the last call again (same K, coefficients, count and P) keeps K2's coordinate cache. */
+IMGCORR_API int imgcorr_set_lens_model(imgcorr_ctx* ctx, const double K[9], const double* dist, int n_dist, const double P[9]);
 
 /* ---- K1: fused dark / flat / nan_to_num / NxN median-threshold ---------------------------------
  * Replaces _correctDarkCurrent + _correctVignetting + _correctArtefacts
